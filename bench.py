@@ -18,8 +18,20 @@ counts slab-generations per second. The generation step needs no collective; the
 distance pass sums the per-pair partial core counts with NCCL inside the library
 (pansim_comm_init_rank; torch.distributed only carries the 128-byte unique id).
 
+--steps K is the number of generations timed: one device-resident batch of K generations after the
+warm-up (at the default K = 100 a window of about 15 ms on a B200 with a 1000 W power limit). --repeats R times R such batches
+(R x K generations) and reports the median batch; at the default R = 1 the `repeats` record holds that
+one batch. The end-to-end record (`e2e`) is the median of 5 runs whatever R is.
+
+--impl reference runs K full cfg2 generations on the host, a few seconds each: pass a small --steps
+for a quick sample.
+
+--dump-outputs DIR writes, after the timed batches, the state a caller of the timed path holds after its
+last generation as DIR/<name>.npy (float32 / float64, see dump_outputs). The inputs are seeded, so two
+builds run with the same arguments can be compared file by file.
+
 Also in the line:
-  repeats        the K-step batch is timed R >= 10 times; value / ms_per_step are the median batch
+  repeats        R, and the fastest / median / slowest of the R batches
   shard_parity   (N > 1) a small column-sharded run equals the unsharded one bit for bit; the run
                  fails when it does not
   cfg2_print_dist  the cfg2 step WITH its per-generation distance pass and on-device statistics
@@ -161,9 +173,8 @@ def run_reference(args, rank, world):
     crate cannot be built here (no cargo), so this is the oracle port."""
     if rank != 0:
         return
-    steps = max(1, args.steps)
-    # bounded sample: each step = one cfg2 generation on the host cores (a few s each)
-    steps_run = min(steps, 3)
+    # each step = one cfg2 generation on the host cores (a few s each)
+    steps_run = args.steps
     pairs = 2000
     threads, t_gen, t_dist = cpu_baseline_sample(args.warmup if args.warmup < 1 else 1, False, pairs)  # warm page cache / omp
     threads, t_gen, t_dist = cpu_baseline_sample(steps_run, True, pairs)
@@ -188,14 +199,21 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100, help="generations in the timed batch")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--impl", default="b200", choices=["b200", "reference"],
+                    help="reference: the CPU oracle port, --steps cfg2 generations at a few seconds each")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-gens", type=int, default=2)
-    ap.add_argument("--repeats", type=int, default=10, help="batches of --steps generations; the median batch is reported")
+    ap.add_argument("--repeats", type=int, default=1, help="timed batches of --steps generations; the median batch is reported")
     ap.add_argument("--no-cfg4", action="store_true", help="skip the cfg4 strong-scaling record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the state after the last timed generation as DIR/<name>.npy (rank 0's slab when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1 or args.repeats < 1:
+        ap.error("--steps and --repeats must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none")
     # stdout carries exactly ONE JSON line: libraries that print there (NCCL's version banner) are
     # sent to stderr, and the line is written to the saved descriptor at the end
     global _JSON_OUT
@@ -246,9 +264,12 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    W = max(3, args.warmup)
-    K = max(1, args.steps)
-    R = max(1, args.repeats)
+    # batches of 8 or more generations launch the selection chain as CUDA graphs, one graph per phase of the
+    # rotating buffers (6 phases), captured on first use: a warm-up of at least 8 keeps the captures out of
+    # the timed batch
+    W = max(8, args.warmup)
+    K = args.steps
+    R = args.repeats
     # this rank's slab: columns [rank*L, (rank+1)*L) of a (world*L)-site alignment
     from pansim_b200.sharding import SITE_ALIGN, ShardedPansim, broadcast_unique_id, column_shards
     L = CFG2["core_size"]
@@ -325,6 +346,8 @@ def main():
     launches = int(tm.launches)
     select_ms, acc_ms = tm.select_ms / K, tm.acc_step_ms / K
     distinct_parents = int(len(np.unique(sim.parents())))      # rows the gather of the last generation actually read
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sim)
     if os.environ.get("BENCH_DIAG") == "1":        # diagnostics: the generation batches only
         if rank == 0:
             print(json.dumps({"diag": os.environ.get("BENCH_DIAG_NAME", ""), "world": world, "backend": backend, "no_comm": no_comm,
@@ -366,7 +389,7 @@ def main():
     # per generation the calls main.rs:435-464 makes, vectors crossing the boundary
     Ke = min(K, 50)
     e2e_runs = []
-    for _ in range(min(R, 5)):
+    for _ in range(5):
         barrier()
         t0 = time.perf_counter()
         for g in range(Ke):
@@ -516,6 +539,25 @@ def main():
         dist.destroy_process_group()
     if shard_parity is False:
         raise SystemExit("bench.py: column-sharded run differs from the unsharded run (shard_parity false)")
+
+
+def dump_outputs(out_dir: str, sim) -> None:
+    """--dump-outputs: what a caller of run_generations holds after the last timed generation (about 33 MB
+    at cfg2). The core state (N x 1.2 Mbp one-hot bytes) is too large to store whole, so a fixed, seeded
+    sample of 4096 sites of every row is written, and every row's A / C / G / T counts over all sites
+    show a change anywhere in the row."""
+    os.makedirs(out_dir, exist_ok=True)
+    core = sim.download_core()
+    sites = np.sort(np.random.default_rng(1).choice(core.shape[1], size=min(4096, core.shape[1]), replace=False))
+    arrays = {
+        "parents": sim.parents().astype(np.float64),
+        "acc": sim.download_acc().astype(np.float32),
+        "core_sample": core[:, sites].astype(np.float32),
+        "core_sample_sites": sites.astype(np.float64),
+        "core_allele_counts": np.stack([np.bincount(row, minlength=9)[[1, 2, 4, 8]] for row in core]).astype(np.float64),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def check_shard_parity(pb, ShardedPansim, rank, world, local_rank, dist, torch) -> bool:
