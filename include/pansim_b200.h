@@ -214,6 +214,37 @@ double pansim_acc_distance(uint32_t inter, uint32_t uni, uint32_t core_genes);
 /* Population::gene_frequencies numerators (population.rs:840-856): counts[G] */
 int pansim_gene_counts(pansim_ctx *ctx, uint32_t *counts);
 
+/* ---- core-genome diversity (extension: the reference has no such output) ----
+ * One column reduction of the packed core alignment on the device (DESIGN.md section 10). Every call
+ * observes the state after recombine(), like the pair calls. On a column shard every field and every SFS
+ * bin is the partial over the shard's sites; the sum over the shards is the whole-alignment value. */
+typedef struct {
+    uint64_t sites;          /* local sites counted (site_end - site_begin)                          */
+    uint64_t segregating;    /* >= 2 alleles present                                                  */
+    uint64_t multiallelic;   /* >= 3 alleles present                                                  */
+    uint64_t pair_diff_sum;  /* sum over sites of sum_{a<b} n_a n_b = sum over pairs i<j of core_diff */
+} pansim_diversity;
+/* per-site allele counts: counts[local_sites][4] = n_A, n_C, n_G, n_T */
+int pansim_core_allele_counts(pansim_ctx *ctx, uint32_t *counts);
+/* the summaries above; sfs[N+1] (may be NULL): sfs[k] = number of sites where k individuals carry an allele
+ * other than the ancestral one, the ancestral row being the row given to pansim_set_initial (uploads do not
+ * change it). Asking for the SFS on a context that never had pansim_set_initial fails with PANSIM_ERR_STATE. */
+int pansim_core_diversity(pansim_ctx *ctx, pansim_diversity *out, uint64_t *sfs /* [N+1] or NULL */);
+/* n generations, each followed by the reduction on the device; with n_pairs > 0 also the --print_dist
+ * pass and its statistics, stats_out[n][4] bit-identical to pansim_run_generations_stats (the pair half
+ * needs the whole alignment or a communicator, like pansim_run_generations_stats) */
+int pansim_run_generations_diversity(pansim_ctx *ctx, uint32_t gen0, uint32_t n, const uint32_t *range1,
+                                     const uint32_t *range2, size_t n_pairs, double *stats_out,
+                                     pansim_diversity *div_out /* [n] */);
+/* out = { pi, theta_W, Tajima's D } from whole-alignment values; needs no device.
+ *   pi = pair_diff_sum / C(N,2)   (mean number of differing sites over all pairs)
+ *   theta_W = S / a1, a1 = sum_{i=1}^{N-1} 1/i, a2 = sum 1/i^2 (ascending i), S = segregating
+ *   D = (pi - S/a1) / sqrt(e1 S + e2 S (S-1)) with b1, b2, c1, c2, e1, e2 of Tajima (1989)
+ * D is NaN when S = 0 or the denominator is 0; all three are NaN when N < 2. With four alleles S counts
+ * sites, not mutations: a site with three alleles carries at least two mutations, so `multiallelic` shows
+ * how far the infinite-sites assumption behind theta_W and D is violated. */
+void pansim_diversity_stats(const pansim_diversity *d, uint32_t pop_size, double out[3]);
+
 /* ---- multi-GPU: column shards of one alignment --------------------------
  * (SURVEY.md 8e; the reference is one shared-memory process, population.rs has no analogue.)
  * Every shard context holds all individuals for [site_begin, site_end) and a replica of the
@@ -260,6 +291,11 @@ int pansim_group_all_pairs(pansim_group *g, size_t chunk_pairs, pansim_pairs_cb 
 /* last walk: wall time (callbacks included), device time of shard 0 inside the reduce-scatters, pairs walked */
 int pansim_group_all_pairs_timing(pansim_group *g, float *wall_ms, float *nccl_ms, uint64_t *pairs);
 int pansim_group_gene_counts(pansim_group *g, uint32_t *counts);                          /* population.rs:840-856 */
+/* whole-alignment diversity: the shard partials summed on the host (sfs [N+1] or NULL) */
+int pansim_group_core_diversity(pansim_group *g, pansim_diversity *out, uint64_t *sfs);
+int pansim_group_run_generations_diversity(pansim_group *g, uint32_t gen0, uint32_t n, const uint32_t *range1,
+                                           const uint32_t *range2, size_t n_pairs, double *stats_out,
+                                           pansim_diversity *div_out);
 int pansim_group_download_acc(pansim_group *g, uint8_t *acc_out);
 int pansim_group_download_core(pansim_group *g, uint8_t *core_onehot_out);               /* [N x core_size] */
 int pansim_group_export_core_csv(pansim_group *g, uint32_t row_begin, uint32_t row_end, char *out);
@@ -279,7 +315,9 @@ int pansim_get_info(pansim_ctx *ctx, pansim_info *out);
 
 /* Device time (ms, CUDA events on the context's stream) of the last
  * pansim_step / pansim_step_with_parents / pansim_run_generations /
- * pansim_pair_counts* call, split by kernel group. */
+ * pansim_pair_counts* call, split by kernel group. After pansim_core_diversity
+ * total_ms is the reduction kernel alone (the diversity batches time like the
+ * other batches). */
 typedef struct {
     float total_ms;
     float core_step_ms;       /* core genome: gather+SNP kernel and the recombination pass (sum over generations) */

@@ -4,7 +4,7 @@ Same long flags (underscores, capitalised --HR_rate / --HGT_rate), same defaults
 same parsing quirks: pop_size/core_size/pan_genes/core_genes/n_gen are parsed as
 f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
-accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs.
+accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity.
 """
 from __future__ import annotations
 
@@ -55,6 +55,10 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--device", type=int, default=0, help="(extension) CUDA device ordinal")
     ap.add_argument("--all_pairs", action="store_true",
                     help="(extension) <outpref>.tsv holds every pair i < j in (i, j) order instead of max_distances sampled pairs")
+    ap.add_argument("--print_diversity", action="store_true",
+                    help="(extension) <outpref>_diversity.tsv: segregating sites, multiallelic sites, pi, Watterson's theta "
+                         "and Tajima's D of the core genome every generation; <outpref>_core_sfs.txt: the site frequency "
+                         "spectrum of the last generation")
     return ap
 
 
@@ -62,8 +66,9 @@ def main(argv=None) -> int:
     ns = vars(build_parser().parse_args(argv))
     device = ns.pop("device")
     all_pairs = ns.pop("all_pairs")
+    print_diversity = ns.pop("print_diversity")
     p = Params(**ns)
-    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs)
+    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity)
     return 0                       # the reference exits 0 even when validation fails (main.rs:195-247)
 
 

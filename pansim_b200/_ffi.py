@@ -30,6 +30,8 @@ EXPORTED = [
     "pansim_group_set_initial", "pansim_group_set_selection", "pansim_group_run_generations", "pansim_group_pair_counts",
     "pansim_group_run_generations_stats", "pansim_group_all_pairs", "pansim_group_all_pairs_timing", "pansim_group_gene_counts",
     "pansim_group_download_acc", "pansim_group_download_core", "pansim_group_export_core_csv",
+    "pansim_core_allele_counts", "pansim_core_diversity", "pansim_run_generations_diversity", "pansim_diversity_stats",
+    "pansim_group_core_diversity", "pansim_group_run_generations_diversity",
 ]
 COMM_ID_BYTES = 128
 
@@ -87,6 +89,11 @@ class EventDump(C.Structure):
         ("hr_seq", C.POINTER(C.c_uint32)), ("hr_value", C.POINTER(C.c_uint8)),
         ("acc_flip_mask", C.POINTER(C.c_uint8)), ("acc_gain_mask", C.POINTER(C.c_uint8)),
     ]
+
+
+class Diversity(C.Structure):
+    _fields_ = [("sites", C.c_uint64), ("segregating", C.c_uint64), ("multiallelic", C.c_uint64),
+                ("pair_diff_sum", C.c_uint64)]
 
 
 PAIRS_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.POINTER(C.c_uint32),
@@ -188,5 +195,11 @@ def lib():
     sig("pansim_group_download_acc", cint, vp, vp)
     sig("pansim_group_download_core", cint, vp, vp)
     sig("pansim_group_export_core_csv", cint, vp, u32, u32, vp)
+    sig("pansim_core_allele_counts", cint, vp, vp)
+    sig("pansim_core_diversity", cint, vp, C.POINTER(Diversity), vp)
+    sig("pansim_run_generations_diversity", cint, vp, u32, u32, vp, vp, sz, vp, vp)
+    sig("pansim_diversity_stats", None, C.POINTER(Diversity), u32, vp)
+    sig("pansim_group_core_diversity", cint, vp, C.POINTER(Diversity), vp)
+    sig("pansim_group_run_generations_diversity", cint, vp, u32, u32, vp, vp, sz, vp, vp)
     _lib = L
     return L

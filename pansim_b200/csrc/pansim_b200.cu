@@ -7,6 +7,7 @@
 #include <chrono>
 #include <cmath>
 #include <cstdio>
+#include <limits>
 #include <cstdlib>
 #include <cstring>
 #include <memory>
@@ -19,6 +20,7 @@
 #include "core_hr.cuh"
 #include "core_mut.cuh"
 #include "distance.cuh"
+#include "diversity.cuh"
 #include "pack.cuh"
 #include "replay.cuh"
 #include "select.cuh"
@@ -235,6 +237,13 @@ struct pansim_ctx {
     cudaStream_t stream_stats2[2] = {nullptr, nullptr};   // statistics kernels of consecutive generations run side by side
     cudaEvent_t ev_pairs[2] = {nullptr, nullptr}, ev_stats[2] = {nullptr, nullptr};
     bool ev_stats_valid[2] = {false, false};
+    // diversity reductions (diversity.cuh): packed copy of the clonal row pansim_set_initial started from (the
+    // ancestral allele of every site, for the SFS), per-call / per-generation results and the SFS bins
+    uint32_t *d_anc = nullptr;
+    bool has_anc = false;
+    unsigned long long *d_div = nullptr, *h_div = nullptr;   // [n][4]: segregating, multiallelic, pair_diff_sum, -
+    size_t div_cap = 0;
+    unsigned long long *d_sfs = nullptr, *h_sfs = nullptr;   // [N + 1]
 
     // column shards of one alignment: NCCL communicator over the shards (comm.hpp). With a communicator the
     // pair-count entry points return whole-alignment core counts (summed over the shards on the device).
@@ -1065,7 +1074,7 @@ void pansim_destroy(pansim_ctx *c)
                     c->d_gain_thr, c->tab_mut.d_thr, c->tab_hr.d_thr, c->d_r1, c->d_r2, c->d_cd, c->d_in, c->d_un,
                     c->d_planes, c->d_work_counter, c->d_replay, c->d_hkeys, c->d_hvals, c->d_stage, c->d_groups, c->d_partner, c->d_orig, c->d_batches, c->d_tile_slots, c->d_tile_orig, c->d_dump_counters, c->d_mut_row, c->d_mut_site,
                     c->d_mut_seq, c->d_mut_allele, c->d_hr_rec, c->d_hr_locus, c->d_hr_donor, c->d_hr_seq,
-                    c->d_hr_value, c->d_dump_flip, c->d_dump_gain};
+                    c->d_hr_value, c->d_dump_flip, c->d_dump_gain, c->d_anc, c->d_div, c->d_sfs};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (auto *e : c->graphs) {
@@ -1087,6 +1096,8 @@ void pansim_destroy(pansim_ctx *c)
     }
     if (c->h_stats) cudaFreeHost(c->h_stats);
     if (c->d_stats) cudaFree(c->d_stats);
+    if (c->h_div) cudaFreeHost(c->h_div);
+    if (c->h_sfs) cudaFreeHost(c->h_sfs);
     for (auto q : c->d_cnt2) if (q) cudaFree(q);
     for (int i = 0; i < 2; i++) {
         if (c->ev_pairs[i]) cudaEventDestroy(c->ev_pairs[i]);
@@ -1459,6 +1470,9 @@ int pansim_set_initial(pansim_ctx *c, const uint8_t *core_row, const uint8_t *ac
         c->core_version++;
         pack_core_kernel<<<div_up64(c->core_stride / 4, 256), 256, 0, c->stream>>>(c->d_stage, c->Ll, 0, 1, dst, c->core_stride, c->d_err);
         LAUNCH_CHECK(c);
+        // the clonal row is the ancestral row of the SFS (pansim_core_diversity); uploads leave it alone
+        if (!c->d_anc) CU(c, cudaMalloc(&c->d_anc, c->core_stride));
+        CU(c, cudaMemcpyAsync(c->d_anc, dst, c->core_stride, cudaMemcpyDeviceToDevice, c->stream));
         if (c->N > 1) {
             const uint64_t vecs = (uint64_t)(c->N - 1) * (c->core_stride / 16);
             replicate_row_kernel<<<div_up64(vecs, 256), 256, 0, c->stream>>>(dst, c->core_stride, c->N);
@@ -1467,6 +1481,7 @@ int pansim_set_initial(pansim_ctx *c, const uint8_t *core_row, const uint8_t *ac
         if (int rc = check_device_flag(c, PANSIM_ERR_INVALID, "core row holds a byte that is not one-hot {1,2,4,8}")) return rc;
     }
     c->has_core = true;
+    c->has_anc = true;
     if (c->G) {
         std::vector<uint8_t> full((size_t)c->N * c->G);
         for (uint32_t r = 0; r < c->N; r++) memcpy(full.data() + (size_t)r * c->G, acc_row, c->G);
@@ -2319,7 +2334,7 @@ static int stats_generation(pansim_ctx *c, uint32_t gen, int slot, size_t P, boo
         CU(c, cudaEventRecord(c->ev_mat, sp));
         CU(c, cudaStreamWaitEvent(c->stream_core, c->ev_mat, 0));       // the next core step reads the materialised rows
     }
-    const int rc = pair_launch(c, P, cd, want_acc ? in : nullptr, want_acc ? un : nullptr);
+    const int rc = P ? pair_launch(c, P, cd, want_acc ? in : nullptr, want_acc ? un : nullptr) : 0;   // P = 0: diversity batch without pairs
     if (rc) { c->ps = c->stream; return rc; }
     *cd_out = cd; *in_out = in; *un_out = un;
     return 0;        // c->ps stays on stream_pairs: the caller's all-reduce and statistics launch follow the pass
@@ -2527,6 +2542,200 @@ int pansim_gene_counts(pansim_ctx *c, uint32_t *counts)
     CU(c, cudaMemcpyAsync(counts, c->d_gain_thr, (size_t)c->G * 4, cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     return 0;
+}
+
+// ---- core-genome diversity (diversity.cuh) ----------------------------------------------------
+static int ensure_div(pansim_ctx *c, size_t n, bool sfs)
+{
+    if (n > c->div_cap) {
+        if (c->d_div) cudaFree(c->d_div);
+        if (c->h_div) cudaFreeHost(c->h_div);
+        c->d_div = nullptr; c->h_div = nullptr; c->div_cap = 0;
+        CU(c, cudaMalloc(&c->d_div, n * 4 * sizeof(unsigned long long)));
+        CU(c, cudaMallocHost(&c->h_div, n * 4 * sizeof(unsigned long long)));
+        c->div_cap = n;
+    }
+    if (sfs && !c->d_sfs) {
+        CU(c, cudaMalloc(&c->d_sfs, ((size_t)c->N + 1) * sizeof(unsigned long long)));
+        CU(c, cudaMallocHost(&c->h_sfs, ((size_t)c->N + 1) * sizeof(unsigned long long)));
+    }
+    return 0;
+}
+
+// the column reduction of the current core buffer on `st`: adds into d_out[0..2] (and d_sfs[0..N]), which
+// the caller has zeroed; the rows must be materialised
+static int launch_diversity(pansim_ctx *c, cudaStream_t st, unsigned long long *d_out, uint4 *d_counts, unsigned long long *d_sfs)
+{
+    if (c->Ll == 0) return 0;
+    DiversityArgs a;
+    a.state = reinterpret_cast<const uint32_t *>(c->core[c->core_cur]);
+    a.row_words = c->core_stride / 4;
+    a.n_sites = c->Ll;
+    a.n_rows = c->N;
+    a.anc = c->d_anc;
+    a.out = d_out;
+    a.counts = d_counts;
+    a.sfs = d_sfs;
+    const uint32_t grid = div_up64(c->Ll, DV_SITES);
+    if (d_counts)
+        diversity_kernel<true, false><<<grid, DV_THREADS, 0, st>>>(a);
+    else if (d_sfs)
+        diversity_kernel<false, true><<<grid, DV_THREADS, std::min<size_t>((size_t)c->N + 1, DV_SFS_BINS) * 4, st>>>(a);
+    else
+        diversity_kernel<false, false><<<grid, DV_THREADS, 0, st>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+static void diversity_from_host(const pansim_ctx *c, const unsigned long long *h, pansim_diversity *out)
+{
+    out->sites = c->Ll;
+    out->segregating = h[0];
+    out->multiallelic = h[1];
+    out->pair_diff_sum = h[2];
+}
+
+// one call's reduction enqueued on c->stream, results into the pinned h_div / h_sfs (the group variant
+// enqueues on every shard before it synchronises)
+static int core_diversity_enqueue(pansim_ctx *c, bool sfs)
+{
+    if (int rc = require_state(c)) return rc;
+    if (sfs && !c->has_anc) FAIL(c, PANSIM_ERR_STATE, "the SFS needs the ancestral row: call pansim_set_initial first");
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (int rc = ensure_div(c, 1, sfs)) return rc;
+    c->ps = c->stream;
+    if (c->Ll)
+        if (int rc = core_materialize(c, c->stream)) return rc;
+    CU(c, cudaMemsetAsync(c->d_div, 0, 4 * sizeof(unsigned long long), c->stream));
+    if (sfs) CU(c, cudaMemsetAsync(c->d_sfs, 0, ((size_t)c->N + 1) * sizeof(unsigned long long), c->stream));
+    timing_begin(c);                    // pansim_get_timing: total_ms = the reduction kernel alone
+    if (int rc = launch_diversity(c, c->stream, c->d_div, nullptr, sfs ? c->d_sfs : nullptr)) return rc;
+    timing_end(c);
+    CU(c, cudaMemcpyAsync(c->h_div, c->d_div, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    if (sfs) CU(c, cudaMemcpyAsync(c->h_sfs, c->d_sfs, ((size_t)c->N + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    return flags_enqueue_readback(c);
+}
+
+static int core_diversity_finish(pansim_ctx *c, pansim_diversity *out, uint64_t *sfs)
+{
+    CU(c, cudaSetDevice(c->cfg.device));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (int rc = flags_inspect(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG)) return rc;
+    diversity_from_host(c, c->h_div, out);
+    if (sfs) memcpy(sfs, c->h_sfs, ((size_t)c->N + 1) * sizeof(uint64_t));
+    return 0;
+}
+
+int pansim_core_allele_counts(pansim_ctx *c, uint32_t *counts)
+{
+    if (!c || !counts) return PANSIM_ERR_INVALID;
+    if (int rc = require_state(c)) return rc;
+    if (c->Ll == 0) return 0;
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (int rc = ensure_div(c, 1, false)) return rc;
+    if (int rc = ensure_stage(c, (size_t)c->Ll * 16)) return rc;
+    c->ps = c->stream;
+    if (int rc = core_materialize(c, c->stream)) return rc;
+    CU(c, cudaMemsetAsync(c->d_div, 0, 4 * sizeof(unsigned long long), c->stream));
+    if (int rc = launch_diversity(c, c->stream, c->d_div, reinterpret_cast<uint4 *>(c->d_stage), nullptr)) return rc;
+    CU(c, cudaMemcpyAsync(counts, c->d_stage, (size_t)c->Ll * 16, cudaMemcpyDeviceToHost, c->stream));
+    return check_device_flag(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG);
+}
+
+int pansim_core_diversity(pansim_ctx *c, pansim_diversity *out, uint64_t *sfs)
+{
+    if (!c || !out) return PANSIM_ERR_INVALID;
+    if (int rc = core_diversity_enqueue(c, sfs != nullptr)) return rc;
+    return core_diversity_finish(c, out, sfs);
+}
+
+// One generation of the diversity batch: stats_generation (the step, then on stream_pairs the materialised
+// rows and, with P > 0, the distance pass) followed on the same stream by the reduction into d_out. Whatever
+// the caller enqueues next on c->ps (all-reduce, statistics launch or the bare ev_pairs record) comes after
+// the reduction, so the back-pressure of generation g + 2 on ev_pairs[slot] also keeps core step g + 2 from
+// overwriting the buffer the reduction reads.
+static int diversity_generation(pansim_ctx *c, uint32_t gen, int slot, size_t P, bool want_acc, unsigned long long *d_out,
+                                uint32_t **cd_out, uint32_t **in_out, uint32_t **un_out)
+{
+    if (int rc = stats_generation(c, gen, slot, P, want_acc, cd_out, in_out, un_out)) return rc;
+    if (int rc = launch_diversity(c, c->ps, d_out, nullptr, nullptr)) { c->ps = c->stream; return rc; }
+    return 0;
+}
+
+// ev_pairs[slot] behind the reduction when no statistics kernel follows (launch_pair_stats records it otherwise)
+static int record_pass_done(pansim_ctx *c, int slot)
+{
+    CU(c, cudaEventRecord(c->ev_pairs[slot], c->ps));
+    c->ev_pairs_valid[slot] = true;
+    return 0;
+}
+
+int pansim_run_generations_diversity(pansim_ctx *c, uint32_t gen0, uint32_t n, const uint32_t *r1, const uint32_t *r2, size_t P,
+                                     double *stats_out, pansim_diversity *div_out)
+{
+    if (!c || !div_out || (P && (!r1 || !r2 || !stats_out))) return PANSIM_ERR_INVALID;
+    if (int rc = require_state(c)) return rc;
+    if (P)
+        if (int rc = require_whole_alignment(c, "pansim_run_generations_diversity with pairs")) return rc;
+    if (n == 0) return 0;
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (P)
+        if (int rc = ensure_pairs(c, P)) return rc;
+    if (int rc = ensure_stats(c, n, P, P > 0)) return rc;
+    if (int rc = ensure_div(c, n, false)) return rc;
+    if (P)
+        if (int rc = pair_prepare(c, r1, r2, P)) return rc;
+    if (c->dump_enabled) CU(c, cudaMemsetAsync(c->d_dump_counters, 0, 2 * sizeof(uint32_t), c->stream));
+    timing_begin(c);
+    CU(c, cudaMemsetAsync(c->d_div, 0, (size_t)n * 4 * sizeof(unsigned long long), c->stream));
+    for (uint32_t g = 0; g < n; g++) {
+        const int slot = (int)(g & 1u);
+        uint32_t *cd = nullptr, *in = nullptr, *un = nullptr;
+        if (int rc = diversity_generation(c, gen0 + g, slot, P, true, c->d_div + (size_t)g * 4, &cd, &in, &un)) return rc;
+        if (P) {
+            if (int rc = comm_allreduce_counts(c, cd, P)) return rc;
+            if (int rc = launch_pair_stats(c, slot, P, cd, in, un, c->d_stats + (size_t)g * 4)) return rc;
+        } else {
+            if (int rc = record_pass_done(c, slot)) return rc;
+        }
+    }
+    if (int rc = stats_batch_end(c)) return rc;
+    timing_end(c);
+    if (P) CU(c, cudaMemcpyAsync(c->h_stats, c->d_stats, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(c->h_div, c->d_div, (size_t)n * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    if (int rc = check_device_flag(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG)) return rc;
+    if (P) memcpy(stats_out, c->h_stats, (size_t)n * 4 * sizeof(double));
+    for (uint32_t g = 0; g < n; g++) diversity_from_host(c, c->h_div + (size_t)g * 4, div_out + g);
+    return 0;
+}
+
+// Tajima (1989), Genetics 123:585-595, eq. 4-9 and 38, evaluated in one fixed order so every host gets the same bits
+void pansim_diversity_stats(const pansim_diversity *d, uint32_t pop_size, double out[3])
+{
+    const double nan = std::numeric_limits<double>::quiet_NaN();
+    if (!d || !out) return;
+    if (pop_size < 2) { out[0] = out[1] = out[2] = nan; return; }
+    const double n = (double)pop_size, S = (double)d->segregating;
+    double a1 = 0.0, a2 = 0.0;
+    for (uint32_t i = 1; i < pop_size; i++) {
+        const double x = (double)i;
+        a1 += 1.0 / x;
+        a2 += 1.0 / (x * x);
+    }
+    const double pairs = (double)((uint64_t)pop_size * (pop_size - 1u) / 2u);
+    const double pi = (double)d->pair_diff_sum / pairs;
+    const double theta_w = S / a1;
+    const double b1 = (n + 1.0) / (3.0 * (n - 1.0));
+    const double b2 = (2.0 * (n * n + n + 3.0)) / (9.0 * n * (n - 1.0));
+    const double c1 = b1 - 1.0 / a1;
+    const double c2 = b2 - (n + 2.0) / (a1 * n) + a2 / (a1 * a1);
+    const double e1 = c1 / a1;
+    const double e2 = c2 / (a1 * a1 + a2);
+    const double var = e1 * S + e2 * S * (S - 1.0);
+    const double den = std::sqrt(var);
+    out[0] = pi;
+    out[1] = theta_w;
+    out[2] = (d->segregating == 0 || !(den > 0.0)) ? nan : (pi - theta_w) / den;
 }
 
 // ---- communicator over column shards (one process per GPU) -------------------

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import OK, PansimError, _ptr, make_config
+from .population import OK, PansimError, _diversity, _pairs_or_none, _ptr, make_config
 
 
 class PansimGroup:
@@ -104,6 +104,41 @@ class PansimGroup:
         wall, nccl, pairs = C.c_float(), C.c_float(), C.c_uint64()
         self._check(self._lib.pansim_group_all_pairs_timing(self._h, C.byref(wall), C.byref(nccl), C.byref(pairs)))
         return dict(wall_ms=wall.value, nccl_ms_shard0=nccl.value, pairs=pairs.value)
+
+    def core_diversity(self, sfs: bool = False):
+        """Whole-alignment diversity (shard partials summed); with sfs=True also the SFS [N + 1] (Pansim.core_diversity)."""
+        d = _ffi.Diversity()
+        h = np.empty(self.N + 1, np.uint64) if sfs else None
+        self._check(self._lib.pansim_group_core_diversity(self._h, C.byref(d), _ptr(h)))
+        return (_diversity(d), h) if sfs else _diversity(d)
+
+    def core_allele_counts(self) -> np.ndarray:
+        """uint32 [core_size, 4] assembled from the shards (Pansim.core_allele_counts per shard context)."""
+        out = np.empty((self.L, 4), np.uint32)
+        for i in range(self.size):
+            h = self._lib.pansim_group_ctx(self._h, i)
+            info = _ffi.Info()
+            self._check(self._lib.pansim_get_info(h, C.byref(info)))
+            part = np.empty((info.local_sites, 4), np.uint32)
+            rc = self._lib.pansim_core_allele_counts(h, _ptr(part))
+            if rc != OK:
+                raise PansimError(rc, self._lib.pansim_last_error(h).decode())
+            begin = self._shard_begin(i)
+            out[begin:begin + info.local_sites] = part
+        return out
+
+    def _shard_begin(self, i: int) -> int:
+        b, e = C.c_uint64(), C.c_uint64()
+        self._check(self._lib.pansim_shard_bounds(self.L, self.size, i, C.byref(b), C.byref(e)))
+        return b.value
+
+    def run_generations_diversity(self, gen0: int, n: int, range1=None, range2=None):
+        """Pansim.run_generations_diversity over the shards: (list of n whole-alignment Diversity, stats or None)."""
+        r1, r2, P = _pairs_or_none(range1, range2)
+        divs = (_ffi.Diversity * max(n, 1))()
+        st = np.empty((n, 4), np.float64) if P else None
+        self._check(self._lib.pansim_group_run_generations_diversity(self._h, gen0, n, _ptr(r1), _ptr(r2), P, _ptr(st), divs))
+        return [_diversity(divs[g]) for g in range(n)], st
 
     def gene_counts(self) -> np.ndarray:
         out = np.empty(self.G, np.uint32)

@@ -42,7 +42,8 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
                              "prop_genes2", "prop_positive", "pos_lambda", "neg_lambda", "seed", "outpref",
                              "threads", "genome_size_penalty", "competition_strength", "device", "gpus"};
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
-                              "all_pairs"};   // all_pairs: extension (every pair i < j in <outpref>.tsv)
+                              "all_pairs", "print_diversity"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                                                                 // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -124,7 +125,7 @@ int main(int argc, char **argv)
     const double pos_lambda = as_f64(fl, "pos_lambda"), neg_lambda = as_f64(fl, "neg_lambda");
     const uint64_t seed = std::strtoull(fl.val["seed"].c_str(), nullptr, 10);
     const bool verbose = fl.sw["verbose"], print_dist = fl.sw["print_dist"], print_matrices = fl.sw["print_matrices"];
-    const bool all_pairs = fl.sw["all_pairs"];
+    const bool all_pairs = fl.sw["all_pairs"], print_diversity = fl.sw["print_diversity"];
     const int n_gpus = std::max(1, std::atoi(fl.val["gpus"].c_str()));       // extension: column shards over N devices of the box
     const bool print_selection = fl.sw["print_selection"], no_control = fl.sw["no_control_genome_size"];
     const double genome_size_penalty = as_f64(fl, "genome_size_penalty"), competition_strength = as_f64(fl, "competition_strength");
@@ -214,6 +215,7 @@ int main(int argc, char **argv)
         pops.set_selection(selection);
         std::vector<double> avg_core(n_gen, 0.0), avg_acc(n_gen, 0.0), std_core(n_gen, 0.0), std_acc(n_gen, 0.0);
         std::vector<double> core_d, acc_d;
+        std::vector<pansim_diversity> diversity;
         auto last_generation_outputs = [&]() {                              // main.rs:467-499
             std::ofstream f(outpref + ".tsv");
             if (all_pairs) {
@@ -233,7 +235,12 @@ int main(int argc, char **argv)
         const bool device_loop = !verbose;
         int first_host_gen = 0;
         if (device_loop) {
-            if (print_dist) {
+            if (print_diversity) {                                          // one batch: reduction (+ --print_dist pass) per generation
+                std::vector<double> st;
+                const std::vector<uint32_t> none;
+                diversity = pops.run_generations_diversity(0, (uint32_t)n_gen, print_dist ? range1 : none, print_dist ? range2 : none, st);
+                for (int j = 0; j < n_gen && print_dist; j++) { avg_core[j] = st[4 * j]; std_core[j] = st[4 * j + 1]; avg_acc[j] = st[4 * j + 2]; std_acc[j] = st[4 * j + 3]; }
+            } else if (print_dist) {
                 const std::vector<double> st = pops.run_generations_stats(0, (uint32_t)n_gen, range1, range2);
                 for (int j = 0; j < n_gen; j++) { avg_core[j] = st[4 * j]; std_core[j] = st[4 * j + 1]; avg_acc[j] = st[4 * j + 2]; std_acc[j] = st[4 * j + 3]; }
             } else {
@@ -244,6 +251,7 @@ int main(int argc, char **argv)
         }
         for (int j = first_host_gen; j < n_gen; j++) {
             pops.step((uint32_t)j);                                         // main.rs:435-464
+            if (print_diversity) diversity.push_back(pops.core_diversity());
             if (j == n_gen - 1) last_generation_outputs();
             if (print_dist) {                                               // main.rs:502-519
                 if (j != n_gen - 1 || all_pairs) pops.pairwise_distances(range1, range2, core_d, acc_d);
@@ -259,6 +267,18 @@ int main(int argc, char **argv)
             std::ofstream f(outpref + "_per_gen.tsv");
             for (int j = 0; j < n_gen; j++)
                 f << fmt(avg_core[j]) << "\t" << fmt(std_core[j]) << "\t" << fmt(avg_acc[j]) << "\t" << fmt(std_acc[j]) << "\n";
+        }
+        if (print_diversity) {                                              // extension: core-genome diversity
+            std::vector<uint64_t> sfs;
+            pops.core_diversity(&sfs);
+            std::ofstream f(outpref + "_diversity.tsv");
+            for (const pansim_diversity &d : diversity) {
+                double st[3];
+                pansim_diversity_stats(&d, (uint32_t)pop_size, st);
+                f << d.segregating << "\t" << d.multiallelic << "\t" << fmt(st[0]) << "\t" << fmt(st[1]) << "\t" << fmt(st[2]) << "\n";
+            }
+            std::ofstream g(outpref + "_core_sfs.txt");
+            for (uint64_t x : sfs) g << x << "\n";
         }
         if (print_matrices) pops.write(outpref);                            // main.rs:550-553
     } catch (const pansim::Error &e) {

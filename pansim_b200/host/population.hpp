@@ -129,6 +129,25 @@ public:
     }
     // main.rs:435-464 for generations gen0 .. gen0+n-1 as one device-resident batch
     void run_generations(uint32_t gen0, uint32_t n) { gcheck(pansim_group_run_generations(grp_, gen0, n)); }
+    // (extension) the same batch with the core-genome diversity reduction after every generation; with pairs
+    // (range1 non-empty) also the --print_dist statistics, stats_out[n*4] as run_generations_stats gives them
+    std::vector<pansim_diversity> run_generations_diversity(uint32_t gen0, uint32_t n, const std::vector<uint32_t> &range1,
+                                                            const std::vector<uint32_t> &range2, std::vector<double> &stats_out)
+    {
+        std::vector<pansim_diversity> out(n);
+        stats_out.assign(range1.empty() ? 0 : (size_t)n * 4, 0.0);
+        gcheck(pansim_group_run_generations_diversity(grp_, gen0, n, range1.data(), range2.data(), range1.size(),
+                                                      stats_out.empty() ? nullptr : stats_out.data(), out.data()));
+        return out;
+    }
+    // (extension) core-genome diversity of the current state over the whole alignment; sfs [N+1] if non-null
+    pansim_diversity core_diversity(std::vector<uint64_t> *sfs = nullptr)
+    {
+        pansim_diversity d;
+        if (sfs) sfs->assign((size_t)cfg_.pop_size + 1, 0);
+        gcheck(pansim_group_core_diversity(grp_, &d, sfs ? sfs->data() : nullptr));
+        return d;
+    }
     // population.rs:840-863: accessory gene frequencies, then core_genes x 1.0
     std::vector<double> gene_frequencies()
     {

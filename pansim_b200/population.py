@@ -11,6 +11,7 @@ boundary (population.rs:822, 828-830, 852).
 from __future__ import annotations
 
 import ctypes as C
+from typing import NamedTuple
 
 import numpy as np
 
@@ -66,6 +67,35 @@ def standard_deviation(values) -> tuple[float, float]:
     d = v - mean
     ss = float(np.cumsum(d * d)[-1])
     return float(np.sqrt(ss / n)), mean
+
+
+class Diversity(NamedTuple):
+    """pansim_diversity: integer summaries of the core alignment (partials over the sites of a column shard)."""
+    sites: int
+    segregating: int
+    multiallelic: int
+    pair_diff_sum: int
+
+
+def _diversity(d: _ffi.Diversity) -> Diversity:
+    return Diversity(d.sites, d.segregating, d.multiallelic, d.pair_diff_sum)
+
+
+def diversity_stats(d: Diversity, pop_size: int) -> tuple[float, float, float]:
+    """(pi, theta_W, Tajima's D) of whole-alignment summaries, evaluated by the library (pansim_diversity_stats)
+    so every host forms the same bits. D is NaN when no site segregates; all three are NaN when pop_size < 2."""
+    out = np.empty(3, np.float64)
+    _ffi.lib().pansim_diversity_stats(C.byref(_ffi.Diversity(*d)), pop_size, _ptr(out))
+    return float(out[0]), float(out[1]), float(out[2])
+
+
+def _pairs_or_none(range1, range2):
+    if range1 is None:
+        return None, None, 0
+    r1 = np.ascontiguousarray(range1, np.uint32)
+    r2 = np.ascontiguousarray(range2, np.uint32)
+    assert r1.shape == r2.shape
+    return r1, r2, len(r1)
 
 
 class Pansim:
@@ -315,6 +345,30 @@ class Pansim:
         self._check(self._lib.pansim_run_generations_stats(self._h, gen0, n, _ptr(r1), _ptr(r2), len(r1), _ptr(out)))
         return out
 
+    # -- core-genome diversity (extension) ---------------------------------
+    def core_allele_counts(self) -> np.ndarray:
+        """Per-site allele counts of the local sites: uint32 [local_sites, 4] = n_A, n_C, n_G, n_T."""
+        out = np.empty((self.local_sites, 4), np.uint32)
+        self._check(self._lib.pansim_core_allele_counts(self._h, _ptr(out)))
+        return out
+
+    def core_diversity(self, sfs: bool = False):
+        """Diversity of the current core state; with sfs=True also (Diversity, sfs[N + 1] uint64), where sfs[k]
+        counts the sites at which k individuals differ from the row given to set_initial."""
+        d = _ffi.Diversity()
+        h = np.empty(self.N + 1, np.uint64) if sfs else None
+        self._check(self._lib.pansim_core_diversity(self._h, C.byref(d), _ptr(h)))
+        return (_diversity(d), h) if sfs else _diversity(d)
+
+    def run_generations_diversity(self, gen0: int, n: int, range1=None, range2=None):
+        """n generations in one device-resident batch, each followed by the diversity reduction: (list of n
+        Diversity, stats). With pairs, stats is the [n, 4] array of run_generations_stats (same bits); else None."""
+        r1, r2, P = _pairs_or_none(range1, range2)
+        divs = (_ffi.Diversity * max(n, 1))()
+        st = np.empty((n, 4), np.float64) if P else None
+        self._check(self._lib.pansim_run_generations_diversity(self._h, gen0, n, _ptr(r1), _ptr(r2), P, _ptr(st), divs))
+        return [_diversity(divs[g]) for g in range(n)], st
+
     # -- multi-GPU: communicator over column shards (one process per GPU) --
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -441,4 +495,4 @@ class Pansim:
                 f.write(",".join(ones + [str(int(x)) for x in acc[r]]) + "\n")
 
 
-__all__ = ["Pansim", "PansimError", "make_config", "standard_deviation", "fmt_f64"]
+__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "make_config", "standard_deviation", "fmt_f64"]

@@ -17,7 +17,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from .params import Derived, Params, derive, fmt_f64, validate
-from .population import Pansim, standard_deviation
+from .population import Pansim, diversity_stats, standard_deviation
 
 
 def selection_coefficients(p: Params, pan_size: int, rng: np.random.Generator) -> np.ndarray:
@@ -59,14 +59,20 @@ class RunResult:
     acc_distances: np.ndarray = None
     gene_freqs: np.ndarray = None            # accessory genes then core_genes ones (population.rs:857-860)
     per_gen: list = field(default_factory=list)   # (avg_core, std_core, avg_acc, std_acc)
+    diversity: list = field(default_factory=list) # per generation: Diversity (--print_diversity)
+    sfs: np.ndarray = None                        # SFS of the last generation (--print_diversity)
     selection: np.ndarray = None
     stdout: list = field(default_factory=list)
 
 
-def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False) -> RunResult | None:
+def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False,
+        print_diversity: bool = False) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
-    in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None."""
+    in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
+    print_diversity (extension): core-genome diversity every generation, written to
+    `<outpref>_diversity.tsv` (segregating, multiallelic, pi, theta_W, Tajima's D) and the site frequency
+    spectrum of the last generation to `<outpref>_core_sfs.txt`."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -114,7 +120,11 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
         device_loop = not p.verbose and not (p.print_dist and all_pairs)
         first_host_gen = 0
         if device_loop:
-            if p.print_dist:
+            if print_diversity:        # one batch: the reduction (and the --print_dist pass) after every generation
+                res.diversity, st = sim.run_generations_diversity(0, p.n_gen, *((r1, r2) if p.print_dist else ()))
+                if p.print_dist:
+                    res.per_gen = [tuple(float(x) for x in row) for row in st]
+            elif p.print_dist:
                 res.per_gen = [tuple(float(x) for x in row) for row in sim.run_generations_stats(0, p.n_gen, r1, r2)]
             else:
                 sim.run_generations(0, p.n_gen)
@@ -122,6 +132,8 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             last_generation_outputs()
         for j in range(first_host_gen, p.n_gen):                                 # main.rs:429
             sim.step(j)                                                          # main.rs:435-464
+            if print_diversity:
+                res.diversity.append(sim.core_diversity())
             if j == p.n_gen - 1:
                 last_generation_outputs()
             if p.print_dist:                                                     # main.rs:502-519
@@ -144,9 +156,24 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             with open(outpref + "_per_gen.tsv", "w") as f:
                 for avg_core, std_core, avg_acc, std_acc in res.per_gen:
                     f.write(f"{fmt_f64(avg_core)}\t{fmt_f64(std_core)}\t{fmt_f64(avg_acc)}\t{fmt_f64(std_acc)}\n")
+        if print_diversity:
+            _, res.sfs = sim.core_diversity(sfs=True)
+            if outpref:
+                write_diversity(outpref, res.diversity, res.sfs, p.pop_size)
         if p.print_matrices and outpref:                                         # main.rs:550-553
             sim.write(outpref)
     return res
+
+
+def write_diversity(outpref: str, diversity, sfs, pop_size: int):
+    """`<outpref>_diversity.tsv`: per generation segregating, multiallelic, pi, theta_W, Tajima's D (no header,
+    like _per_gen.tsv); `<outpref>_core_sfs.txt`: the N + 1 SFS bins, one per line."""
+    with open(outpref + "_diversity.tsv", "w") as f:
+        for d in diversity:
+            pi, tw, td = diversity_stats(d, pop_size)
+            f.write(f"{d.segregating}\t{d.multiallelic}\t{fmt_f64(pi)}\t{fmt_f64(tw)}\t{fmt_f64(td)}\n")
+    with open(outpref + "_core_sfs.txt", "w") as f:
+        f.write("".join(f"{int(x)}\n" for x in sfs))
 
 
 def summarize(core_d, acc_d, gene_freqs, n_acc_genes: int) -> dict:
