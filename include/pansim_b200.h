@@ -245,6 +245,28 @@ int pansim_run_generations_diversity(pansim_ctx *ctx, uint32_t gen0, uint32_t n,
  * how far the infinite-sites assumption behind theta_W and D is violated. */
 void pansim_diversity_stats(const pansim_diversity *d, uint32_t pop_size, double out[3]);
 
+/* ---- core-genome VCF (extension: the reference writes the alignment only as _core_genome.csv) ----
+ * The alignment as VCF 4.2 text, expanded on the device and streamed to the file through the pinned
+ * double-buffered pipeline of pansim_write_core_csv (DESIGN.md section 11). Header (each line ends in \n):
+ *   ##fileformat=VCFv4.2 / ##source=pansim_b200 / ##contig=<ID=core,length=core_size> /
+ *   ##FORMAT=<ID=GT,Number=1,Type=String,Description="Genotype"> /
+ *   #CHROM POS ID REF ALT QUAL FILTER INFO FORMAT ind_0 .. ind_{N-1}   (tab-separated; ind_i is row i)
+ * Then, in position order, one line per site where some row carries an allele other than the ancestral one:
+ *   core POS . REF ALT . . . GT g_0 .. g_{N-1}
+ * POS = global site index + 1; REF = the site's letter in the row given to pansim_set_initial (uploads do not
+ * change it, as for the SFS); ALT = the other letters with a count above zero, in A,C,G,T order, comma-separated;
+ * g_i = 0 for REF, else 1 + the index of row i's letter in ALT (haploid, one digit). A site fixed for another
+ * letter is written (ALT of one letter, every g_i = 1); a site where every row carries REF is not. A line is
+ * 19 + digits(POS) + 2 |ALT| + 2 N bytes. The state is read after recombine(), like every reader.
+ * Without pansim_set_initial the calls fail with PANSIM_ERR_STATE; a failed or short write fails with
+ * PANSIM_ERR_INVALID. bytes_out (may be NULL) = bytes written. A column-shard context writes its own lines
+ * with global POS: the header-less bodies of the shards, concatenated in shard order, are the whole body. */
+int pansim_write_core_vcf(pansim_ctx *ctx, const char *path, int with_header, uint64_t *bytes_out);
+/* measurement: the site pass (allele counts, line descriptors, offset scan, chunking) and the expansion of
+ * every chunk into device memory, each `repeats` times with no copy to the host; mean device ms of one
+ * pass (CUDA events) and the bytes of text (header excluded) */
+int pansim_core_vcf_kernel_ms(pansim_ctx *ctx, uint32_t repeats, float *site_ms, float *expand_ms, uint64_t *text_bytes);
+
 /* ---- multi-GPU: column shards of one alignment --------------------------
  * (SURVEY.md 8e; the reference is one shared-memory process, population.rs has no analogue.)
  * Every shard context holds all individuals for [site_begin, site_end) and a replica of the
@@ -299,6 +321,8 @@ int pansim_group_run_generations_diversity(pansim_group *g, uint32_t gen0, uint3
 int pansim_group_download_acc(pansim_group *g, uint8_t *acc_out);
 int pansim_group_download_core(pansim_group *g, uint8_t *core_onehot_out);               /* [N x core_size] */
 int pansim_group_export_core_csv(pansim_group *g, uint32_t row_begin, uint32_t row_end, char *out);
+/* the whole-alignment VCF of pansim_write_core_vcf: the header once, then every shard's lines in shard order */
+int pansim_group_write_core_vcf(pansim_group *g, const char *path, uint64_t *bytes_out);
 
 /* ---- introspection / instrumentation ----------------------------------- */
 typedef struct {

@@ -4,7 +4,7 @@ Same long flags (underscores, capitalised --HR_rate / --HGT_rate), same defaults
 same parsing quirks: pop_size/core_size/pan_genes/core_genes/n_gen are parsed as
 f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
-accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity.
+accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf.
 """
 from __future__ import annotations
 
@@ -59,6 +59,9 @@ def build_parser() -> argparse.ArgumentParser:
                     help="(extension) <outpref>_diversity.tsv: segregating sites, multiallelic sites, pi, Watterson's theta "
                          "and Tajima's D of the core genome every generation; <outpref>_core_sfs.txt: the site frequency "
                          "spectrum of the last generation")
+    ap.add_argument("--print_vcf", action="store_true",
+                    help="(extension) <outpref>_core_genome.vcf: the core alignment of the last generation as VCF, one "
+                         "line per site that differs from the initial row, haploid genotypes against it")
     return ap
 
 
@@ -67,8 +70,9 @@ def main(argv=None) -> int:
     device = ns.pop("device")
     all_pairs = ns.pop("all_pairs")
     print_diversity = ns.pop("print_diversity")
+    print_vcf = ns.pop("print_vcf")
     p = Params(**ns)
-    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity)
+    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf)
     return 0                       # the reference exits 0 even when validation fails (main.rs:195-247)
 
 

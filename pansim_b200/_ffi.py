@@ -32,6 +32,7 @@ EXPORTED = [
     "pansim_group_download_acc", "pansim_group_download_core", "pansim_group_export_core_csv",
     "pansim_core_allele_counts", "pansim_core_diversity", "pansim_run_generations_diversity", "pansim_diversity_stats",
     "pansim_group_core_diversity", "pansim_group_run_generations_diversity",
+    "pansim_write_core_vcf", "pansim_group_write_core_vcf", "pansim_core_vcf_kernel_ms",
 ]
 COMM_ID_BYTES = 128
 
@@ -201,5 +202,8 @@ def lib():
     sig("pansim_diversity_stats", None, C.POINTER(Diversity), u32, vp)
     sig("pansim_group_core_diversity", cint, vp, C.POINTER(Diversity), vp)
     sig("pansim_group_run_generations_diversity", cint, vp, u32, u32, vp, vp, sz, vp, vp)
+    sig("pansim_write_core_vcf", cint, vp, C.c_char_p, cint, C.POINTER(C.c_uint64))
+    sig("pansim_group_write_core_vcf", cint, vp, C.c_char_p, C.POINTER(C.c_uint64))
+    sig("pansim_core_vcf_kernel_ms", cint, vp, u32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint64))
     _lib = L
     return L

@@ -24,6 +24,7 @@
 #include "pack.cuh"
 #include "replay.cuh"
 #include "select.cuh"
+#include "vcf.cuh"
 
 using namespace pansim;
 
@@ -258,10 +259,15 @@ struct pansim_ctx {
     uint32_t *d_hvals = nullptr;
     size_t hash_cap = 0;
 
-    // CSV export: two device + two pinned host chunks (double buffering), completion events
-    char *d_csv[2] = {nullptr, nullptr}, *h_csv[2] = {nullptr, nullptr};
-    cudaEvent_t ev_csv[2] = {nullptr, nullptr};
-    size_t csv_cap = 0;
+    // text export (CSV, VCF): two device + two pinned host chunks (double buffering), completion events
+    char *d_txt[2] = {nullptr, nullptr}, *h_txt[2] = {nullptr, nullptr};
+    cudaEvent_t ev_txt[2] = {nullptr, nullptr};
+    size_t txt_cap = 0;
+    // VCF export (vcf.cuh): per-site allele counts, line descriptors and offsets, scan blocks, chunk bounds
+    uint4 *d_vcf_counts = nullptr;
+    uint8_t *d_vcf_desc = nullptr;
+    unsigned long long *d_vcf_off = nullptr, *d_vcf_block = nullptr, *d_vcf_bounds = nullptr;
+    uint32_t *d_vcf_nchunks = nullptr;
     // staging for upload/download
     uint8_t *d_stage = nullptr;
     size_t stage_cap = 0;
@@ -1074,7 +1080,8 @@ void pansim_destroy(pansim_ctx *c)
                     c->d_gain_thr, c->tab_mut.d_thr, c->tab_hr.d_thr, c->d_r1, c->d_r2, c->d_cd, c->d_in, c->d_un,
                     c->d_planes, c->d_work_counter, c->d_replay, c->d_hkeys, c->d_hvals, c->d_stage, c->d_groups, c->d_partner, c->d_orig, c->d_batches, c->d_tile_slots, c->d_tile_orig, c->d_dump_counters, c->d_mut_row, c->d_mut_site,
                     c->d_mut_seq, c->d_mut_allele, c->d_hr_rec, c->d_hr_locus, c->d_hr_donor, c->d_hr_seq,
-                    c->d_hr_value, c->d_dump_flip, c->d_dump_gain, c->d_anc, c->d_div, c->d_sfs};
+                    c->d_hr_value, c->d_dump_flip, c->d_dump_gain, c->d_anc, c->d_div, c->d_sfs,
+                    c->d_vcf_counts, c->d_vcf_desc, c->d_vcf_off, c->d_vcf_block, c->d_vcf_bounds, c->d_vcf_nchunks};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (auto *e : c->graphs) {
@@ -1090,9 +1097,9 @@ void pansim_destroy(pansim_ctx *c)
     }
     if (c->h_avg) cudaFreeHost(c->h_avg);
     for (int b = 0; b < 2; b++) {
-        if (c->h_csv[b]) cudaFreeHost(c->h_csv[b]);
-        if (c->d_csv[b]) cudaFree(c->d_csv[b]);
-        if (c->ev_csv[b]) cudaEventDestroy(c->ev_csv[b]);
+        if (c->h_txt[b]) cudaFreeHost(c->h_txt[b]);
+        if (c->d_txt[b]) cudaFree(c->d_txt[b]);
+        if (c->ev_txt[b]) cudaEventDestroy(c->ev_txt[b]);
     }
     if (c->h_stats) cudaFreeHost(c->h_stats);
     if (c->d_stats) cudaFree(c->d_stats);
@@ -1512,11 +1519,54 @@ int pansim_download_core(pansim_ctx *c, uint8_t *out)
     return 0;
 }
 
-// `A,C,G,T\n` rows of _core_genome.csv (population.rs:877-879), expanded on the GPU and streamed out
-// through two pinned host buffers: while chunk k is handed to `sink` (copied into the caller's buffer,
-// or written to a file), the kernel and the device-to-host copy of chunk k+1 are in flight.
-// sink(chunk_ptr, bytes) returns 0 to go on.
+// the two device and two pinned host chunks of the text exports, each at least `bytes`
+static int ensure_txt_staging(pansim_ctx *c, size_t bytes, const char *what)
+{
+    if (bytes <= c->txt_cap) return 0;
+    for (int b = 0; b < 2; b++) {
+        if (c->h_txt[b]) cudaFreeHost(c->h_txt[b]);
+        if (c->d_txt[b]) cudaFree(c->d_txt[b]);
+        c->h_txt[b] = nullptr; c->d_txt[b] = nullptr;
+    }
+    c->txt_cap = 0;
+    for (int b = 0; b < 2; b++) {
+        if (cudaMallocHost(&c->h_txt[b], bytes) != cudaSuccess || cudaMalloc(&c->d_txt[b], bytes) != cudaSuccess)
+            FAIL(c, PANSIM_ERR_NOMEM, "staging buffers of %zu bytes for the %s export failed", bytes, what);
+        if (!c->ev_txt[b]) CU(c, cudaEventCreateWithFlags(&c->ev_txt[b], cudaEventDisableTiming));
+    }
+    c->txt_cap = bytes;
+    return 0;
+}
+
+// Text expanded on the GPU chunk by chunk and streamed out through two pinned host buffers: while chunk k
+// is handed to `sink` (copied into the caller's buffer, or written to a file), the kernel and the
+// device-to-host copy of chunk k+1 are in flight. expand(k, dst, &bytes) enqueues the kernel of chunk k on
+// c->stream, which writes `bytes` (at most cap) bytes at dst; sink(chunk_ptr, bytes) returns 0 to go on.
 extern "C++" {
+template <typename Expand, typename Sink>
+static int stream_text_chunks(pansim_ctx *c, size_t n_chunks, size_t cap, const char *what, Expand &&expand, Sink &&sink)
+{
+    if (n_chunks == 0) return 0;
+    if (int rc = ensure_txt_staging(c, cap, what)) return rc;
+    size_t bytes[2] = {0, 0};
+    auto enqueue = [&](size_t k, int b) -> int {
+        if (int rc = expand(k, c->d_txt[b], &bytes[b])) return rc;
+        CU(c, cudaMemcpyAsync(c->h_txt[b], c->d_txt[b], bytes[b], cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaEventRecord(c->ev_txt[b], c->stream));
+        return 0;
+    };
+    int b = 0;
+    if (int rc = enqueue(0, 0)) return rc;
+    for (size_t k = 0; k < n_chunks; k++, b ^= 1) {
+        if (k + 1 < n_chunks)
+            if (int rc = enqueue(k + 1, b ^ 1)) return rc;                 // next chunk in flight while this one is consumed
+        CU(c, cudaEventSynchronize(c->ev_txt[b]));
+        if (sink(c->h_txt[b], bytes[b])) FAIL(c, PANSIM_ERR_INVALID, "%s export: the sink failed (short write?)", what);
+    }
+    return 0;
+}
+
+// `A,C,G,T\n` rows of _core_genome.csv (population.rs:877-879), a chunk of rows per kernel
 template <typename Sink>
 static int export_core_csv_stream(pansim_ctx *c, uint32_t row_begin, uint32_t row_end, Sink &&sink)
 {
@@ -1529,39 +1579,16 @@ static int export_core_csv_stream(pansim_ctx *c, uint32_t row_begin, uint32_t ro
     const size_t chunk_target = 32ull << 20;
     const uint32_t rows_per = (uint32_t)std::max<size_t>(1, chunk_target / row_bytes);
     const size_t chunk_bytes = (size_t)std::min<uint32_t>(rows_per, row_end - row_begin) * row_bytes;
-    if (chunk_bytes > c->csv_cap) {
-        for (int b = 0; b < 2; b++) {
-            if (c->h_csv[b]) cudaFreeHost(c->h_csv[b]);
-            if (c->d_csv[b]) cudaFree(c->d_csv[b]);
-            c->h_csv[b] = nullptr; c->d_csv[b] = nullptr;
-        }
-        c->csv_cap = 0;
-        for (int b = 0; b < 2; b++) {
-            if (cudaMallocHost(&c->h_csv[b], chunk_bytes) != cudaSuccess || cudaMalloc(&c->d_csv[b], chunk_bytes) != cudaSuccess)
-                FAIL(c, PANSIM_ERR_NOMEM, "staging buffers of %zu bytes for the CSV export failed", chunk_bytes);
-            if (!c->ev_csv[b]) CU(c, cudaEventCreateWithFlags(&c->ev_csv[b], cudaEventDisableTiming));
-        }
-        c->csv_cap = chunk_bytes;
-    }
+    const size_t n_chunks = (row_end - row_begin + (size_t)rows_per - 1) / rows_per;
     const uint64_t wpr = (c->Ll + 15) / 16;
-    auto enqueue = [&](uint32_t r0, int b) -> int {
+    return stream_text_chunks(c, n_chunks, chunk_bytes, "CSV", [&](size_t k, char *dst, size_t *bytes) -> int {
+        const uint32_t r0 = row_begin + (uint32_t)k * rows_per;
         const uint32_t nr = std::min(rows_per, row_end - r0);
-        export_core_csv_kernel<<<div_up64((uint64_t)nr * wpr, 256), 256, 0, c->stream>>>(c->core[c->core_cur], c->core_stride, c->Ll, r0, nr, c->d_csv[b]);
+        export_core_csv_kernel<<<div_up64((uint64_t)nr * wpr, 256), 256, 0, c->stream>>>(c->core[c->core_cur], c->core_stride, c->Ll, r0, nr, dst);
         LAUNCH_CHECK(c);
-        CU(c, cudaMemcpyAsync(c->h_csv[b], c->d_csv[b], (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, c->stream));
-        CU(c, cudaEventRecord(c->ev_csv[b], c->stream));
+        *bytes = (size_t)nr * row_bytes;
         return 0;
-    };
-    int b = 0;
-    if (int rc = enqueue(row_begin, 0)) return rc;
-    for (uint32_t r0 = row_begin; r0 < row_end; r0 += rows_per, b ^= 1) {
-        const uint32_t nr = std::min(rows_per, row_end - r0);
-        if (r0 + rows_per < row_end)
-            if (int rc = enqueue(r0 + rows_per, b ^ 1)) return rc;         // next chunk in flight while this one is consumed
-        CU(c, cudaEventSynchronize(c->ev_csv[b]));
-        if (sink(c->h_csv[b], (size_t)nr * row_bytes)) FAIL(c, PANSIM_ERR_INVALID, "CSV export: the sink failed (short write?)");
-    }
-    return 0;
+    }, sink);
 }
 }  // extern "C++"
 
@@ -2736,6 +2763,184 @@ void pansim_diversity_stats(const pansim_diversity *d, uint32_t pop_size, double
     out[0] = pi;
     out[1] = theta_w;
     out[2] = (d->segregating == 0 || !(den > 0.0)) ? nan : (pi - theta_w) / den;
+}
+
+// ---- core-genome VCF (vcf.cuh) ----------------------------------------------------------------
+constexpr unsigned long long VCF_CHUNK_BYTES = 32ull << 20;     // text per chunk (one line where a line is longer)
+
+static int ensure_vcf(pansim_ctx *c)
+{
+    if (c->d_vcf_nchunks) return 0;
+    const size_t blocks = div_up64(c->Ll, VS_SITES);
+    CU(c, cudaMalloc(&c->d_vcf_counts, (size_t)c->Ll * sizeof(uint4)));
+    CU(c, cudaMalloc(&c->d_vcf_desc, blocks * VS_SITES));
+    CU(c, cudaMalloc(&c->d_vcf_off, ((size_t)c->Ll + 1) * sizeof(unsigned long long)));
+    CU(c, cudaMalloc(&c->d_vcf_block, blocks * sizeof(unsigned long long)));
+    CU(c, cudaMalloc(&c->d_vcf_bounds, 2 * ((size_t)c->Ll + 1) * sizeof(unsigned long long)));
+    CU(c, cudaMalloc(&c->d_vcf_nchunks, sizeof(uint32_t)));
+    return 0;
+}
+
+// the site pass on c->stream over materialised rows: allele counts (the counts instance of the diversity
+// reduction), descriptors, line offsets (d_vcf_off[Ll] = the whole text) and the chunk bounds
+static int vcf_site_pass(pansim_ctx *c)
+{
+    CU(c, cudaMemsetAsync(c->d_div, 0, 4 * sizeof(unsigned long long), c->stream));
+    if (int rc = launch_diversity(c, c->stream, c->d_div, c->d_vcf_counts, nullptr)) return rc;
+    VcfSiteArgs a;
+    a.counts = c->d_vcf_counts;
+    a.anc = c->d_anc;
+    a.n_sites = c->Ll;
+    a.pos0 = c->site_begin + 1;
+    a.n_rows = c->N;
+    a.desc = c->d_vcf_desc;
+    a.off = c->d_vcf_off;
+    a.block = c->d_vcf_block;
+    const uint32_t blocks = div_up64(c->Ll, VS_SITES);
+    vcf_site_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    vcf_scan_blocks_kernel<<<1, VS_SCAN_THREADS, 0, c->stream>>>(a.block, blocks, c->d_vcf_off + c->Ll);
+    LAUNCH_CHECK(c);
+    vcf_offsets_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    vcf_chunk_kernel<<<1, VS_SCAN_THREADS, 0, c->stream>>>(c->d_vcf_off, c->Ll, VCF_CHUNK_BYTES, c->d_vcf_bounds, c->d_vcf_nchunks);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// materialise, run the site pass and read back the chunk bounds only: bounds[2k] = first site of chunk k,
+// bounds[2k + 1] = its byte offset, the last pair = (Ll, whole text). Empty for a context without sites.
+static int vcf_prepare(pansim_ctx *c, std::vector<unsigned long long> &bounds)
+{
+    bounds.clear();
+    if (int rc = require_state(c)) return rc;
+    if (!c->has_anc) FAIL(c, PANSIM_ERR_STATE, "the VCF needs the ancestral row: call pansim_set_initial first");
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (c->Ll == 0) return 0;
+    if (int rc = ensure_div(c, 1, false)) return rc;
+    if (int rc = ensure_vcf(c)) return rc;
+    c->ps = c->stream;
+    if (int rc = core_materialize(c, c->stream)) return rc;
+    if (int rc = check_hr_flag(c)) return rc;
+    if (int rc = vcf_site_pass(c)) return rc;
+    uint32_t n = 0;
+    CU(c, cudaMemcpyAsync(&n, c->d_vcf_nchunks, sizeof n, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    bounds.resize(2 * ((size_t)n + 1));
+    CU(c, cudaMemcpyAsync(bounds.data(), c->d_vcf_bounds, bounds.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+// the lines of chunk k (bounds of vcf_prepare) into dst
+static int launch_vcf_expand(pansim_ctx *c, const unsigned long long *bk, char *dst)
+{
+    VcfExpandArgs a;
+    a.state = reinterpret_cast<const uint32_t *>(c->core[c->core_cur]);
+    a.row_words = c->core_stride / 4;
+    a.n_rows = c->N;
+    a.desc = c->d_vcf_desc;
+    a.off = c->d_vcf_off;
+    a.site0 = bk[0];
+    a.site1 = bk[2];
+    a.base = bk[1];
+    a.pos0 = c->site_begin + 1;
+    a.out = dst;
+    if (bk[3] == bk[1]) return 0;                                   // no line in the chunk
+    const dim3 grid(div_up64(a.site1, VX_SITES) - (uint32_t)(a.site0 / VX_SITES), div_up64(c->N, VX_ROWS));
+    vcf_expand_kernel<<<grid, VX_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+static size_t vcf_max_chunk(const std::vector<unsigned long long> &bd)
+{
+    size_t cap = 0;
+    for (size_t k = 0; k + 3 < bd.size(); k += 2) cap = std::max<size_t>(cap, bd[k + 3] - bd[k + 1]);
+    return cap;
+}
+
+// header lines of the file: the contig is the whole alignment, sample ind_i is row i
+static std::string vcf_header(uint64_t core_size, uint32_t N)
+{
+    std::string h = "##fileformat=VCFv4.2\n##source=pansim_b200\n##contig=<ID=core,length=" + std::to_string(core_size) +
+                    ">\n##FORMAT=<ID=GT,Number=1,Type=String,Description=\"Genotype\">\n"
+                    "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT";
+    h.reserve(h.size() + (size_t)N * 12 + 1);
+    for (uint32_t i = 0; i < N; i++) {
+        h += "\tind_";
+        h += std::to_string(i);
+    }
+    h += '\n';
+    return h;
+}
+
+// the one writer behind pansim_write_core_vcf and pansim_group_write_core_vcf: optionally the header, then
+// the context's lines with global POS, appended to f; *total counts the bytes handed to f
+static int write_core_vcf_to(pansim_ctx *c, FILE *f, bool header, uint64_t *total)
+{
+    std::vector<unsigned long long> bd;
+    if (int rc = vcf_prepare(c, bd)) return rc;
+    auto sink = [&](const char *p, size_t n) { *total += n; return fwrite(p, 1, n, f) == n ? 0 : 1; };
+    if (header) {
+        const std::string h = vcf_header(c->L, c->N);
+        if (sink(h.data(), h.size())) FAIL(c, PANSIM_ERR_INVALID, "VCF export: writing the header failed");
+    }
+    const size_t cap = vcf_max_chunk(bd);
+    if (cap == 0) return 0;                                         // no site differs from the ancestral row
+    const size_t n_chunks = bd.size() / 2 - 1;
+    return stream_text_chunks(c, n_chunks, cap, "VCF", [&](size_t k, char *dst, size_t *bytes) -> int {
+        *bytes = bd[2 * k + 3] - bd[2 * k + 1];
+        return launch_vcf_expand(c, &bd[2 * k], dst);
+    }, sink);
+}
+
+int pansim_write_core_vcf(pansim_ctx *c, const char *path, int with_header, uint64_t *bytes_out)
+{
+    if (!c || !path) return PANSIM_ERR_INVALID;
+    if (int rc = require_state(c)) return rc;
+    if (!c->has_anc) FAIL(c, PANSIM_ERR_STATE, "the VCF needs the ancestral row: call pansim_set_initial first");
+    FILE *f = fopen(path, "wb");
+    if (!f) FAIL(c, PANSIM_ERR_INVALID, "cannot create %s", path);
+    uint64_t total = 0;
+    const int rc = write_core_vcf_to(c, f, with_header != 0, &total);
+    const int rc2 = fclose(f);
+    if (bytes_out) *bytes_out = total;
+    if (rc) return rc;
+    if (rc2) FAIL(c, PANSIM_ERR_INVALID, "closing %s failed", path);
+    return 0;
+}
+
+int pansim_core_vcf_kernel_ms(pansim_ctx *c, uint32_t repeats, float *site_ms, float *expand_ms, uint64_t *text_bytes)
+{
+    if (!c || !repeats) return PANSIM_ERR_INVALID;
+    std::vector<unsigned long long> bd;
+    if (int rc = vcf_prepare(c, bd)) return rc;                     // also the warm-up of the site pass
+    if (bd.empty()) FAIL(c, PANSIM_ERR_INVALID, "no core sites on this context");
+    if (int rc = ensure_txt_staging(c, std::max<size_t>(1, vcf_max_chunk(bd)), "VCF")) return rc;
+    const size_t n_chunks = bd.size() / 2 - 1;
+    for (size_t k = 0; k < n_chunks; k++)                           // warm-up of the expansion
+        if (int rc = launch_vcf_expand(c, &bd[2 * k], c->d_txt[k & 1])) return rc;
+    cudaEvent_t ev[3];
+    for (auto &e : ev) CU(c, cudaEventCreate(&e));
+    int rc = 0;
+    cudaEventRecord(ev[0], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++) rc = vcf_site_pass(c);
+    cudaEventRecord(ev[1], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++)
+        for (size_t k = 0; k < n_chunks && !rc; k++) rc = launch_vcf_expand(c, &bd[2 * k], c->d_txt[k & 1]);
+    cudaEventRecord(ev[2], c->stream);
+    const cudaError_t e = cudaEventSynchronize(ev[2]);
+    float t0 = 0.f, t1 = 0.f;
+    cudaEventElapsedTime(&t0, ev[0], ev[1]);
+    cudaEventElapsedTime(&t1, ev[1], ev[2]);
+    for (auto &x : ev) cudaEventDestroy(x);
+    if (rc) return rc;
+    if (e != cudaSuccess) FAIL(c, PANSIM_ERR_CUDA, "VCF kernels failed: %s", cudaGetErrorString(e));
+    if (site_ms) *site_ms = t0 / (float)repeats;
+    if (expand_ms) *expand_ms = t1 / (float)repeats;
+    if (text_bytes) *text_bytes = bd.back();
+    return 0;
 }
 
 // ---- communicator over column shards (one process per GPU) -------------------

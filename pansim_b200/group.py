@@ -155,6 +155,12 @@ class PansimGroup:
         self._check(self._lib.pansim_group_download_core(self._h, _ptr(out)))
         return out
 
+    def write_core_vcf(self, path: str) -> int:
+        """The whole-alignment VCF (Pansim.write_core_vcf): header once, then every shard's lines; bytes written."""
+        n = C.c_uint64(0)
+        self._check(self._lib.pansim_group_write_core_vcf(self._h, path.encode(), C.byref(n)))
+        return n.value
+
     def export_core_csv(self, row_begin: int, row_end: int) -> bytes:
         out = np.empty((row_end - row_begin) * 2 * self.L, np.uint8)
         self._check(self._lib.pansim_group_export_core_csv(self._h, row_begin, row_end, _ptr(out)))

@@ -42,8 +42,9 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
                              "prop_genes2", "prop_positive", "pos_lambda", "neg_lambda", "seed", "outpref",
                              "threads", "genome_size_penalty", "competition_strength", "device", "gpus"};
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
-                              "all_pairs", "print_diversity"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
-                                                                 // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt)
+                              "all_pairs", "print_diversity", "print_vcf"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                                                                              // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
+                                                                              // print_vcf (<outpref>_core_genome.vcf)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -125,7 +126,7 @@ int main(int argc, char **argv)
     const double pos_lambda = as_f64(fl, "pos_lambda"), neg_lambda = as_f64(fl, "neg_lambda");
     const uint64_t seed = std::strtoull(fl.val["seed"].c_str(), nullptr, 10);
     const bool verbose = fl.sw["verbose"], print_dist = fl.sw["print_dist"], print_matrices = fl.sw["print_matrices"];
-    const bool all_pairs = fl.sw["all_pairs"], print_diversity = fl.sw["print_diversity"];
+    const bool all_pairs = fl.sw["all_pairs"], print_diversity = fl.sw["print_diversity"], print_vcf = fl.sw["print_vcf"];
     const int n_gpus = std::max(1, std::atoi(fl.val["gpus"].c_str()));       // extension: column shards over N devices of the box
     const bool print_selection = fl.sw["print_selection"], no_control = fl.sw["no_control_genome_size"];
     const double genome_size_penalty = as_f64(fl, "genome_size_penalty"), competition_strength = as_f64(fl, "competition_strength");
@@ -281,6 +282,7 @@ int main(int argc, char **argv)
             for (uint64_t x : sfs) g << x << "\n";
         }
         if (print_matrices) pops.write(outpref);                            // main.rs:550-553
+        if (print_vcf) pops.write_core_vcf(outpref + "_core_genome.vcf");   // extension: the last generation as VCF
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)
         std::fprintf(stderr, "pansim: %s\n", e.what());

@@ -174,6 +174,13 @@ public:
     }
     // population.rs:865-897 `write` for both populations
     void write(const std::string &outpref);
+    // (extension) the core alignment as VCF against the initial row, all shards in one file; bytes written
+    uint64_t write_core_vcf(const std::string &path)
+    {
+        uint64_t n = 0;
+        gcheck(pansim_group_write_core_vcf(grp_, path.c_str(), &n));
+        return n;
+    }
 
     pansim_ctx *raw() { return ctx_; }          // shard 0 (the whole run when n_gpus() == 1)
     pansim_group *group() { return grp_; }

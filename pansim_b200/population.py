@@ -486,6 +486,21 @@ class Pansim:
         self._check(self._lib.pansim_write_core_csv(self._h, path.encode(), C.byref(n)))
         return n.value
 
+    def write_core_vcf(self, path: str, header: bool = True) -> int:
+        """The core alignment as VCF 4.2 (include/pansim_b200.h): one line per site where some row differs from
+        the row given to set_initial, haploid GT against it. A column-shard context writes its own lines with
+        global POS; header=False leaves out the header, so the shards' bodies can be concatenated. Bytes written."""
+        n = C.c_uint64(0)
+        self._check(self._lib.pansim_write_core_vcf(self._h, path.encode(), int(header), C.byref(n)))
+        return n.value
+
+    def vcf_kernel_ms(self, repeats: int = 10) -> tuple[float, float, int]:
+        """Measurement: device ms of one VCF site pass and of one expansion of every chunk (no copy), and the
+        bytes of text (header excluded)."""
+        site, expand, n = C.c_float(), C.c_float(), C.c_uint64()
+        self._check(self._lib.pansim_core_vcf_kernel_ms(self._h, repeats, C.byref(site), C.byref(expand), C.byref(n)))
+        return site.value, expand.value, n.value
+
     def write(self, outpref: str):
         self.write_core_csv(outpref + "_core_genome.csv")
         acc = self.download_acc()

@@ -66,13 +66,15 @@ class RunResult:
 
 
 def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False,
-        print_diversity: bool = False) -> RunResult | None:
+        print_diversity: bool = False, print_vcf: bool = False) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
     print_diversity (extension): core-genome diversity every generation, written to
     `<outpref>_diversity.tsv` (segregating, multiallelic, pi, theta_W, Tajima's D) and the site frequency
-    spectrum of the last generation to `<outpref>_core_sfs.txt`."""
+    spectrum of the last generation to `<outpref>_core_sfs.txt`.
+    print_vcf (extension): the core alignment of the last generation as `<outpref>_core_genome.vcf`, written
+    after the other outputs (Pansim.write_core_vcf)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -162,6 +164,8 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
                 write_diversity(outpref, res.diversity, res.sfs, p.pop_size)
         if p.print_matrices and outpref:                                         # main.rs:550-553
             sim.write(outpref)
+        if print_vcf and outpref:
+            sim.write_core_vcf(outpref + "_core_genome.vcf")
     return res
 
 
