@@ -267,6 +267,49 @@ int pansim_write_core_vcf(pansim_ctx *ctx, const char *path, int with_header, ui
  * pass (CUDA events) and the bytes of text (header excluded) */
 int pansim_core_vcf_kernel_ms(pansim_ctx *ctx, uint32_t repeats, float *site_ms, float *expand_ms, uint64_t *text_bytes);
 
+/* ---- core-genome linkage disequilibrium (extension: the reference has no two-site statistic) ----
+ * r^2 and four-gamete pairs binned by the distance between two sites, the joint counts of the site pairs formed
+ * on the tensor cores (DESIGN.md section 12). The state is read after recombine(), like every reader.
+ * Let n = N. At a local site a row is DERIVED when its letter differs from the site's letter in the ancestral row
+ * (the row given to pansim_set_initial), the convention of the SFS and of VCF GT != 0; multiallelic sites are
+ * collapsed to derived / ancestral. a = the derived count of a site; the site is USED when
+ * 1 <= min_minor <= min(a, n - a). The pairs are used sites i < j (global 0-based indices) with
+ * 1 <= d = j - i <= max_dist; pair (i, j) goes to bin b = (d - 1) / bin_width. There are
+ * n_bins = ceil(max_dist / bin_width) bins; bin b covers distances b*w + 1 .. min((b + 1)*w, max_dist).
+ * Per pair, with c = the number of rows derived at both sites:
+ *   D = n*c - a_i*a_j, exact in int64;
+ *   inv_x = 1.0 / (double)(a_x*(n - a_x)), the product exact, the division IEEE round-to-nearest, once per site;
+ *   r2 = (((double)D * (double)D) * inv_i) * inv_j, each product rounded on its own (no fused or reordered operation);
+ *   q = round-half-even(r2 * 2^32) as uint64;
+ *   four gametes iff c > 0, a_i - c > 0, a_j - c > 0 and n - a_i - a_j + c > 0.
+ * |D| <= n^2/4 < 2^53, so D, a(n - a) and their conversions to double are exact for every N a context can hold.
+ * Per bin the call returns the pairs, the four-gamete pairs and sum q as an exact 128-bit integer (r2_hi, r2_lo).
+ * Every output is an integer: neither the grid nor the shard split changes a bit.
+ *
+ * next: NULL, or the context holding the sites right after ctx's (next.site_begin == ctx.site_end, same N). Without
+ * it ctx counts the pairs whose sites both lie in its own range. With it ctx also counts the pairs whose second site
+ * lies among next's first max_dist sites, made on next's device and copied over as a halo (cudaMemcpyPeerAsync);
+ * pairs with both sites in the halo belong to next. sites_used (may be NULL) counts ctx's own used sites only. So
+ * over column shards s = 0..k-1 the sum of pansim_core_ld(shard s, shard s+1) is the single-context result bit for
+ * bit; pansim_group_core_ld is that sum. Under a communicator (pansim_comm_init_rank) a rank's call counts only its
+ * own pairs: there is no halo exchange between processes.
+ * Errors: no pansim_set_initial -> PANSIM_ERR_STATE; max_dist, bin_width or min_minor = 0, a next that is not
+ * adjacent or has another N, or max_dist above next's local sites (group: above the narrowest shard) ->
+ * PANSIM_ERR_INVALID. The context keeps working after a refused call. The site-major bit rows (one bit per row and
+ * used site) are allocated on first use and kept with the context. */
+typedef struct { uint32_t max_dist, bin_width, min_minor; } pansim_ld_params;
+typedef struct { uint64_t pairs, four_gamete, r2_hi, r2_lo; } pansim_ld_bin;
+int pansim_core_ld(pansim_ctx *ctx, pansim_ctx *next, const pansim_ld_params *p,
+                   pansim_ld_bin *bins /* [n_bins] */, uint64_t *sites_used);
+/* measurement (next = NULL): the site pass (allele counts, used sites, scan, compaction), the transpose to bit rows
+ * and the pair pass (tile list and pair kernel), each `repeats` times after one warm-up call; mean device ms of one
+ * pass (CUDA events) and the pairs counted */
+int pansim_core_ld_kernel_ms(pansim_ctx *ctx, const pansim_ld_params *p, uint32_t repeats,
+                             float *site_ms, float *transpose_ms, float *pair_ms, uint64_t *pairs);
+/* mean r^2 of a bin, needs no device: (ldexp((double)r2_hi, 32) + ldexp((double)r2_lo, -32)) / (double)pairs in
+ * that order, NaN when pairs = 0, so every host prints the same digits */
+double pansim_ld_mean_r2(const pansim_ld_bin *b);
+
 /* ---- multi-GPU: column shards of one alignment --------------------------
  * (SURVEY.md 8e; the reference is one shared-memory process, population.rs has no analogue.)
  * Every shard context holds all individuals for [site_begin, site_end) and a replica of the
@@ -323,6 +366,9 @@ int pansim_group_download_core(pansim_group *g, uint8_t *core_onehot_out);      
 int pansim_group_export_core_csv(pansim_group *g, uint32_t row_begin, uint32_t row_end, char *out);
 /* the whole-alignment VCF of pansim_write_core_vcf: the header once, then every shard's lines in shard order */
 int pansim_group_write_core_vcf(pansim_group *g, const char *path, uint64_t *bytes_out);
+
+/* pansim_core_ld over the whole alignment: every shard with the next one as its halo, summed on the host */
+int pansim_group_core_ld(pansim_group *g, const pansim_ld_params *p, pansim_ld_bin *bins, uint64_t *sites_used);
 
 /* ---- introspection / instrumentation ----------------------------------- */
 typedef struct {

@@ -4,7 +4,8 @@ Same long flags (underscores, capitalised --HR_rate / --HGT_rate), same defaults
 same parsing quirks: pop_size/core_size/pan_genes/core_genes/n_gen are parsed as
 f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
-accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf.
+accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
+--print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor.
 """
 from __future__ import annotations
 
@@ -62,6 +63,13 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--print_vcf", action="store_true",
                     help="(extension) <outpref>_core_genome.vcf: the core alignment of the last generation as VCF, one "
                          "line per site that differs from the initial row, haploid genotypes against it")
+    ap.add_argument("--print_ld", action="store_true",
+                    help="(extension) <outpref>_core_ld.tsv: linkage disequilibrium of the core genome of the last generation, "
+                         "one line per distance bin: dist_lo, dist_hi, site pairs, pairs with four gametes, mean r^2")
+    ap.add_argument("--ld_max_dist", type=int, default=10000, help="(extension) largest site distance of --print_ld")
+    ap.add_argument("--ld_bin_width", type=int, default=100, help="(extension) distances per bin of --print_ld")
+    ap.add_argument("--ld_min_minor", type=int, default=1,
+                    help="(extension) --print_ld uses sites where at least this many rows are derived and at least this many are not")
     return ap
 
 
@@ -71,8 +79,9 @@ def main(argv=None) -> int:
     all_pairs = ns.pop("all_pairs")
     print_diversity = ns.pop("print_diversity")
     print_vcf = ns.pop("print_vcf")
+    ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
     p = Params(**ns)
-    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf)
+    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf, **ld)
     return 0                       # the reference exits 0 even when validation fails (main.rs:195-247)
 
 

@@ -33,6 +33,7 @@ EXPORTED = [
     "pansim_core_allele_counts", "pansim_core_diversity", "pansim_run_generations_diversity", "pansim_diversity_stats",
     "pansim_group_core_diversity", "pansim_group_run_generations_diversity",
     "pansim_write_core_vcf", "pansim_group_write_core_vcf", "pansim_core_vcf_kernel_ms",
+    "pansim_core_ld", "pansim_group_core_ld", "pansim_core_ld_kernel_ms", "pansim_ld_mean_r2",
 ]
 COMM_ID_BYTES = 128
 
@@ -95,6 +96,14 @@ class EventDump(C.Structure):
 class Diversity(C.Structure):
     _fields_ = [("sites", C.c_uint64), ("segregating", C.c_uint64), ("multiallelic", C.c_uint64),
                 ("pair_diff_sum", C.c_uint64)]
+
+
+class LdParams(C.Structure):
+    _fields_ = [("max_dist", C.c_uint32), ("bin_width", C.c_uint32), ("min_minor", C.c_uint32)]
+
+
+class LdBin(C.Structure):
+    _fields_ = [("pairs", C.c_uint64), ("four_gamete", C.c_uint64), ("r2_hi", C.c_uint64), ("r2_lo", C.c_uint64)]
 
 
 PAIRS_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.POINTER(C.c_uint32),
@@ -205,5 +214,10 @@ def lib():
     sig("pansim_write_core_vcf", cint, vp, C.c_char_p, cint, C.POINTER(C.c_uint64))
     sig("pansim_group_write_core_vcf", cint, vp, C.c_char_p, C.POINTER(C.c_uint64))
     sig("pansim_core_vcf_kernel_ms", cint, vp, u32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint64))
+    sig("pansim_core_ld", cint, vp, vp, C.POINTER(LdParams), C.POINTER(LdBin), C.POINTER(C.c_uint64))
+    sig("pansim_group_core_ld", cint, vp, C.POINTER(LdParams), C.POINTER(LdBin), C.POINTER(C.c_uint64))
+    sig("pansim_core_ld_kernel_ms", cint, vp, C.POINTER(LdParams), u32, C.POINTER(C.c_float), C.POINTER(C.c_float),
+        C.POINTER(C.c_float), C.POINTER(C.c_uint64))
+    sig("pansim_ld_mean_r2", dbl, C.POINTER(LdBin))
     _lib = L
     return L

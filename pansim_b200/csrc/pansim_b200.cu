@@ -21,6 +21,7 @@
 #include "core_mut.cuh"
 #include "distance.cuh"
 #include "diversity.cuh"
+#include "ld.cuh"
 #include "pack.cuh"
 #include "replay.cuh"
 #include "select.cuh"
@@ -268,6 +269,21 @@ struct pansim_ctx {
     uint8_t *d_vcf_desc = nullptr;
     unsigned long long *d_vcf_off = nullptr, *d_vcf_block = nullptr, *d_vcf_bounds = nullptr;
     uint32_t *d_vcf_nchunks = nullptr;
+    // core LD (ld.cuh): allele counts, used-site ranks, the compacted used sites (position, derived count, 1 / (a (n - a)))
+    // and their site-major derived bit rows. `ld` holds the context's own used sites followed by the halo copied from
+    // the next shard; `ld_halo` is the halo this context makes of its first sites when it is the next of another one.
+    struct LdBuf {
+        uint4 *counts = nullptr;
+        unsigned long long *block = nullptr;
+        uint32_t *rank = nullptr, *pos = nullptr, *a = nullptr, *x = nullptr;
+        double *inv = nullptr;
+        size_t site_cap = 0, used_cap = 0, x_cap = 0;
+    } ld, ld_halo;
+    unsigned long long *d_ld_tiles = nullptr, *d_ld_bins = nullptr;   // tile-pair offsets [I tiles + 1], bins [n][4]
+    size_t ld_tiles_cap = 0, ld_bins_cap = 0;
+    unsigned long long *h_ld = nullptr, *h_ld_bins = nullptr;         // pinned: own / halo used sites, tile pairs; bins
+    size_t h_ld_bins_cap = 0;
+    cudaEvent_t ev_ld = nullptr;                                       // the halo of this context is ready
     // staging for upload/download
     uint8_t *d_stage = nullptr;
     size_t stage_cap = 0;
@@ -1084,6 +1100,16 @@ void pansim_destroy(pansim_ctx *c)
                     c->d_vcf_counts, c->d_vcf_desc, c->d_vcf_off, c->d_vcf_block, c->d_vcf_bounds, c->d_vcf_nchunks};
     for (void *p : ptrs)
         if (p) cudaFree(p);
+    for (auto *b : {&c->ld, &c->ld_halo}) {
+        void *lp[] = {b->counts, b->block, b->rank, b->pos, b->a, b->x, b->inv};
+        for (void *p : lp)
+            if (p) cudaFree(p);
+    }
+    if (c->d_ld_tiles) cudaFree(c->d_ld_tiles);
+    if (c->d_ld_bins) cudaFree(c->d_ld_bins);
+    if (c->h_ld) cudaFreeHost(c->h_ld);
+    if (c->h_ld_bins) cudaFreeHost(c->h_ld_bins);
+    if (c->ev_ld) cudaEventDestroy(c->ev_ld);
     for (auto *e : c->graphs) {
         if (e->exec) cudaGraphExecDestroy(e->exec);
         e->pool.destroy();
@@ -2941,6 +2967,371 @@ int pansim_core_vcf_kernel_ms(pansim_ctx *c, uint32_t repeats, float *site_ms, f
     if (expand_ms) *expand_ms = t1 / (float)repeats;
     if (text_bytes) *text_bytes = bd.back();
     return 0;
+}
+
+// ---- core-genome linkage disequilibrium (ld.cuh) ---------------------------------------------
+using LdBuf = pansim_ctx::LdBuf;
+
+// counts and ranks of n_sites sites, the compacted arrays of n_used used sites (grown, never shrunk)
+static int ld_ensure_sites(pansim_ctx *c, LdBuf &b, size_t n_sites, size_t n_used)
+{
+    if (n_sites > b.site_cap) {
+        for (void *p : {(void *)b.counts, (void *)b.block, (void *)b.rank})
+            if (p) cudaFree(p);
+        b.counts = nullptr; b.block = nullptr; b.rank = nullptr; b.site_cap = 0;
+        CU(c, cudaMalloc(&b.counts, n_sites * sizeof(uint4)));
+        CU(c, cudaMalloc(&b.block, ((size_t)div_up64(n_sites, VS_SITES) + 1) * sizeof(unsigned long long)));
+        CU(c, cudaMalloc(&b.rank, n_sites * sizeof(uint32_t)));
+        b.site_cap = n_sites;
+    }
+    if (n_used > b.used_cap) {
+        for (void *p : {(void *)b.pos, (void *)b.a, (void *)b.inv})
+            if (p) cudaFree(p);
+        b.pos = nullptr; b.a = nullptr; b.inv = nullptr; b.used_cap = 0;
+        CU(c, cudaMalloc(&b.pos, n_used * sizeof(uint32_t)));
+        CU(c, cudaMalloc(&b.a, n_used * sizeof(uint32_t)));
+        CU(c, cudaMalloc(&b.inv, n_used * sizeof(double)));
+        b.used_cap = n_used;
+    }
+    return 0;
+}
+
+// the site-major bit rows of n_used used sites (kept with the context, like the intersection matrix)
+static int ld_ensure_x(pansim_ctx *c, LdBuf &b, size_t n_used)
+{
+    const size_t bytes = std::max<size_t>(1, n_used) * ld_row_words(c->N) * sizeof(uint32_t);
+    if (bytes <= b.x_cap) return 0;
+    if (b.x) cudaFree(b.x);
+    b.x = nullptr; b.x_cap = 0;
+    if (cudaMalloc(&b.x, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL(c, PANSIM_ERR_NOMEM, "cudaMalloc of %zu bytes (LD bit rows) failed", bytes);
+    }
+    b.x_cap = bytes;
+    return 0;
+}
+
+static int ld_ensure_host(pansim_ctx *c, size_t n_bins)
+{
+    if (!c->h_ld) CU(c, cudaMallocHost(&c->h_ld, 4 * sizeof(unsigned long long)));
+    if (!c->ev_ld) CU(c, cudaEventCreateWithFlags(&c->ev_ld, cudaEventDisableTiming));
+    if (n_bins > c->h_ld_bins_cap) {
+        if (c->h_ld_bins) cudaFreeHost(c->h_ld_bins);
+        c->h_ld_bins = nullptr; c->h_ld_bins_cap = 0;
+        CU(c, cudaMallocHost(&c->h_ld_bins, n_bins * 4 * sizeof(unsigned long long)));
+        c->h_ld_bins_cap = n_bins;
+    }
+    return 0;
+}
+
+// site pass over the first n local sites of c (materialised rows) into b on c->stream: allele counts, used sites,
+// their ranks and compacted arrays; the number of used sites is b.block[n_blocks], copied to *h_used if given
+static int ld_site_pass(pansim_ctx *c, LdBuf &b, uint64_t n, uint32_t min_minor, unsigned long long *h_used)
+{
+    DiversityArgs d;
+    d.state = reinterpret_cast<const uint32_t *>(c->core[c->core_cur]);
+    d.row_words = c->core_stride / 4;
+    d.n_sites = n;
+    d.n_rows = c->N;
+    d.anc = c->d_anc;
+    d.out = c->d_div;
+    d.counts = b.counts;
+    d.sfs = nullptr;
+    CU(c, cudaMemsetAsync(c->d_div, 0, 4 * sizeof(unsigned long long), c->stream));
+    diversity_kernel<true, false><<<div_up64(n, DV_SITES), DV_THREADS, 0, c->stream>>>(d);
+    LAUNCH_CHECK(c);
+    LdSiteArgs a;
+    a.counts = b.counts;
+    a.anc = c->d_anc;
+    a.n_sites = n;
+    a.n_rows = c->N;
+    a.min_minor = min_minor;
+    a.pos0 = (uint32_t)c->site_begin;
+    a.block = b.block;
+    a.rank = b.rank;
+    a.pos = b.pos;
+    a.a = b.a;
+    a.inv = b.inv;
+    const uint32_t blocks = div_up64(n, VS_SITES);
+    ld_site_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    vcf_scan_blocks_kernel<<<1, VS_SCAN_THREADS, 0, c->stream>>>(b.block, blocks, b.block + blocks);
+    LAUNCH_CHECK(c);
+    ld_compact_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    if (h_used) CU(c, cudaMemcpyAsync(h_used, b.block + blocks, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+}
+
+// derived bit rows of the used sites among the first n local sites of c into x (row k = rank k)
+static int ld_transpose(pansim_ctx *c, const LdBuf &b, uint64_t n, uint32_t *x)
+{
+    LdTransposeArgs a;
+    a.state = reinterpret_cast<const uint32_t *>(c->core[c->core_cur]);
+    a.row_words = c->core_stride / 4;
+    a.n_rows = c->N;
+    a.n_sites = n;
+    a.anc = c->d_anc;
+    a.rank = b.rank;
+    a.kw = ld_row_words(c->N);
+    a.x = x;
+    const dim3 grid(div_up64(n, LT_SITES), div_up64((uint64_t)a.kw * 32, LT_ROWS));
+    ld_transpose_kernel<<<grid, LT_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// tile-pair offsets of the `own` used sites against all `own + halo` of them; the total goes to *h_tiles if given
+static int ld_tile_list(pansim_ctx *c, uint64_t own, uint64_t all, uint32_t max_dist, unsigned long long *h_tiles)
+{
+    const uint32_t n_i = div_up64(own, LD_TILE);
+    if ((size_t)n_i + 1 > c->ld_tiles_cap) {
+        if (c->d_ld_tiles) cudaFree(c->d_ld_tiles);
+        c->d_ld_tiles = nullptr; c->ld_tiles_cap = 0;
+        CU(c, cudaMalloc(&c->d_ld_tiles, ((size_t)n_i + 1) * sizeof(unsigned long long)));
+        c->ld_tiles_cap = (size_t)n_i + 1;
+    }
+    ld_tiles_kernel<<<div_up64(n_i, 256), 256, 0, c->stream>>>(c->ld.pos, (uint32_t)own, (uint32_t)all, max_dist, c->d_ld_tiles);
+    LAUNCH_CHECK(c);
+    vcf_scan_blocks_kernel<<<1, VS_SCAN_THREADS, 0, c->stream>>>(c->d_ld_tiles, n_i, c->d_ld_tiles + n_i);
+    LAUNCH_CHECK(c);
+    if (h_tiles) CU(c, cudaMemcpyAsync(h_tiles, c->d_ld_tiles + n_i, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+}
+
+static uint32_t ld_n_bins(const pansim_ld_params *p) { return (uint32_t)(((uint64_t)p->max_dist + p->bin_width - 1) / p->bin_width); }
+
+// zeroed bins, then the pair kernel over `tiles` tile pairs
+static int ld_pairs(pansim_ctx *c, const pansim_ld_params *p, uint64_t own, uint64_t all, uint64_t tiles)
+{
+    const uint32_t n_bins = ld_n_bins(p);
+    if (n_bins > c->ld_bins_cap) {
+        if (c->d_ld_bins) cudaFree(c->d_ld_bins);
+        c->d_ld_bins = nullptr; c->ld_bins_cap = 0;
+        CU(c, cudaMalloc(&c->d_ld_bins, (size_t)n_bins * 4 * sizeof(unsigned long long)));
+        c->ld_bins_cap = n_bins;
+    }
+    CU(c, cudaMemsetAsync(c->d_ld_bins, 0, (size_t)n_bins * 4 * sizeof(unsigned long long), c->stream));
+    if (!tiles) return 0;
+    if (tiles > 0x7FFFFFFFull) FAIL(c, PANSIM_ERR_INVALID, "%llu LD tile pairs: more than one launch holds", (unsigned long long)tiles);
+    LdPairArgs a;
+    a.x = c->ld.x;
+    a.kw = ld_row_words(c->N);
+    a.k_iters = a.kw * 32 / LD_KB;
+    a.pos = c->ld.pos;
+    a.a = c->ld.a;
+    a.inv = c->ld.inv;
+    a.n_own = (uint32_t)own;
+    a.n_all = (uint32_t)all;
+    a.n_rows = c->N;
+    a.max_dist = p->max_dist;
+    a.bin_width = p->bin_width;
+    a.n_bins = n_bins;
+    a.tile_off = c->d_ld_tiles;
+    a.n_i = div_up64(own, LD_TILE);
+    a.bins = c->d_ld_bins;
+    const size_t smem = ld_pair_smem_bytes(n_bins);
+    CU(c, cudaFuncSetAttribute(ld_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ld_pair_kernel<<<(uint32_t)tiles, LD_THREADS, smem, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// Refusals leave the context as it was. Errors of `next` are reported on c.
+static int ld_validate(pansim_ctx *c, pansim_ctx *next, const pansim_ld_params *p)
+{
+    if (!p->max_dist || !p->bin_width || !p->min_minor) FAIL(c, PANSIM_ERR_INVALID, "LD: max_dist, bin_width and min_minor must be >= 1");
+    if (int rc = require_state(c)) return rc;
+    if (!c->has_anc) FAIL(c, PANSIM_ERR_STATE, "LD needs the ancestral row: call pansim_set_initial first");
+    if (c->site_end > 0xFFFFFFFFull) FAIL(c, PANSIM_ERR_INVALID, "LD: site positions above 2^32-1");
+    if (next) {
+        if (next == c || next->N != c->N || next->site_begin != c->site_end)
+            FAIL(c, PANSIM_ERR_INVALID, "LD: next must hold the sites right after this context's, with the same pop_size");
+        if (!next->has_core || !next->has_anc) FAIL(c, PANSIM_ERR_STATE, "LD: the next context has no state or no ancestral row");
+        if (p->max_dist > next->Ll) FAIL(c, PANSIM_ERR_INVALID, "LD: max_dist %u exceeds the %llu sites of the next context", p->max_dist, (unsigned long long)next->Ll);
+    }
+    return 0;
+}
+
+// One context's share of the LD pass in three enqueued phases; between them the host reads the used-site and
+// tile-pair counts. A list of jobs runs every phase on all of them before it waits, so the devices overlap.
+struct LdJob {
+    pansim_ctx *c, *next;
+    uint64_t own = 0, halo = 0, tiles = 0;
+};
+
+static int ld_sync(pansim_ctx *c)
+{
+    CU(c, cudaSetDevice(c->cfg.device));
+    CU(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+// a failure on `next` reported on c
+static int ld_on_next(pansim_ctx *c, pansim_ctx *next, int rc)
+{
+    if (rc) c->err = "next context: " + next->err;
+    return rc;
+}
+
+static int ld_phase_sites(LdJob &j, const pansim_ld_params *p)
+{
+    pansim_ctx *c = j.c, *nx = j.next;
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (int rc = ensure_div(c, 1, false)) return rc;
+    if (int rc = ld_ensure_host(c, ld_n_bins(p))) return rc;
+    if (int rc = ld_ensure_sites(c, c->ld, c->Ll, c->Ll + (nx ? p->max_dist : 0))) return rc;
+    c->ps = c->stream;
+    if (int rc = core_materialize(c, c->stream)) return rc;
+    if (int rc = check_hr_flag(c)) return rc;
+    c->h_ld[1] = 0;
+    if (int rc = ld_site_pass(c, c->ld, c->Ll, p->min_minor, c->h_ld)) return rc;
+    if (nx) {
+        CU(c, cudaSetDevice(nx->cfg.device));
+        int rc = ensure_div(nx, 1, false);
+        if (!rc) rc = ld_ensure_sites(nx, nx->ld_halo, p->max_dist, p->max_dist);
+        if (!rc) rc = ld_ensure_host(nx, 1);
+        if (!rc) { nx->ps = nx->stream; rc = core_materialize(nx, nx->stream); }
+        if (!rc) rc = check_hr_flag(nx);
+        if (!rc) rc = ld_site_pass(nx, nx->ld_halo, p->max_dist, p->min_minor, c->h_ld + 1);
+        if (rc) return ld_on_next(c, nx, rc);
+    }
+    return 0;
+}
+
+static int ld_phase_rows(LdJob &j, const pansim_ld_params *p)
+{
+    pansim_ctx *c = j.c, *nx = j.next;
+    if (int rc = ld_sync(c)) return rc;
+    if (nx)
+        if (int rc = ld_sync(nx)) return ld_on_next(c, nx, rc);
+    j.own = c->h_ld[0];
+    j.halo = nx ? c->h_ld[1] : 0;
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (!j.own) return 0;
+    const uint64_t kw = ld_row_words(c->N);
+    if (int rc = ld_ensure_x(c, c->ld, j.own + j.halo)) return rc;
+    if (int rc = ld_transpose(c, c->ld, c->Ll, c->ld.x)) return rc;
+    if (j.halo) {
+        // the halo: the used sites among the next context's first max_dist sites, made on its device and stream,
+        // then copied behind ctx's own used sites
+        CU(c, cudaSetDevice(nx->cfg.device));
+        int rc = ld_ensure_x(nx, nx->ld_halo, j.halo);
+        if (!rc) rc = ld_transpose(nx, nx->ld_halo, p->max_dist, nx->ld_halo.x);
+        if (!rc && cudaEventRecord(nx->ev_ld, nx->stream) != cudaSuccess) { nx->err = "cudaEventRecord failed"; rc = PANSIM_ERR_CUDA; }
+        if (rc) return ld_on_next(c, nx, rc);
+        CU(c, cudaSetDevice(c->cfg.device));
+        CU(c, cudaStreamWaitEvent(c->stream, nx->ev_ld, 0));
+        const LdBuf &h = nx->ld_halo;
+        struct Part { void *dst; const void *src; size_t bytes; } parts[] = {
+            {c->ld.x + j.own * kw, h.x, j.halo * kw * sizeof(uint32_t)}, {c->ld.pos + j.own, h.pos, j.halo * sizeof(uint32_t)},
+            {c->ld.a + j.own, h.a, j.halo * sizeof(uint32_t)}, {c->ld.inv + j.own, h.inv, j.halo * sizeof(double)}};
+        for (const Part &q : parts) {
+            if (c->cfg.device == nx->cfg.device) CU(c, cudaMemcpyAsync(q.dst, q.src, q.bytes, cudaMemcpyDeviceToDevice, c->stream));
+            else CU(c, cudaMemcpyPeerAsync(q.dst, c->cfg.device, q.src, nx->cfg.device, q.bytes, c->stream));
+        }
+    }
+    return ld_tile_list(c, j.own, j.own + j.halo, p->max_dist, c->h_ld + 2);
+}
+
+static int ld_phase_pairs(LdJob &j, const pansim_ld_params *p)
+{
+    pansim_ctx *c = j.c;
+    if (int rc = ld_sync(c)) return rc;
+    j.tiles = j.own ? c->h_ld[2] : 0;
+    if (int rc = ld_pairs(c, p, j.own, j.own + j.halo, j.tiles)) return rc;
+    CU(c, cudaMemcpyAsync(c->h_ld_bins, c->d_ld_bins, (size_t)ld_n_bins(p) * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    return flags_enqueue_readback(c);
+}
+
+// adds job j's bins into out (the 128-bit sums with carry)
+static int ld_finish(LdJob &j, const pansim_ld_params *p, pansim_ld_bin *out, uint64_t *used)
+{
+    pansim_ctx *c = j.c;
+    if (int rc = ld_sync(c)) return rc;
+    if (int rc = flags_inspect(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG)) return rc;
+    for (uint32_t b = 0; b < ld_n_bins(p); b++) {
+        const unsigned long long *h = c->h_ld_bins + 4 * (size_t)b;
+        out[b].pairs += h[0];
+        out[b].four_gamete += h[1];
+        const uint64_t lo = out[b].r2_lo + h[3];
+        out[b].r2_hi += h[2] + (lo < h[3] ? 1u : 0u);
+        out[b].r2_lo = lo;
+    }
+    *used += j.own;
+    return 0;
+}
+
+// the phases over all jobs; on failure *failed = the job's index
+static int ld_run(std::vector<LdJob> &jobs, const pansim_ld_params *p, pansim_ld_bin *bins, uint64_t *used, size_t *failed)
+{
+    memset(bins, 0, (size_t)ld_n_bins(p) * sizeof(pansim_ld_bin));
+    *used = 0;
+    for (auto phase : {ld_phase_sites, ld_phase_rows, ld_phase_pairs})
+        for (size_t i = 0; i < jobs.size(); i++)
+            if (int rc = phase(jobs[i], p)) { *failed = i; return rc; }
+    for (size_t i = 0; i < jobs.size(); i++)
+        if (int rc = ld_finish(jobs[i], p, bins, used)) { *failed = i; return rc; }
+    return 0;
+}
+
+int pansim_core_ld(pansim_ctx *c, pansim_ctx *next, const pansim_ld_params *p, pansim_ld_bin *bins, uint64_t *sites_used)
+{
+    if (!c || !p || !bins) return PANSIM_ERR_INVALID;
+    if (int rc = ld_validate(c, next, p)) return rc;
+    std::vector<LdJob> jobs{{c, next}};
+    uint64_t used = 0;
+    size_t failed = 0;
+    if (int rc = ld_run(jobs, p, bins, &used, &failed)) return rc;
+    if (sites_used) *sites_used = used;
+    return 0;
+}
+
+int pansim_core_ld_kernel_ms(pansim_ctx *c, const pansim_ld_params *p, uint32_t repeats, float *site_ms, float *transpose_ms,
+                             float *pair_ms, uint64_t *pairs)
+{
+    if (!c || !p || !repeats) return PANSIM_ERR_INVALID;
+    if (int rc = ld_validate(c, nullptr, p)) return rc;
+    std::vector<LdJob> jobs{{c, nullptr}};
+    std::vector<pansim_ld_bin> bins(ld_n_bins(p));
+    uint64_t used = 0;
+    size_t failed = 0;
+    if (int rc = ld_run(jobs, p, bins.data(), &used, &failed)) return rc;       // also the warm-up
+    const LdJob &j = jobs[0];
+    cudaEvent_t ev[4];
+    for (auto &e : ev) CU(c, cudaEventCreate(&e));
+    int rc = 0;
+    cudaEventRecord(ev[0], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++) rc = ld_site_pass(c, c->ld, c->Ll, p->min_minor, nullptr);
+    cudaEventRecord(ev[1], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc && j.own; r++) rc = ld_transpose(c, c->ld, c->Ll, c->ld.x);
+    cudaEventRecord(ev[2], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc && j.own; r++) {
+        rc = ld_tile_list(c, j.own, j.own, p->max_dist, nullptr);
+        if (!rc) rc = ld_pairs(c, p, j.own, j.own, j.tiles);
+    }
+    cudaEventRecord(ev[3], c->stream);
+    const cudaError_t e = cudaEventSynchronize(ev[3]);
+    float t[3] = {0.f, 0.f, 0.f};
+    for (int k = 0; k < 3; k++) cudaEventElapsedTime(&t[k], ev[k], ev[k + 1]);
+    for (auto &x : ev) cudaEventDestroy(x);
+    if (rc) return rc;
+    if (e != cudaSuccess) FAIL(c, PANSIM_ERR_CUDA, "LD kernels failed: %s", cudaGetErrorString(e));
+    if (site_ms) *site_ms = t[0] / (float)repeats;
+    if (transpose_ms) *transpose_ms = t[1] / (float)repeats;
+    if (pair_ms) *pair_ms = t[2] / (float)repeats;
+    if (pairs) {
+        *pairs = 0;
+        for (const pansim_ld_bin &b : bins) *pairs += b.pairs;
+    }
+    return 0;
+}
+
+// mean r^2 of a bin from its exact integer sum; the same bits on every host
+double pansim_ld_mean_r2(const pansim_ld_bin *b)
+{
+    if (!b || !b->pairs) return std::numeric_limits<double>::quiet_NaN();
+    return (std::ldexp((double)b->r2_hi, 32) + std::ldexp((double)b->r2_lo, -32)) / (double)b->pairs;
 }
 
 // ---- communicator over column shards (one process per GPU) -------------------

@@ -13,7 +13,8 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import OK, PansimError, _diversity, _pairs_or_none, _ptr, make_config
+from .population import (OK, CoreLD, PansimError, _core_ld, _diversity, _ld_bins, _ld_params, _pairs_or_none, _ptr,
+                         make_config)
 
 
 class PansimGroup:
@@ -139,6 +140,14 @@ class PansimGroup:
         st = np.empty((n, 4), np.float64) if P else None
         self._check(self._lib.pansim_group_run_generations_diversity(self._h, gen0, n, _ptr(r1), _ptr(r2), P, _ptr(st), divs))
         return [_diversity(divs[g]) for g in range(n)], st
+
+    def core_ld(self, max_dist: int = 10000, bin_width: int = 100, min_minor: int = 1) -> CoreLD:
+        """Whole-alignment LD bins (Pansim.core_ld): every shard with the next one as its halo, summed."""
+        bins, n = _ld_bins(max_dist, bin_width)
+        used = C.c_uint64(0)
+        self._check(self._lib.pansim_group_core_ld(self._h, C.byref(_ld_params(max_dist, bin_width, min_minor)), bins,
+                                                   C.byref(used)))
+        return _core_ld(bins, n, max_dist, bin_width, used.value)
 
     def gene_counts(self) -> np.ndarray:
         out = np.empty(self.G, np.uint32)

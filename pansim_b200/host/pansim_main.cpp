@@ -6,6 +6,7 @@
 // same call order per generation (main.rs:429-528) and the same six output files with
 // Rust's `{}` float formatting. Host randomness (selection coefficients, initial rows,
 // pair sampling) uses std::mt19937_64 in place of rand's StdRng.
+#include <algorithm>
 #include <charconv>
 #include <cmath>
 #include <cstdio>
@@ -40,11 +41,13 @@ struct Flags {
 const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes", "avg_gene_freq", "n_gen",
                              "max_distances", "core_mu", "HR_rate", "HGT_rate", "rate_genes1", "rate_genes2",
                              "prop_genes2", "prop_positive", "pos_lambda", "neg_lambda", "seed", "outpref",
-                             "threads", "genome_size_penalty", "competition_strength", "device", "gpus"};
+                             "threads", "genome_size_penalty", "competition_strength", "device", "gpus",
+                             "ld_max_dist", "ld_bin_width", "ld_min_minor"};       // extensions: --print_ld bins
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
-                              "all_pairs", "print_diversity", "print_vcf"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "all_pairs", "print_diversity", "print_vcf", "print_ld"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
-                                                                              // print_vcf (<outpref>_core_genome.vcf)
+                                                                              // print_vcf (<outpref>_core_genome.vcf),
+                                                                              // print_ld (<outpref>_core_ld.tsv)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -53,7 +56,8 @@ bool parse(int argc, char **argv, Flags &f)
              {"HR_rate", "0.05"}, {"HGT_rate", "0.05"}, {"rate_genes1", "1.0"}, {"rate_genes2", "1000.0"},
              {"prop_genes2", "0.1"}, {"prop_positive", "-0.1"}, {"pos_lambda", "10.0"}, {"neg_lambda", "10.0"},
              {"seed", "0"}, {"outpref", "distances"}, {"threads", "1"}, {"genome_size_penalty", "0.99"},
-             {"competition_strength", "0.0"}, {"device", "0"}, {"gpus", "1"}};
+             {"competition_strength", "0.0"}, {"device", "0"}, {"gpus", "1"},
+             {"ld_max_dist", "10000"}, {"ld_bin_width", "100"}, {"ld_min_minor", "1"}};
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         if (a == "--help" || a == "-h") {
@@ -127,6 +131,10 @@ int main(int argc, char **argv)
     const uint64_t seed = std::strtoull(fl.val["seed"].c_str(), nullptr, 10);
     const bool verbose = fl.sw["verbose"], print_dist = fl.sw["print_dist"], print_matrices = fl.sw["print_matrices"];
     const bool all_pairs = fl.sw["all_pairs"], print_diversity = fl.sw["print_diversity"], print_vcf = fl.sw["print_vcf"];
+    const bool print_ld = fl.sw["print_ld"];
+    const pansim_ld_params ld_params = {(uint32_t)std::strtoul(fl.val["ld_max_dist"].c_str(), nullptr, 10),
+                                        (uint32_t)std::strtoul(fl.val["ld_bin_width"].c_str(), nullptr, 10),
+                                        (uint32_t)std::strtoul(fl.val["ld_min_minor"].c_str(), nullptr, 10)};
     const int n_gpus = std::max(1, std::atoi(fl.val["gpus"].c_str()));       // extension: column shards over N devices of the box
     const bool print_selection = fl.sw["print_selection"], no_control = fl.sw["no_control_genome_size"];
     const double genome_size_penalty = as_f64(fl, "genome_size_penalty"), competition_strength = as_f64(fl, "competition_strength");
@@ -283,6 +291,14 @@ int main(int argc, char **argv)
         }
         if (print_matrices) pops.write(outpref);                            // main.rs:550-553
         if (print_vcf) pops.write_core_vcf(outpref + "_core_genome.vcf");   // extension: the last generation as VCF
+        if (print_ld) {                                                     // extension: LD of the last generation by distance
+            std::ofstream f(outpref + "_core_ld.tsv");
+            const std::vector<pansim_ld_bin> bins = pops.core_ld(ld_params);
+            for (size_t b = 0; b < bins.size(); b++) {
+                const uint64_t lo = (uint64_t)b * ld_params.bin_width + 1, hi = std::min<uint64_t>(lo + ld_params.bin_width - 1, ld_params.max_dist);
+                f << lo << "\t" << hi << "\t" << bins[b].pairs << "\t" << bins[b].four_gamete << "\t" << fmt(pansim_ld_mean_r2(&bins[b])) << "\n";
+            }
+        }
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)
         std::fprintf(stderr, "pansim: %s\n", e.what());

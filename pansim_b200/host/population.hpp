@@ -182,6 +182,16 @@ public:
         return n;
     }
 
+    // (extension) LD of the core alignment by site distance over all shards: n_bins = ceil(max_dist / bin_width) bins
+    std::vector<pansim_ld_bin> core_ld(const pansim_ld_params &p, uint64_t *sites_used = nullptr)
+    {
+        const uint64_t n = p.bin_width ? ((uint64_t)p.max_dist + p.bin_width - 1) / p.bin_width : 0;
+        std::vector<pansim_ld_bin> bins(std::max<uint64_t>(n, 1));
+        gcheck(pansim_group_core_ld(grp_, &p, bins.data(), sites_used));
+        bins.resize(n);
+        return bins;
+    }
+
     pansim_ctx *raw() { return ctx_; }          // shard 0 (the whole run when n_gpus() == 1)
     pansim_group *group() { return grp_; }
     const pansim_config &config() const { return cfg_; }

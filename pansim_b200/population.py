@@ -89,6 +89,43 @@ def diversity_stats(d: Diversity, pop_size: int) -> tuple[float, float, float]:
     return float(out[0]), float(out[1]), float(out[2])
 
 
+class CoreLD(NamedTuple):
+    """LD bins of pansim_core_ld (include/pansim_b200.h): per bin its distances dist_lo..dist_hi, the site pairs, the
+    pairs showing four gametes, the exact sum of r^2 in units of 2^-32 and the mean r^2 (NaN for an empty bin); and
+    the used sites counted."""
+    dist_lo: np.ndarray
+    dist_hi: np.ndarray
+    pairs: np.ndarray
+    four_gamete: np.ndarray
+    r2_sum: list
+    mean_r2: np.ndarray
+    sites_used: int
+
+
+def _ld_params(max_dist: int, bin_width: int, min_minor: int) -> _ffi.LdParams:
+    return _ffi.LdParams(max_dist, bin_width, min_minor)
+
+
+def _ld_bins(max_dist: int, bin_width: int):
+    n = -(-max_dist // bin_width) if max_dist > 0 and bin_width > 0 else 1
+    return (_ffi.LdBin * max(n, 1))(), n
+
+
+def _core_ld(bins, n: int, max_dist: int, bin_width: int, used: int) -> CoreLD:
+    lib = _ffi.lib()
+    lo = np.arange(n, dtype=np.int64) * bin_width + 1
+    hi = np.minimum(lo + bin_width - 1, max_dist)
+    return CoreLD(lo, hi, np.array([b.pairs for b in bins[:n]], np.uint64),
+                  np.array([b.four_gamete for b in bins[:n]], np.uint64),
+                  [(b.r2_hi << 64) | b.r2_lo for b in bins[:n]],
+                  np.array([lib.pansim_ld_mean_r2(C.byref(b)) for b in bins[:n]], np.float64), used)
+
+
+def ld_mean_r2(pairs: int, r2_sum: int) -> float:
+    """Mean r^2 of a bin from its pair count and exact r^2 sum (units of 2^-32), formed by the library."""
+    return _ffi.lib().pansim_ld_mean_r2(C.byref(_ffi.LdBin(pairs, 0, r2_sum >> 64, r2_sum & (2 ** 64 - 1))))
+
+
 def _pairs_or_none(range1, range2):
     if range1 is None:
         return None, None, 0
@@ -369,6 +406,24 @@ class Pansim:
         self._check(self._lib.pansim_run_generations_diversity(self._h, gen0, n, _ptr(r1), _ptr(r2), P, _ptr(st), divs))
         return [_diversity(divs[g]) for g in range(n)], st
 
+    # -- core-genome linkage disequilibrium (extension) --------------------
+    def core_ld(self, max_dist: int = 10000, bin_width: int = 100, min_minor: int = 1, next: "Pansim | None" = None) -> CoreLD:
+        """r^2 and four-gamete pairs of the used sites binned by distance (pansim_core_ld). `next` is the context
+        holding the sites right after this one's: its first max_dist sites are then the halo of this context, so the
+        sum over the shards chained this way equals the single-context result."""
+        bins, n = _ld_bins(max_dist, bin_width)
+        used = C.c_uint64(0)
+        self._check(self._lib.pansim_core_ld(self._h, next._h if next is not None else None,
+                                             C.byref(_ld_params(max_dist, bin_width, min_minor)), bins, C.byref(used)))
+        return _core_ld(bins, n, max_dist, bin_width, used.value)
+
+    def ld_kernel_ms(self, max_dist: int = 10000, bin_width: int = 100, min_minor: int = 1, repeats: int = 10):
+        """Measurement: device ms of one site pass, one transpose and one pair pass, and the pairs counted."""
+        s, t, q, n = C.c_float(), C.c_float(), C.c_float(), C.c_uint64()
+        self._check(self._lib.pansim_core_ld_kernel_ms(self._h, C.byref(_ld_params(max_dist, bin_width, min_minor)), repeats,
+                                                       C.byref(s), C.byref(t), C.byref(q), C.byref(n)))
+        return s.value, t.value, q.value, n.value
+
     # -- multi-GPU: communicator over column shards (one process per GPU) --
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -510,4 +565,4 @@ class Pansim:
                 f.write(",".join(ones + [str(int(x)) for x in acc[r]]) + "\n")
 
 
-__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "make_config", "standard_deviation", "fmt_f64"]
+__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "make_config", "standard_deviation", "fmt_f64"]

@@ -61,12 +61,14 @@ class RunResult:
     per_gen: list = field(default_factory=list)   # (avg_core, std_core, avg_acc, std_acc)
     diversity: list = field(default_factory=list) # per generation: Diversity (--print_diversity)
     sfs: np.ndarray = None                        # SFS of the last generation (--print_diversity)
+    ld: object = None                             # CoreLD of the last generation (--print_ld)
     selection: np.ndarray = None
     stdout: list = field(default_factory=list)
 
 
 def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False,
-        print_diversity: bool = False, print_vcf: bool = False) -> RunResult | None:
+        print_diversity: bool = False, print_vcf: bool = False, print_ld: bool = False, ld_max_dist: int = 10000,
+        ld_bin_width: int = 100, ld_min_minor: int = 1) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -74,7 +76,10 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     `<outpref>_diversity.tsv` (segregating, multiallelic, pi, theta_W, Tajima's D) and the site frequency
     spectrum of the last generation to `<outpref>_core_sfs.txt`.
     print_vcf (extension): the core alignment of the last generation as `<outpref>_core_genome.vcf`, written
-    after the other outputs (Pansim.write_core_vcf)."""
+    after the other outputs (Pansim.write_core_vcf).
+    print_ld (extension): linkage disequilibrium of the core alignment of the last generation as
+    `<outpref>_core_ld.tsv`, written after the other outputs (Pansim.core_ld with ld_max_dist, ld_bin_width,
+    ld_min_minor; write_core_ld)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -166,7 +171,19 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             sim.write(outpref)
         if print_vcf and outpref:
             sim.write_core_vcf(outpref + "_core_genome.vcf")
+        if print_ld:
+            res.ld = sim.core_ld(ld_max_dist, ld_bin_width, ld_min_minor)
+            if outpref:
+                write_core_ld(outpref, res.ld)
     return res
+
+
+def write_core_ld(outpref: str, ld):
+    """`<outpref>_core_ld.tsv`: one line per distance bin (no header): dist_lo, dist_hi, pairs, four-gamete pairs,
+    mean r^2 (NaN for an empty bin)."""
+    with open(outpref + "_core_ld.tsv", "w") as f:
+        for lo, hi, n, fg, r2 in zip(ld.dist_lo, ld.dist_hi, ld.pairs, ld.four_gamete, ld.mean_r2):
+            f.write(f"{int(lo)}\t{int(hi)}\t{int(n)}\t{int(fg)}\t{fmt_f64(float(r2))}\n")
 
 
 def write_diversity(outpref: str, diversity, sfs, pop_size: int):
