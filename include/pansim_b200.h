@@ -310,6 +310,62 @@ int pansim_core_ld_kernel_ms(pansim_ctx *ctx, const pansim_ld_params *p, uint32_
  * that order, NaN when pairs = 0, so every host prints the same digits */
 double pansim_ld_mean_r2(const pansim_ld_bin *b);
 
+/* ---- clonal genealogy (extension: the reference keeps no pedigree) -------
+ * The parent vectors the generations were drawn with, recorded on the device, and the genealogy of the present
+ * population traced from them (DESIGN.md section 13). Both populations share it: next_generation gathers the core and
+ * the accessory rows by the same vector.
+ *
+ * Record. Once recording is enabled, each call that advances the population by one generation appends that
+ * generation's parent vector H (u32[N], child -> parent index in the previous generation): pansim_step,
+ * pansim_run_generations, pansim_run_generations_stats, pansim_run_generations_diversity, pansim_step_with_parents,
+ * pansim_next_generation and pansim_step_replay. The record keeps the last `capacity` vectors as a ring. Let T be the
+ * number of vectors kept, H_1 .. H_T oldest first. Generation 0 is the population before H_1; generation T is the
+ * present. pansim_set_initial, pansim_upload_core, pansim_upload_acc and enabling again clear the record (T = 0).
+ *
+ * Lineages: a_T(i) = i, a_{t-1}(i) = H_t[a_t(i)].
+ * Nodes:
+ *   - Leaves are nodes 0 .. N-1. Leaf i is present individual i: time 0, individual = i.
+ *   - An internal node is created at generation t for each individual x such that at least two distinct
+ *     generation-(t+1) ancestors of present individuals have x as their parent: |{a_{t+1}(i) : a_t(i) = x}| >= 2.
+ *     Its time is T - t and its individual is x.
+ *   - Internal nodes are numbered N, N+1, ... from the present backwards (time ascending); within one generation
+ *     they are ordered by the smallest leaf below them, ascending.
+ *   - If more than one lineage remains at generation 0, a virtual root is added last: time T, individual =
+ *     0xFFFFFFFF, its children the remaining lineages' top nodes. Otherwise the last merge (the MRCA) is the root,
+ *     and the trace stops there even when t > 0.
+ *   - The root's parent is 0xFFFFFFFF. There are at most 2N nodes, and every parent has a larger id than its child.
+ * TMRCA(i, j) = the time of the lowest common ancestor of leaves i and j: 0 for i = j, T under a virtual root
+ * ("not coalesced within the record").
+ * Newick: a leaf is `ind_<i>` (the sample names of the VCF); an internal node is `(` its children, `,`-separated,
+ * `)` with no label; every non-root node is followed by `:` and its branch length parent.time - time as a decimal
+ * integer; children are ordered by the smallest leaf below them, ascending; the text ends with `;` and `\n`. With
+ * N = 1 the tree is `ind_0;\n`. This ordering makes the string canonical: the same history gives the same bytes on
+ * every host and every shard count. Every output is an integer; no grid, stream or shard split changes a byte.
+ *
+ * Cost while recording: one device-to-device copy of N x 4 bytes per generation on a stream of its own, ordered after
+ * the parent draw by an event; the selection chain, its graphs and the core step are unchanged. With recording off no
+ * call, event or graph differs. The trace (one CTA) and the TMRCA walk run when asked for.
+ *
+ * pansim_enable_genealogy allocates the ring, capacity x N x 4 bytes of device memory (plus 52 N bytes for the trace);
+ * a failed allocation returns PANSIM_ERR_NOMEM and leaves recording off. capacity = 0 turns recording off and frees
+ * the ring. pansim_genealogy traces on the device and copies back the node table (nodes[2N], may be NULL) and the
+ * summary; lineages_at_start = 1 means the MRCA was found. pansim_genealogy_history copies the record itself,
+ * out[kept][N] oldest first. pansim_genealogy_tmrca uses the device node table of the current record (traced again
+ * if the record changed since the last trace); an index >= N returns PANSIM_ERR_INVALID. Before
+ * pansim_enable_genealogy these return PANSIM_ERR_STATE. The context keeps working after a refused call. */
+typedef struct { uint32_t parent, individual, time; } pansim_genealogy_node;
+typedef struct { uint64_t generations_total; uint32_t generations_kept, n_nodes, lineages_at_start; } pansim_genealogy_info;
+int pansim_enable_genealogy(pansim_ctx *ctx, uint32_t capacity);
+int pansim_genealogy(pansim_ctx *ctx, pansim_genealogy_node *nodes /* [2N] */, pansim_genealogy_info *info);
+int pansim_genealogy_history(pansim_ctx *ctx, uint32_t *out /* [kept][N], oldest first */);
+int pansim_genealogy_tmrca(pansim_ctx *ctx, const uint32_t *r1, const uint32_t *r2, size_t n_pairs, uint32_t *tmrca);
+/* Newick text of a node table (as pansim_genealogy returns it; n_leaves = N), needs no device. Iterative: any depth.
+ * *len = the length of the text, terminating NUL excluded. out = NULL: only *len. Otherwise cap must hold the text
+ * and its NUL; if it does not, PANSIM_ERR_INVALID with *len set. A table that is not a tree of that shape (root not
+ * last, a parent not above its child, a leaf as parent, a branch of negative length) -> PANSIM_ERR_INVALID. */
+int pansim_genealogy_newick(const pansim_genealogy_node *nodes, uint32_t n_nodes, uint32_t n_leaves, char *out,
+                            size_t cap, size_t *len);
+
 /* ---- multi-GPU: column shards of one alignment --------------------------
  * (SURVEY.md 8e; the reference is one shared-memory process, population.rs has no analogue.)
  * Every shard context holds all individuals for [site_begin, site_end) and a replica of the
@@ -369,6 +425,12 @@ int pansim_group_write_core_vcf(pansim_group *g, const char *path, uint64_t *byt
 
 /* pansim_core_ld over the whole alignment: every shard with the next one as its halo, summed on the host */
 int pansim_group_core_ld(pansim_group *g, const pansim_ld_params *p, pansim_ld_bin *bins, uint64_t *sites_used);
+
+/* the clonal genealogy of the group: every shard draws the same parents, so shard 0 records and answers. Under a
+ * communicator (one process per GPU) every rank records its own identical copy; nothing is exchanged. */
+int pansim_group_enable_genealogy(pansim_group *g, uint32_t capacity);
+int pansim_group_genealogy(pansim_group *g, pansim_genealogy_node *nodes, pansim_genealogy_info *info);
+int pansim_group_genealogy_tmrca(pansim_group *g, const uint32_t *r1, const uint32_t *r2, size_t n_pairs, uint32_t *tmrca);
 
 /* ---- introspection / instrumentation ----------------------------------- */
 typedef struct {

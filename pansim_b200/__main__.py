@@ -5,7 +5,7 @@ same parsing quirks: pop_size/core_size/pan_genes/core_genes/n_gen are parsed as
 f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
 accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
---print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor.
+--print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy.
 """
 from __future__ import annotations
 
@@ -70,6 +70,10 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--ld_bin_width", type=int, default=100, help="(extension) distances per bin of --print_ld")
     ap.add_argument("--ld_min_minor", type=int, default=1,
                     help="(extension) --print_ld uses sites where at least this many rows are derived and at least this many are not")
+    ap.add_argument("--print_genealogy", action="store_true",
+                    help="(extension) record the parents of every generation; <outpref>_genealogy.nwk: the clonal genealogy of "
+                         "the last generation as Newick (leaves ind_<i>, branch lengths in generations); <outpref>_tmrca.tsv: "
+                         "the TMRCA of the pair on each line of <outpref>.tsv")
     return ap
 
 
@@ -79,9 +83,11 @@ def main(argv=None) -> int:
     all_pairs = ns.pop("all_pairs")
     print_diversity = ns.pop("print_diversity")
     print_vcf = ns.pop("print_vcf")
+    print_genealogy = ns.pop("print_genealogy")
     ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
     p = Params(**ns)
-    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf, **ld)
+    run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf,
+        print_genealogy=print_genealogy, **ld)
     return 0                       # the reference exits 0 even when validation fails (main.rs:195-247)
 
 

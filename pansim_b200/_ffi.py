@@ -34,6 +34,8 @@ EXPORTED = [
     "pansim_group_core_diversity", "pansim_group_run_generations_diversity",
     "pansim_write_core_vcf", "pansim_group_write_core_vcf", "pansim_core_vcf_kernel_ms",
     "pansim_core_ld", "pansim_group_core_ld", "pansim_core_ld_kernel_ms", "pansim_ld_mean_r2",
+    "pansim_enable_genealogy", "pansim_genealogy", "pansim_genealogy_history", "pansim_genealogy_tmrca",
+    "pansim_genealogy_newick", "pansim_group_enable_genealogy", "pansim_group_genealogy", "pansim_group_genealogy_tmrca",
 ]
 COMM_ID_BYTES = 128
 
@@ -104,6 +106,15 @@ class LdParams(C.Structure):
 
 class LdBin(C.Structure):
     _fields_ = [("pairs", C.c_uint64), ("four_gamete", C.c_uint64), ("r2_hi", C.c_uint64), ("r2_lo", C.c_uint64)]
+
+
+class GenealogyNode(C.Structure):
+    _fields_ = [("parent", C.c_uint32), ("individual", C.c_uint32), ("time", C.c_uint32)]
+
+
+class GenealogyInfo(C.Structure):
+    _fields_ = [("generations_total", C.c_uint64), ("generations_kept", C.c_uint32), ("n_nodes", C.c_uint32),
+                ("lineages_at_start", C.c_uint32)]
 
 
 PAIRS_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.POINTER(C.c_uint32),
@@ -219,5 +230,13 @@ def lib():
     sig("pansim_core_ld_kernel_ms", cint, vp, C.POINTER(LdParams), u32, C.POINTER(C.c_float), C.POINTER(C.c_float),
         C.POINTER(C.c_float), C.POINTER(C.c_uint64))
     sig("pansim_ld_mean_r2", dbl, C.POINTER(LdBin))
+    sig("pansim_enable_genealogy", cint, vp, u32)
+    sig("pansim_genealogy", cint, vp, vp, C.POINTER(GenealogyInfo))
+    sig("pansim_genealogy_history", cint, vp, vp)
+    sig("pansim_genealogy_tmrca", cint, vp, vp, vp, sz, vp)
+    sig("pansim_genealogy_newick", cint, vp, u32, u32, vp, sz, C.POINTER(sz))
+    sig("pansim_group_enable_genealogy", cint, vp, u32)
+    sig("pansim_group_genealogy", cint, vp, vp, C.POINTER(GenealogyInfo))
+    sig("pansim_group_genealogy_tmrca", cint, vp, vp, vp, sz, vp)
     _lib = L
     return L

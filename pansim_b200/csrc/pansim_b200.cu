@@ -21,6 +21,7 @@
 #include "core_mut.cuh"
 #include "distance.cuh"
 #include "diversity.cuh"
+#include "genealogy.cuh"
 #include "ld.cuh"
 #include "pack.cuh"
 #include "replay.cuh"
@@ -284,6 +285,20 @@ struct pansim_ctx {
     unsigned long long *h_ld = nullptr, *h_ld_bins = nullptr;         // pinned: own / halo used sites, tile pairs; bins
     size_t h_ld_bins_cap = 0;
     cudaEvent_t ev_ld = nullptr;                                       // the halo of this context is ready
+    // clonal genealogy (genealogy.cuh): a ring of the last gen_cap parent vectors, each copied on stream_gen behind
+    // ev_parents[i]; next_parents_buffer waits on ev_gen_done[i] before buffer i is rewritten. The trace and the
+    // TMRCA walk run on stream_gen too, so they follow every copy enqueued before them.
+    cudaStream_t stream_gen = nullptr;
+    cudaEvent_t ev_gen_done[3] = {nullptr, nullptr, nullptr};
+    bool gen_done_valid[3] = {false, false, false};
+    uint32_t *d_gen_ring = nullptr;      // [gen_cap][N]
+    uint32_t *d_gen_scratch = nullptr;   // trace scratch and node table, gen_scratch_words(N) words
+    uint32_t gen_cap = 0;                // 0: recording off
+    uint64_t gen_total = 0;              // vectors appended since the last reset
+    uint64_t gen_epoch = 1, gen_traced = 0;   // bumped by every append and reset / the record the node table is of
+    uint32_t gen_nodes = 0, gen_lineages = 0;
+    uint32_t *d_gen_pairs = nullptr;     // TMRCA: r1, r2, result
+    size_t gen_pair_cap = 0;
     // staging for upload/download
     uint8_t *d_stage = nullptr;
     size_t stage_cap = 0;
@@ -902,15 +917,39 @@ int require_state(pansim_ctx *c)
 }
 
 // Rotate to the next parents buffer. The buffer was last read by the core step
-// issued three generations ago: the selection chain must not overwrite it before
-// that kernel has finished.
+// issued three generations ago (and by the genealogy copy of that generation): the
+// selection chain must not overwrite it before that kernel has finished.
 int next_parents_buffer(pansim_ctx *c)
 {
     c->parents_idx = (c->parents_idx + 1) % 3;
     const int i = c->parents_idx;
     if (c->core_done_valid[i]) CU(c, cudaStreamWaitEvent(c->stream, c->ev_core_done[i], 0));
+    if (c->gen_done_valid[i]) CU(c, cudaStreamWaitEvent(c->stream, c->ev_gen_done[i], 0));
     c->d_parents = c->d_parents_buf[i];
     return 0;
+}
+
+// With genealogy recording on: append the current parents vector (ev_parents[i] recorded behind it) to the ring,
+// one device-to-device copy on stream_gen into the slot the host already knows
+int genealogy_record(pansim_ctx *c)
+{
+    if (!c->gen_cap) return 0;
+    const int i = c->parents_idx;
+    CU(c, cudaStreamWaitEvent(c->stream_gen, c->ev_parents[i], 0));
+    uint32_t *dst = c->d_gen_ring + (size_t)(c->gen_total % c->gen_cap) * c->N;
+    CU(c, cudaMemcpyAsync(dst, c->d_parents, (size_t)c->N * 4, cudaMemcpyDeviceToDevice, c->stream_gen));
+    CU(c, cudaEventRecord(c->ev_gen_done[i], c->stream_gen));
+    c->gen_done_valid[i] = true;
+    c->gen_total++;
+    c->gen_epoch++;
+    return 0;
+}
+
+// the state was replaced: the record starts again (T = 0)
+void genealogy_reset(pansim_ctx *c)
+{
+    c->gen_total = 0;
+    c->gen_epoch++;
 }
 
 // accessory step on the chain stream, fused core step on the core stream; both
@@ -921,6 +960,7 @@ int launch_core_part(pansim_ctx *c, uint32_t gen)
     const int i = c->parents_idx;
     CU(c, cudaEventRecord(c->ev_parents[i], c->stream));
     CU(c, cudaStreamWaitEvent(c->stream_core, c->ev_parents[i], 0));
+    if (int rc = genealogy_record(c)) return rc;
     {
         ScopedSpan s(c, TG_CORE, c->stream_core);
         if (int rc = launch_core_step(c, gen, true, c->stream_core)) return rc;
@@ -1110,6 +1150,9 @@ void pansim_destroy(pansim_ctx *c)
     if (c->h_ld) cudaFreeHost(c->h_ld);
     if (c->h_ld_bins) cudaFreeHost(c->h_ld_bins);
     if (c->ev_ld) cudaEventDestroy(c->ev_ld);
+    if (c->stream_gen) { cudaStreamSynchronize(c->stream_gen); cudaStreamDestroy(c->stream_gen); }
+    for (auto e : c->ev_gen_done) if (e) cudaEventDestroy(e);
+    for (void *p : {(void *)c->d_gen_ring, (void *)c->d_gen_scratch, (void *)c->d_gen_pairs}) if (p) cudaFree(p);
     for (auto *e : c->graphs) {
         if (e->exec) cudaGraphExecDestroy(e->exec);
         e->pool.destroy();
@@ -1450,7 +1493,7 @@ int pansim_upload_core(pansim_ctx *c, const uint8_t *bytes)
 {
     if (!c || !bytes) return PANSIM_ERR_INVALID;
     CU(c, cudaSetDevice(c->cfg.device));
-    if (c->Ll == 0) { c->has_core = true; return 0; }
+    if (c->Ll == 0) { c->has_core = true; genealogy_reset(c); return 0; }
     // stage at most ~256 MiB of host bytes at a time
     uint32_t rows_per = (uint32_t)std::max<uint64_t>(1, (256ull << 20) / c->Ll);
     if (rows_per > c->N) rows_per = c->N;
@@ -1459,6 +1502,7 @@ int pansim_upload_core(pansim_ctx *c, const uint8_t *bytes)
     uint8_t *dst = c->core[c->core_cur];
     c->hr_pending = false;                       // the state is replaced
     c->core_version++;
+    genealogy_reset(c);
     for (uint32_t r0 = 0; r0 < c->N; r0 += rows_per) {
         const uint32_t nr = std::min(rows_per, c->N - r0);
         CU(c, cudaMemcpyAsync(c->d_stage, bytes + (size_t)r0 * c->Ll, (size_t)nr * c->Ll, cudaMemcpyHostToDevice, c->stream));
@@ -1476,6 +1520,7 @@ int pansim_upload_acc(pansim_ctx *c, const uint8_t *bytes)
     if (!c || (!bytes && c->G)) return PANSIM_ERR_INVALID;
     CU(c, cudaSetDevice(c->cfg.device));
     if (int rc = join_fitness(c)) return rc;
+    genealogy_reset(c);
     if (c->G) {
         if (int rc = ensure_stage(c, (size_t)c->N * c->G)) return rc;
         CU(c, cudaMemcpyAsync(c->d_stage, bytes, (size_t)c->N * c->G, cudaMemcpyHostToDevice, c->stream));
@@ -1494,6 +1539,7 @@ int pansim_set_initial(pansim_ctx *c, const uint8_t *core_row, const uint8_t *ac
 {
     if (!c || !core_row || (!acc_row && c->G)) return PANSIM_ERR_INVALID;
     CU(c, cudaSetDevice(c->cfg.device));
+    genealogy_reset(c);
     if (c->Ll) {
         if (int rc = ensure_stage(c, (size_t)c->Ll)) return rc;
         CU(c, cudaMemcpyAsync(c->d_stage, core_row + c->site_begin, c->Ll, cudaMemcpyHostToDevice, c->stream));
@@ -1863,6 +1909,10 @@ int pansim_next_generation(pansim_ctx *c, const uint32_t *parents)
     CU(c, cudaSetDevice(c->cfg.device));
     if (int rc = next_parents_buffer(c)) return rc;
     if (int rc = upload_parents(c, parents)) return rc;
+    if (c->gen_cap) {
+        CU(c, cudaEventRecord(c->ev_parents[c->parents_idx], c->stream));
+        if (int rc = genealogy_record(c)) return rc;
+    }
     timing_begin(c);
     if (int rc = join_fitness(c)) return rc;
     if (c->G) {
@@ -3332,6 +3382,206 @@ double pansim_ld_mean_r2(const pansim_ld_bin *b)
 {
     if (!b || !b->pairs) return std::numeric_limits<double>::quiet_NaN();
     return (std::ldexp((double)b->r2_hi, 32) + std::ldexp((double)b->r2_lo, -32)) / (double)b->pairs;
+}
+
+// ---- clonal genealogy (genealogy.cuh, DESIGN.md section 13) ------------------
+// trace scratch and node table: owner, cnt, newid [N]; lineage nodes and ancestors [2][N] each; parent, individual,
+// time [2N] each; n_nodes and lineages_at_start
+static size_t gen_scratch_words(uint32_t N) { return (size_t)13 * N + 2; }
+
+int pansim_enable_genealogy(pansim_ctx *c, uint32_t capacity)
+{
+    if (!c) return PANSIM_ERR_INVALID;
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (c->stream_gen) CU(c, cudaStreamSynchronize(c->stream_gen));
+    for (uint32_t **p : {&c->d_gen_ring, &c->d_gen_scratch, &c->d_gen_pairs}) {
+        if (*p) cudaFree(*p);
+        *p = nullptr;
+    }
+    c->gen_pair_cap = 0;
+    c->gen_cap = 0;
+    for (bool &v : c->gen_done_valid) v = false;
+    genealogy_reset(c);
+    if (capacity == 0) return 0;
+    if (!c->stream_gen) {
+        CU(c, cudaStreamCreateWithFlags(&c->stream_gen, cudaStreamNonBlocking));
+        for (auto &e : c->ev_gen_done) CU(c, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    }
+    const bool fits = (uint64_t)capacity <= (uint64_t)SIZE_MAX / 4 / c->N;
+    if (!fits || cudaMalloc(&c->d_gen_ring, (size_t)capacity * c->N * 4) != cudaSuccess ||
+        cudaMalloc(&c->d_gen_scratch, gen_scratch_words(c->N) * 4) != cudaSuccess) {
+        cudaGetLastError();
+        for (uint32_t **p : {&c->d_gen_ring, &c->d_gen_scratch}) {
+            if (*p) cudaFree(*p);
+            *p = nullptr;
+        }
+        FAIL(c, PANSIM_ERR_NOMEM, "genealogy ring of %u x %u parent vectors: cudaMalloc failed; recording stays off", capacity, c->N);
+    }
+    c->gen_cap = capacity;
+    return 0;
+}
+
+// the node table of the current record on the device (traced again only when the record changed)
+static int genealogy_trace(pansim_ctx *c, GenealogyTrace &a)
+{
+    const uint32_t N = c->N;
+    uint32_t *w = c->d_gen_scratch;
+    a.ring = c->d_gen_ring;
+    a.cap = c->gen_cap;
+    a.N = N;
+    a.T = (uint32_t)std::min<uint64_t>(c->gen_total, c->gen_cap);
+    a.base = (uint32_t)((c->gen_total - a.T) % c->gen_cap);
+    a.owner = w; a.cnt = w + N; a.newid = w + 2 * (size_t)N;
+    a.lin_node[0] = w + 3 * (size_t)N; a.lin_node[1] = w + 4 * (size_t)N;
+    a.lin_anc[0] = w + 5 * (size_t)N; a.lin_anc[1] = w + 6 * (size_t)N;
+    a.parent = w + 7 * (size_t)N; a.individual = w + 9 * (size_t)N; a.time = w + 11 * (size_t)N;
+    a.out = w + 13 * (size_t)N;
+    if (c->gen_traced == c->gen_epoch) return 0;
+    genealogy_trace_kernel<<<1, GT_THREADS, 0, c->stream_gen>>>(a);
+    LAUNCH_CHECK(c);
+    uint32_t out[2];
+    CU(c, cudaMemcpyAsync(out, a.out, sizeof out, cudaMemcpyDeviceToHost, c->stream_gen));
+    CU(c, cudaStreamSynchronize(c->stream_gen));
+    c->gen_nodes = out[0];
+    c->gen_lineages = out[1];
+    c->gen_traced = c->gen_epoch;
+    return 0;
+}
+
+static int genealogy_require(pansim_ctx *c)
+{
+    if (!c->gen_cap) FAIL(c, PANSIM_ERR_STATE, "genealogy recording is off: call pansim_enable_genealogy first");
+    CU(c, cudaSetDevice(c->cfg.device));
+    return 0;
+}
+
+int pansim_genealogy(pansim_ctx *c, pansim_genealogy_node *nodes, pansim_genealogy_info *info)
+{
+    if (!c) return PANSIM_ERR_INVALID;
+    if (int rc = genealogy_require(c)) return rc;
+    GenealogyTrace a;
+    if (int rc = genealogy_trace(c, a)) return rc;
+    if (nodes) {
+        const size_t n = c->gen_nodes;
+        std::vector<uint32_t> h(3 * n);
+        CU(c, cudaMemcpyAsync(h.data(), a.parent, n * 4, cudaMemcpyDeviceToHost, c->stream_gen));
+        CU(c, cudaMemcpyAsync(h.data() + n, a.individual, n * 4, cudaMemcpyDeviceToHost, c->stream_gen));
+        CU(c, cudaMemcpyAsync(h.data() + 2 * n, a.time, n * 4, cudaMemcpyDeviceToHost, c->stream_gen));
+        CU(c, cudaStreamSynchronize(c->stream_gen));
+        for (size_t k = 0; k < n; k++) nodes[k] = {h[k], h[n + k], h[2 * n + k]};
+    }
+    if (info) {
+        info->generations_total = c->gen_total;
+        info->generations_kept = a.T;
+        info->n_nodes = c->gen_nodes;
+        info->lineages_at_start = c->gen_lineages;
+    }
+    return 0;
+}
+
+int pansim_genealogy_history(pansim_ctx *c, uint32_t *out)
+{
+    if (!c || !out) return PANSIM_ERR_INVALID;
+    if (int rc = genealogy_require(c)) return rc;
+    const uint64_t T = std::min<uint64_t>(c->gen_total, c->gen_cap);
+    const uint64_t base = (c->gen_total - T) % c->gen_cap;
+    const uint64_t first = std::min<uint64_t>(T, c->gen_cap - base);        // oldest vectors up to the end of the ring
+    const size_t row = (size_t)c->N * 4;
+    if (first) CU(c, cudaMemcpyAsync(out, c->d_gen_ring + base * c->N, first * row, cudaMemcpyDeviceToHost, c->stream_gen));
+    if (T > first) CU(c, cudaMemcpyAsync(out + first * c->N, c->d_gen_ring, (T - first) * row, cudaMemcpyDeviceToHost, c->stream_gen));
+    CU(c, cudaStreamSynchronize(c->stream_gen));
+    return 0;
+}
+
+int pansim_genealogy_tmrca(pansim_ctx *c, const uint32_t *r1, const uint32_t *r2, size_t P, uint32_t *tmrca)
+{
+    if (!c || (P && (!r1 || !r2 || !tmrca))) return PANSIM_ERR_INVALID;
+    if (int rc = genealogy_require(c)) return rc;
+    for (size_t k = 0; k < P; k++)
+        if (r1[k] >= c->N || r2[k] >= c->N) FAIL(c, PANSIM_ERR_INVALID, "TMRCA pair %zu = (%u, %u): index >= pop_size %u", k, r1[k], r2[k], c->N);
+    GenealogyTrace a;
+    if (int rc = genealogy_trace(c, a)) return rc;
+    if (P == 0) return 0;
+    if (P > c->gen_pair_cap) {
+        if (c->d_gen_pairs) cudaFree(c->d_gen_pairs);
+        c->d_gen_pairs = nullptr;
+        c->gen_pair_cap = 0;
+        if (cudaMalloc(&c->d_gen_pairs, 3 * P * 4) != cudaSuccess) { cudaGetLastError(); FAIL(c, PANSIM_ERR_NOMEM, "cudaMalloc for %zu TMRCA pairs failed", P); }
+        c->gen_pair_cap = P;
+    }
+    uint32_t *d1 = c->d_gen_pairs, *d2 = d1 + P, *dt = d2 + P;
+    CU(c, cudaMemcpyAsync(d1, r1, P * 4, cudaMemcpyHostToDevice, c->stream_gen));
+    CU(c, cudaMemcpyAsync(d2, r2, P * 4, cudaMemcpyHostToDevice, c->stream_gen));
+    const unsigned grid = (unsigned)std::min<uint64_t>(div_up64(P, 256), (uint64_t)c->sm_count * 16);
+    genealogy_tmrca_kernel<<<grid, 256, 0, c->stream_gen>>>(a.parent, a.time, d1, d2, P, dt);
+    LAUNCH_CHECK(c);
+    CU(c, cudaMemcpyAsync(tmrca, dt, P * 4, cudaMemcpyDeviceToHost, c->stream_gen));
+    CU(c, cudaStreamSynchronize(c->stream_gen));
+    return 0;
+}
+
+// Newick of a node table, no device. A checked table has its root last and every other node's parent above it, so
+// the tree is walked with an explicit stack (no recursion: a caterpillar of any size is fine).
+int pansim_genealogy_newick(const pansim_genealogy_node *nodes, uint32_t n_nodes, uint32_t n_leaves, char *out,
+                            size_t cap, size_t *len)
+{
+    if (!nodes || !len || n_leaves == 0 || n_nodes < n_leaves || (uint64_t)n_nodes > 2ull * n_leaves) return PANSIM_ERR_INVALID;
+    const uint32_t root = n_nodes - 1;
+    if (nodes[root].parent != GEN_NONE) return PANSIM_ERR_INVALID;
+    for (uint32_t k = 0; k < root; k++) {
+        const uint32_t p = nodes[k].parent;
+        if (p <= k || p < n_leaves || p >= n_nodes || nodes[p].time < nodes[k].time) return PANSIM_ERR_INVALID;
+    }
+    // smallest leaf below every node; the children of every node in that order (CSR)
+    std::vector<uint32_t> minleaf(n_nodes, GEN_NONE), first(n_nodes + 1, 0), child(root);
+    for (uint32_t k = 0; k < n_leaves; k++) minleaf[k] = k;
+    for (uint32_t k = 0; k < root; k++) {
+        minleaf[nodes[k].parent] = std::min(minleaf[nodes[k].parent], minleaf[k]);
+        first[nodes[k].parent + 1]++;
+    }
+    for (uint32_t k = 0; k < n_nodes; k++) first[k + 1] += first[k];
+    std::vector<uint32_t> order(root), fill(first.begin(), first.end() - 1);
+    for (uint32_t k = 0; k < root; k++) order[k] = k;
+    std::sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return minleaf[x] != minleaf[y] ? minleaf[x] < minleaf[y] : x < y; });
+    for (uint32_t k : order) child[fill[nodes[k].parent]++] = k;
+    size_t pos = 0;
+    auto put = [&](const char *s, size_t n) {
+        if (out && pos + n <= cap) memcpy(out + pos, s, n);
+        pos += n;
+    };
+    auto put_u = [&](const char *prefix, size_t np, uint32_t v) {
+        char b[24];
+        const int n = snprintf(b, sizeof b, "%u", v);
+        put(prefix, np);
+        put(b, (size_t)n);
+    };
+    auto enter = [&](uint32_t v) {
+        if (v < n_leaves) put_u("ind_", 4, v);
+        else put("(", 1);
+    };
+    struct Frame { uint32_t node, next; };
+    std::vector<Frame> stack{{root, 0}};
+    enter(root);
+    while (!stack.empty()) {
+        const uint32_t v = stack.back().node, i = stack.back().next;
+        if (v >= n_leaves && first[v] + i < first[v + 1]) {
+            if (i) put(",", 1);
+            const uint32_t ch = child[first[v] + i];
+            stack.back().next++;
+            enter(ch);
+            stack.push_back({ch, 0});
+            continue;
+        }
+        if (v >= n_leaves) put(")", 1);
+        if (v != root) put_u(":", 1, nodes[nodes[v].parent].time - nodes[v].time);
+        stack.pop_back();
+    }
+    put(";\n", 2);
+    *len = pos;
+    if (!out) return 0;
+    if (cap < pos + 1) return PANSIM_ERR_INVALID;
+    out[pos] = '\0';
+    return 0;
 }
 
 // ---- communicator over column shards (one process per GPU) -------------------

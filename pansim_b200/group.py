@@ -13,8 +13,8 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import (OK, CoreLD, PansimError, _core_ld, _diversity, _ld_bins, _ld_params, _pairs_or_none, _ptr,
-                         make_config)
+from .population import (OK, CoreLD, Genealogy, PansimError, _core_ld, _diversity, _genealogy, _genealogy_history,
+                         _ld_bins, _ld_params, _pairs_or_none, _ptr, _tmrca, make_config)
 
 
 class PansimGroup:
@@ -148,6 +148,24 @@ class PansimGroup:
         self._check(self._lib.pansim_group_core_ld(self._h, C.byref(_ld_params(max_dist, bin_width, min_minor)), bins,
                                                    C.byref(used)))
         return _core_ld(bins, n, max_dist, bin_width, used.value)
+
+    def enable_genealogy(self, capacity: int):
+        """Pansim.enable_genealogy for the group: shard 0 records (every shard draws the same parents)."""
+        self._check(self._lib.pansim_group_enable_genealogy(self._h, capacity))
+
+    def genealogy(self) -> Genealogy:
+        return _genealogy(lambda nodes, info: self._lib.pansim_group_genealogy(self._h, nodes, info), self._check, self.N)
+
+    def genealogy_history(self) -> np.ndarray:
+        h = self._lib.pansim_group_ctx(self._h, 0)
+
+        def check(rc):
+            if rc != OK:
+                raise PansimError(rc, self._lib.pansim_last_error(h).decode())
+        return _genealogy_history(self._lib, h, check, self.N)
+
+    def tmrca(self, range1, range2) -> np.ndarray:
+        return _tmrca(lambda *a: self._lib.pansim_group_genealogy_tmrca(self._h, *a), self._check, range1, range2)
 
     def gene_counts(self) -> np.ndarray:
         out = np.empty(self.G, np.uint32)

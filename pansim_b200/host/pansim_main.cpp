@@ -44,10 +44,11 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
                              "threads", "genome_size_penalty", "competition_strength", "device", "gpus",
                              "ld_max_dist", "ld_bin_width", "ld_min_minor"};       // extensions: --print_ld bins
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
-                              "all_pairs", "print_diversity", "print_vcf", "print_ld"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
                                                                               // print_vcf (<outpref>_core_genome.vcf),
-                                                                              // print_ld (<outpref>_core_ld.tsv)
+                                                                              // print_ld (<outpref>_core_ld.tsv),
+                                                                              // print_genealogy (<outpref>_genealogy.nwk, <outpref>_tmrca.tsv)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -131,7 +132,7 @@ int main(int argc, char **argv)
     const uint64_t seed = std::strtoull(fl.val["seed"].c_str(), nullptr, 10);
     const bool verbose = fl.sw["verbose"], print_dist = fl.sw["print_dist"], print_matrices = fl.sw["print_matrices"];
     const bool all_pairs = fl.sw["all_pairs"], print_diversity = fl.sw["print_diversity"], print_vcf = fl.sw["print_vcf"];
-    const bool print_ld = fl.sw["print_ld"];
+    const bool print_ld = fl.sw["print_ld"], print_genealogy = fl.sw["print_genealogy"];
     const pansim_ld_params ld_params = {(uint32_t)std::strtoul(fl.val["ld_max_dist"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_bin_width"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_min_minor"].c_str(), nullptr, 10)};
@@ -222,6 +223,7 @@ int main(int argc, char **argv)
         pansim::Populations pops(cfg, n_gpus);
         pops.set_initial(core_row, acc_row);
         pops.set_selection(selection);
+        if (print_genealogy) pops.enable_genealogy((uint32_t)n_gen);       // extension: after set_initial, which clears the record
         std::vector<double> avg_core(n_gen, 0.0), avg_acc(n_gen, 0.0), std_core(n_gen, 0.0), std_acc(n_gen, 0.0);
         std::vector<double> core_d, acc_d;
         std::vector<pansim_diversity> diversity;
@@ -297,6 +299,21 @@ int main(int argc, char **argv)
             for (size_t b = 0; b < bins.size(); b++) {
                 const uint64_t lo = (uint64_t)b * ld_params.bin_width + 1, hi = std::min<uint64_t>(lo + ld_params.bin_width - 1, ld_params.max_dist);
                 f << lo << "\t" << hi << "\t" << bins[b].pairs << "\t" << bins[b].four_gamete << "\t" << fmt(pansim_ld_mean_r2(&bins[b])) << "\n";
+            }
+        }
+        if (print_genealogy) {                                              // extension: the genealogy of the last generation
+            std::ofstream(outpref + "_genealogy.nwk", std::ios::binary) << pops.newick(pops.genealogy());
+            // one TMRCA per line of <outpref>.tsv: the sampled pairs, or every pair i < j in (i, j) order by row blocks
+            std::ofstream f(outpref + "_tmrca.tsv");
+            auto put = [&](const std::vector<uint32_t> &t) { for (uint32_t x : t) f << x << "\n"; };
+            if (!all_pairs) {
+                put(pops.tmrca(range1, range2));
+            } else {
+                std::vector<uint32_t> ii, jj;
+                for (uint32_t i = 0; i + 1 < (uint32_t)pop_size; i++) {
+                    for (uint32_t j = i + 1; j < (uint32_t)pop_size; j++) { ii.push_back(i); jj.push_back(j); }
+                    if (ii.size() >= 4000000 || i + 2 == (uint32_t)pop_size) { put(pops.tmrca(ii, jj)); ii.clear(); jj.clear(); }
+                }
             }
         }
     } catch (const pansim::Error &e) {

@@ -192,6 +192,36 @@ public:
         return bins;
     }
 
+    // (extension) record the parent vector of every generation from now on, the last `capacity` kept (0: off)
+    void enable_genealogy(uint32_t capacity) { gcheck(pansim_group_enable_genealogy(grp_, capacity)); }
+    // (extension) the clonal genealogy of the present population: the node table, and its summary if info is non-null
+    std::vector<pansim_genealogy_node> genealogy(pansim_genealogy_info *info = nullptr)
+    {
+        std::vector<pansim_genealogy_node> nodes(2 * (size_t)cfg_.pop_size);
+        pansim_genealogy_info i;
+        gcheck(pansim_group_genealogy(grp_, nodes.data(), &i));
+        nodes.resize(i.n_nodes);
+        if (info) *info = i;
+        return nodes;
+    }
+    // (extension) TMRCA of each pair (range1[k], range2[k]), in generations
+    std::vector<uint32_t> tmrca(const std::vector<uint32_t> &range1, const std::vector<uint32_t> &range2)
+    {
+        std::vector<uint32_t> out(range1.size());
+        gcheck(pansim_group_genealogy_tmrca(grp_, range1.data(), range2.data(), range1.size(), out.data()));
+        return out;
+    }
+    // (extension) the canonical Newick text of a node table (pansim_genealogy_newick)
+    std::string newick(const std::vector<pansim_genealogy_node> &nodes)
+    {
+        size_t len = 0;
+        check_newick(pansim_genealogy_newick(nodes.data(), (uint32_t)nodes.size(), cfg_.pop_size, nullptr, 0, &len));
+        std::string s(len + 1, '\0');
+        check_newick(pansim_genealogy_newick(nodes.data(), (uint32_t)nodes.size(), cfg_.pop_size, &s[0], s.size(), &len));
+        s.resize(len);
+        return s;
+    }
+
     pansim_ctx *raw() { return ctx_; }          // shard 0 (the whole run when n_gpus() == 1)
     pansim_group *group() { return grp_; }
     const pansim_config &config() const { return cfg_; }
@@ -204,6 +234,10 @@ private:
     void gcheck(int rc)
     {
         if (rc != PANSIM_OK) throw Error(rc, pansim_group_last_error(grp_));
+    }
+    void check_newick(int rc)
+    {
+        if (rc != PANSIM_OK) throw Error(rc, "pansim_genealogy_newick: the node table is not a tree of that shape");
     }
     // host-driven operators work on one context; a sharded run uses the device-resident calls
     void single(const char *what)

@@ -126,6 +126,66 @@ def ld_mean_r2(pairs: int, r2_sum: int) -> float:
     return _ffi.lib().pansim_ld_mean_r2(C.byref(_ffi.LdBin(pairs, 0, r2_sum >> 64, r2_sum & (2 ** 64 - 1))))
 
 
+class Genealogy(NamedTuple):
+    """The clonal genealogy of the present population (pansim_genealogy, include/pansim_b200.h): per node its parent
+    (0xFFFFFFFF at the root), the individual it stands for (0xFFFFFFFF at a virtual root) and its time in generations
+    before the present; leaves are nodes 0 .. n_leaves-1. generations_total vectors were recorded since the last
+    reset, generations_kept of them are traced; lineages_at_start = 1 means the MRCA was found."""
+    parent: np.ndarray
+    individual: np.ndarray
+    time: np.ndarray
+    generations_total: int
+    generations_kept: int
+    n_nodes: int
+    lineages_at_start: int
+    n_leaves: int
+
+    def newick(self) -> str:
+        """The canonical Newick text (leaves `ind_<i>`, integer branch lengths), formatted by the library."""
+        return genealogy_newick(self.parent, self.individual, self.time, self.n_leaves)
+
+
+def genealogy_newick(parent, individual, time, n_leaves: int) -> str:
+    """pansim_genealogy_newick of a node table given as three arrays (no device)."""
+    lib = _ffi.lib()
+    table = np.ascontiguousarray(np.stack([np.asarray(parent), np.asarray(individual), np.asarray(time)], axis=1), np.uint32)
+    n = C.c_size_t(0)
+    rc = lib.pansim_genealogy_newick(_ptr(table), len(table), n_leaves, None, 0, C.byref(n))
+    if rc != OK:
+        raise PansimError(rc, "pansim_genealogy_newick: not a tree of that shape")
+    buf = C.create_string_buffer(n.value + 1)
+    rc = lib.pansim_genealogy_newick(_ptr(table), len(table), n_leaves, buf, n.value + 1, C.byref(n))
+    if rc != OK:
+        raise PansimError(rc, "pansim_genealogy_newick failed")
+    return buf.raw[:n.value].decode()
+
+
+def _genealogy(call, check, N: int) -> Genealogy:
+    nodes = np.empty((2 * N, 3), np.uint32)
+    info = _ffi.GenealogyInfo()
+    check(call(_ptr(nodes), C.byref(info)))
+    t = nodes[:info.n_nodes]
+    return Genealogy(t[:, 0].copy(), t[:, 1].copy(), t[:, 2].copy(), info.generations_total, info.generations_kept,
+                     info.n_nodes, info.lineages_at_start, N)
+
+
+def _genealogy_history(lib, h, check, N: int) -> np.ndarray:
+    info = _ffi.GenealogyInfo()
+    check(lib.pansim_genealogy(h, None, C.byref(info)))
+    out = np.empty((info.generations_kept, N), np.uint32)
+    check(lib.pansim_genealogy_history(h, _ptr(out)))
+    return out
+
+
+def _tmrca(call, check, range1, range2) -> np.ndarray:
+    r1 = np.ascontiguousarray(range1, np.uint32)
+    r2 = np.ascontiguousarray(range2, np.uint32)
+    assert r1.shape == r2.shape
+    out = np.empty(len(r1), np.uint32)
+    check(call(_ptr(r1), _ptr(r2), len(r1), _ptr(out)))
+    return out
+
+
 def _pairs_or_none(range1, range2):
     if range1 is None:
         return None, None, 0
@@ -424,6 +484,24 @@ class Pansim:
                                                        C.byref(s), C.byref(t), C.byref(q), C.byref(n)))
         return s.value, t.value, q.value, n.value
 
+    # -- clonal genealogy (extension) ---------------------------------------
+    def enable_genealogy(self, capacity: int):
+        """Record the parent vector of every generation from now on, keeping the last `capacity` (0: stop and free)."""
+        self._check(self._lib.pansim_enable_genealogy(self._h, capacity))
+
+    def genealogy(self) -> Genealogy:
+        """The genealogy of the present population traced on the device from the record."""
+        return _genealogy(lambda nodes, info: self._lib.pansim_genealogy(self._h, nodes, info), self._check, self.N)
+
+    def genealogy_history(self) -> np.ndarray:
+        """The record itself: uint32 [kept, N], oldest generation first; row t maps child -> parent index."""
+        return _genealogy_history(self._lib, self._h, self._check, self.N)
+
+    def tmrca(self, range1, range2) -> np.ndarray:
+        """Time to the most recent common ancestor of each pair (generations; the kept generations when the pair has
+        not coalesced within the record)."""
+        return _tmrca(lambda *a: self._lib.pansim_genealogy_tmrca(self._h, *a), self._check, range1, range2)
+
     # -- multi-GPU: communicator over column shards (one process per GPU) --
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -565,4 +643,5 @@ class Pansim:
                 f.write(",".join(ones + [str(int(x)) for x in acc[r]]) + "\n")
 
 
-__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "make_config", "standard_deviation", "fmt_f64"]
+__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "Genealogy", "genealogy_newick",
+           "make_config", "standard_deviation", "fmt_f64"]

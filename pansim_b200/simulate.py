@@ -62,13 +62,15 @@ class RunResult:
     diversity: list = field(default_factory=list) # per generation: Diversity (--print_diversity)
     sfs: np.ndarray = None                        # SFS of the last generation (--print_diversity)
     ld: object = None                             # CoreLD of the last generation (--print_ld)
+    genealogy: object = None                      # Genealogy of the last generation (--print_genealogy)
+    tmrca: np.ndarray = None                      # TMRCA of the sampled pairs (--print_genealogy without --all_pairs)
     selection: np.ndarray = None
     stdout: list = field(default_factory=list)
 
 
 def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False,
         print_diversity: bool = False, print_vcf: bool = False, print_ld: bool = False, ld_max_dist: int = 10000,
-        ld_bin_width: int = 100, ld_min_minor: int = 1) -> RunResult | None:
+        ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -79,7 +81,10 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     after the other outputs (Pansim.write_core_vcf).
     print_ld (extension): linkage disequilibrium of the core alignment of the last generation as
     `<outpref>_core_ld.tsv`, written after the other outputs (Pansim.core_ld with ld_max_dist, ld_bin_width,
-    ld_min_minor; write_core_ld)."""
+    ld_min_minor; write_core_ld).
+    print_genealogy (extension): the parents of every generation are recorded on the device from generation 0;
+    after the other outputs the genealogy of the last generation goes to `<outpref>_genealogy.nwk` and the TMRCA of
+    the pair on each line of `<outpref>.tsv` to `<outpref>_tmrca.tsv` (write_genealogy)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -104,6 +109,8 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     with Pansim.from_params(p, device=device) as sim:
         sim.set_initial(core_row, acc_row)
         sim.set_selection(sel)
+        if print_genealogy:
+            sim.enable_genealogy(p.n_gen)                                        # after set_initial, which clears the record
         def last_generation_outputs():                                           # main.rs:467-499
             if not all_pairs:
                 res.core_distances, res.acc_distances = sim.pairwise_distances(r1, r2)
@@ -175,7 +182,29 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             res.ld = sim.core_ld(ld_max_dist, ld_bin_width, ld_min_minor)
             if outpref:
                 write_core_ld(outpref, res.ld)
+        if print_genealogy:
+            res.genealogy = sim.genealogy()
+            if not all_pairs:
+                res.tmrca = sim.tmrca(r1, r2)
+            if outpref:
+                write_genealogy(outpref, sim, res.genealogy, None if all_pairs else res.tmrca)
     return res
+
+
+def write_genealogy(outpref: str, sim, genealogy, tmrca):
+    """`<outpref>_genealogy.nwk`: the Newick text; `<outpref>_tmrca.tsv`: one integer per line, the TMRCA of the
+    pair on the same line of `<outpref>.tsv` (tmrca = None: every pair i < j in (i, j) order, by row blocks)."""
+    with open(outpref + "_genealogy.nwk", "w") as f:
+        f.write(genealogy.newick())
+    with open(outpref + "_tmrca.tsv", "w") as f:
+        if tmrca is not None:
+            f.write("".join(f"{int(x)}\n" for x in tmrca))
+            return
+        N = sim.N
+        for i0, i1 in sim.row_blocks():
+            ii = np.repeat(np.arange(i0, i1, dtype=np.uint32), [N - 1 - i for i in range(i0, i1)])
+            jj = np.concatenate([np.arange(i + 1, N, dtype=np.uint32) for i in range(i0, i1)])
+            f.write("".join(f"{int(x)}\n" for x in sim.tmrca(ii, jj)))
 
 
 def write_core_ld(outpref: str, ld):
