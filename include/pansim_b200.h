@@ -267,6 +267,37 @@ int pansim_write_core_vcf(pansim_ctx *ctx, const char *path, int with_header, ui
  * pass (CUDA events) and the bytes of text (header excluded) */
 int pansim_core_vcf_kernel_ms(pansim_ctx *ctx, uint32_t repeats, float *site_ms, float *expand_ms, uint64_t *text_bytes);
 
+/* ---- core-genome FASTA alignment (extension: the reference writes the alignment only as _core_genome.csv) ----
+ * The alignment as FASTA text for phylogenetic and clustering tools (IQ-TREE, RAxML-NG, FastTree, Gubbins,
+ * snp-dists), expanded on the device and streamed to the file through the pinned double-buffered pipeline of
+ * pansim_write_core_csv (DESIGN.md section 14).
+ *   Whole mode (snps_only = 0): every site of the alignment is a column, in position order.
+ *   SNP mode (snps_only != 0): a column is a site where at least two letters are present among the N rows; the
+ *     number of columns equals pansim_diversity.segregating. A site fixed for a non-ancestral letter is not a
+ *     column. This is the column selection snp-sites makes on a gap-free alignment; it is not the VCF's rule
+ *     (pansim_write_core_vcf writes every site that differs from the ancestral row, fixed ones included).
+ *   Constant-site counts: const_counts[4] holds, for the sites that are not columns, the number whose letter is
+ *     A, C, G and T (in whole mode all four are 0). const_counts summed plus the number of columns equals the
+ *     context's sites; in SNP mode they are what IQ-TREE's -fconst a,c,g,t takes.
+ *   Bytes: for each row i = 0 .. N-1 in order, one record: ">ind_<i>\n" (the VCF sample names and the Newick leaf
+ *     names of the genealogy), the row's letters of the columns (uppercase ACGT, one line, no wrapping), "\n". A
+ *     record is 7 + digits(i) + columns bytes; record i starts at byte i (7 + columns) + sum over j < i of digits(j).
+ *     With zero columns each record is ">ind_<i>\n\n".
+ * The state is read after recombine(), like every reader. The calls need a state (pansim_set_initial or an upload;
+ * otherwise PANSIM_ERR_STATE) but not the ancestral row. A path that cannot be created, or a failed or short write,
+ * gives PANSIM_ERR_INVALID. The context keeps working after a refused call. columns_out, const_counts (4 values) and
+ * bytes_out may be NULL. */
+int pansim_write_core_fasta(pansim_ctx *ctx, const char *path, int snps_only, uint64_t *columns_out, uint64_t *const_counts /* [4] or NULL */, uint64_t *bytes_out);
+/* The letters of rows [row_begin, row_end): `columns` bytes per row, rows back to back, no headers or separators;
+ * *columns_out = the context's columns. out = NULL: only *columns_out. A range past N -> PANSIM_ERR_INVALID. On a
+ * column shard the columns are the shard's own: polymorphism is decided per column, so the shards' letters of a row,
+ * concatenated in shard order, are the whole row's letters, and their column and constant-site counts sum. */
+int pansim_export_core_fasta_rows(pansim_ctx *ctx, int snps_only, uint32_t row_begin, uint32_t row_end, char *out, uint64_t *columns_out);
+/* measurement: the site pass (SNP mode: allele counts, polymorphic sites, scan, column list; whole mode: nothing)
+ * and the expansion of every chunk of records into device memory, each `repeats` times after a warm-up, with no
+ * copy to the host; mean device ms of one pass (CUDA events) and the bytes of the file */
+int pansim_core_fasta_kernel_ms(pansim_ctx *ctx, int snps_only, uint32_t repeats, float *site_ms, float *expand_ms, uint64_t *text_bytes);
+
 /* ---- core-genome linkage disequilibrium (extension: the reference has no two-site statistic) ----
  * r^2 and four-gamete pairs binned by the distance between two sites, the joint counts of the site pairs formed
  * on the tensor cores (DESIGN.md section 12). The state is read after recombine(), like every reader.
@@ -422,6 +453,9 @@ int pansim_group_download_core(pansim_group *g, uint8_t *core_onehot_out);      
 int pansim_group_export_core_csv(pansim_group *g, uint32_t row_begin, uint32_t row_end, char *out);
 /* the whole-alignment VCF of pansim_write_core_vcf: the header once, then every shard's lines in shard order */
 int pansim_group_write_core_vcf(pansim_group *g, const char *path, uint64_t *bytes_out);
+/* the whole-alignment FASTA of pansim_write_core_fasta, by row blocks: every shard's letters, the records written
+ * on the host; columns and constant-site counts are the sums over the shards */
+int pansim_group_write_core_fasta(pansim_group *g, const char *path, int snps_only, uint64_t *columns_out, uint64_t *const_counts, uint64_t *bytes_out);
 
 /* pansim_core_ld over the whole alignment: every shard with the next one as its halo, summed on the host */
 int pansim_group_core_ld(pansim_group *g, const pansim_ld_params *p, pansim_ld_bin *bins, uint64_t *sites_used);

@@ -5,7 +5,7 @@ same parsing quirks: pop_size/core_size/pan_genes/core_genes/n_gen are parsed as
 f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
 accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
---print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy.
+--print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy, --print_fasta, --print_snp_alignment.
 """
 from __future__ import annotations
 
@@ -74,6 +74,13 @@ def build_parser() -> argparse.ArgumentParser:
                     help="(extension) record the parents of every generation; <outpref>_genealogy.nwk: the clonal genealogy of "
                          "the last generation as Newick (leaves ind_<i>, branch lengths in generations); <outpref>_tmrca.tsv: "
                          "the TMRCA of the pair on each line of <outpref>.tsv")
+    ap.add_argument("--print_fasta", action="store_true",
+                    help="(extension) <outpref>_core_genome.fasta: the core alignment of the last generation as FASTA, one "
+                         "record ind_<i> per individual, every site")
+    ap.add_argument("--print_snp_alignment", action="store_true",
+                    help="(extension) <outpref>_core_snps.fasta: the same records with only the sites where two or more "
+                         "letters are present; <outpref>_core_snps_fconst.txt: the constant sites by letter, nA,nC,nG,nT "
+                         "(IQ-TREE -fconst)")
     return ap
 
 
@@ -84,10 +91,12 @@ def main(argv=None) -> int:
     print_diversity = ns.pop("print_diversity")
     print_vcf = ns.pop("print_vcf")
     print_genealogy = ns.pop("print_genealogy")
+    print_fasta = ns.pop("print_fasta")
+    print_snp_alignment = ns.pop("print_snp_alignment")
     ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
     p = Params(**ns)
     run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf,
-        print_genealogy=print_genealogy, **ld)
+        print_genealogy=print_genealogy, print_fasta=print_fasta, print_snp_alignment=print_snp_alignment, **ld)
     return 0                       # the reference exits 0 even when validation fails (main.rs:195-247)
 
 

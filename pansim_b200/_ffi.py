@@ -33,6 +33,7 @@ EXPORTED = [
     "pansim_core_allele_counts", "pansim_core_diversity", "pansim_run_generations_diversity", "pansim_diversity_stats",
     "pansim_group_core_diversity", "pansim_group_run_generations_diversity",
     "pansim_write_core_vcf", "pansim_group_write_core_vcf", "pansim_core_vcf_kernel_ms",
+    "pansim_write_core_fasta", "pansim_export_core_fasta_rows", "pansim_group_write_core_fasta", "pansim_core_fasta_kernel_ms",
     "pansim_core_ld", "pansim_group_core_ld", "pansim_core_ld_kernel_ms", "pansim_ld_mean_r2",
     "pansim_enable_genealogy", "pansim_genealogy", "pansim_genealogy_history", "pansim_genealogy_tmrca",
     "pansim_genealogy_newick", "pansim_group_enable_genealogy", "pansim_group_genealogy", "pansim_group_genealogy_tmrca",
@@ -225,6 +226,10 @@ def lib():
     sig("pansim_write_core_vcf", cint, vp, C.c_char_p, cint, C.POINTER(C.c_uint64))
     sig("pansim_group_write_core_vcf", cint, vp, C.c_char_p, C.POINTER(C.c_uint64))
     sig("pansim_core_vcf_kernel_ms", cint, vp, u32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint64))
+    sig("pansim_write_core_fasta", cint, vp, C.c_char_p, cint, C.POINTER(C.c_uint64), vp, C.POINTER(C.c_uint64))
+    sig("pansim_export_core_fasta_rows", cint, vp, cint, u32, u32, vp, C.POINTER(C.c_uint64))
+    sig("pansim_group_write_core_fasta", cint, vp, C.c_char_p, cint, C.POINTER(C.c_uint64), vp, C.POINTER(C.c_uint64))
+    sig("pansim_core_fasta_kernel_ms", cint, vp, cint, u32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint64))
     sig("pansim_core_ld", cint, vp, vp, C.POINTER(LdParams), C.POINTER(LdBin), C.POINTER(C.c_uint64))
     sig("pansim_group_core_ld", cint, vp, C.POINTER(LdParams), C.POINTER(LdBin), C.POINTER(C.c_uint64))
     sig("pansim_core_ld_kernel_ms", cint, vp, C.POINTER(LdParams), u32, C.POINTER(C.c_float), C.POINTER(C.c_float),

@@ -27,6 +27,7 @@
 #include "replay.cuh"
 #include "select.cuh"
 #include "vcf.cuh"
+#include "fasta.cuh"
 
 using namespace pansim;
 
@@ -265,11 +266,16 @@ struct pansim_ctx {
     char *d_txt[2] = {nullptr, nullptr}, *h_txt[2] = {nullptr, nullptr};
     cudaEvent_t ev_txt[2] = {nullptr, nullptr};
     size_t txt_cap = 0;
-    // VCF export (vcf.cuh): per-site allele counts, line descriptors and offsets, scan blocks, chunk bounds
+    // VCF export (vcf.cuh): per-site allele counts (shared with the FASTA export), line descriptors and offsets,
+    // scan blocks, chunk bounds
     uint4 *d_vcf_counts = nullptr;
     uint8_t *d_vcf_desc = nullptr;
     unsigned long long *d_vcf_off = nullptr, *d_vcf_block = nullptr, *d_vcf_bounds = nullptr;
     uint32_t *d_vcf_nchunks = nullptr;
+    // FASTA export (fasta.cuh), SNP mode: polymorphic sites per scan block (+ total), constant-site letters, the
+    // column list; pinned read-back of the column count and the constant-site letters
+    unsigned long long *d_fa_block = nullptr, *d_fa_const = nullptr, *h_fa = nullptr;
+    uint32_t *d_fa_cols = nullptr;
     // core LD (ld.cuh): allele counts, used-site ranks, the compacted used sites (position, derived count, 1 / (a (n - a)))
     // and their site-major derived bit rows. `ld` holds the context's own used sites followed by the halo copied from
     // the next shard; `ld_halo` is the halo this context makes of its first sites when it is the next of another one.
@@ -1137,7 +1143,8 @@ void pansim_destroy(pansim_ctx *c)
                     c->d_planes, c->d_work_counter, c->d_replay, c->d_hkeys, c->d_hvals, c->d_stage, c->d_groups, c->d_partner, c->d_orig, c->d_batches, c->d_tile_slots, c->d_tile_orig, c->d_dump_counters, c->d_mut_row, c->d_mut_site,
                     c->d_mut_seq, c->d_mut_allele, c->d_hr_rec, c->d_hr_locus, c->d_hr_donor, c->d_hr_seq,
                     c->d_hr_value, c->d_dump_flip, c->d_dump_gain, c->d_anc, c->d_div, c->d_sfs,
-                    c->d_vcf_counts, c->d_vcf_desc, c->d_vcf_off, c->d_vcf_block, c->d_vcf_bounds, c->d_vcf_nchunks};
+                    c->d_vcf_counts, c->d_vcf_desc, c->d_vcf_off, c->d_vcf_block, c->d_vcf_bounds, c->d_vcf_nchunks,
+                    c->d_fa_block, c->d_fa_const, c->d_fa_cols};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (auto *b : {&c->ld, &c->ld_halo}) {
@@ -1148,6 +1155,7 @@ void pansim_destroy(pansim_ctx *c)
     if (c->d_ld_tiles) cudaFree(c->d_ld_tiles);
     if (c->d_ld_bins) cudaFree(c->d_ld_bins);
     if (c->h_ld) cudaFreeHost(c->h_ld);
+    if (c->h_fa) cudaFreeHost(c->h_fa);
     if (c->h_ld_bins) cudaFreeHost(c->h_ld_bins);
     if (c->ev_ld) cudaEventDestroy(c->ev_ld);
     if (c->stream_gen) { cudaStreamSynchronize(c->stream_gen); cudaStreamDestroy(c->stream_gen); }
@@ -2844,11 +2852,27 @@ void pansim_diversity_stats(const pansim_diversity *d, uint32_t pop_size, double
 // ---- core-genome VCF (vcf.cuh) ----------------------------------------------------------------
 constexpr unsigned long long VCF_CHUNK_BYTES = 32ull << 20;     // text per chunk (one line where a line is longer)
 
+// *slot = bytes of device memory unless already allocated; a failed allocation leaves *slot null
+static int alloc_once(pansim_ctx *c, void **slot, size_t bytes)
+{
+    if (*slot) return 0;
+    void *p = nullptr;
+    CU(c, cudaMalloc(&p, bytes));
+    *slot = p;
+    return 0;
+}
+
+// the per-site allele counts of the VCF and FASTA site passes (one buffer: each pass fills it before it reads it)
+static int ensure_site_counts(pansim_ctx *c)
+{
+    return alloc_once(c, reinterpret_cast<void **>(&c->d_vcf_counts), (size_t)c->Ll * sizeof(uint4));
+}
+
 static int ensure_vcf(pansim_ctx *c)
 {
+    if (int rc = ensure_site_counts(c)) return rc;
     if (c->d_vcf_nchunks) return 0;
     const size_t blocks = div_up64(c->Ll, VS_SITES);
-    CU(c, cudaMalloc(&c->d_vcf_counts, (size_t)c->Ll * sizeof(uint4)));
     CU(c, cudaMalloc(&c->d_vcf_desc, blocks * VS_SITES));
     CU(c, cudaMalloc(&c->d_vcf_off, ((size_t)c->Ll + 1) * sizeof(unsigned long long)));
     CU(c, cudaMalloc(&c->d_vcf_block, blocks * sizeof(unsigned long long)));
@@ -3016,6 +3040,202 @@ int pansim_core_vcf_kernel_ms(pansim_ctx *c, uint32_t repeats, float *site_ms, f
     if (site_ms) *site_ms = t0 / (float)repeats;
     if (expand_ms) *expand_ms = t1 / (float)repeats;
     if (text_bytes) *text_bytes = bd.back();
+    return 0;
+}
+
+// ---- core-genome FASTA (fasta.cuh) ------------------------------------------------------------
+constexpr uint64_t FASTA_CHUNK_BYTES = 32ull << 20;   // text per chunk: whole records (one record where a record is longer)
+
+// every buffer is allocated on its own when missing, so a failed allocation leaves nothing to leak on the next call
+static int ensure_fasta(pansim_ctx *c)
+{
+    if (int rc = ensure_site_counts(c)) return rc;
+    const size_t blocks = div_up64(c->Ll, VS_SITES);
+    if (int rc = alloc_once(c, reinterpret_cast<void **>(&c->d_fa_block), (blocks + 1) * sizeof(unsigned long long))) return rc;
+    if (int rc = alloc_once(c, reinterpret_cast<void **>(&c->d_fa_const), 4 * sizeof(unsigned long long))) return rc;
+    if (int rc = alloc_once(c, reinterpret_cast<void **>(&c->d_fa_cols), (size_t)c->Ll * sizeof(uint32_t))) return rc;
+    if (!c->h_fa) {
+        void *p = nullptr;
+        CU(c, cudaMallocHost(&p, 5 * sizeof(unsigned long long)));
+        c->h_fa = static_cast<unsigned long long *>(p);
+    }
+    return 0;
+}
+
+// the SNP-mode site pass on c->stream over materialised rows: allele counts (the counts instance of the diversity
+// reduction), polymorphic sites and constant-site letters per block, the scan of the blocks and the column list
+static int fasta_site_pass(pansim_ctx *c)
+{
+    CU(c, cudaMemsetAsync(c->d_div, 0, 4 * sizeof(unsigned long long), c->stream));
+    CU(c, cudaMemsetAsync(c->d_fa_const, 0, 4 * sizeof(unsigned long long), c->stream));
+    if (int rc = launch_diversity(c, c->stream, c->d_div, c->d_vcf_counts, nullptr)) return rc;
+    FastaSiteArgs a;
+    a.counts = c->d_vcf_counts;
+    a.n_sites = c->Ll;
+    a.block = c->d_fa_block;
+    a.consts = c->d_fa_const;
+    a.cols = c->d_fa_cols;
+    const uint32_t blocks = div_up64(c->Ll, VS_SITES);
+    fasta_site_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    vcf_scan_blocks_kernel<<<1, VS_SCAN_THREADS, 0, c->stream>>>(a.block, blocks, a.block + blocks);
+    LAUNCH_CHECK(c);
+    fasta_compact_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// Materialise the rows and, in SNP mode, enqueue the site pass and the read-back of the column count and the
+// constant-site letters into h_fa, without waiting for them (the group enqueues on every shard first). Whole mode
+// needs no pass: every local site is a column.
+static int fasta_enqueue(pansim_ctx *c, bool snps)
+{
+    if (int rc = require_state(c)) return rc;
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (c->Ll == 0) return 0;
+    c->ps = c->stream;
+    if (int rc = core_materialize(c, c->stream)) return rc;
+    if (int rc = check_hr_flag(c)) return rc;
+    if (!snps) return 0;
+    if (int rc = ensure_div(c, 1, false)) return rc;
+    if (int rc = ensure_fasta(c)) return rc;
+    if (int rc = fasta_site_pass(c)) return rc;
+    CU(c, cudaMemcpyAsync(c->h_fa, c->d_fa_block + div_up64(c->Ll, VS_SITES), sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(c->h_fa + 1, c->d_fa_const, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+}
+
+// the column count and constant-site letters of fasta_enqueue, once it has finished
+static int fasta_columns(pansim_ctx *c, bool snps, uint64_t *cols, uint64_t consts[4])
+{
+    for (int k = 0; k < 4; k++) consts[k] = 0;
+    *cols = snps ? 0 : c->Ll;
+    if (!snps || c->Ll == 0) return 0;
+    CU(c, cudaSetDevice(c->cfg.device));
+    CU(c, cudaStreamSynchronize(c->stream));
+    *cols = c->h_fa[0];
+    for (int k = 0; k < 4; k++) consts[k] = c->h_fa[1 + k];
+    return 0;
+}
+
+// rows [r0, r1) with `cols` columns into dst on c->stream: whole records when framed, the letters only otherwise
+static int launch_fasta_expand(pansim_ctx *c, bool snps, uint64_t cols, uint32_t r0, uint32_t r1, bool framed, char *dst)
+{
+    if (r0 == r1 || (!framed && cols == 0)) return 0;
+    FastaExpandArgs a;
+    a.state = reinterpret_cast<const uint32_t *>(c->core[c->core_cur]);
+    a.row_words = c->core_stride / 4;
+    a.cols = snps ? c->d_fa_cols : nullptr;
+    a.n_cols = cols;
+    a.row0 = r0;
+    a.row1 = r1;
+    a.framed = framed ? 1u : 0u;
+    a.out = dst;
+    const dim3 grid(std::max<uint32_t>(1, div_up64(cols, FX_COLS)), div_up64(r1 - r0, FX_ROWS));
+    fasta_expand_kernel<<<grid, FX_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// rows per chunk of at most FASTA_CHUNK_BYTES when a row takes at most row_bytes (at least one row)
+static uint32_t fasta_rows_per_chunk(uint64_t row_bytes, uint32_t n_rows)
+{
+    return (uint32_t)std::min<uint64_t>(std::max<uint32_t>(1, n_rows), std::max<uint64_t>(1, FASTA_CHUNK_BYTES / std::max<uint64_t>(1, row_bytes)));
+}
+
+// the largest record of rows below n_rows
+static uint64_t fasta_max_record(uint32_t n_rows, uint64_t cols) { return 7 + vcf_digits(n_rows ? n_rows - 1 : 0) + cols; }
+
+// rows [row_begin, row_end) streamed to sink in chunks of whole records (framed) or of letter rows
+extern "C++" {
+template <typename Sink>
+static int fasta_stream(pansim_ctx *c, bool snps, uint64_t cols, uint32_t row_begin, uint32_t row_end, bool framed, Sink &&sink)
+{
+    const uint64_t row_bytes = framed ? fasta_max_record(row_end, cols) : cols;
+    if (row_begin == row_end || row_bytes == 0) return 0;
+    const uint32_t rows_per = fasta_rows_per_chunk(row_bytes, row_end - row_begin);
+    const size_t n_chunks = div_up64(row_end - row_begin, rows_per);
+    return stream_text_chunks(c, n_chunks, (size_t)rows_per * row_bytes, "FASTA", [&](size_t k, char *dst, size_t *bytes) -> int {
+        const uint32_t r0 = row_begin + (uint32_t)k * rows_per, r1 = std::min(row_end, r0 + rows_per);
+        *bytes = framed ? fasta_record_offset(r1, cols) - fasta_record_offset(r0, cols) : (uint64_t)(r1 - r0) * cols;
+        return launch_fasta_expand(c, snps, cols, r0, r1, framed, dst);
+    }, sink);
+}
+}  // extern "C++"
+
+int pansim_write_core_fasta(pansim_ctx *c, const char *path, int snps_only, uint64_t *columns_out, uint64_t *const_counts,
+                            uint64_t *bytes_out)
+{
+    if (!c || !path) return PANSIM_ERR_INVALID;
+    if (int rc = require_state(c)) return rc;
+    const bool snps = snps_only != 0;
+    FILE *f = fopen(path, "wb");
+    if (!f) FAIL(c, PANSIM_ERR_INVALID, "cannot create %s", path);
+    uint64_t total = 0, cols = 0, consts[4];
+    int rc = fasta_enqueue(c, snps);
+    if (!rc) rc = fasta_columns(c, snps, &cols, consts);
+    if (!rc) rc = fasta_stream(c, snps, cols, 0, c->N, true, [&](const char *p, size_t n) { total += n; return fwrite(p, 1, n, f) == n ? 0 : 1; });
+    const int rc2 = fclose(f);
+    if (bytes_out) *bytes_out = total;
+    if (rc) return rc;
+    if (rc2) FAIL(c, PANSIM_ERR_INVALID, "closing %s failed", path);
+    if (columns_out) *columns_out = cols;
+    if (const_counts) memcpy(const_counts, consts, sizeof consts);
+    return 0;
+}
+
+int pansim_export_core_fasta_rows(pansim_ctx *c, int snps_only, uint32_t row_begin, uint32_t row_end, char *out, uint64_t *columns_out)
+{
+    if (!c) return PANSIM_ERR_INVALID;
+    if (row_begin > row_end || row_end > c->N) FAIL(c, PANSIM_ERR_INVALID, "rows [%u, %u) out of range", row_begin, row_end);
+    const bool snps = snps_only != 0;
+    uint64_t cols = 0, consts[4];
+    if (int rc = fasta_enqueue(c, snps)) return rc;
+    if (int rc = fasta_columns(c, snps, &cols, consts)) return rc;
+    if (columns_out) *columns_out = cols;
+    if (!out) return 0;
+    char *dst = out;
+    return fasta_stream(c, snps, cols, row_begin, row_end, false, [&](const char *p, size_t n) { memcpy(dst, p, n); dst += n; return 0; });
+}
+
+int pansim_core_fasta_kernel_ms(pansim_ctx *c, int snps_only, uint32_t repeats, float *site_ms, float *expand_ms, uint64_t *text_bytes)
+{
+    if (!c || !repeats) return PANSIM_ERR_INVALID;
+    const bool snps = snps_only != 0;
+    uint64_t cols = 0, consts[4];
+    if (int rc = fasta_enqueue(c, snps)) return rc;                 // also the warm-up of the site pass
+    if (int rc = fasta_columns(c, snps, &cols, consts)) return rc;
+    if (c->Ll == 0) FAIL(c, PANSIM_ERR_INVALID, "no core sites on this context");
+    const uint64_t row_bytes = fasta_max_record(c->N, cols);
+    const uint32_t rows_per = fasta_rows_per_chunk(row_bytes, c->N);
+    const size_t n_chunks = div_up64(c->N, rows_per);
+    if (int rc = ensure_txt_staging(c, (size_t)rows_per * row_bytes, "FASTA")) return rc;
+    auto expand_all = [&]() -> int {
+        for (size_t k = 0; k < n_chunks; k++) {
+            const uint32_t r0 = (uint32_t)k * rows_per, r1 = std::min(c->N, r0 + rows_per);
+            if (int rc = launch_fasta_expand(c, snps, cols, r0, r1, true, c->d_txt[k & 1])) return rc;
+        }
+        return 0;
+    };
+    if (int rc = expand_all()) return rc;                           // warm-up of the expansion
+    cudaEvent_t ev[3];
+    for (auto &e : ev) CU(c, cudaEventCreate(&e));
+    int rc = 0;
+    cudaEventRecord(ev[0], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc && snps; r++) rc = fasta_site_pass(c);
+    cudaEventRecord(ev[1], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++) rc = expand_all();
+    cudaEventRecord(ev[2], c->stream);
+    const cudaError_t e = cudaEventSynchronize(ev[2]);
+    float t0 = 0.f, t1 = 0.f;
+    cudaEventElapsedTime(&t0, ev[0], ev[1]);
+    cudaEventElapsedTime(&t1, ev[1], ev[2]);
+    for (auto &x : ev) cudaEventDestroy(x);
+    if (rc) return rc;
+    if (e != cudaSuccess) FAIL(c, PANSIM_ERR_CUDA, "FASTA kernels failed: %s", cudaGetErrorString(e));
+    if (site_ms) *site_ms = t0 / (float)repeats;
+    if (expand_ms) *expand_ms = t1 / (float)repeats;
+    if (text_bytes) *text_bytes = fasta_record_offset(c->N, cols);
     return 0;
 }
 

@@ -13,8 +13,8 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import (OK, CoreLD, Genealogy, PansimError, _core_ld, _diversity, _genealogy, _genealogy_history,
-                         _ld_bins, _ld_params, _pairs_or_none, _ptr, _tmrca, make_config)
+from .population import (OK, CoreFasta, CoreLD, Genealogy, PansimError, _core_ld, _diversity, _genealogy, _genealogy_history,
+                         _ld_bins, _ld_params, _pairs_or_none, _ptr, _tmrca, _write_fasta, make_config)
 
 
 class PansimGroup:
@@ -187,6 +187,11 @@ class PansimGroup:
         n = C.c_uint64(0)
         self._check(self._lib.pansim_group_write_core_vcf(self._h, path.encode(), C.byref(n)))
         return n.value
+
+    def write_core_fasta(self, path: str, snps_only: bool = False) -> CoreFasta:
+        """The whole-alignment FASTA (Pansim.write_core_fasta): the shards' letters of every row in shard order; the
+        columns and constant-site counts are summed over the shards."""
+        return _write_fasta(lambda *a: self._lib.pansim_group_write_core_fasta(self._h, *a), self._check, path, snps_only)
 
     def export_core_csv(self, row_begin: int, row_end: int) -> bytes:
         out = np.empty((row_end - row_begin) * 2 * self.L, np.uint8)

@@ -44,11 +44,14 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
                              "threads", "genome_size_penalty", "competition_strength", "device", "gpus",
                              "ld_max_dist", "ld_bin_width", "ld_min_minor"};       // extensions: --print_ld bins
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
-                              "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy",
+                              "print_fasta", "print_snp_alignment"};          // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
                                                                               // print_vcf (<outpref>_core_genome.vcf),
                                                                               // print_ld (<outpref>_core_ld.tsv),
-                                                                              // print_genealogy (<outpref>_genealogy.nwk, <outpref>_tmrca.tsv)
+                                                                              // print_genealogy (<outpref>_genealogy.nwk, <outpref>_tmrca.tsv),
+                                                                              // print_fasta (<outpref>_core_genome.fasta),
+                                                                              // print_snp_alignment (<outpref>_core_snps.fasta, <outpref>_core_snps_fconst.txt)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -133,6 +136,7 @@ int main(int argc, char **argv)
     const bool verbose = fl.sw["verbose"], print_dist = fl.sw["print_dist"], print_matrices = fl.sw["print_matrices"];
     const bool all_pairs = fl.sw["all_pairs"], print_diversity = fl.sw["print_diversity"], print_vcf = fl.sw["print_vcf"];
     const bool print_ld = fl.sw["print_ld"], print_genealogy = fl.sw["print_genealogy"];
+    const bool print_fasta = fl.sw["print_fasta"], print_snp_alignment = fl.sw["print_snp_alignment"];
     const pansim_ld_params ld_params = {(uint32_t)std::strtoul(fl.val["ld_max_dist"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_bin_width"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_min_minor"].c_str(), nullptr, 10)};
@@ -315,6 +319,12 @@ int main(int argc, char **argv)
                     if (ii.size() >= 4000000 || i + 2 == (uint32_t)pop_size) { put(pops.tmrca(ii, jj)); ii.clear(); jj.clear(); }
                 }
             }
+        }
+        if (print_fasta) pops.write_core_fasta(outpref + "_core_genome.fasta", false);   // extension: the last generation as FASTA
+        if (print_snp_alignment) {                                          // extension: its polymorphic columns, constant sites for -fconst
+            uint64_t consts[4];
+            pops.write_core_fasta(outpref + "_core_snps.fasta", true, consts);
+            std::ofstream(outpref + "_core_snps_fconst.txt") << consts[0] << "," << consts[1] << "," << consts[2] << "," << consts[3] << "\n";
         }
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)

@@ -181,6 +181,14 @@ public:
         gcheck(pansim_group_write_core_vcf(grp_, path.c_str(), &n));
         return n;
     }
+    // (extension) the core alignment as FASTA, every site or (snps_only) the polymorphic columns, all shards in one
+    // file; the constant-site counts by letter go to const_counts[4] if given; bytes written
+    uint64_t write_core_fasta(const std::string &path, bool snps_only, uint64_t *const_counts = nullptr)
+    {
+        uint64_t n = 0;
+        gcheck(pansim_group_write_core_fasta(grp_, path.c_str(), snps_only ? 1 : 0, nullptr, const_counts, &n));
+        return n;
+    }
 
     // (extension) LD of the core alignment by site distance over all shards: n_bins = ceil(max_dist / bin_width) bins
     std::vector<pansim_ld_bin> core_ld(const pansim_ld_params &p, uint64_t *sites_used = nullptr)

@@ -89,6 +89,21 @@ def diversity_stats(d: Diversity, pop_size: int) -> tuple[float, float, float]:
     return float(out[0]), float(out[1]), float(out[2])
 
 
+class CoreFasta(NamedTuple):
+    """What a FASTA writer wrote (include/pansim_b200.h): bytes of the file, columns per record and, for the sites
+    that are not columns, how many carry A, C, G and T (all 0 in whole mode; IQ-TREE's -fconst in SNP mode)."""
+    bytes: int
+    columns: int
+    const_counts: np.ndarray
+
+
+def _write_fasta(call, check, path: str, snps_only: bool) -> CoreFasta:
+    cols, n = C.c_uint64(0), C.c_uint64(0)
+    consts = np.zeros(4, np.uint64)
+    check(call(path.encode(), int(snps_only), C.byref(cols), _ptr(consts), C.byref(n)))
+    return CoreFasta(n.value, cols.value, consts)
+
+
 class CoreLD(NamedTuple):
     """LD bins of pansim_core_ld (include/pansim_b200.h): per bin its distances dist_lo..dist_hi, the site pairs, the
     pairs showing four gametes, the exact sum of r^2 in units of 2^-32 and the mean r^2 (NaN for an empty bin); and
@@ -632,6 +647,34 @@ class Pansim:
         bytes of text (header excluded)."""
         site, expand, n = C.c_float(), C.c_float(), C.c_uint64()
         self._check(self._lib.pansim_core_vcf_kernel_ms(self._h, repeats, C.byref(site), C.byref(expand), C.byref(n)))
+        return site.value, expand.value, n.value
+
+    def write_core_fasta(self, path: str, snps_only: bool = False) -> CoreFasta:
+        """The core alignment as FASTA (include/pansim_b200.h): one record `>ind_<i>` per row, every site as a column
+        or, with snps_only, the sites where two or more letters are present (snp-sites' selection). Returns the
+        bytes written, the columns and the constant-site counts by letter (A, C, G, T)."""
+        return _write_fasta(lambda *a: self._lib.pansim_write_core_fasta(self._h, *a), self._check, path, snps_only)
+
+    def export_core_fasta_rows(self, row_begin: int, row_end: int, snps_only: bool = False) -> np.ndarray:
+        """The FASTA letters of rows [row_begin, row_end) without headers: uint8 [rows, columns] of ASCII ACGT. On a
+        column shard the columns are the shard's own; the shards' arrays, concatenated along axis 1 in shard order,
+        are the whole alignment's. In whole mode the columns are the local sites; in SNP mode a first call (out = NULL)
+        asks for their number, which repeats the site pass of the second (0.1-0.6 ms on a B200 at 1 000 to
+        10 000 x 1.2 Mbp, profiles/r07_fasta_bench.json)."""
+        cols = C.c_uint64(self.local_sites)
+        if snps_only:
+            self._check(self._lib.pansim_export_core_fasta_rows(self._h, 1, row_begin, row_end, None, C.byref(cols)))
+        out = np.empty((max(0, row_end - row_begin), cols.value), np.uint8)
+        self._check(self._lib.pansim_export_core_fasta_rows(self._h, int(snps_only), row_begin, row_end, _ptr(out),
+                                                            C.byref(cols)))
+        return out
+
+    def fasta_kernel_ms(self, snps_only: bool = False, repeats: int = 10) -> tuple[float, float, int]:
+        """Measurement: device ms of one FASTA site pass (SNP mode) and of one expansion of every chunk of records
+        (no copy), and the bytes of the file."""
+        site, expand, n = C.c_float(), C.c_float(), C.c_uint64()
+        self._check(self._lib.pansim_core_fasta_kernel_ms(self._h, int(snps_only), repeats, C.byref(site), C.byref(expand),
+                                                          C.byref(n)))
         return site.value, expand.value, n.value
 
     def write(self, outpref: str):

@@ -70,7 +70,8 @@ class RunResult:
 
 def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False,
         print_diversity: bool = False, print_vcf: bool = False, print_ld: bool = False, ld_max_dist: int = 10000,
-        ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False) -> RunResult | None:
+        ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False, print_fasta: bool = False,
+        print_snp_alignment: bool = False) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -84,7 +85,11 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     ld_min_minor; write_core_ld).
     print_genealogy (extension): the parents of every generation are recorded on the device from generation 0;
     after the other outputs the genealogy of the last generation goes to `<outpref>_genealogy.nwk` and the TMRCA of
-    the pair on each line of `<outpref>.tsv` to `<outpref>_tmrca.tsv` (write_genealogy)."""
+    the pair on each line of `<outpref>.tsv` to `<outpref>_tmrca.tsv` (write_genealogy).
+    print_fasta / print_snp_alignment (extension): after the other outputs, the core alignment of the last generation
+    as `<outpref>_core_genome.fasta` (every site) / `<outpref>_core_snps.fasta` (the sites where two or more letters
+    are present) with `<outpref>_core_snps_fconst.txt`, the constant sites by letter as `nA,nC,nG,nT`
+    (Pansim.write_core_fasta)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -188,6 +193,12 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
                 res.tmrca = sim.tmrca(r1, r2)
             if outpref:
                 write_genealogy(outpref, sim, res.genealogy, None if all_pairs else res.tmrca)
+        if print_fasta and outpref:
+            sim.write_core_fasta(outpref + "_core_genome.fasta")
+        if print_snp_alignment and outpref:
+            consts = sim.write_core_fasta(outpref + "_core_snps.fasta", snps_only=True).const_counts
+            with open(outpref + "_core_snps_fconst.txt", "w") as f:
+                f.write(",".join(str(int(x)) for x in consts) + "\n")
     return res
 
 
