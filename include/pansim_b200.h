@@ -341,6 +341,39 @@ int pansim_core_ld_kernel_ms(pansim_ctx *ctx, const pansim_ld_params *p, uint32_
  * that order, NaN when pairs = 0, so every host prints the same digits */
 double pansim_ld_mean_r2(const pansim_ld_bin *b);
 
+/* ---- accessory-gene linkage (extension: the reference writes single-gene frequencies only) ----
+ * r^2, associated, dissociated and four-gamete gene pairs by compartment class, the joint presence counts of the
+ * gene pairs formed on the tensor cores (DESIGN.md section 15). Presence is absolute, so no ancestral row is needed.
+ * Let n = N. Gene g in [0, G) is PRESENT in row r when its bit is set; a_g = the rows carrying g (the numbers
+ * pansim_gene_counts returns). group(g) = 1 if n_compartments == 2 and comp_lo[1] <= g < comp_hi[1], else 0 (with
+ * both compartments, group 1 is the genes of --rate_genes2, main.rs:341-367). A gene is USED when
+ * 1 <= min_minor <= min(a, n - a); genes at or past G are never used. The pairs are all pairs of used genes g < h
+ * (there is no window: gene indices carry no position); the class of a pair is group(g) + group(h):
+ * 0 = "0-0", 1 = "0-1", 2 = "1-1". Per pair, with c = the rows carrying both genes, exactly as pansim_core_ld:
+ *   D = n*c - a_g*a_h, exact in int64;
+ *   inv_x = 1.0 / (double)(a_x*(n - a_x)), the product exact, the division IEEE round-to-nearest, once per gene;
+ *   r2 = (((double)D * (double)D) * inv_g) * inv_h, each product rounded on its own;
+ *   q = round-half-even(r2 * 2^32) as uint64;
+ *   four gametes iff c > 0, a_g - c > 0, a_h - c > 0 and n - a_g - a_h + c > 0;
+ *   the pair is ASSOCIATED when D > 0 and DISSOCIATED when D < 0;
+ *   its r^2 histogram bin is b = min((q * r2_bins) >> 32, r2_bins - 1) in uint64 (q <= 2^32, r2_bins <= 1024).
+ * Per class the call returns the pairs, the four-gamete pairs and sum q as an exact 128-bit integer in `ld` (so
+ * pansim_ld_mean_r2(&classes[k].ld) is the class mean), and the associated and dissociated pairs;
+ * hist[class * r2_bins + b] = the pairs of that class in bin b; genes_used[group] = the used genes of each group.
+ * Every output is an integer: neither the grid nor the shard count changes a bit. G = 0 or N < 2 gives all zeros.
+ * Errors: no state (pansim_set_initial or pansim_upload_acc) -> PANSIM_ERR_STATE; r2_bins = 0, r2_bins > 1024 or
+ * min_minor = 0 -> PANSIM_ERR_INVALID. The context keeps working after a refused call. The gene-major presence bit
+ * rows (one bit per row and used gene) are allocated on first use and kept with the context. */
+typedef struct { uint32_t r2_bins, min_minor; } pansim_gene_ld_params;
+typedef struct { pansim_ld_bin ld; uint64_t associated, dissociated; } pansim_gene_ld_class;
+int pansim_gene_ld(pansim_ctx *ctx, const pansim_gene_ld_params *p, pansim_gene_ld_class classes[3],
+                   uint64_t *hist /* [3][r2_bins] or NULL */, uint64_t genes_used[2] /* or NULL */);
+/* measurement: the gene pass (presence counts, used genes, scan, compaction), the transpose to bit rows and the
+ * pair pass (zeroed outputs and pair kernel), each `repeats` times after one warm-up call; mean device ms of one
+ * pass (CUDA events) and the pairs counted */
+int pansim_gene_ld_kernel_ms(pansim_ctx *ctx, const pansim_gene_ld_params *p, uint32_t repeats,
+                             float *gene_ms, float *transpose_ms, float *pair_ms, uint64_t *pairs);
+
 /* ---- clonal genealogy (extension: the reference keeps no pedigree) -------
  * The parent vectors the generations were drawn with, recorded on the device, and the genealogy of the present
  * population traced from them (DESIGN.md section 13). Both populations share it: next_generation gathers the core and
@@ -459,6 +492,11 @@ int pansim_group_write_core_fasta(pansim_group *g, const char *path, int snps_on
 
 /* pansim_core_ld over the whole alignment: every shard with the next one as its halo, summed on the host */
 int pansim_group_core_ld(pansim_group *g, const pansim_ld_params *p, pansim_ld_bin *bins, uint64_t *sites_used);
+
+/* pansim_gene_ld of the group: the accessory matrix is replicated in every shard, so shard 0 answers. Under a
+ * communicator every rank computes the same whole result; nothing is exchanged. */
+int pansim_group_gene_ld(pansim_group *g, const pansim_gene_ld_params *p, pansim_gene_ld_class classes[3],
+                         uint64_t *hist, uint64_t genes_used[2]);
 
 /* the clonal genealogy of the group: every shard draws the same parents, so shard 0 records and answers. Under a
  * communicator (one process per GPU) every rank records its own identical copy; nothing is exchanged. */

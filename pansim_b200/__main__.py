@@ -5,7 +5,8 @@ same parsing quirks: pop_size/core_size/pan_genes/core_genes/n_gen are parsed as
 f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
 accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
---print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy, --print_fasta, --print_snp_alignment.
+--print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy, --print_fasta, --print_snp_alignment,
+--print_gene_ld, --gene_ld_bins, --gene_ld_min_minor.
 """
 from __future__ import annotations
 
@@ -81,6 +82,13 @@ def build_parser() -> argparse.ArgumentParser:
                     help="(extension) <outpref>_core_snps.fasta: the same records with only the sites where two or more "
                          "letters are present; <outpref>_core_snps_fconst.txt: the constant sites by letter, nA,nC,nG,nT "
                          "(IQ-TREE -fconst)")
+    ap.add_argument("--print_gene_ld", action="store_true",
+                    help="(extension) <outpref>_gene_ld.tsv: linkage of the accessory genes of the last generation, one line "
+                         "per class of gene pair (0-0, 0-1, 1-1 by compartment): class, gene pairs, pairs with four gametes, "
+                         "associated pairs, dissociated pairs, mean r^2, then the r^2 histogram")
+    ap.add_argument("--gene_ld_bins", type=int, default=20, help="(extension) r^2 histogram bins of --print_gene_ld (1..1024)")
+    ap.add_argument("--gene_ld_min_minor", type=int, default=1,
+                    help="(extension) --print_gene_ld uses genes present in at least this many rows and absent from at least this many")
     return ap
 
 
@@ -94,6 +102,7 @@ def main(argv=None) -> int:
     print_fasta = ns.pop("print_fasta")
     print_snp_alignment = ns.pop("print_snp_alignment")
     ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
+    ld.update({k: ns.pop(k) for k in ("print_gene_ld", "gene_ld_bins", "gene_ld_min_minor")})
     p = Params(**ns)
     run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf,
         print_genealogy=print_genealogy, print_fasta=print_fasta, print_snp_alignment=print_snp_alignment, **ld)

@@ -35,6 +35,7 @@ EXPORTED = [
     "pansim_write_core_vcf", "pansim_group_write_core_vcf", "pansim_core_vcf_kernel_ms",
     "pansim_write_core_fasta", "pansim_export_core_fasta_rows", "pansim_group_write_core_fasta", "pansim_core_fasta_kernel_ms",
     "pansim_core_ld", "pansim_group_core_ld", "pansim_core_ld_kernel_ms", "pansim_ld_mean_r2",
+    "pansim_gene_ld", "pansim_group_gene_ld", "pansim_gene_ld_kernel_ms",
     "pansim_enable_genealogy", "pansim_genealogy", "pansim_genealogy_history", "pansim_genealogy_tmrca",
     "pansim_genealogy_newick", "pansim_group_enable_genealogy", "pansim_group_genealogy", "pansim_group_genealogy_tmrca",
 ]
@@ -107,6 +108,14 @@ class LdParams(C.Structure):
 
 class LdBin(C.Structure):
     _fields_ = [("pairs", C.c_uint64), ("four_gamete", C.c_uint64), ("r2_hi", C.c_uint64), ("r2_lo", C.c_uint64)]
+
+
+class GeneLdParams(C.Structure):
+    _fields_ = [("r2_bins", C.c_uint32), ("min_minor", C.c_uint32)]
+
+
+class GeneLdClass(C.Structure):
+    _fields_ = [("ld", LdBin), ("associated", C.c_uint64), ("dissociated", C.c_uint64)]
 
 
 class GenealogyNode(C.Structure):
@@ -235,6 +244,10 @@ def lib():
     sig("pansim_core_ld_kernel_ms", cint, vp, C.POINTER(LdParams), u32, C.POINTER(C.c_float), C.POINTER(C.c_float),
         C.POINTER(C.c_float), C.POINTER(C.c_uint64))
     sig("pansim_ld_mean_r2", dbl, C.POINTER(LdBin))
+    sig("pansim_gene_ld", cint, vp, C.POINTER(GeneLdParams), C.POINTER(GeneLdClass), vp, vp)
+    sig("pansim_group_gene_ld", cint, vp, C.POINTER(GeneLdParams), C.POINTER(GeneLdClass), vp, vp)
+    sig("pansim_gene_ld_kernel_ms", cint, vp, C.POINTER(GeneLdParams), u32, C.POINTER(C.c_float), C.POINTER(C.c_float),
+        C.POINTER(C.c_float), C.POINTER(C.c_uint64))
     sig("pansim_enable_genealogy", cint, vp, u32)
     sig("pansim_genealogy", cint, vp, vp, C.POINTER(GenealogyInfo))
     sig("pansim_genealogy_history", cint, vp, vp)

@@ -21,6 +21,7 @@
 #include "core_mut.cuh"
 #include "distance.cuh"
 #include "diversity.cuh"
+#include "gene_ld.cuh"
 #include "genealogy.cuh"
 #include "ld.cuh"
 #include "pack.cuh"
@@ -291,6 +292,15 @@ struct pansim_ctx {
     unsigned long long *h_ld = nullptr, *h_ld_bins = nullptr;         // pinned: own / halo used sites, tile pairs; bins
     size_t h_ld_bins_cap = 0;
     cudaEvent_t ev_ld = nullptr;                                       // the halo of this context is ready
+    // accessory-gene LD (gene_ld.cuh): presence counts and ranks of the G genes, the compacted used genes (presence
+    // count, group, 1 / (a (n - a))), their gene-major presence bit rows, and the outputs (class totals, histogram,
+    // used genes of group 1), mirrored in pinned host memory
+    struct GeneLdBuf {
+        uint32_t *counts = nullptr, *rank = nullptr, *a = nullptr, *grp = nullptr, *x = nullptr;
+        double *inv = nullptr;
+        unsigned long long *block = nullptr, *out = nullptr, *h_out = nullptr;
+        size_t x_cap = 0, out_cap = 0;
+    } gl;
     // clonal genealogy (genealogy.cuh): a ring of the last gen_cap parent vectors, each copied on stream_gen behind
     // ev_parents[i]; next_parents_buffer waits on ev_gen_done[i] before buffer i is rewritten. The trace and the
     // TMRCA walk run on stream_gen too, so they follow every copy enqueued before them.
@@ -1158,6 +1168,12 @@ void pansim_destroy(pansim_ctx *c)
     if (c->h_fa) cudaFreeHost(c->h_fa);
     if (c->h_ld_bins) cudaFreeHost(c->h_ld_bins);
     if (c->ev_ld) cudaEventDestroy(c->ev_ld);
+    {
+        void *gp[] = {c->gl.counts, c->gl.rank, c->gl.a, c->gl.grp, c->gl.x, c->gl.inv, c->gl.block, c->gl.out};
+        for (void *p : gp)
+            if (p) cudaFree(p);
+        if (c->gl.h_out) cudaFreeHost(c->gl.h_out);
+    }
     if (c->stream_gen) { cudaStreamSynchronize(c->stream_gen); cudaStreamDestroy(c->stream_gen); }
     for (auto e : c->ev_gen_done) if (e) cudaEventDestroy(e);
     for (void *p : {(void *)c->d_gen_ring, (void *)c->d_gen_scratch, (void *)c->d_gen_pairs}) if (p) cudaFree(p);
@@ -3602,6 +3618,222 @@ double pansim_ld_mean_r2(const pansim_ld_bin *b)
 {
     if (!b || !b->pairs) return std::numeric_limits<double>::quiet_NaN();
     return (std::ldexp((double)b->r2_hi, 32) + std::ldexp((double)b->r2_lo, -32)) / (double)b->pairs;
+}
+
+// ---- accessory-gene LD (gene_ld.cuh, DESIGN.md section 15) ---------------------------------------
+// output words: the class totals, the histogram [3][r2_bins], then the used genes of group 1
+static size_t gene_ld_out_words(uint32_t r2_bins) { return GL_OUT_CLASSES + 3 * (size_t)r2_bins + 1; }
+
+// the per-gene arrays (G is fixed per context, so they are allocated once) and the outputs for r2_bins
+static int gene_ld_ensure(pansim_ctx *c, uint32_t r2_bins)
+{
+    auto &b = c->gl;
+    if (!b.counts) {
+        const size_t G = c->G;
+        CU(c, cudaMalloc(&b.counts, G * sizeof(uint32_t)));
+        CU(c, cudaMalloc(&b.rank, G * sizeof(uint32_t)));
+        CU(c, cudaMalloc(&b.a, G * sizeof(uint32_t)));
+        CU(c, cudaMalloc(&b.grp, G * sizeof(uint32_t)));
+        CU(c, cudaMalloc(&b.inv, G * sizeof(double)));
+        CU(c, cudaMalloc(&b.block, ((size_t)div_up64(G, VS_SITES) + 1) * sizeof(unsigned long long)));
+    }
+    const size_t words = gene_ld_out_words(r2_bins);
+    if (words > b.out_cap) {
+        if (b.out) cudaFree(b.out);
+        if (b.h_out) cudaFreeHost(b.h_out);
+        b.out = nullptr; b.h_out = nullptr; b.out_cap = 0;
+        CU(c, cudaMalloc(&b.out, words * sizeof(unsigned long long)));
+        CU(c, cudaMallocHost(&b.h_out, words * sizeof(unsigned long long)));
+        b.out_cap = words;
+    }
+    return 0;
+}
+
+// the gene-major bit rows of n_used used genes (kept with the context, like the core LD rows)
+static int gene_ld_ensure_x(pansim_ctx *c, size_t n_used)
+{
+    const size_t bytes = std::max<size_t>(1, n_used) * ld_row_words(c->N) * sizeof(uint32_t);
+    if (bytes <= c->gl.x_cap) return 0;
+    if (c->gl.x) cudaFree(c->gl.x);
+    c->gl.x = nullptr; c->gl.x_cap = 0;
+    if (cudaMalloc(&c->gl.x, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL(c, PANSIM_ERR_NOMEM, "cudaMalloc of %zu bytes (gene LD bit rows) failed", bytes);
+    }
+    c->gl.x_cap = bytes;
+    return 0;
+}
+
+// gene pass on c->stream: presence counts (K8), used genes, their ranks and compacted arrays, the used genes of
+// group 1 (zeroed here); the number of used genes is block[n_blocks], copied to *h_used if given
+static int gene_ld_gene_pass(pansim_ctx *c, const pansim_gene_ld_params *p, uint32_t r2_bins, unsigned long long *h_used)
+{
+    auto &b = c->gl;
+    acc_gene_counts_kernel<<<c->acc_words, 256, 0, c->stream>>>(c->acc[c->acc_cur], c->N, c->G, c->acc_stride_words, b.counts);
+    LAUNCH_CHECK(c);
+    unsigned long long *used1 = b.out + gene_ld_out_words(r2_bins) - 1;
+    CU(c, cudaMemsetAsync(used1, 0, sizeof(unsigned long long), c->stream));
+    GeneLdArgs a;
+    a.counts = b.counts;
+    a.n_genes = c->G;
+    a.n_rows = c->N;
+    a.min_minor = p->min_minor;
+    const bool two = c->cfg.n_compartments == 2;
+    a.lo1 = two ? c->cfg.comp_lo[1] : 0u;
+    a.hi1 = two ? c->cfg.comp_hi[1] : 0u;
+    a.block = b.block;
+    a.rank = b.rank;
+    a.a = b.a;
+    a.grp = b.grp;
+    a.inv = b.inv;
+    a.used1 = used1;
+    const uint32_t blocks = div_up64(c->G, VS_SITES);
+    gene_ld_mark_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    vcf_scan_blocks_kernel<<<1, VS_SCAN_THREADS, 0, c->stream>>>(b.block, blocks, b.block + blocks);
+    LAUNCH_CHECK(c);
+    gene_ld_compact_kernel<<<blocks, VS_THREADS, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    if (h_used) CU(c, cudaMemcpyAsync(h_used, b.block + blocks, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+}
+
+// presence bit rows of the used genes into gl.x (row k = rank k)
+static int gene_ld_transpose(pansim_ctx *c)
+{
+    GeneLdTransposeArgs a;
+    a.state = c->acc[c->acc_cur];
+    a.stride_words = c->acc_stride_words;
+    a.n_rows = c->N;
+    a.n_genes = c->G;
+    a.rank = c->gl.rank;
+    a.kw = ld_row_words(c->N);
+    a.x = c->gl.x;
+    const dim3 grid(c->acc_words, div_up64(a.kw / 2, GT_WARPS));
+    gene_ld_transpose_kernel<<<grid, GT_WARPS * 32, 0, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+static uint64_t gene_ld_tile_pairs(uint64_t used)
+{
+    const uint64_t t = (used + LD_TILE - 1) / LD_TILE;
+    return t * (t + 1) / 2;
+}
+
+// zeroed class totals and histogram, then the pair kernel over every tile pair of the `used` genes
+static int gene_ld_pairs(pansim_ctx *c, uint32_t r2_bins, uint64_t used)
+{
+    CU(c, cudaMemsetAsync(c->gl.out, 0, (GL_OUT_CLASSES + 3 * (size_t)r2_bins) * sizeof(unsigned long long), c->stream));
+    if (used < 2) return 0;
+    const uint64_t tiles = gene_ld_tile_pairs(used);
+    if (tiles > 0x7FFFFFFFull) FAIL(c, PANSIM_ERR_INVALID, "%llu gene LD tile pairs: more than one launch holds", (unsigned long long)tiles);
+    GeneLdPairArgs a;
+    a.x = c->gl.x;
+    a.kw = ld_row_words(c->N);
+    a.k_iters = a.kw * 32 / LD_KB;
+    a.a = c->gl.a;
+    a.grp = c->gl.grp;
+    a.inv = c->gl.inv;
+    a.n_used = (uint32_t)used;
+    a.n_rows = c->N;
+    a.n_tiles = div_up64(used, LD_TILE);
+    a.r2_bins = r2_bins;
+    a.out = c->gl.out;
+    const size_t smem = gene_ld_pair_smem_bytes(r2_bins);
+    CU(c, cudaFuncSetAttribute(gene_ld_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    gene_ld_pair_kernel<<<(uint32_t)tiles, LD_THREADS, smem, c->stream>>>(a);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// Refusals leave the context as it was.
+static int gene_ld_validate(pansim_ctx *c, const pansim_gene_ld_params *p)
+{
+    if (!p->r2_bins || p->r2_bins > GL_MAX_BINS || !p->min_minor)
+        FAIL(c, PANSIM_ERR_INVALID, "gene LD: r2_bins must be 1..%u and min_minor >= 1", GL_MAX_BINS);
+    if (!c->has_acc) FAIL(c, PANSIM_ERR_STATE, "gene LD: no accessory state: call pansim_set_initial or pansim_upload_acc first");
+    return 0;
+}
+
+// the gene pass, the transpose and the pair pass into the pinned outputs (G >= 1, N >= 2); *used = the used genes
+static int gene_ld_run(pansim_ctx *c, const pansim_gene_ld_params *p, uint64_t *used)
+{
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (int rc = gene_ld_ensure(c, p->r2_bins)) return rc;
+    const size_t words = gene_ld_out_words(p->r2_bins);
+    unsigned long long *h_used = c->gl.h_out + words - 1;                      // overwritten by the readback below
+    if (int rc = gene_ld_gene_pass(c, p, p->r2_bins, h_used)) return rc;
+    CU(c, cudaStreamSynchronize(c->stream));
+    *used = *h_used;
+    if (*used >= 2) {
+        if (int rc = gene_ld_ensure_x(c, *used)) return rc;
+        if (int rc = gene_ld_transpose(c)) return rc;
+    }
+    if (int rc = gene_ld_pairs(c, p->r2_bins, *used)) return rc;
+    CU(c, cudaMemcpyAsync(c->gl.h_out, c->gl.out, words * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int pansim_gene_ld(pansim_ctx *c, const pansim_gene_ld_params *p, pansim_gene_ld_class classes[3], uint64_t *hist, uint64_t genes_used[2])
+{
+    if (!c || !p || !classes) return PANSIM_ERR_INVALID;
+    if (int rc = gene_ld_validate(c, p)) return rc;
+    memset(classes, 0, 3 * sizeof(pansim_gene_ld_class));
+    if (hist) memset(hist, 0, 3 * (size_t)p->r2_bins * sizeof(uint64_t));
+    uint64_t used = 0, used1 = 0;
+    if (c->G && c->N >= 2) {                                                     // otherwise no gene is used
+        if (int rc = gene_ld_run(c, p, &used)) return rc;
+        const unsigned long long *h = c->gl.h_out;
+        for (int k = 0; k < 3; k++) {
+            const unsigned long long *w = h + GL_CLASS_WORDS * k;
+            classes[k].ld = {w[0], w[1], w[2], w[3]};
+            classes[k].associated = w[4];
+            classes[k].dissociated = w[5];
+        }
+        if (hist)
+            for (size_t b = 0; b < 3 * (size_t)p->r2_bins; b++) hist[b] = h[GL_OUT_CLASSES + b];
+        used1 = h[gene_ld_out_words(p->r2_bins) - 1];
+    }
+    if (genes_used) {
+        genes_used[0] = used - used1;
+        genes_used[1] = used1;
+    }
+    return 0;
+}
+
+int pansim_gene_ld_kernel_ms(pansim_ctx *c, const pansim_gene_ld_params *p, uint32_t repeats, float *gene_ms, float *transpose_ms,
+                             float *pair_ms, uint64_t *pairs)
+{
+    if (!c || !p || !repeats) return PANSIM_ERR_INVALID;
+    pansim_gene_ld_class cls[3];
+    uint64_t gu[2];
+    if (int rc = pansim_gene_ld(c, p, cls, nullptr, gu)) return rc;           // also the warm-up
+    const uint64_t used = gu[0] + gu[1];
+    float t[3] = {0.f, 0.f, 0.f};
+    if (c->G && c->N >= 2) {
+        cudaEvent_t ev[4];
+        for (auto &e : ev) CU(c, cudaEventCreate(&e));
+        int rc = 0;
+        cudaEventRecord(ev[0], c->stream);
+        for (uint32_t r = 0; r < repeats && !rc; r++) rc = gene_ld_gene_pass(c, p, p->r2_bins, nullptr);
+        cudaEventRecord(ev[1], c->stream);
+        for (uint32_t r = 0; r < repeats && !rc && used >= 2; r++) rc = gene_ld_transpose(c);
+        cudaEventRecord(ev[2], c->stream);
+        for (uint32_t r = 0; r < repeats && !rc; r++) rc = gene_ld_pairs(c, p->r2_bins, used);
+        cudaEventRecord(ev[3], c->stream);
+        const cudaError_t e = cudaEventSynchronize(ev[3]);
+        for (int k = 0; k < 3; k++) cudaEventElapsedTime(&t[k], ev[k], ev[k + 1]);
+        for (auto &x : ev) cudaEventDestroy(x);
+        if (rc) return rc;
+        if (e != cudaSuccess) FAIL(c, PANSIM_ERR_CUDA, "gene LD kernels failed: %s", cudaGetErrorString(e));
+    }
+    if (gene_ms) *gene_ms = t[0] / (float)repeats;
+    if (transpose_ms) *transpose_ms = t[1] / (float)repeats;
+    if (pair_ms) *pair_ms = t[2] / (float)repeats;
+    if (pairs) *pairs = cls[0].ld.pairs + cls[1].ld.pairs + cls[2].ld.pairs;
+    return 0;
 }
 
 // ---- clonal genealogy (genealogy.cuh, DESIGN.md section 13) ------------------

@@ -13,8 +13,8 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import (OK, CoreFasta, CoreLD, Genealogy, PansimError, _core_ld, _diversity, _genealogy, _genealogy_history,
-                         _ld_bins, _ld_params, _pairs_or_none, _ptr, _tmrca, _write_fasta, make_config)
+from .population import (OK, CoreFasta, CoreLD, GeneLD, Genealogy, PansimError, _core_ld, _diversity, _gene_ld, _genealogy,
+                         _genealogy_history, _ld_bins, _ld_params, _pairs_or_none, _ptr, _tmrca, _write_fasta, make_config)
 
 
 class PansimGroup:
@@ -148,6 +148,10 @@ class PansimGroup:
         self._check(self._lib.pansim_group_core_ld(self._h, C.byref(_ld_params(max_dist, bin_width, min_minor)), bins,
                                                    C.byref(used)))
         return _core_ld(bins, n, max_dist, bin_width, used.value)
+
+    def gene_ld(self, r2_bins: int = 20, min_minor: int = 1) -> GeneLD:
+        """Accessory-gene linkage (Pansim.gene_ld): the accessory matrix is replicated, so shard 0 answers."""
+        return _gene_ld(lambda *a: self._lib.pansim_group_gene_ld(self._h, *a), self._check, r2_bins, min_minor)
 
     def enable_genealogy(self, capacity: int):
         """Pansim.enable_genealogy for the group: shard 0 records (every shard draws the same parents)."""

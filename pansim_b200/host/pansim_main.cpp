@@ -42,16 +42,18 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
                              "max_distances", "core_mu", "HR_rate", "HGT_rate", "rate_genes1", "rate_genes2",
                              "prop_genes2", "prop_positive", "pos_lambda", "neg_lambda", "seed", "outpref",
                              "threads", "genome_size_penalty", "competition_strength", "device", "gpus",
-                             "ld_max_dist", "ld_bin_width", "ld_min_minor"};       // extensions: --print_ld bins
+                             "ld_max_dist", "ld_bin_width", "ld_min_minor",        // extensions: --print_ld bins,
+                             "gene_ld_bins", "gene_ld_min_minor"};                 // --print_gene_ld histogram and genes
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
                               "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy",
-                              "print_fasta", "print_snp_alignment"};          // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "print_fasta", "print_snp_alignment", "print_gene_ld"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
                                                                               // print_vcf (<outpref>_core_genome.vcf),
                                                                               // print_ld (<outpref>_core_ld.tsv),
                                                                               // print_genealogy (<outpref>_genealogy.nwk, <outpref>_tmrca.tsv),
                                                                               // print_fasta (<outpref>_core_genome.fasta),
-                                                                              // print_snp_alignment (<outpref>_core_snps.fasta, <outpref>_core_snps_fconst.txt)
+                                                                              // print_snp_alignment (<outpref>_core_snps.fasta, <outpref>_core_snps_fconst.txt),
+                                                                              // print_gene_ld (<outpref>_gene_ld.tsv)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -61,7 +63,8 @@ bool parse(int argc, char **argv, Flags &f)
              {"prop_genes2", "0.1"}, {"prop_positive", "-0.1"}, {"pos_lambda", "10.0"}, {"neg_lambda", "10.0"},
              {"seed", "0"}, {"outpref", "distances"}, {"threads", "1"}, {"genome_size_penalty", "0.99"},
              {"competition_strength", "0.0"}, {"device", "0"}, {"gpus", "1"},
-             {"ld_max_dist", "10000"}, {"ld_bin_width", "100"}, {"ld_min_minor", "1"}};
+             {"ld_max_dist", "10000"}, {"ld_bin_width", "100"}, {"ld_min_minor", "1"},
+             {"gene_ld_bins", "20"}, {"gene_ld_min_minor", "1"}};
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         if (a == "--help" || a == "-h") {
@@ -140,6 +143,9 @@ int main(int argc, char **argv)
     const pansim_ld_params ld_params = {(uint32_t)std::strtoul(fl.val["ld_max_dist"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_bin_width"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_min_minor"].c_str(), nullptr, 10)};
+    const bool print_gene_ld = fl.sw["print_gene_ld"];
+    const pansim_gene_ld_params gene_ld_params = {(uint32_t)std::strtoul(fl.val["gene_ld_bins"].c_str(), nullptr, 10),
+                                                  (uint32_t)std::strtoul(fl.val["gene_ld_min_minor"].c_str(), nullptr, 10)};
     const int n_gpus = std::max(1, std::atoi(fl.val["gpus"].c_str()));       // extension: column shards over N devices of the box
     const bool print_selection = fl.sw["print_selection"], no_control = fl.sw["no_control_genome_size"];
     const double genome_size_penalty = as_f64(fl, "genome_size_penalty"), competition_strength = as_f64(fl, "competition_strength");
@@ -325,6 +331,18 @@ int main(int argc, char **argv)
             uint64_t consts[4];
             pops.write_core_fasta(outpref + "_core_snps.fasta", true, consts);
             std::ofstream(outpref + "_core_snps_fconst.txt") << consts[0] << "," << consts[1] << "," << consts[2] << "," << consts[3] << "\n";
+        }
+        if (print_gene_ld) {                                                // extension: linkage of the accessory genes by class
+            std::vector<uint64_t> hist;
+            const std::array<pansim_gene_ld_class, 3> cls = pops.gene_ld(gene_ld_params, &hist);
+            const char *label[3] = {"0-0", "0-1", "1-1"};
+            std::ofstream f(outpref + "_gene_ld.tsv");
+            for (int k = 0; k < 3; k++) {
+                f << label[k] << "\t" << cls[k].ld.pairs << "\t" << cls[k].ld.four_gamete << "\t" << cls[k].associated << "\t"
+                  << cls[k].dissociated << "\t" << fmt(pansim_ld_mean_r2(&cls[k].ld));
+                for (uint32_t b = 0; b < gene_ld_params.r2_bins; b++) f << "\t" << hist[(size_t)k * gene_ld_params.r2_bins + b];
+                f << "\n";
+            }
         }
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)

@@ -8,6 +8,7 @@
 // meaning and error behaviour follow population.rs; errors surface as
 // pansim::Error (the reference panics via unwrap()).
 #pragma once
+#include <array>
 #include <cmath>
 #include <cstdint>
 #include <stdexcept>
@@ -198,6 +199,18 @@ public:
         gcheck(pansim_group_core_ld(grp_, &p, bins.data(), sites_used));
         bins.resize(n);
         return bins;
+    }
+
+    // (extension) linkage of the accessory genes by class (0-0, 0-1, 1-1); the r^2 histogram [3][r2_bins] goes to
+    // *hist and the used genes of each group to genes_used[2] if given. The accessory matrix is replicated, so
+    // shard 0 answers.
+    std::array<pansim_gene_ld_class, 3> gene_ld(const pansim_gene_ld_params &p, std::vector<uint64_t> *hist = nullptr,
+                                                uint64_t *genes_used = nullptr)
+    {
+        std::array<pansim_gene_ld_class, 3> cls{};
+        if (hist) hist->assign(3 * (size_t)(p.r2_bins <= 1024 ? p.r2_bins : 0), 0);
+        gcheck(pansim_group_gene_ld(grp_, &p, cls.data(), hist && !hist->empty() ? hist->data() : nullptr, genes_used));
+        return cls;
     }
 
     // (extension) record the parent vector of every generation from now on, the last `capacity` kept (0: off)

@@ -141,6 +141,39 @@ def ld_mean_r2(pairs: int, r2_sum: int) -> float:
     return _ffi.lib().pansim_ld_mean_r2(C.byref(_ffi.LdBin(pairs, 0, r2_sum >> 64, r2_sum & (2 ** 64 - 1))))
 
 
+GENE_LD_CLASSES = ("0-0", "0-1", "1-1")
+
+
+class GeneLD(NamedTuple):
+    """Accessory-gene linkage of pansim_gene_ld (include/pansim_b200.h), one entry per class of gene pair in the order
+    of `classes` (the groups of the two genes: 0-0, 0-1, 1-1): the gene pairs, those showing four gametes, the
+    associated (D > 0) and dissociated (D < 0) ones, the exact sum of r^2 in units of 2^-32 and the mean r^2 (NaN for
+    an empty class); hist [3, r2_bins] the pairs per r^2 bin, and genes_used [2] the used genes of each group."""
+    classes: tuple
+    pairs: np.ndarray
+    four_gamete: np.ndarray
+    associated: np.ndarray
+    dissociated: np.ndarray
+    r2_sum: list
+    mean_r2: np.ndarray
+    hist: np.ndarray
+    genes_used: np.ndarray
+
+
+def _gene_ld(call, check, r2_bins: int, min_minor: int) -> GeneLD:
+    """call(params, classes, hist, genes_used) -> status; the histogram is only allocated for a valid r2_bins (the
+    library refuses the others before writing)."""
+    cls = (_ffi.GeneLdClass * 3)()
+    hist = np.zeros((3, r2_bins if 1 <= r2_bins <= 1024 else 0), np.uint64)
+    used = np.zeros(2, np.uint64)
+    check(call(C.byref(_ffi.GeneLdParams(r2_bins, min_minor)), cls, _ptr(hist) if hist.size else None, _ptr(used)))
+    lib = _ffi.lib()
+    return GeneLD(GENE_LD_CLASSES, np.array([c.ld.pairs for c in cls], np.uint64),
+                  np.array([c.ld.four_gamete for c in cls], np.uint64), np.array([c.associated for c in cls], np.uint64),
+                  np.array([c.dissociated for c in cls], np.uint64), [(c.ld.r2_hi << 64) | c.ld.r2_lo for c in cls],
+                  np.array([lib.pansim_ld_mean_r2(C.byref(c.ld)) for c in cls], np.float64), hist, used)
+
+
 class Genealogy(NamedTuple):
     """The clonal genealogy of the present population (pansim_genealogy, include/pansim_b200.h): per node its parent
     (0xFFFFFFFF at the root), the individual it stands for (0xFFFFFFFF at a virtual root) and its time in generations
@@ -499,6 +532,19 @@ class Pansim:
                                                        C.byref(s), C.byref(t), C.byref(q), C.byref(n)))
         return s.value, t.value, q.value, n.value
 
+    # -- accessory-gene linkage (extension) ---------------------------------
+    def gene_ld(self, r2_bins: int = 20, min_minor: int = 1) -> GeneLD:
+        """r^2, associated, dissociated and four-gamete pairs of the used accessory genes by compartment class, and
+        the r^2 histogram of each class (pansim_gene_ld)."""
+        return _gene_ld(lambda *a: self._lib.pansim_gene_ld(self._h, *a), self._check, r2_bins, min_minor)
+
+    def gene_ld_kernel_ms(self, r2_bins: int = 20, min_minor: int = 1, repeats: int = 10):
+        """Measurement: device ms of one gene pass, one transpose and one pair pass, and the pairs counted."""
+        g, t, q, n = C.c_float(), C.c_float(), C.c_float(), C.c_uint64()
+        self._check(self._lib.pansim_gene_ld_kernel_ms(self._h, C.byref(_ffi.GeneLdParams(r2_bins, min_minor)), repeats,
+                                                       C.byref(g), C.byref(t), C.byref(q), C.byref(n)))
+        return g.value, t.value, q.value, n.value
+
     # -- clonal genealogy (extension) ---------------------------------------
     def enable_genealogy(self, capacity: int):
         """Record the parent vector of every generation from now on, keeping the last `capacity` (0: stop and free)."""
@@ -686,5 +732,5 @@ class Pansim:
                 f.write(",".join(ones + [str(int(x)) for x in acc[r]]) + "\n")
 
 
-__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "Genealogy", "genealogy_newick",
+__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "GeneLD", "Genealogy", "genealogy_newick",
            "make_config", "standard_deviation", "fmt_f64"]

@@ -62,6 +62,7 @@ class RunResult:
     diversity: list = field(default_factory=list) # per generation: Diversity (--print_diversity)
     sfs: np.ndarray = None                        # SFS of the last generation (--print_diversity)
     ld: object = None                             # CoreLD of the last generation (--print_ld)
+    gene_ld: object = None                        # GeneLD of the last generation (--print_gene_ld)
     genealogy: object = None                      # Genealogy of the last generation (--print_genealogy)
     tmrca: np.ndarray = None                      # TMRCA of the sampled pairs (--print_genealogy without --all_pairs)
     selection: np.ndarray = None
@@ -71,7 +72,8 @@ class RunResult:
 def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pairs: bool = False,
         print_diversity: bool = False, print_vcf: bool = False, print_ld: bool = False, ld_max_dist: int = 10000,
         ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False, print_fasta: bool = False,
-        print_snp_alignment: bool = False) -> RunResult | None:
+        print_snp_alignment: bool = False, print_gene_ld: bool = False, gene_ld_bins: int = 20,
+        gene_ld_min_minor: int = 1) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -89,7 +91,9 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     print_fasta / print_snp_alignment (extension): after the other outputs, the core alignment of the last generation
     as `<outpref>_core_genome.fasta` (every site) / `<outpref>_core_snps.fasta` (the sites where two or more letters
     are present) with `<outpref>_core_snps_fconst.txt`, the constant sites by letter as `nA,nC,nG,nT`
-    (Pansim.write_core_fasta)."""
+    (Pansim.write_core_fasta).
+    print_gene_ld (extension): linkage of the accessory genes of the last generation as `<outpref>_gene_ld.tsv`,
+    written after every other output (Pansim.gene_ld with gene_ld_bins, gene_ld_min_minor; write_gene_ld)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -199,7 +203,20 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             consts = sim.write_core_fasta(outpref + "_core_snps.fasta", snps_only=True).const_counts
             with open(outpref + "_core_snps_fconst.txt", "w") as f:
                 f.write(",".join(str(int(x)) for x in consts) + "\n")
+        if print_gene_ld:
+            res.gene_ld = sim.gene_ld(gene_ld_bins, gene_ld_min_minor)
+            if outpref:
+                write_gene_ld(outpref, res.gene_ld)
     return res
+
+
+def write_gene_ld(outpref: str, gl):
+    """`<outpref>_gene_ld.tsv`: one line per class of gene pair, 0-0, 0-1, 1-1 (no header): class, pairs, four-gamete
+    pairs, associated, dissociated, mean r^2 (NaN for an empty class), then the r^2 histogram counts."""
+    with open(outpref + "_gene_ld.tsv", "w") as f:
+        for k, label in enumerate(gl.classes):
+            f.write("\t".join([label, str(int(gl.pairs[k])), str(int(gl.four_gamete[k])), str(int(gl.associated[k])),
+                               str(int(gl.dissociated[k])), fmt_f64(float(gl.mean_r2[k])), *(str(int(x)) for x in gl.hist[k])]) + "\n")
 
 
 def write_genealogy(outpref: str, sim, genealogy, tmrca):
