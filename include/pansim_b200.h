@@ -374,6 +374,48 @@ int pansim_gene_ld(pansim_ctx *ctx, const pansim_gene_ld_params *p, pansim_gene_
 int pansim_gene_ld_kernel_ms(pansim_ctx *ctx, const pansim_gene_ld_params *p, uint32_t repeats,
                              float *gene_ms, float *transpose_ms, float *pair_ms, uint64_t *pairs);
 
+/* ---- pangenome accumulation curves and gene frequency spectrum (extension: the reference writes _freqs.txt) ----
+ * Roary's pangenome summaries of the accessory state (DESIGN.md section 16). N = pop_size, G = pan_size (the matrix
+ * genes), c0 = cfg.core_genes: the c0 genes are carried by every row and are not in the matrix (_freqs.txt appends
+ * them as 1.0, pansim_acc_distance adds them). a_g = the rows carrying matrix gene g (the numbers pansim_gene_counts
+ * returns). Bits at or past G in a row's last word are never counted.
+ * ORDERS. Order p (0 <= p < P) is a permutation o_p of 0..N-1 drawn by Fisher-Yates: start from the identity; for
+ * i = N-1 down to 1 swap o[i] and o[j], j = (uint32)(((uint64)r * (i+1)) >> 32), r = .x of philox4x32_10 (common.cuh)
+ * with key = (lo32(seed), hi32(seed)) and counter = {i, p, 0, PANSIM_GENE_ACC_ORDER_TAG}. No simulation stream has
+ * that counter word 3 (theirs are (stream << 16) | q below 0x00090000, or 0x01000000 + e for recombination events).
+ * The draw touches no simulation stream and changes no state.
+ * CURVES. x_k = row o_p[k-1], k = 1..N; per order and k:
+ *   pan(k)    = c0 + the matrix genes present in at least one of x_1..x_k;
+ *   core(k)   = c0 + the matrix genes present in all of x_1..x_k;
+ *   new(k)    = the matrix genes present in x_k and in none of x_1..x_{k-1}, + c0 when k = 1 (pan(k) = sum_{j<=k} new(j));
+ *   unique(k) = the matrix genes present in exactly one of x_1..x_k, + c0 when k = 1 (every gene is unique then).
+ * Every value is a uint32 (<= G + c0); no output depends on the grid, the chunking or the shard count.
+ * SPECTRUM. spectrum[k], k = 0..N = the matrix genes with a_g = k, + c0 in bin N. Bin 0 holds the matrix genes no row
+ * carries; they are not in the pangenome.
+ * CLASSES (Roary's thresholds as integer tests on a gene carried by a >= 1 rows): core if 100 a >= 99 N, else soft
+ * core if 100 a >= 95 N, else shell if 100 a >= 15 N, else cloud; total = the sum of the four. The c0 genes are core.
+ * The integer rule is the definition; Roary's floating-point rounding at a boundary is not promised.
+ * The state is read like pansim_gene_counts: acc[acc_cur] on the context's stream, so it follows every enqueued step.
+ * Errors: no accessory state (pansim_set_initial or pansim_upload_acc) -> PANSIM_ERR_STATE; n_perms = 0 or
+ * n_perms > PANSIM_GENE_ACC_MAX_PERMS -> PANSIM_ERR_INVALID. The context keeps working after a refused call. The
+ * orders, per-step counts and curves (32 bytes per order and row) are allocated on first use and kept with the context;
+ * the orders stay on the device unless `orders` is non-NULL. */
+#define PANSIM_GENE_ACC_ORDER_TAG 0x00A00000u
+#define PANSIM_GENE_ACC_MAX_PERMS 10000u
+/* every output is [n_perms][N] and may be NULL */
+int pansim_gene_accumulation(pansim_ctx *ctx, uint64_t seed, uint32_t n_perms, uint32_t *orders, uint32_t *pan,
+                             uint32_t *core, uint32_t *new_genes, uint32_t *unique);
+/* measurement: the order draw and the accumulation (zeroed counts, chunk summaries, walk, curves), each `repeats`
+ * times after one warm-up call; mean device ms of one pass (CUDA events); bytes_read = n_perms * N * ceil(G/32) * 4,
+ * the rows as the walk reads them */
+int pansim_gene_accumulation_kernel_ms(pansim_ctx *ctx, uint64_t seed, uint32_t n_perms, uint32_t repeats,
+                                       float *order_ms, float *accum_ms, uint64_t *bytes_read);
+/* spectrum[N + 1] as above (presence counts of acc_gene_counts_kernel, binned on the device) */
+int pansim_gene_spectrum(pansim_ctx *ctx, uint64_t *spectrum);
+/* out = { core, soft core, shell, cloud, total } of a spectrum[pop_size + 1]; needs no device, so every host prints
+ * the same numbers */
+void pansim_pangenome_classes(const uint64_t *spectrum, uint32_t pop_size, uint64_t out[5]);
+
 /* ---- clonal genealogy (extension: the reference keeps no pedigree) -------
  * The parent vectors the generations were drawn with, recorded on the device, and the genealogy of the present
  * population traced from them (DESIGN.md section 13). Both populations share it: next_generation gathers the core and
@@ -497,6 +539,12 @@ int pansim_group_core_ld(pansim_group *g, const pansim_ld_params *p, pansim_ld_b
  * communicator every rank computes the same whole result; nothing is exchanged. */
 int pansim_group_gene_ld(pansim_group *g, const pansim_gene_ld_params *p, pansim_gene_ld_class classes[3],
                          uint64_t *hist, uint64_t genes_used[2]);
+
+/* pansim_gene_accumulation and pansim_gene_spectrum of the group: the accessory matrix is replicated, so shard 0
+ * answers. Under a communicator every rank computes the same whole result; nothing is exchanged. */
+int pansim_group_gene_accumulation(pansim_group *g, uint64_t seed, uint32_t n_perms, uint32_t *orders, uint32_t *pan,
+                                   uint32_t *core, uint32_t *new_genes, uint32_t *unique);
+int pansim_group_gene_spectrum(pansim_group *g, uint64_t *spectrum);
 
 /* the clonal genealogy of the group: every shard draws the same parents, so shard 0 records and answers. Under a
  * communicator (one process per GPU) every rank records its own identical copy; nothing is exchanged. */

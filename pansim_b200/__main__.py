@@ -6,7 +6,7 @@ f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
 accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
 --print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy, --print_fasta, --print_snp_alignment,
---print_gene_ld, --gene_ld_bins, --gene_ld_min_minor.
+--print_gene_ld, --gene_ld_bins, --gene_ld_min_minor, --print_gene_accumulation, --gene_accumulation_perms.
 """
 from __future__ import annotations
 
@@ -89,6 +89,13 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--gene_ld_bins", type=int, default=20, help="(extension) r^2 histogram bins of --print_gene_ld (1..1024)")
     ap.add_argument("--gene_ld_min_minor", type=int, default=1,
                     help="(extension) --print_gene_ld uses genes present in at least this many rows and absent from at least this many")
+    ap.add_argument("--print_gene_accumulation", action="store_true",
+                    help="(extension) Roary's pangenome summaries of the last generation: <outpref>_number_of_genes_in_pan_genome"
+                         ".Rtab, _number_of_conserved_genes.Rtab, _number_of_new_genes.Rtab, _number_of_unique_genes.Rtab (one "
+                         "line per random order of the genomes, keyed by --seed); <outpref>_gene_spectrum.txt; "
+                         "<outpref>_summary_statistics.txt (core, soft-core, shell, cloud genes)")
+    ap.add_argument("--gene_accumulation_perms", type=int, default=100,
+                    help="(extension) random orders of --print_gene_accumulation (1..10000)")
     return ap
 
 
@@ -102,7 +109,8 @@ def main(argv=None) -> int:
     print_fasta = ns.pop("print_fasta")
     print_snp_alignment = ns.pop("print_snp_alignment")
     ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
-    ld.update({k: ns.pop(k) for k in ("print_gene_ld", "gene_ld_bins", "gene_ld_min_minor")})
+    ld.update({k: ns.pop(k) for k in ("print_gene_ld", "gene_ld_bins", "gene_ld_min_minor", "print_gene_accumulation",
+                                      "gene_accumulation_perms")})
     p = Params(**ns)
     run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf,
         print_genealogy=print_genealogy, print_fasta=print_fasta, print_snp_alignment=print_snp_alignment, **ld)

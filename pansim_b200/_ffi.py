@@ -36,6 +36,8 @@ EXPORTED = [
     "pansim_write_core_fasta", "pansim_export_core_fasta_rows", "pansim_group_write_core_fasta", "pansim_core_fasta_kernel_ms",
     "pansim_core_ld", "pansim_group_core_ld", "pansim_core_ld_kernel_ms", "pansim_ld_mean_r2",
     "pansim_gene_ld", "pansim_group_gene_ld", "pansim_gene_ld_kernel_ms",
+    "pansim_gene_accumulation", "pansim_group_gene_accumulation", "pansim_gene_accumulation_kernel_ms",
+    "pansim_gene_spectrum", "pansim_group_gene_spectrum", "pansim_pangenome_classes",
     "pansim_enable_genealogy", "pansim_genealogy", "pansim_genealogy_history", "pansim_genealogy_tmrca",
     "pansim_genealogy_newick", "pansim_group_enable_genealogy", "pansim_group_genealogy", "pansim_group_genealogy_tmrca",
 ]
@@ -248,6 +250,13 @@ def lib():
     sig("pansim_group_gene_ld", cint, vp, C.POINTER(GeneLdParams), C.POINTER(GeneLdClass), vp, vp)
     sig("pansim_gene_ld_kernel_ms", cint, vp, C.POINTER(GeneLdParams), u32, C.POINTER(C.c_float), C.POINTER(C.c_float),
         C.POINTER(C.c_float), C.POINTER(C.c_uint64))
+    sig("pansim_gene_accumulation", cint, vp, C.c_uint64, u32, vp, vp, vp, vp, vp)
+    sig("pansim_group_gene_accumulation", cint, vp, C.c_uint64, u32, vp, vp, vp, vp, vp)
+    sig("pansim_gene_accumulation_kernel_ms", cint, vp, C.c_uint64, u32, u32, C.POINTER(C.c_float), C.POINTER(C.c_float),
+        C.POINTER(C.c_uint64))
+    sig("pansim_gene_spectrum", cint, vp, vp)
+    sig("pansim_group_gene_spectrum", cint, vp, vp)
+    sig("pansim_pangenome_classes", None, vp, u32, vp)
     sig("pansim_enable_genealogy", cint, vp, u32)
     sig("pansim_genealogy", cint, vp, vp, C.POINTER(GenealogyInfo))
     sig("pansim_genealogy_history", cint, vp, vp)

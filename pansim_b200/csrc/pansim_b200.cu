@@ -25,6 +25,7 @@
 #include "genealogy.cuh"
 #include "ld.cuh"
 #include "pack.cuh"
+#include "pangenome.cuh"
 #include "replay.cuh"
 #include "select.cuh"
 #include "vcf.cuh"
@@ -301,6 +302,16 @@ struct pansim_ctx {
         unsigned long long *block = nullptr, *out = nullptr, *h_out = nullptr;
         size_t x_cap = 0, out_cap = 0;
     } gl;
+    // pangenome accumulation (pangenome.cuh): the orders, the per-step deltas (also the swap indices of an order draw
+    // that does not fit in shared memory), the chunk summaries and the four curves, sized for perm_cap orders; the
+    // gene frequency spectrum
+    struct GeneAccBuf {
+        uint32_t *orders = nullptr, *delta = nullptr, *summary = nullptr, *curves = nullptr;
+        size_t perm_cap = 0, summary_cap = 0;
+        unsigned long long *spectrum = nullptr;
+        int walk_slots = 0;          // resident walk CTAs of the device (per SM x SMs), queried on first use
+        int order_smem_max = 0;      // shared memory a CTA can opt in to (the order draw's limit), queried on first use
+    } ga;
     // clonal genealogy (genealogy.cuh): a ring of the last gen_cap parent vectors, each copied on stream_gen behind
     // ev_parents[i]; next_parents_buffer waits on ev_gen_done[i] before buffer i is rewritten. The trace and the
     // TMRCA walk run on stream_gen too, so they follow every copy enqueued before them.
@@ -1173,6 +1184,8 @@ void pansim_destroy(pansim_ctx *c)
         for (void *p : gp)
             if (p) cudaFree(p);
         if (c->gl.h_out) cudaFreeHost(c->gl.h_out);
+        for (void *p : {(void *)c->ga.orders, (void *)c->ga.delta, (void *)c->ga.summary, (void *)c->ga.curves, (void *)c->ga.spectrum})
+            if (p) cudaFree(p);
     }
     if (c->stream_gen) { cudaStreamSynchronize(c->stream_gen); cudaStreamDestroy(c->stream_gen); }
     for (auto e : c->ev_gen_done) if (e) cudaEventDestroy(e);
@@ -3834,6 +3847,202 @@ int pansim_gene_ld_kernel_ms(pansim_ctx *c, const pansim_gene_ld_params *p, uint
     if (pair_ms) *pair_ms = t[2] / (float)repeats;
     if (pairs) *pairs = cls[0].ld.pairs + cls[1].ld.pairs + cls[2].ld.pairs;
     return 0;
+}
+
+// ---- pangenome accumulation and gene frequency spectrum (pangenome.cuh, DESIGN.md section 16) ------------------
+static_assert(PG_ORDER_TAG == PANSIM_GENE_ACC_ORDER_TAG, "the order draw's counter word is documented in the header");
+static_assert(PANSIM_GENE_ACC_MAX_PERMS <= 65535u, "orders are grid.z of the walk");
+// Chunks of the N steps of an order: one, unless the word slices x orders leave resident walk CTAs unused; then as
+// many as fill at most one wave of them (a partial second wave would run at a fraction of the SMs), each chunk at
+// least 256 steps and a whole number of batches.
+static void gene_acc_plan(const pansim_ctx *c, uint32_t P, uint32_t *chunk_rows, uint32_t *n_chunks)
+{
+    const uint64_t base = (uint64_t)div_up64(c->acc_words, PG_SLICE_WORDS) * P, slots = (uint64_t)std::max(1, c->ga.walk_slots);
+    uint64_t chunks = 1;
+    if (base && base < slots) chunks = std::max<uint64_t>(1, std::min<uint64_t>(slots / base, c->N / 256));
+    *chunk_rows = div_up64(div_up64(c->N, chunks), PG_BATCH) * PG_BATCH;
+    *n_chunks = div_up64(c->N, *chunk_rows);
+}
+
+// orders, deltas and curves for P orders (kept with the context, grown when P grows) and the chunk summaries
+static int gene_acc_ensure(pansim_ctx *c, uint32_t P, uint32_t n_chunks)
+{
+    auto &b = c->ga;
+    if (P > b.perm_cap) {
+        for (uint32_t **q : {&b.orders, &b.delta, &b.curves})
+            if (*q) { cudaFree(*q); *q = nullptr; }
+        b.perm_cap = 0;
+        const size_t pn = (size_t)P * c->N * sizeof(uint32_t);
+        if (cudaMalloc(&b.orders, pn) != cudaSuccess || cudaMalloc(&b.delta, pn * PG_STATS) != cudaSuccess ||
+            cudaMalloc(&b.curves, pn * 4) != cudaSuccess) {
+            cudaGetLastError();
+            FAIL(c, PANSIM_ERR_NOMEM, "cudaMalloc of %zu bytes (gene accumulation, %u orders) failed", pn * 8, P);
+        }
+        b.perm_cap = P;
+    }
+    const size_t words = n_chunks > 1 ? (size_t)P * n_chunks * 3 * c->acc_words : 0;
+    if (words > b.summary_cap) {
+        if (b.summary) cudaFree(b.summary);
+        b.summary = nullptr; b.summary_cap = 0;
+        if (cudaMalloc(&b.summary, words * sizeof(uint32_t)) != cudaSuccess) {
+            cudaGetLastError();
+            FAIL(c, PANSIM_ERR_NOMEM, "cudaMalloc of %zu bytes (gene accumulation chunk summaries) failed", words * 4);
+        }
+        b.summary_cap = words;
+    }
+    return 0;
+}
+
+// P orders into ga.orders; the swap indices go to shared memory when 8 N bytes fit, else to ga.delta
+static int gene_acc_orders(pansim_ctx *c, uint64_t seed, uint32_t P)
+{
+    PgOrderArgs a;
+    a.rk = philox_key_schedule(make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+    a.n_rows = c->N;
+    a.orders = c->ga.orders;
+    a.scratch = c->ga.delta;
+    const size_t smem = 2 * (size_t)c->N * sizeof(uint32_t);
+    if (smem <= (size_t)c->ga.order_smem_max) {
+        pg_order_kernel<true><<<P, PG_ORDER_THREADS, smem, c->stream>>>(a);
+    } else {
+        pg_order_kernel<false><<<P, PG_ORDER_THREADS, 0, c->stream>>>(a);
+    }
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// the walk over the orders in ga.orders (zeroed deltas, chunk summaries, walk) and the curves
+static int gene_acc_accumulate(pansim_ctx *c, uint32_t P, uint32_t chunk_rows, uint32_t n_chunks)
+{
+    auto &b = c->ga;
+    const size_t pn = (size_t)P * c->N;
+    CU(c, cudaMemsetAsync(b.delta, 0, pn * PG_STATS * sizeof(uint32_t), c->stream));
+    if (c->G) {
+        PgWalkArgs a;
+        a.state = c->acc[c->acc_cur];
+        a.stride_words = c->acc_stride_words;
+        a.n_words = c->acc_words;
+        a.n_genes = c->G;
+        a.n_rows = c->N;
+        a.orders = b.orders;
+        a.chunk_rows = chunk_rows;
+        a.n_chunks = n_chunks;
+        a.summary = b.summary;
+        a.delta = b.delta;
+        const uint32_t slices = div_up64(c->acc_words, PG_SLICE_WORDS);
+        if (n_chunks > 1) {
+            pg_summary_kernel<<<dim3(slices, n_chunks - 1, P), PG_SLICE_WORDS, 0, c->stream>>>(a);
+            LAUNCH_CHECK(c);
+        }
+        pg_walk_kernel<<<dim3(slices, n_chunks, P), PG_SLICE_WORDS, 0, c->stream>>>(a);
+        LAUNCH_CHECK(c);
+    }
+    PgCurveArgs q;
+    q.delta = b.delta;
+    q.n_rows = c->N;
+    q.c0 = c->cfg.core_genes;
+    q.pan = b.curves;
+    q.core = b.curves + pn;
+    q.new_genes = b.curves + 2 * pn;
+    q.unique = b.curves + 3 * pn;
+    pg_curves_kernel<<<P, PG_SCAN_THREADS, 0, c->stream>>>(q);
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// Refusals leave the context as it was.
+static int gene_acc_prepare(pansim_ctx *c, uint32_t n_perms, uint32_t *chunk_rows, uint32_t *n_chunks)
+{
+    if (!n_perms || n_perms > PANSIM_GENE_ACC_MAX_PERMS)
+        FAIL(c, PANSIM_ERR_INVALID, "gene accumulation: n_perms must be 1..%u", PANSIM_GENE_ACC_MAX_PERMS);
+    if (!c->has_acc) FAIL(c, PANSIM_ERR_STATE, "gene accumulation: no accessory state: call pansim_set_initial or pansim_upload_acc first");
+    CU(c, cudaSetDevice(c->cfg.device));
+    if (!c->ga.walk_slots) {       // device limits of the launches, once per context
+        int per_sm = 0;
+        CU(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pg_walk_kernel, PG_SLICE_WORDS, 0));
+        CU(c, cudaDeviceGetAttribute(&c->ga.order_smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->cfg.device));
+        CU(c, cudaFuncSetAttribute(pg_order_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->ga.order_smem_max));
+        c->ga.walk_slots = std::max(1, per_sm) * std::max(1, c->sm_count);
+    }
+    gene_acc_plan(c, n_perms, chunk_rows, n_chunks);
+    return gene_acc_ensure(c, n_perms, *n_chunks);
+}
+
+int pansim_gene_accumulation(pansim_ctx *c, uint64_t seed, uint32_t n_perms, uint32_t *orders, uint32_t *pan, uint32_t *core,
+                             uint32_t *new_genes, uint32_t *unique)
+{
+    if (!c) return PANSIM_ERR_INVALID;
+    uint32_t chunk_rows = 0, n_chunks = 0;
+    if (int rc = gene_acc_prepare(c, n_perms, &chunk_rows, &n_chunks)) return rc;
+    if (int rc = gene_acc_orders(c, seed, n_perms)) return rc;
+    if (int rc = gene_acc_accumulate(c, n_perms, chunk_rows, n_chunks)) return rc;
+    const size_t pn = (size_t)n_perms * c->N;
+    if (orders) CU(c, cudaMemcpyAsync(orders, c->ga.orders, pn * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    uint32_t *out[4] = {pan, core, new_genes, unique};
+    for (int k = 0; k < 4; k++)
+        if (out[k]) CU(c, cudaMemcpyAsync(out[k], c->ga.curves + k * pn, pn * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int pansim_gene_accumulation_kernel_ms(pansim_ctx *c, uint64_t seed, uint32_t n_perms, uint32_t repeats, float *order_ms,
+                                       float *accum_ms, uint64_t *bytes_read)
+{
+    if (!c || !repeats) return PANSIM_ERR_INVALID;
+    if (int rc = pansim_gene_accumulation(c, seed, n_perms, nullptr, nullptr, nullptr, nullptr, nullptr)) return rc;   // also the warm-up
+    uint32_t chunk_rows = 0, n_chunks = 0;
+    gene_acc_plan(c, n_perms, &chunk_rows, &n_chunks);
+    cudaEvent_t ev[3];
+    for (auto &e : ev) CU(c, cudaEventCreate(&e));
+    int rc = 0;
+    cudaEventRecord(ev[0], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++) rc = gene_acc_orders(c, seed, n_perms);
+    cudaEventRecord(ev[1], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++) rc = gene_acc_accumulate(c, n_perms, chunk_rows, n_chunks);
+    cudaEventRecord(ev[2], c->stream);
+    const cudaError_t e = cudaEventSynchronize(ev[2]);
+    float t[2] = {0.f, 0.f};
+    for (int k = 0; k < 2; k++) cudaEventElapsedTime(&t[k], ev[k], ev[k + 1]);
+    for (auto &x : ev) cudaEventDestroy(x);
+    if (rc) return rc;
+    if (e != cudaSuccess) FAIL(c, PANSIM_ERR_CUDA, "gene accumulation kernels failed: %s", cudaGetErrorString(e));
+    if (order_ms) *order_ms = t[0] / (float)repeats;
+    if (accum_ms) *accum_ms = t[1] / (float)repeats;
+    if (bytes_read) *bytes_read = (uint64_t)n_perms * c->N * c->acc_words * sizeof(uint32_t);
+    return 0;
+}
+
+int pansim_gene_spectrum(pansim_ctx *c, uint64_t *spectrum)
+{
+    if (!c || !spectrum) return PANSIM_ERR_INVALID;
+    if (!c->has_acc) FAIL(c, PANSIM_ERR_STATE, "gene spectrum: no accessory state: call pansim_set_initial or pansim_upload_acc first");
+    CU(c, cudaSetDevice(c->cfg.device));
+    const size_t bytes = ((size_t)c->N + 1) * sizeof(unsigned long long);
+    if (!c->ga.spectrum) CU(c, cudaMalloc(&c->ga.spectrum, bytes));
+    CU(c, cudaMemsetAsync(c->ga.spectrum, 0, bytes, c->stream));
+    if (c->G) {
+        acc_gene_counts_kernel<<<c->acc_words, 256, 0, c->stream>>>(c->acc[c->acc_cur], c->N, c->G, c->acc_stride_words, c->d_gain_thr);
+        LAUNCH_CHECK(c);
+        pg_spectrum_kernel<<<div_up64(c->G, 256), 256, 0, c->stream>>>(c->d_gain_thr, c->G, c->ga.spectrum);
+        LAUNCH_CHECK(c);
+    }
+    CU(c, cudaMemcpyAsync(spectrum, c->ga.spectrum, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    spectrum[c->N] += c->cfg.core_genes;
+    return 0;
+}
+
+void pansim_pangenome_classes(const uint64_t *spectrum, uint32_t pop_size, uint64_t out[5])
+{
+    if (!out) return;
+    for (int k = 0; k < 5; k++) out[k] = 0;
+    if (!spectrum) return;
+    const uint64_t n = pop_size;
+    for (uint64_t a = 1; a <= n; a++) {
+        const uint64_t h = 100 * a;
+        out[h >= 99 * n ? 0 : h >= 95 * n ? 1 : h >= 15 * n ? 2 : 3] += spectrum[a];
+    }
+    out[4] = out[0] + out[1] + out[2] + out[3];
 }
 
 // ---- clonal genealogy (genealogy.cuh, DESIGN.md section 13) ------------------

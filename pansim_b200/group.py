@@ -13,8 +13,9 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import (OK, CoreFasta, CoreLD, GeneLD, Genealogy, PansimError, _core_ld, _diversity, _gene_ld, _genealogy,
-                         _genealogy_history, _ld_bins, _ld_params, _pairs_or_none, _ptr, _tmrca, _write_fasta, make_config)
+from .population import (OK, CoreFasta, CoreLD, GeneAccumulation, GeneLD, Genealogy, PansimError, _core_ld, _diversity,
+                         _gene_accumulation, _gene_ld, _gene_spectrum, _genealogy, _genealogy_history, _ld_bins, _ld_params,
+                         _pairs_or_none, _ptr, _tmrca, _write_fasta, make_config)
 
 
 class PansimGroup:
@@ -152,6 +153,16 @@ class PansimGroup:
     def gene_ld(self, r2_bins: int = 20, min_minor: int = 1) -> GeneLD:
         """Accessory-gene linkage (Pansim.gene_ld): the accessory matrix is replicated, so shard 0 answers."""
         return _gene_ld(lambda *a: self._lib.pansim_group_gene_ld(self._h, *a), self._check, r2_bins, min_minor)
+
+    def gene_accumulation(self, n_perms: int = 100, seed: int | None = None) -> GeneAccumulation:
+        """Pangenome accumulation curves (Pansim.gene_accumulation): the accessory matrix is replicated, so shard 0
+        answers."""
+        return _gene_accumulation(lambda *a: self._lib.pansim_group_gene_accumulation(self._h, *a), self._check, self.N,
+                                  n_perms, self.cfg.seed if seed is None else seed)
+
+    def gene_spectrum(self) -> np.ndarray:
+        """The gene frequency spectrum (Pansim.gene_spectrum), answered by shard 0."""
+        return _gene_spectrum(lambda *a: self._lib.pansim_group_gene_spectrum(self._h, *a), self._check, self.N)
 
     def enable_genealogy(self, capacity: int):
         """Pansim.enable_genealogy for the group: shard 0 records (every shard draws the same parents)."""

@@ -43,17 +43,21 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
                              "prop_genes2", "prop_positive", "pos_lambda", "neg_lambda", "seed", "outpref",
                              "threads", "genome_size_penalty", "competition_strength", "device", "gpus",
                              "ld_max_dist", "ld_bin_width", "ld_min_minor",        // extensions: --print_ld bins,
-                             "gene_ld_bins", "gene_ld_min_minor"};                 // --print_gene_ld histogram and genes
+                             "gene_ld_bins", "gene_ld_min_minor",                  // --print_gene_ld histogram and genes,
+                             "gene_accumulation_perms"};                           // --print_gene_accumulation orders
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
                               "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy",
-                              "print_fasta", "print_snp_alignment", "print_gene_ld"};   // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "print_fasta", "print_snp_alignment", "print_gene_ld",
+                              "print_gene_accumulation"};                     // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
                                                                               // print_vcf (<outpref>_core_genome.vcf),
                                                                               // print_ld (<outpref>_core_ld.tsv),
                                                                               // print_genealogy (<outpref>_genealogy.nwk, <outpref>_tmrca.tsv),
                                                                               // print_fasta (<outpref>_core_genome.fasta),
                                                                               // print_snp_alignment (<outpref>_core_snps.fasta, <outpref>_core_snps_fconst.txt),
-                                                                              // print_gene_ld (<outpref>_gene_ld.tsv)
+                                                                              // print_gene_ld (<outpref>_gene_ld.tsv),
+                                                                              // print_gene_accumulation (<outpref>_number_of_*.Rtab,
+                                                                              //   <outpref>_gene_spectrum.txt, <outpref>_summary_statistics.txt)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -64,7 +68,7 @@ bool parse(int argc, char **argv, Flags &f)
              {"seed", "0"}, {"outpref", "distances"}, {"threads", "1"}, {"genome_size_penalty", "0.99"},
              {"competition_strength", "0.0"}, {"device", "0"}, {"gpus", "1"},
              {"ld_max_dist", "10000"}, {"ld_bin_width", "100"}, {"ld_min_minor", "1"},
-             {"gene_ld_bins", "20"}, {"gene_ld_min_minor", "1"}};
+             {"gene_ld_bins", "20"}, {"gene_ld_min_minor", "1"}, {"gene_accumulation_perms", "100"}};
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         if (a == "--help" || a == "-h") {
@@ -144,6 +148,8 @@ int main(int argc, char **argv)
                                         (uint32_t)std::strtoul(fl.val["ld_bin_width"].c_str(), nullptr, 10),
                                         (uint32_t)std::strtoul(fl.val["ld_min_minor"].c_str(), nullptr, 10)};
     const bool print_gene_ld = fl.sw["print_gene_ld"];
+    const bool print_gene_accumulation = fl.sw["print_gene_accumulation"];
+    const uint32_t gene_accumulation_perms = (uint32_t)std::strtoul(fl.val["gene_accumulation_perms"].c_str(), nullptr, 10);
     const pansim_gene_ld_params gene_ld_params = {(uint32_t)std::strtoul(fl.val["gene_ld_bins"].c_str(), nullptr, 10),
                                                   (uint32_t)std::strtoul(fl.val["gene_ld_min_minor"].c_str(), nullptr, 10)};
     const int n_gpus = std::max(1, std::atoi(fl.val["gpus"].c_str()));       // extension: column shards over N devices of the box
@@ -343,6 +349,30 @@ int main(int argc, char **argv)
                 for (uint32_t b = 0; b < gene_ld_params.r2_bins; b++) f << "\t" << hist[(size_t)k * gene_ld_params.r2_bins + b];
                 f << "\n";
             }
+        }
+        if (print_gene_accumulation) {                                      // extension: Roary's pangenome summaries
+            const auto acc = pops.gene_accumulation(seed, gene_accumulation_perms);
+            const size_t N = pop_size;
+            const std::pair<const char *, const std::vector<uint32_t> *> curves[4] = {
+                {"genes_in_pan_genome", &acc.pan}, {"conserved_genes", &acc.core}, {"new_genes", &acc.new_genes},
+                {"unique_genes", &acc.unique}};
+            for (const auto &c : curves) {
+                std::ofstream f(outpref + "_number_of_" + c.first + ".Rtab");
+                for (size_t p = 0; p < gene_accumulation_perms; p++)
+                    for (size_t k = 0; k < N; k++) f << (*c.second)[p * N + k] << (k + 1 < N ? "\t" : "\n");
+            }
+            const std::vector<uint64_t> spectrum = pops.gene_spectrum();
+            {
+                std::ofstream f(outpref + "_gene_spectrum.txt");
+                for (uint64_t x : spectrum) f << x << "\n";
+            }
+            uint64_t cls[5];
+            pansim_pangenome_classes(spectrum.data(), (uint32_t)N, cls);
+            const char *label[5] = {"Core genes\t(99% <= strains <= 100%)", "Soft core genes\t(95% <= strains < 99%)",
+                                    "Shell genes\t(15% <= strains < 95%)", "Cloud genes\t(0% <= strains < 15%)",
+                                    "Total genes\t(0% <= strains <= 100%)"};
+            std::ofstream f(outpref + "_summary_statistics.txt");
+            for (int k = 0; k < 5; k++) f << label[k] << "\t" << cls[k] << "\n";
         }
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)

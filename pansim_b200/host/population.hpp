@@ -213,6 +213,26 @@ public:
         return cls;
     }
 
+    // (extension) pangenome accumulation curves over n_perms random orders of the rows drawn from seed, each
+    // [n_perms][N] row-major; the accessory matrix is replicated, so shard 0 answers
+    struct GeneAccumulation { std::vector<uint32_t> orders, pan, core, new_genes, unique; };
+    GeneAccumulation gene_accumulation(uint64_t seed, uint32_t n_perms)
+    {
+        GeneAccumulation r;
+        const size_t n = n_perms <= PANSIM_GENE_ACC_MAX_PERMS ? (size_t)n_perms * cfg_.pop_size : 0;
+        for (auto *v : {&r.orders, &r.pan, &r.core, &r.new_genes, &r.unique}) v->assign(n, 0);
+        gcheck(pansim_group_gene_accumulation(grp_, seed, n_perms, r.orders.data(), r.pan.data(), r.core.data(),
+                                              r.new_genes.data(), r.unique.data()));
+        return r;
+    }
+    // (extension) the gene frequency spectrum [N + 1]: genes carried by k rows, core_genes in bin N
+    std::vector<uint64_t> gene_spectrum()
+    {
+        std::vector<uint64_t> s((size_t)cfg_.pop_size + 1);
+        gcheck(pansim_group_gene_spectrum(grp_, s.data()));
+        return s;
+    }
+
     // (extension) record the parent vector of every generation from now on, the last `capacity` kept (0: off)
     void enable_genealogy(uint32_t capacity) { gcheck(pansim_group_enable_genealogy(grp_, capacity)); }
     // (extension) the clonal genealogy of the present population: the node table, and its summary if info is non-null

@@ -174,6 +174,50 @@ def _gene_ld(call, check, r2_bins: int, min_minor: int) -> GeneLD:
                   np.array([lib.pansim_ld_mean_r2(C.byref(c.ld)) for c in cls], np.float64), hist, used)
 
 
+GENE_ACC_MAX_PERMS = 10000      # PANSIM_GENE_ACC_MAX_PERMS
+
+
+class GeneAccumulation(NamedTuple):
+    """Pangenome accumulation curves of pansim_gene_accumulation (include/pansim_b200.h), each uint32 [P, N]: the
+    random orders of the rows, and per order and number of genomes k = 1..N the pan genes, the core (conserved)
+    genes, the new genes and the unique genes (Roary's four .Rtab curves). The core_genes count in pan and core at
+    every k, and in new and unique at k = 1."""
+    orders: np.ndarray
+    pan: np.ndarray
+    core: np.ndarray
+    new: np.ndarray
+    unique: np.ndarray
+
+
+def _gene_accumulation(call, check, N: int, n_perms: int, seed: int) -> GeneAccumulation:
+    """call(seed, n_perms, orders, pan, core, new, unique) -> status; the arrays are only sized for a valid n_perms
+    (the library refuses the others before writing)."""
+    P = n_perms if 1 <= n_perms <= GENE_ACC_MAX_PERMS else 0
+    out = [np.empty((P, N), np.uint32) for _ in range(5)]
+    check(call(seed, n_perms, *[_ptr(a) for a in out]))
+    return GeneAccumulation(*out)
+
+
+def _gene_spectrum(call, check, N: int) -> np.ndarray:
+    out = np.empty(N + 1, np.uint64)
+    check(call(_ptr(out)))
+    return out
+
+
+PANGENOME_CLASSES = ("core", "soft_core", "shell", "cloud", "total")
+
+
+def pangenome_classes(spectrum, pop_size: int) -> tuple[int, int, int, int, int]:
+    """(core, soft core, shell, cloud, total) genes of a gene frequency spectrum [pop_size + 1] by Roary's
+    thresholds as integer tests, evaluated by the library (pansim_pangenome_classes) so every host prints the same."""
+    spec = np.ascontiguousarray(spectrum, np.uint64)
+    if spec.shape != (pop_size + 1,):
+        raise ValueError(f"spectrum must have pop_size + 1 = {pop_size + 1} bins, not {spec.shape}")
+    out = np.zeros(5, np.uint64)
+    _ffi.lib().pansim_pangenome_classes(_ptr(spec), pop_size, _ptr(out))
+    return tuple(int(x) for x in out)
+
+
 class Genealogy(NamedTuple):
     """The clonal genealogy of the present population (pansim_genealogy, include/pansim_b200.h): per node its parent
     (0xFFFFFFFF at the root), the individual it stands for (0xFFFFFFFF at a virtual root) and its time in generations
@@ -545,6 +589,24 @@ class Pansim:
                                                        C.byref(g), C.byref(t), C.byref(q), C.byref(n)))
         return g.value, t.value, q.value, n.value
 
+    # -- pangenome accumulation (extension) ---------------------------------
+    def gene_accumulation(self, n_perms: int = 100, seed: int | None = None) -> GeneAccumulation:
+        """Pan, core, new and unique genes against the number of genomes over n_perms random orders of the rows,
+        the orders drawn on the device from `seed` (None: the context's seed) (pansim_gene_accumulation)."""
+        return _gene_accumulation(lambda *a: self._lib.pansim_gene_accumulation(self._h, *a), self._check, self.N, n_perms,
+                                  self.cfg.seed if seed is None else seed)
+
+    def gene_accumulation_kernel_ms(self, n_perms: int = 100, seed: int | None = None, repeats: int = 10):
+        """Measurement: device ms of one order draw and of one accumulation, and the row bytes the walk reads."""
+        o, a, n = C.c_float(), C.c_float(), C.c_uint64()
+        self._check(self._lib.pansim_gene_accumulation_kernel_ms(self._h, self.cfg.seed if seed is None else seed, n_perms,
+                                                                 repeats, C.byref(o), C.byref(a), C.byref(n)))
+        return o.value, a.value, n.value
+
+    def gene_spectrum(self) -> np.ndarray:
+        """uint64 [N + 1]: the accessory genes carried by k rows, the core_genes added to bin N (pansim_gene_spectrum)."""
+        return _gene_spectrum(lambda *a: self._lib.pansim_gene_spectrum(self._h, *a), self._check, self.N)
+
     # -- clonal genealogy (extension) ---------------------------------------
     def enable_genealogy(self, capacity: int):
         """Record the parent vector of every generation from now on, keeping the last `capacity` (0: stop and free)."""
@@ -732,5 +794,5 @@ class Pansim:
                 f.write(",".join(ones + [str(int(x)) for x in acc[r]]) + "\n")
 
 
-__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "GeneLD", "Genealogy", "genealogy_newick",
-           "make_config", "standard_deviation", "fmt_f64"]
+__all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "GeneLD", "GeneAccumulation",
+           "pangenome_classes", "Genealogy", "genealogy_newick", "make_config", "standard_deviation", "fmt_f64"]

@@ -17,7 +17,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from .params import Derived, Params, derive, fmt_f64, validate
-from .population import Pansim, diversity_stats, standard_deviation
+from .population import Pansim, diversity_stats, pangenome_classes, standard_deviation
 
 
 def selection_coefficients(p: Params, pan_size: int, rng: np.random.Generator) -> np.ndarray:
@@ -63,6 +63,8 @@ class RunResult:
     sfs: np.ndarray = None                        # SFS of the last generation (--print_diversity)
     ld: object = None                             # CoreLD of the last generation (--print_ld)
     gene_ld: object = None                        # GeneLD of the last generation (--print_gene_ld)
+    gene_accumulation: object = None              # GeneAccumulation of the last generation (--print_gene_accumulation)
+    gene_spectrum: np.ndarray = None              # gene frequency spectrum of the last generation (--print_gene_accumulation)
     genealogy: object = None                      # Genealogy of the last generation (--print_genealogy)
     tmrca: np.ndarray = None                      # TMRCA of the sampled pairs (--print_genealogy without --all_pairs)
     selection: np.ndarray = None
@@ -73,7 +75,8 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
         print_diversity: bool = False, print_vcf: bool = False, print_ld: bool = False, ld_max_dist: int = 10000,
         ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False, print_fasta: bool = False,
         print_snp_alignment: bool = False, print_gene_ld: bool = False, gene_ld_bins: int = 20,
-        gene_ld_min_minor: int = 1) -> RunResult | None:
+        gene_ld_min_minor: int = 1, print_gene_accumulation: bool = False,
+        gene_accumulation_perms: int = 100) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -93,7 +96,11 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     are present) with `<outpref>_core_snps_fconst.txt`, the constant sites by letter as `nA,nC,nG,nT`
     (Pansim.write_core_fasta).
     print_gene_ld (extension): linkage of the accessory genes of the last generation as `<outpref>_gene_ld.tsv`,
-    written after every other output (Pansim.gene_ld with gene_ld_bins, gene_ld_min_minor; write_gene_ld)."""
+    written after every other output (Pansim.gene_ld with gene_ld_bins, gene_ld_min_minor; write_gene_ld).
+    print_gene_accumulation (extension): after every other output, Roary's pangenome summaries of the last generation:
+    the accumulation curves over gene_accumulation_perms random orders keyed by p.seed, the gene frequency spectrum
+    and the core / soft-core / shell / cloud counts (Pansim.gene_accumulation, Pansim.gene_spectrum;
+    write_gene_accumulation)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -207,7 +214,33 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             res.gene_ld = sim.gene_ld(gene_ld_bins, gene_ld_min_minor)
             if outpref:
                 write_gene_ld(outpref, res.gene_ld)
+        if print_gene_accumulation:
+            res.gene_accumulation = sim.gene_accumulation(gene_accumulation_perms, p.seed)
+            res.gene_spectrum = sim.gene_spectrum()
+            if outpref:
+                write_gene_accumulation(outpref, res.gene_accumulation, res.gene_spectrum)
     return res
+
+
+ROARY_CLASSES = ("Core genes\t(99% <= strains <= 100%)", "Soft core genes\t(95% <= strains < 99%)",
+                 "Shell genes\t(15% <= strains < 95%)", "Cloud genes\t(0% <= strains < 15%)",
+                 "Total genes\t(0% <= strains <= 100%)")
+
+
+def write_gene_accumulation(outpref: str, acc, spectrum):
+    """Roary's pangenome files: `<outpref>_number_of_genes_in_pan_genome.Rtab`, `_number_of_conserved_genes.Rtab`,
+    `_number_of_new_genes.Rtab` and `_number_of_unique_genes.Rtab` (one line per order, N tab-separated counts for
+    k = 1..N, no header); `<outpref>_gene_spectrum.txt` (N + 1 lines, genes carried by k rows); and
+    `<outpref>_summary_statistics.txt` (core, soft-core, shell, cloud and total genes, Roary's layout)."""
+    for name, curve in (("genes_in_pan_genome", acc.pan), ("conserved_genes", acc.core), ("new_genes", acc.new),
+                        ("unique_genes", acc.unique)):
+        with open(f"{outpref}_number_of_{name}.Rtab", "w") as f:
+            f.write("".join("\t".join(map(str, row.tolist())) + "\n" for row in curve))
+    with open(outpref + "_gene_spectrum.txt", "w") as f:
+        f.write("".join(f"{int(x)}\n" for x in spectrum))
+    classes = pangenome_classes(spectrum, len(spectrum) - 1)
+    with open(outpref + "_summary_statistics.txt", "w") as f:
+        f.write("".join(f"{label}\t{n}\n" for label, n in zip(ROARY_CLASSES, classes)))
 
 
 def write_gene_ld(outpref: str, gl):
