@@ -472,6 +472,52 @@ int pansim_genealogy_tmrca(pansim_ctx *ctx, const uint32_t *r1, const uint32_t *
 int pansim_genealogy_newick(const pansim_genealogy_node *nodes, uint32_t n_nodes, uint32_t n_leaves, char *out,
                             size_t cap, size_t *len);
 
+/* ---- parsimony on the true genealogy (extension) --------------------------
+ * How many changes each core site and each accessory gene needs on a rooted tree of the present rows (DESIGN.md
+ * section 17): the per-character, per-branch and summary counts of homoplasy tools, on the genealogy the run made.
+ * TREE. A node table parent[n_nodes]: leaves are nodes 0 .. N-1, leaf i = row i; every non-root node has a parent with
+ * a larger id (ascending ids visit children before parents); the root is the last node, parent 0xFFFFFFFF; every
+ * internal node has at least 2 children, so N <= n_nodes <= 2N - 1 (with N = 1 the single leaf is the root).
+ * pansim_genealogy's table satisfies this (pass its .parent column); any rooted tree over the rows does once it is
+ * renumbered in postorder. A table that breaks a rule -> PANSIM_ERR_INVALID (checked on the host).
+ * CHARACTERS. Core: every site of the context's local column range, state = the letter, A < C < G < T. Genes: the G
+ * matrix genes, state = absent < present. Padding (the tail of a row's last word, region padding, bits at or past G)
+ * never counts.
+ * SCORE (Hartigan 1973; Fitch 1971 on binary nodes). A leaf's set is {its state}. An internal node v with children
+ * u_1 .. u_k: n_x = |{j : x in S(u_j)}|, m_v = max_x n_x, S(v) = {x : n_x = m_v}, and v contributes k - m_v.
+ * score(c) = the sum over internal nodes = the least number of branches whose ends differ at c over all assignments
+ * of states to the internal nodes. A node with k >= 3 children is a hard polytomy: each child branch is a branch.
+ * SUMMARY. characters; variable = characters with >= 2 states among the leaves; tree_length S = sum of scores;
+ * min_changes M = sum (distinct states - 1); max_changes G = sum (N - max_x count_x), the score on a star tree;
+ * homoplastic = characters with score > distinct - 1. pansim_parsimony_indices (no device) forms CI = M / S and
+ * RI = (G - S) / (G - M), NaN where the denominator is 0, so every host prints the same bytes.
+ * RECONSTRUCTION (one optimal assignment, fixed by rule). The root takes the smallest state of S(root); a non-root
+ * internal node takes its parent's state if that is in its set, else the smallest state of its set; a leaf takes its
+ * own state. branch_changes[v] (core) = the characters whose state at v differs from the state at parent(v);
+ * gains[v] / losses[v] (genes) = the characters absent at the parent and present at v / the reverse. Root entries
+ * are 0. The rule is optimal (the cost of v's subtree and branch given the parent state y is s_v + [y not in S(v)]),
+ * so sum_v branch_changes[v] = S (core) and sum_v gains[v] + losses[v] = S (genes).
+ * Every output is an integer: no slab count, grid or shard split changes a bit. The state is read on the context's
+ * stream after every enqueued step (pending recombination applied first). Every output pointer may be NULL.
+ * Scratch: (n_nodes - N) x 16 bytes per column of 32 sites (core) or x 8 bytes per word of 32 genes, allocated for the
+ * call in slabs of columns under a budget (the smaller of 16 GiB and half the free device memory;
+ * PANSIM_PARSIMONY_SCRATCH_MB overrides it) and freed before it returns.
+ * Errors: no state (pansim_set_initial or pansim_upload_*) -> PANSIM_ERR_STATE; a bad table -> PANSIM_ERR_INVALID;
+ * scratch that cannot be allocated -> PANSIM_ERR_NOMEM. The context keeps working after a refused call. */
+typedef struct { uint64_t characters, variable, tree_length, min_changes, max_changes, homoplastic; } pansim_parsimony;
+int pansim_core_parsimony(pansim_ctx *ctx, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out,
+                          uint32_t *site_changes /* [local L] */, uint64_t *branch_changes /* [n_nodes] */);
+int pansim_gene_parsimony(pansim_ctx *ctx, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out,
+                          uint32_t *gene_changes /* [G] */, uint64_t *gains /* [n_nodes] */, uint64_t *losses /* [n_nodes] */);
+/* measurement: the parsimony kernels of one call (every slab; genes != 0: the gene pass) `repeats` times after one
+ * warm-up pass; mean device ms of one pass (CUDA events); bytes_read = columns x (2 N x row bytes of a column + (3 x
+ * internal nodes - 1) x set bytes), the rows and scratch as the walk reads them; slabs = the slabs of one pass.
+ * Any output may be NULL. */
+int pansim_parsimony_kernel_ms(pansim_ctx *ctx, const uint32_t *parent, uint32_t n_nodes, int genes, uint32_t repeats,
+                               float *ms, uint64_t *bytes_read, uint32_t *slabs);
+/* CI and RI of a summary (either may be NULL); needs no device */
+void pansim_parsimony_indices(const pansim_parsimony *p, double *ci, double *ri);
+
 /* ---- multi-GPU: column shards of one alignment --------------------------
  * (SURVEY.md 8e; the reference is one shared-memory process, population.rs has no analogue.)
  * Every shard context holds all individuals for [site_begin, site_end) and a replica of the
@@ -551,6 +597,15 @@ int pansim_group_gene_spectrum(pansim_group *g, uint64_t *spectrum);
 int pansim_group_enable_genealogy(pansim_group *g, uint32_t capacity);
 int pansim_group_genealogy(pansim_group *g, pansim_genealogy_node *nodes, pansim_genealogy_info *info);
 int pansim_group_genealogy_tmrca(pansim_group *g, const uint32_t *r1, const uint32_t *r2, size_t n_pairs, uint32_t *tmrca);
+
+/* parsimony of the group on a node table over its rows. Core: every shard answers for its columns; the summaries and
+ * branch changes are summed and site_changes holds the shards' sites concatenated in shard (= site) order. Genes: the
+ * accessory matrix is replicated, so shard 0 answers. Under a communicator a rank covers its own columns, as
+ * pansim_core_ld does; nothing is exchanged. */
+int pansim_group_core_parsimony(pansim_group *g, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out,
+                                uint32_t *site_changes, uint64_t *branch_changes);
+int pansim_group_gene_parsimony(pansim_group *g, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out,
+                                uint32_t *gene_changes, uint64_t *gains, uint64_t *losses);
 
 /* ---- introspection / instrumentation ----------------------------------- */
 typedef struct {

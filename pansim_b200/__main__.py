@@ -6,7 +6,8 @@ f64 and rounded (main.rs:155-167) so `--pop_size 1e3` works; max_distances,
 threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
 accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
 --print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy, --print_fasta, --print_snp_alignment,
---print_gene_ld, --gene_ld_bins, --gene_ld_min_minor, --print_gene_accumulation, --gene_accumulation_perms.
+--print_gene_ld, --gene_ld_bins, --gene_ld_min_minor, --print_gene_accumulation, --gene_accumulation_perms,
+--print_parsimony.
 """
 from __future__ import annotations
 
@@ -96,6 +97,10 @@ def build_parser() -> argparse.ArgumentParser:
                          "<outpref>_summary_statistics.txt (core, soft-core, shell, cloud genes)")
     ap.add_argument("--gene_accumulation_perms", type=int, default=100,
                     help="(extension) random orders of --print_gene_accumulation (1..10000)")
+    ap.add_argument("--print_parsimony", action="store_true",
+                    help="(extension) parsimony changes on the true genealogy of the last generation: <outpref>_parsimony.tsv "
+                         "(core and gene summaries with CI and RI), <outpref>_core_site_changes.txt, <outpref>_gene_changes.txt, "
+                         "<outpref>_branch_changes.tsv")
     return ap
 
 
@@ -110,7 +115,7 @@ def main(argv=None) -> int:
     print_snp_alignment = ns.pop("print_snp_alignment")
     ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
     ld.update({k: ns.pop(k) for k in ("print_gene_ld", "gene_ld_bins", "gene_ld_min_minor", "print_gene_accumulation",
-                                      "gene_accumulation_perms")})
+                                      "gene_accumulation_perms", "print_parsimony")})
     p = Params(**ns)
     run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf,
         print_genealogy=print_genealogy, print_fasta=print_fasta, print_snp_alignment=print_snp_alignment, **ld)

@@ -38,6 +38,8 @@ EXPORTED = [
     "pansim_gene_ld", "pansim_group_gene_ld", "pansim_gene_ld_kernel_ms",
     "pansim_gene_accumulation", "pansim_group_gene_accumulation", "pansim_gene_accumulation_kernel_ms",
     "pansim_gene_spectrum", "pansim_group_gene_spectrum", "pansim_pangenome_classes",
+    "pansim_core_parsimony", "pansim_gene_parsimony", "pansim_parsimony_kernel_ms", "pansim_parsimony_indices",
+    "pansim_group_core_parsimony", "pansim_group_gene_parsimony",
     "pansim_enable_genealogy", "pansim_genealogy", "pansim_genealogy_history", "pansim_genealogy_tmrca",
     "pansim_genealogy_newick", "pansim_group_enable_genealogy", "pansim_group_genealogy", "pansim_group_genealogy_tmrca",
 ]
@@ -118,6 +120,11 @@ class GeneLdParams(C.Structure):
 
 class GeneLdClass(C.Structure):
     _fields_ = [("ld", LdBin), ("associated", C.c_uint64), ("dissociated", C.c_uint64)]
+
+
+class Parsimony(C.Structure):
+    _fields_ = [("characters", C.c_uint64), ("variable", C.c_uint64), ("tree_length", C.c_uint64),
+                ("min_changes", C.c_uint64), ("max_changes", C.c_uint64), ("homoplastic", C.c_uint64)]
 
 
 class GenealogyNode(C.Structure):
@@ -257,6 +264,13 @@ def lib():
     sig("pansim_gene_spectrum", cint, vp, vp)
     sig("pansim_group_gene_spectrum", cint, vp, vp)
     sig("pansim_pangenome_classes", None, vp, u32, vp)
+    sig("pansim_core_parsimony", cint, vp, vp, u32, C.POINTER(Parsimony), vp, vp)
+    sig("pansim_gene_parsimony", cint, vp, vp, u32, C.POINTER(Parsimony), vp, vp, vp)
+    sig("pansim_group_core_parsimony", cint, vp, vp, u32, C.POINTER(Parsimony), vp, vp)
+    sig("pansim_group_gene_parsimony", cint, vp, vp, u32, C.POINTER(Parsimony), vp, vp, vp)
+    sig("pansim_parsimony_kernel_ms", cint, vp, vp, u32, cint, u32, C.POINTER(C.c_float), C.POINTER(C.c_uint64),
+        C.POINTER(C.c_uint32))
+    sig("pansim_parsimony_indices", None, C.POINTER(Parsimony), C.POINTER(C.c_double), C.POINTER(C.c_double))
     sig("pansim_enable_genealogy", cint, vp, u32)
     sig("pansim_genealogy", cint, vp, vp, C.POINTER(GenealogyInfo))
     sig("pansim_genealogy_history", cint, vp, vp)

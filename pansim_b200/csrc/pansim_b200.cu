@@ -26,6 +26,7 @@
 #include "ld.cuh"
 #include "pack.cuh"
 #include "pangenome.cuh"
+#include "parsimony.cuh"
 #include "replay.cuh"
 #include "select.cuh"
 #include "vcf.cuh"
@@ -4043,6 +4044,228 @@ void pansim_pangenome_classes(const uint64_t *spectrum, uint32_t pop_size, uint6
         out[h >= 99 * n ? 0 : h >= 95 * n ? 1 : h >= 15 * n ? 2 : 3] += spectrum[a];
     }
     out[4] = out[0] + out[1] + out[2] + out[3];
+}
+
+// ---- parsimony on a node table (parsimony.cuh, DESIGN.md section 17) ---------
+// Default scratch budget of one call: the smaller of 16 GiB and half the free device memory.
+// PANSIM_PARSIMONY_SCRATCH_MB=<n> replaces it (a small value forces many slabs; the results are the same).
+constexpr uint64_t PS_BUDGET_CAP_MB = 16384;
+
+// The rules of the node table (include/pansim_b200.h), checked on the host. On success csr = child_off[n_internal + 1]
+// followed by child[n_nodes - 1]: the children of each internal node in ascending id.
+static int parsimony_tree(pansim_ctx *c, const uint32_t *parent, uint32_t n_nodes, std::vector<uint32_t> &csr)
+{
+    const uint32_t N = c->N;
+    if (!parent) FAIL(c, PANSIM_ERR_INVALID, "parsimony: null node table");
+    if (n_nodes < N || (uint64_t)n_nodes > 2ull * N - 1)
+        FAIL(c, PANSIM_ERR_INVALID, "parsimony: %u nodes for %u leaves (a tree has N .. 2N - 1)", n_nodes, N);
+    const uint32_t root = n_nodes - 1, n_int = n_nodes - N;
+    if (parent[root] != GEN_NONE) FAIL(c, PANSIM_ERR_INVALID, "parsimony: the last node (%u) must be the root, parent 0xFFFFFFFF", root);
+    csr.assign((size_t)n_int + 1 + root, 0);
+    for (uint32_t k = 0; k < root; k++) {
+        const uint32_t p = parent[k];
+        if (p <= k || p < N || p >= n_nodes)
+            FAIL(c, PANSIM_ERR_INVALID, "parsimony: node %u has parent %u (an internal node with a larger id)", k, p);
+        csr[p - N + 1]++;
+    }
+    for (uint32_t v = 0; v < n_int; v++)
+        if (csr[v + 1] < 2) FAIL(c, PANSIM_ERR_INVALID, "parsimony: internal node %u has %u children (at least 2)", N + v, csr[v + 1]);
+    for (uint32_t v = 0; v < n_int; v++) csr[v + 1] += csr[v];
+    std::vector<uint32_t> fill(csr.begin(), csr.begin() + n_int);
+    uint32_t *child = csr.data() + n_int + 1;
+    for (uint32_t k = 0; k < root; k++) child[fill[parent[k] - N]++] = k;
+    return 0;
+}
+
+// the device buffers of one call, freed when it returns
+struct ParsimonyCall {
+    uint32_t *tree = nullptr, *scores = nullptr;
+    unsigned long long *out = nullptr;       // summary [5], then the branch arrays [NB][n_nodes]
+    void *scratch = nullptr;
+    uint32_t cols_slab = 0, n_nodes = 0, nb = 1;
+    uint64_t n_chars = 0, n_cols = 0;
+    size_t smem = 0;
+    bool genes = false;
+    ParsimonyArgs a{};
+    ~ParsimonyCall()
+    {
+        for (void *p : {(void *)tree, (void *)scores, (void *)out, scratch})
+            if (p) cudaFree(p);
+    }
+};
+
+static uint64_t parsimony_budget()
+{
+    if (const char *e = std::getenv("PANSIM_PARSIMONY_SCRATCH_MB"))
+        if (const uint64_t mb = std::strtoull(e, nullptr, 10)) return mb << 20;
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); free_b = 0; }
+    return std::min<uint64_t>(PS_BUDGET_CAP_MB << 20, free_b / 2);
+}
+
+// Checks, the per-character counts, the buffers and the uploaded table; refusals leave the context as it was.
+static int parsimony_prepare(pansim_ctx *c, bool genes, const uint32_t *parent, uint32_t n_nodes, ParsimonyCall &w)
+{
+    if (int rc = require_state(c)) return rc;
+    std::vector<uint32_t> csr;
+    if (int rc = parsimony_tree(c, parent, n_nodes, csr)) return rc;
+    CU(c, cudaSetDevice(c->cfg.device));
+    const uint32_t N = c->N, n_int = n_nodes - N, ns = genes ? 2 : 4;
+    w.genes = genes;
+    w.n_nodes = n_nodes;
+    w.nb = genes ? 2 : 1;
+    w.n_chars = genes ? c->G : c->Ll;
+    w.n_cols = (w.n_chars + 31) / 32;
+    const uint64_t pad_cols = (w.n_cols + PS_THREADS - 1) / PS_THREADS * PS_THREADS;
+    uint64_t cols = n_int ? parsimony_budget() / ((uint64_t)n_int * ns * 4) : pad_cols;
+    cols = std::min(pad_cols, std::max<uint64_t>(PS_THREADS, cols / PS_THREADS * PS_THREADS));
+    w.cols_slab = (uint32_t)std::min<uint64_t>(cols, 0x7FFFFF80ull);
+    const size_t out_words = 5 + (size_t)w.nb * n_nodes;
+    auto alloc = [&](void **p, size_t bytes, const char *what) -> int {
+        if (cudaMalloc(p, bytes) != cudaSuccess) {
+            cudaGetLastError();
+            *p = nullptr;
+            FAIL(c, PANSIM_ERR_NOMEM, "parsimony: cudaMalloc of %zu bytes (%s) failed", bytes, what);
+        }
+        return 0;
+    };
+    if (int rc = alloc((void **)&w.tree, csr.size() * 4, "node table")) return rc;
+    if (int rc = alloc((void **)&w.out, out_words * 8, "results")) return rc;
+    if (int rc = alloc((void **)&w.scores, std::max<uint64_t>(w.n_chars, 1) * 4, "character scores")) return rc;
+    if (n_int && w.n_cols)
+        if (int rc = alloc(&w.scratch, (size_t)n_int * w.cols_slab * ns * 4, "scratch")) return rc;
+    CU(c, cudaMemcpyAsync(w.tree, csr.data(), csr.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    const uint32_t *rows = nullptr;
+    uint64_t row_words = 0;
+    if (!genes) {
+        if (c->Ll) {
+            if (int rc = ensure_div(c, 1, false)) return rc;
+            if (int rc = ensure_site_counts(c)) return rc;
+            c->ps = c->stream;
+            if (int rc = core_materialize(c, c->stream)) return rc;
+            CU(c, cudaMemsetAsync(c->d_div, 0, 4 * sizeof(unsigned long long), c->stream));
+            if (int rc = launch_diversity(c, c->stream, c->d_div, c->d_vcf_counts, nullptr)) return rc;
+        }
+        rows = reinterpret_cast<const uint32_t *>(c->core[c->core_cur]);
+        row_words = c->core_stride / 4;
+    } else {
+        if (c->G) {
+            acc_gene_counts_kernel<<<c->acc_words, 256, 0, c->stream>>>(c->acc[c->acc_cur], c->N, c->G, c->acc_stride_words, c->d_gain_thr);
+            LAUNCH_CHECK(c);
+        }
+        rows = c->acc[c->acc_cur];
+        row_words = c->acc_stride_words;
+    }
+    ParsimonyArgs &a = w.a;
+    a.rows = rows;
+    a.row_words = row_words;
+    a.n_leaves = N;
+    a.n_internal = n_int;
+    a.child_off = w.tree;
+    a.child = w.tree + n_int + 1;
+    a.col0 = 0;
+    a.cols_pad = w.cols_slab;
+    a.n_cols = w.n_cols;
+    a.n_chars = w.n_chars;
+    a.dmax = 32u - (uint32_t)__builtin_clz(N);
+    a.scratch = w.scratch;
+    a.site_counts = c->d_vcf_counts;
+    a.gene_counts = c->d_gain_thr;
+    a.scores = w.scores;
+    a.summary = w.out;
+    a.branch0 = w.out + 5;
+    a.branch1 = w.out + 5 + (genes ? n_nodes : 0);
+    w.smem = (size_t)ns * a.dmax * PS_THREADS * 4;
+    if (w.smem > 48 * 1024) {
+        const cudaError_t e = genes ? cudaFuncSetAttribute(parsimony_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)w.smem)
+                                    : cudaFuncSetAttribute(parsimony_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)w.smem);
+        CU(c, e);
+    }
+    return 0;
+}
+
+// zeroed results, then the slabs of columns one after the other on c->stream
+static int parsimony_launch(pansim_ctx *c, ParsimonyCall &w)
+{
+    CU(c, cudaMemsetAsync(w.out, 0, (5 + (size_t)w.nb * w.n_nodes) * 8, c->stream));
+    for (uint64_t col0 = 0; col0 < w.n_cols; col0 += w.cols_slab) {
+        ParsimonyArgs a = w.a;
+        a.col0 = col0;
+        const uint64_t cols = std::min<uint64_t>(w.cols_slab, w.n_cols - col0);
+        const uint32_t grid = div_up64(cols, PS_THREADS);
+        if (w.genes)
+            parsimony_kernel<2><<<grid, PS_THREADS, w.smem, c->stream>>>(a);
+        else
+            parsimony_kernel<4><<<grid, PS_THREADS, w.smem, c->stream>>>(a);
+        LAUNCH_CHECK(c);
+    }
+    return 0;
+}
+
+static int parsimony_call(pansim_ctx *c, bool genes, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out,
+                          uint32_t *chars, uint64_t *branch0, uint64_t *branch1)
+{
+    if (!c) return PANSIM_ERR_INVALID;
+    ParsimonyCall w;
+    if (int rc = parsimony_prepare(c, genes, parent, n_nodes, w)) return rc;
+    if (int rc = parsimony_launch(c, w)) return rc;
+    unsigned long long sum[5];
+    CU(c, cudaMemcpyAsync(sum, w.out, sizeof sum, cudaMemcpyDeviceToHost, c->stream));
+    if (chars && w.n_chars) CU(c, cudaMemcpyAsync(chars, w.scores, w.n_chars * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (branch0) CU(c, cudaMemcpyAsync(branch0, w.a.branch0, (size_t)n_nodes * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (branch1) CU(c, cudaMemcpyAsync(branch1, w.a.branch1, (size_t)n_nodes * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (int rc = check_device_flag(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG)) return rc;
+    if (out) *out = {w.n_chars, sum[0], sum[1], sum[2], sum[3], sum[4]};
+    return 0;
+}
+
+int pansim_core_parsimony(pansim_ctx *c, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out, uint32_t *site_changes,
+                          uint64_t *branch_changes)
+{
+    return parsimony_call(c, false, parent, n_nodes, out, site_changes, branch_changes, nullptr);
+}
+
+int pansim_gene_parsimony(pansim_ctx *c, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out, uint32_t *gene_changes,
+                          uint64_t *gains, uint64_t *losses)
+{
+    return parsimony_call(c, true, parent, n_nodes, out, gene_changes, gains, losses);
+}
+
+int pansim_parsimony_kernel_ms(pansim_ctx *c, const uint32_t *parent, uint32_t n_nodes, int genes, uint32_t repeats, float *ms,
+                               uint64_t *bytes_read, uint32_t *slabs)
+{
+    if (!c || !repeats) return PANSIM_ERR_INVALID;
+    ParsimonyCall w;
+    if (int rc = parsimony_prepare(c, genes != 0, parent, n_nodes, w)) return rc;
+    if (int rc = parsimony_launch(c, w)) return rc;      // warm-up
+    cudaEvent_t ev[2];
+    for (auto &e : ev) CU(c, cudaEventCreate(&e));
+    int rc = 0;
+    cudaEventRecord(ev[0], c->stream);
+    for (uint32_t r = 0; r < repeats && !rc; r++) rc = parsimony_launch(c, w);
+    cudaEventRecord(ev[1], c->stream);
+    const cudaError_t e = cudaEventSynchronize(ev[1]);
+    float t = 0.f;
+    cudaEventElapsedTime(&t, ev[0], ev[1]);
+    for (auto &x : ev) cudaEventDestroy(x);
+    if (rc) return rc;
+    if (e != cudaSuccess) FAIL(c, PANSIM_ERR_CUDA, "parsimony kernel failed: %s", cudaGetErrorString(e));
+    if (ms) *ms = t / (float)repeats;
+    // per column: every leaf read twice (8 / 4 bytes), every non-root internal set read twice (as a child going up,
+    // then as a child going down), the root's set and every internal node's assigned state read once (16 / 8 bytes)
+    const uint64_t leaf_b = genes ? 4 : 8, set_b = genes ? 8 : 16, n_int = n_nodes - c->N;
+    if (bytes_read) *bytes_read = w.n_cols * (2 * (uint64_t)c->N * leaf_b + (n_int ? 3 * n_int - 1 : 0) * set_b);
+    if (slabs) *slabs = (uint32_t)((w.n_cols + w.cols_slab - 1) / w.cols_slab);
+    return 0;
+}
+
+void pansim_parsimony_indices(const pansim_parsimony *p, double *ci, double *ri)
+{
+    const double nan = std::numeric_limits<double>::quiet_NaN();
+    if (!p) return;
+    const double S = (double)p->tree_length, M = (double)p->min_changes, G = (double)p->max_changes;
+    if (ci) *ci = p->tree_length ? M / S : nan;
+    if (ri) *ri = p->max_changes != p->min_changes ? (G - S) / (G - M) : nan;
 }
 
 // ---- clonal genealogy (genealogy.cuh, DESIGN.md section 13) ------------------

@@ -13,9 +13,10 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import (OK, CoreFasta, CoreLD, GeneAccumulation, GeneLD, Genealogy, PansimError, _core_ld, _diversity,
-                         _gene_accumulation, _gene_ld, _gene_spectrum, _genealogy, _genealogy_history, _ld_bins, _ld_params,
-                         _pairs_or_none, _ptr, _tmrca, _write_fasta, make_config)
+from .population import (OK, CoreFasta, CoreLD, CoreParsimony, GeneAccumulation, GeneLD, GeneParsimony, Genealogy, PansimError,
+                         _core_ld, _diversity, _gene_accumulation, _gene_ld, _gene_spectrum, _genealogy, _genealogy_history,
+                         _ld_bins, _ld_params, _pairs_or_none, _parent_table, _parsimony, _ptr, _tmrca, _write_fasta,
+                         make_config)
 
 
 class PansimGroup:
@@ -163,6 +164,17 @@ class PansimGroup:
     def gene_spectrum(self) -> np.ndarray:
         """The gene frequency spectrum (Pansim.gene_spectrum), answered by shard 0."""
         return _gene_spectrum(lambda *a: self._lib.pansim_group_gene_spectrum(self._h, *a), self._check, self.N)
+
+    def core_parsimony(self, genealogy=None) -> CoreParsimony:
+        """Pansim.core_parsimony over the whole alignment: every shard scores its sites, the results are summed and the
+        site scores concatenated in site order."""
+        parent = _parent_table(self.genealogy() if genealogy is None else genealogy)
+        return _parsimony(lambda *a: self._lib.pansim_group_core_parsimony(self._h, *a), self._check, parent, self.L, False)
+
+    def gene_parsimony(self, genealogy=None) -> GeneParsimony:
+        """Pansim.gene_parsimony: the accessory matrix is replicated, so shard 0 answers."""
+        parent = _parent_table(self.genealogy() if genealogy is None else genealogy)
+        return _parsimony(lambda *a: self._lib.pansim_group_gene_parsimony(self._h, *a), self._check, parent, self.G, True)
 
     def enable_genealogy(self, capacity: int):
         """Pansim.enable_genealogy for the group: shard 0 records (every shard draws the same parents)."""

@@ -48,7 +48,7 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
                               "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy",
                               "print_fasta", "print_snp_alignment", "print_gene_ld",
-                              "print_gene_accumulation"};                     // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "print_gene_accumulation", "print_parsimony"};  // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
                                                                               // print_vcf (<outpref>_core_genome.vcf),
                                                                               // print_ld (<outpref>_core_ld.tsv),
@@ -57,7 +57,9 @@ const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection",
                                                                               // print_snp_alignment (<outpref>_core_snps.fasta, <outpref>_core_snps_fconst.txt),
                                                                               // print_gene_ld (<outpref>_gene_ld.tsv),
                                                                               // print_gene_accumulation (<outpref>_number_of_*.Rtab,
-                                                                              //   <outpref>_gene_spectrum.txt, <outpref>_summary_statistics.txt)
+                                                                              //   <outpref>_gene_spectrum.txt, <outpref>_summary_statistics.txt),
+                                                                              // print_parsimony (<outpref>_parsimony.tsv, <outpref>_core_site_changes.txt,
+                                                                              //   <outpref>_gene_changes.txt, <outpref>_branch_changes.tsv)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -149,6 +151,7 @@ int main(int argc, char **argv)
                                         (uint32_t)std::strtoul(fl.val["ld_min_minor"].c_str(), nullptr, 10)};
     const bool print_gene_ld = fl.sw["print_gene_ld"];
     const bool print_gene_accumulation = fl.sw["print_gene_accumulation"];
+    const bool print_parsimony = fl.sw["print_parsimony"];
     const uint32_t gene_accumulation_perms = (uint32_t)std::strtoul(fl.val["gene_accumulation_perms"].c_str(), nullptr, 10);
     const pansim_gene_ld_params gene_ld_params = {(uint32_t)std::strtoul(fl.val["gene_ld_bins"].c_str(), nullptr, 10),
                                                   (uint32_t)std::strtoul(fl.val["gene_ld_min_minor"].c_str(), nullptr, 10)};
@@ -239,7 +242,7 @@ int main(int argc, char **argv)
         pansim::Populations pops(cfg, n_gpus);
         pops.set_initial(core_row, acc_row);
         pops.set_selection(selection);
-        if (print_genealogy) pops.enable_genealogy((uint32_t)n_gen);       // extension: after set_initial, which clears the record
+        if (print_genealogy || print_parsimony) pops.enable_genealogy((uint32_t)n_gen);   // extension: after set_initial, which clears the record
         std::vector<double> avg_core(n_gen, 0.0), avg_acc(n_gen, 0.0), std_core(n_gen, 0.0), std_acc(n_gen, 0.0);
         std::vector<double> core_d, acc_d;
         std::vector<pansim_diversity> diversity;
@@ -373,6 +376,44 @@ int main(int argc, char **argv)
                                     "Total genes\t(0% <= strains <= 100%)"};
             std::ofstream f(outpref + "_summary_statistics.txt");
             for (int k = 0; k < 5; k++) f << label[k] << "\t" << cls[k] << "\n";
+        }
+        if (print_parsimony) {                                              // extension: parsimony on the true genealogy
+            const std::vector<pansim_genealogy_node> nodes = pops.genealogy();
+            const size_t n = nodes.size();
+            std::vector<uint32_t> parent(n), first(n, (uint32_t)pop_size), below(n, 0);
+            for (size_t k = 0; k < n; k++) parent[k] = nodes[k].parent;
+            const auto core = pops.core_parsimony(parent);
+            const auto genes = pops.gene_parsimony(parent);
+            {
+                std::ofstream f(outpref + "_parsimony.tsv");
+                const std::pair<const char *, const pansim_parsimony *> rows[2] = {{"core", &core.summary}, {"genes", &genes.summary}};
+                for (const auto &r : rows) {
+                    const pansim_parsimony &q = *r.second;
+                    double ci = 0.0, ri = 0.0;
+                    pansim_parsimony_indices(&q, &ci, &ri);
+                    f << r.first << "\t" << q.characters << "\t" << q.variable << "\t" << q.tree_length << "\t" << q.min_changes
+                      << "\t" << q.max_changes << "\t" << q.homoplastic << "\t" << fmt(ci) << "\t" << fmt(ri) << "\n";
+                }
+            }
+            {
+                std::ofstream f(outpref + "_core_site_changes.txt");
+                for (uint32_t x : core.site_changes) f << x << "\n";
+            }
+            {
+                std::ofstream f(outpref + "_gene_changes.txt");
+                for (uint32_t x : genes.gene_changes) f << x << "\n";
+            }
+            // (first leaf, leaves below) of every node: the key of a clade in _genealogy.nwk, whose internal nodes
+            // carry no label
+            for (size_t k = 0; k < (size_t)pop_size && k < n; k++) { first[k] = (uint32_t)k; below[k] = 1; }
+            for (size_t k = 0; k + 1 < n; k++) {
+                first[parent[k]] = std::min(first[parent[k]], first[k]);
+                below[parent[k]] += below[k];
+            }
+            std::ofstream f(outpref + "_branch_changes.tsv");
+            for (size_t k = 0; k + 1 < n; k++)
+                f << k << "\t" << parent[k] << "\t" << first[k] << "\t" << below[k] << "\t" << nodes[parent[k]].time - nodes[k].time
+                  << "\t" << core.branch_changes[k] << "\t" << genes.gains[k] << "\t" << genes.losses[k] << "\n";
         }
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)

@@ -252,6 +252,29 @@ public:
         gcheck(pansim_group_genealogy_tmrca(grp_, range1.data(), range2.data(), range1.size(), out.data()));
         return out;
     }
+    // (extension) parsimony changes of the core sites / accessory genes on a node table given as its parent column
+    // (pansim_group_core_parsimony / pansim_group_gene_parsimony)
+    struct CoreParsimony { pansim_parsimony summary; std::vector<uint32_t> site_changes; std::vector<uint64_t> branch_changes; };
+    CoreParsimony core_parsimony(const std::vector<uint32_t> &parent)
+    {
+        CoreParsimony r{};
+        r.site_changes.assign(cfg_.core_size, 0);
+        r.branch_changes.assign(parent.size(), 0);
+        gcheck(pansim_group_core_parsimony(grp_, parent.data(), (uint32_t)parent.size(), &r.summary, r.site_changes.data(),
+                                           r.branch_changes.data()));
+        return r;
+    }
+    struct GeneParsimony { pansim_parsimony summary; std::vector<uint32_t> gene_changes; std::vector<uint64_t> gains, losses; };
+    GeneParsimony gene_parsimony(const std::vector<uint32_t> &parent)
+    {
+        GeneParsimony r{};
+        r.gene_changes.assign(cfg_.pan_size, 0);
+        r.gains.assign(parent.size(), 0);
+        r.losses.assign(parent.size(), 0);
+        gcheck(pansim_group_gene_parsimony(grp_, parent.data(), (uint32_t)parent.size(), &r.summary, r.gene_changes.data(),
+                                           r.gains.data(), r.losses.data()));
+        return r;
+    }
     // (extension) the canonical Newick text of a node table (pansim_genealogy_newick)
     std::string newick(const std::vector<pansim_genealogy_node> &nodes)
     {

@@ -218,6 +218,69 @@ def pangenome_classes(spectrum, pop_size: int) -> tuple[int, int, int, int, int]
     return tuple(int(x) for x in out)
 
 
+PARSIMONY_FIELDS = ("characters", "variable", "tree_length", "min_changes", "max_changes", "homoplastic")
+
+
+class CoreParsimony(NamedTuple):
+    """Parsimony of the core sites on a node table (pansim_core_parsimony, include/pansim_b200.h): the summary, the
+    consistency and retention indices (NaN for a zero denominator), the score of every local site (uint32, position
+    order) and the changes on the branch above every node (uint64 [n_nodes], 0 at the root)."""
+    characters: int
+    variable: int
+    tree_length: int
+    min_changes: int
+    max_changes: int
+    homoplastic: int
+    ci: float
+    ri: float
+    site_changes: np.ndarray
+    branch_changes: np.ndarray
+
+
+class GeneParsimony(NamedTuple):
+    """Parsimony of the accessory genes on a node table (pansim_gene_parsimony): the summary, CI and RI, the score of
+    every matrix gene (uint32, _pangenome.csv column order) and the gains and losses on the branch above every node
+    (uint64 [n_nodes], 0 at the root)."""
+    characters: int
+    variable: int
+    tree_length: int
+    min_changes: int
+    max_changes: int
+    homoplastic: int
+    ci: float
+    ri: float
+    gene_changes: np.ndarray
+    gains: np.ndarray
+    losses: np.ndarray
+
+
+def parsimony_indices(summary) -> tuple[float, float]:
+    """(CI, RI) = (M / S, (G - S) / (G - M)) of a parsimony summary (anything with the six summary fields), NaN for a
+    zero denominator, evaluated by the library (pansim_parsimony_indices) so every host prints the same."""
+    p = _ffi.Parsimony(*(int(getattr(summary, f)) for f in PARSIMONY_FIELDS))
+    ci, ri = C.c_double(), C.c_double()
+    _ffi.lib().pansim_parsimony_indices(C.byref(p), C.byref(ci), C.byref(ri))
+    return ci.value, ri.value
+
+
+def _parent_table(genealogy) -> np.ndarray:
+    """The parent column of a Genealogy, or a parent array itself, as contiguous uint32."""
+    parent = genealogy.parent if hasattr(genealogy, "parent") else genealogy
+    return np.ascontiguousarray(parent, np.uint32)
+
+
+def _parsimony(call, check, parent: np.ndarray, n_chars: int, genes: bool):
+    """call(parent, n_nodes, &summary, chars, branch arrays...) -> status."""
+    n = len(parent)
+    s = _ffi.Parsimony()
+    chars = np.zeros(n_chars, np.uint32)
+    branches = [np.zeros(n, np.uint64) for _ in range(2 if genes else 1)]
+    check(call(_ptr(parent), n, C.byref(s), _ptr(chars), *[_ptr(b) for b in branches]))
+    head = tuple(int(getattr(s, f)) for f in PARSIMONY_FIELDS)
+    ci, ri = parsimony_indices(s)
+    return (GeneParsimony if genes else CoreParsimony)(*head, ci, ri, chars, *branches)
+
+
 class Genealogy(NamedTuple):
     """The clonal genealogy of the present population (pansim_genealogy, include/pansim_b200.h): per node its parent
     (0xFFFFFFFF at the root), the individual it stands for (0xFFFFFFFF at a virtual root) and its time in generations
@@ -625,6 +688,26 @@ class Pansim:
         not coalesced within the record)."""
         return _tmrca(lambda *a: self._lib.pansim_genealogy_tmrca(self._h, *a), self._check, range1, range2)
 
+    # -- parsimony on the genealogy (extension) ------------------------------
+    def core_parsimony(self, genealogy=None) -> CoreParsimony:
+        """Parsimony changes of every local core site on a node table: a Genealogy, a parent array, or None for
+        self.genealogy() (pansim_core_parsimony)."""
+        parent = _parent_table(self.genealogy() if genealogy is None else genealogy)
+        return _parsimony(lambda *a: self._lib.pansim_core_parsimony(self._h, *a), self._check, parent, self.local_sites, False)
+
+    def gene_parsimony(self, genealogy=None) -> GeneParsimony:
+        """Parsimony changes, gains and losses of every accessory gene on a node table (pansim_gene_parsimony)."""
+        parent = _parent_table(self.genealogy() if genealogy is None else genealogy)
+        return _parsimony(lambda *a: self._lib.pansim_gene_parsimony(self._h, *a), self._check, parent, self.G, True)
+
+    def parsimony_kernel_ms(self, genealogy=None, genes: bool = False, repeats: int = 10):
+        """Measurement: device ms of one parsimony pass (every slab), the bytes its walk reads, and the slabs."""
+        parent = _parent_table(self.genealogy() if genealogy is None else genealogy)
+        ms, nb, sl = C.c_float(), C.c_uint64(), C.c_uint32()
+        self._check(self._lib.pansim_parsimony_kernel_ms(self._h, _ptr(parent), len(parent), int(genes), repeats,
+                                                         C.byref(ms), C.byref(nb), C.byref(sl)))
+        return ms.value, nb.value, sl.value
+
     # -- multi-GPU: communicator over column shards (one process per GPU) --
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -795,4 +878,5 @@ class Pansim:
 
 
 __all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "GeneLD", "GeneAccumulation",
-           "pangenome_classes", "Genealogy", "genealogy_newick", "make_config", "standard_deviation", "fmt_f64"]
+           "pangenome_classes", "CoreParsimony", "GeneParsimony", "parsimony_indices", "Genealogy", "genealogy_newick",
+           "make_config", "standard_deviation", "fmt_f64"]

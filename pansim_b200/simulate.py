@@ -66,6 +66,8 @@ class RunResult:
     gene_accumulation: object = None              # GeneAccumulation of the last generation (--print_gene_accumulation)
     gene_spectrum: np.ndarray = None              # gene frequency spectrum of the last generation (--print_gene_accumulation)
     genealogy: object = None                      # Genealogy of the last generation (--print_genealogy)
+    core_parsimony: object = None                 # CoreParsimony on the genealogy (--print_parsimony)
+    gene_parsimony: object = None                 # GeneParsimony on the genealogy (--print_parsimony)
     tmrca: np.ndarray = None                      # TMRCA of the sampled pairs (--print_genealogy without --all_pairs)
     selection: np.ndarray = None
     stdout: list = field(default_factory=list)
@@ -76,7 +78,7 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
         ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False, print_fasta: bool = False,
         print_snp_alignment: bool = False, print_gene_ld: bool = False, gene_ld_bins: int = 20,
         gene_ld_min_minor: int = 1, print_gene_accumulation: bool = False,
-        gene_accumulation_perms: int = 100) -> RunResult | None:
+        gene_accumulation_perms: int = 100, print_parsimony: bool = False) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -100,7 +102,10 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     print_gene_accumulation (extension): after every other output, Roary's pangenome summaries of the last generation:
     the accumulation curves over gene_accumulation_perms random orders keyed by p.seed, the gene frequency spectrum
     and the core / soft-core / shell / cloud counts (Pansim.gene_accumulation, Pansim.gene_spectrum;
-    write_gene_accumulation)."""
+    write_gene_accumulation).
+    print_parsimony (extension): the parents are recorded from generation 0 as for print_genealogy (without its files
+    unless that is also given); after every other output, the parsimony changes of the core sites and the accessory
+    genes on the genealogy of the last generation (Pansim.core_parsimony, Pansim.gene_parsimony; write_parsimony)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -125,7 +130,7 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     with Pansim.from_params(p, device=device) as sim:
         sim.set_initial(core_row, acc_row)
         sim.set_selection(sel)
-        if print_genealogy:
+        if print_genealogy or print_parsimony:
             sim.enable_genealogy(p.n_gen)                                        # after set_initial, which clears the record
         def last_generation_outputs():                                           # main.rs:467-499
             if not all_pairs:
@@ -219,7 +224,50 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             res.gene_spectrum = sim.gene_spectrum()
             if outpref:
                 write_gene_accumulation(outpref, res.gene_accumulation, res.gene_spectrum)
+        if print_parsimony:
+            g = res.genealogy if res.genealogy is not None else sim.genealogy()
+            res.core_parsimony = sim.core_parsimony(g)
+            res.gene_parsimony = sim.gene_parsimony(g)
+            if outpref:
+                write_parsimony(outpref, g, res.core_parsimony, res.gene_parsimony)
     return res
+
+
+def clades(parent, n_leaves: int) -> tuple[np.ndarray, np.ndarray]:
+    """(first leaf, leaves below) of every node of a node table whose parents have larger ids. Every internal node
+    has at least two children, so the pair identifies a clade: the key that joins a per-branch table to a Newick text
+    whose internal nodes carry no label."""
+    parent = np.asarray(parent, np.int64)
+    n = len(parent)
+    first = np.full(n, n_leaves, np.int64)
+    below = np.zeros(n, np.int64)
+    first[:n_leaves] = np.arange(n_leaves)
+    below[:n_leaves] = 1
+    for k in range(n - 1):
+        q = parent[k]
+        first[q] = min(first[q], first[k])
+        below[q] += below[k]
+    return first, below
+
+
+def write_parsimony(outpref: str, genealogy, core, genes):
+    """`<outpref>_parsimony.tsv`: two lines, `core` then `genes`, each characters, variable, tree length, min changes,
+    max changes, homoplastic, CI, RI (no header; NaN for an empty denominator); `<outpref>_core_site_changes.txt`: the
+    score of each core site in position order; `<outpref>_gene_changes.txt`: the score of each matrix gene in
+    `_pangenome.csv` column order; `<outpref>_branch_changes.tsv`: per non-root node in id order, no header: node,
+    parent, first leaf, leaves below, branch length (generations), core changes, gene gains, gene losses."""
+    with open(outpref + "_parsimony.tsv", "w") as f:
+        for name, r in (("core", core), ("genes", genes)):
+            f.write("\t".join([name] + [str(int(x)) for x in r[:6]] + [fmt_f64(r.ci), fmt_f64(r.ri)]) + "\n")
+    with open(outpref + "_core_site_changes.txt", "w") as f:
+        f.write("".join(f"{x}\n" for x in core.site_changes.tolist()))
+    with open(outpref + "_gene_changes.txt", "w") as f:
+        f.write("".join(f"{x}\n" for x in genes.gene_changes.tolist()))
+    parent, time = genealogy.parent, genealogy.time
+    first, below = clades(parent, genealogy.n_leaves)
+    with open(outpref + "_branch_changes.tsv", "w") as f:
+        f.write("".join(f"{k}\t{parent[k]}\t{first[k]}\t{below[k]}\t{time[parent[k]] - time[k]}\t{core.branch_changes[k]}\t"
+                        f"{genes.gains[k]}\t{genes.losses[k]}\n" for k in range(len(parent) - 1)))
 
 
 ROARY_CLASSES = ("Core genes\t(99% <= strains <= 100%)", "Soft core genes\t(95% <= strains < 99%)",
