@@ -41,8 +41,13 @@
 //
 // Data movement: warp-private TMA pipelines (cp.async.bulk global->shared with
 // mbarrier completion from the PARENT's row, cp.async.bulk shared->global into
-// the child's row), three 2 KiB stages per warp, no CTA-wide barrier in the
-// steady state.
+// the child's row), two 2 KiB stages per warp, no CTA-wide barrier in the
+// steady state. One item keeps a warp busy far longer than a load takes, so a
+// load issued one item ahead is hidden. Two stages and a 48-register budget
+// (40 used) leave a quarter of each SM's registers and ~38 KB of its shared
+// memory free at four resident CTAs: the selection chain of the next
+// generation runs there beside the core kernel instead of waiting for core
+// CTAs to retire (DESIGN.md section 5).
 #pragma once
 #include "common.cuh"
 #include "core_hr.cuh"
@@ -56,15 +61,23 @@ namespace pansim {
 #define PANSIM_CM_MAXREG 0          // > 0: cap registers per thread with __maxnreg__ instead of the launch bound
 #endif
 constexpr int CM_WARPS = PANSIM_CM_WARPS;
+// PANSIM_CM_STAGES=3 PANSIM_CM_CTAS=4 builds the earlier three-stage ring (58 registers) for comparison
 #ifndef PANSIM_CM_STAGES
-#define PANSIM_CM_STAGES 3
+#define PANSIM_CM_STAGES 2
 #endif
 #ifndef PANSIM_CM_CTAS
-#define PANSIM_CM_CTAS 4
+#define PANSIM_CM_CTAS 5
+#endif
+#ifndef PANSIM_CM_RESIDENT
+#define PANSIM_CM_RESIDENT 4
 #endif
 constexpr int CM_STAGES = PANSIM_CM_STAGES;       // 2 KiB stages per warp
 constexpr int CM_CTAS_PER_SM = PANSIM_CM_CTAS;    // launch bound (register budget = 65536 / (256 * CTAs))
-// Two stages: the load of item j+1 is issued early in item j (after its Philox calls), once the bulk
+// CTAs resident per SM at most: the host sizes the dynamic shared memory of a CTA so that no more fit.
+// At cfg2, 4 resident CTAs of the two-stage kernel: 143.8-144.3 us per generation; 5 (40 warps, the
+// chain squeezed out of every scheduler): 152.3-152.5.
+constexpr int CM_RESIDENT_CTAS = PANSIM_CM_RESIDENT;
+// Two stages: the load of item j+1 is issued in item j, after its recombination apply, once the bulk
 // store of item j-1 has finished reading the stage it reuses. Three stages: issued at the end of
 // item j-1, two items ahead.
 constexpr bool CM_LATE_LOAD = CM_STAGES == 2;
@@ -355,7 +368,9 @@ template <bool RNG, bool DUMP>
 __device__ __forceinline__ void mut_cta_items(const CoreMutArgs &a, const MutSmem &m, uint32_t item_begin,
                                               uint32_t item_end, uint32_t blk_regs, uint32_t blk_reg0)
 {
-    const uint32_t warp = threadIdx.x >> 5;
+    // REDUX writes a uniform register: everything a warp derives from its index (item cursor, stage and
+    // mbarrier addresses) can then live in uniform registers instead of taking one register per lane
+    const uint32_t warp = __reduce_max_sync(0xffffffffu, threadIdx.x >> 5);
     uint32_t lane = threadIdx.x & 31;
     asm volatile("" : "+r"(lane));          // keep it in a register (otherwise %tid.x is re-read at every use)
     const uint32_t gen_off = a.gen_dev ? __ldg(a.gen_dev) : 0u;
@@ -368,25 +383,33 @@ __device__ __forceinline__ void mut_cta_items(const CoreMutArgs &a, const MutSme
     const uint32_t n_my = (item_end - gw + CM_WARPS - 1) / CM_WARPS;
     const uint32_t d_row = CM_WARPS / blk_regs, d_reg = CM_WARPS % blk_regs;
 
-    // the load side runs CM_STAGES-1 items ahead with its own (row, reg, stage) cursor (lane 0 only)
-    uint32_t l_row = gw / blk_regs, l_reg = gw % blk_regs, l_stage = 0;
-    // parent rows are kept in registers and re-read only when a cursor moves on to another row (a warp
+    // parent rows are kept in registers and re-read only when an item moves on to another row (a warp
     // stays on one row for many items when the row has more regions than the CTA has warps)
 #define PANSIM_CM_PARENT(r_) (a.parents ? __ldg(a.parents + (r_)) : (r_))
-    uint32_t l_prow = PANSIM_CM_PARENT(l_row);
     // shared-space addresses, computed once and made opaque so that they stay in registers (otherwise
     // they are re-derived from %cluster_ctaid and the carve-up arithmetic at every use)
     uint32_t stages_s = smem_u32(stages), bars_s = smem_u32(bars), lut_s = smem_u32(m.lut);
     asm volatile("" : "+r"(stages_s), "+r"(bars_s), "+r"(lut_s));
     const uint32_t tab_s = lut_s + CM_LUT_BYTES, hr_thr_s = tab_s + (CM_GUIDE_WORDS + a.mut_size) * 4u;
     const uint8_t *old_blk = a.old_state + (uint64_t)blk_reg0 * REGION_BYTES;
-#define PANSIM_CM_ISSUE_LOAD()                                                                               \
+    // TMA load of (parent row p, block region r) into stage st (lane 0)
+#define PANSIM_CM_LOAD(p_, r_, st_)                                                                          \
     do {                                                                                                     \
-        const uint8_t *src_ = old_blk + (uint64_t)l_prow * a.row_stride + l_reg * REGION_BYTES;              \
-        const uint32_t bar_ = bars_s + l_stage * 8u;                                                         \
+        const uint8_t *src_ = old_blk + (uint64_t)(p_) * a.row_stride + (r_) * REGION_BYTES;                \
+        const uint32_t bar_ = bars_s + (st_) * 8u;                                                           \
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_), "n"(REGION_BYTES) : "memory"); \
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" \
-                     ::"r"(stages_s + l_stage * REGION_BYTES), "l"(src_), "n"(REGION_BYTES), "r"(bar_) : "memory"); \
+                     ::"r"(stages_s + (st_) * REGION_BYTES), "l"(src_), "n"(REGION_BYTES), "r"(bar_) : "memory"); \
+    } while (0)
+
+    uint32_t row = gw / blk_regs, breg = gw % blk_regs;
+    uint32_t prow = PANSIM_CM_PARENT(row);          // parent of `row`
+    // Two stages: the load of item j+1 is issued by item j itself, from the (row, region, parent) it computes
+    // for the next item anyway. Three stages: the load side runs two items ahead with its own cursor (lane 0).
+    uint32_t l_row = row, l_reg = breg, l_prow = prow, l_stage = 0;
+#define PANSIM_CM_ISSUE_LOAD()                                                                               \
+    do {                                                                                                     \
+        PANSIM_CM_LOAD(l_prow, l_reg, l_stage);                                                              \
         l_stage = l_stage == (uint32_t)(CM_STAGES - 1) ? 0u : l_stage + 1u;                                  \
         uint32_t nr_ = l_row + d_row;                                                                        \
         l_reg += d_reg;                                                                                      \
@@ -398,17 +421,18 @@ __device__ __forceinline__ void mut_cta_items(const CoreMutArgs &a, const MutSme
     } while (0)
 
     if (lane == 0) {
-        const uint32_t ahead = CM_LATE_LOAD ? 1u : (uint32_t)(CM_STAGES - 1);
-        const uint32_t pre = n_my < ahead ? n_my : ahead;
+        if (CM_LATE_LOAD) {
+            PANSIM_CM_LOAD(prow, breg, 0u);
+        } else {
+            const uint32_t pre = min(n_my, (uint32_t)(CM_STAGES - 1));
 #pragma unroll 1
-        for (uint32_t jj = 0; jj < pre; jj++) PANSIM_CM_ISSUE_LOAD();
+            for (uint32_t jj = 0; jj < pre; jj++) PANSIM_CM_ISSUE_LOAD();
+        }
     }
 
-    uint32_t row = gw / blk_regs, breg = gw % blk_regs;
     if (RNG) mut_const_wait(m);
     const bool hr_on = RNG && a.hr_nsub != 0u;
     HrWindow hw_cur{0u, 0u, 0u};
-    uint32_t prow = hr_on ? PANSIM_CM_PARENT(row) : 0u, nprow = prow;      // parent of `row` / of the next item's row
     if (hr_on) hw_cur = hr_window_fetch(a, hr_gen, m.hr_thr, hr_thr_s, prow, blk_reg0 + breg, lane, 0u, 0u);
     uint32_t s = 0, par = 0;                 // stage of item j and the phase parity of its mbarrier
     for (uint32_t j = 0; j < n_my; j++) {
@@ -431,31 +455,30 @@ __device__ __forceinline__ void mut_cta_items(const CoreMutArgs &a, const MutSme
             k = poisson_fast_s(tab_s, a.mut_kmax, c0.x);
             if (a.mut_nsub > 1) k += mut_count_extra(mctr, a.key, tab, a.mut_nsub, a.mut_kmax);
         }
-
-        if (CM_LATE_LOAD && lane == 0 && j + 1 < n_my) {
-            bulk_wait_read<0>();          // the store of item j-1 has left the stage item j+1 goes into
-            PANSIM_CM_ISSUE_LOAD();
-        }
         mbar_wait_s(bars_s + s * 8u, par);
 
-        if (hr_on) {
+        if (hr_on && hw_cur.K) {
             // ---- recombination of the previous generation on the parent's row (population.rs:725-748):
             // windows in draw order, so a later event of a cell overwrites an earlier one ----
-            if (hw_cur.K) {
-                hr_window_apply(sw_s, hw_cur);
+            hr_window_apply(sw_s, hw_cur);
 #pragma unroll 1
-                for (uint32_t base = 32u; base < hw_cur.K; base += 32u)
-                    hr_window_apply(sw_s, hr_window_fetch(a, hr_gen, m.hr_thr, hr_thr_s, prow, reg, lane, base, hw_cur.K));
-            }
-            // first window of the NEXT item, fetched into the registers just consumed: its donor
-            // loads are in flight while this item's SNP events are applied
-            if (j + 1 < n_my) {
-                uint32_t nrow = row + d_row, nreg = breg + d_reg;
-                if (nreg >= blk_regs) { nreg -= blk_regs; nrow++; }
-                nprow = nrow == row ? prow : PANSIM_CM_PARENT(nrow);
-                hw_cur = hr_window_fetch(a, hr_gen, m.hr_thr, hr_thr_s, nprow, blk_reg0 + nreg, lane, 0u, 0u);
-            }
+            for (uint32_t base = 32u; base < hw_cur.K; base += 32u)
+                hr_window_apply(sw_s, hr_window_fetch(a, hr_gen, m.hr_thr, hr_thr_s, prow, reg, lane, base, hw_cur.K));
         }
+        // the next item: its row, region and parent
+        const bool more = j + 1 < n_my;
+        uint32_t nrow = row + d_row, nreg = breg + d_reg;
+        if (nreg >= blk_regs) { nreg -= blk_regs; nrow++; }
+        const uint32_t nprow = (!more || nrow == row) ? prow : PANSIM_CM_PARENT(nrow);
+        if (CM_LATE_LOAD && lane == 0 && more) {
+            // issued after the recombination apply rather than before the mbarrier wait: by now the bulk store
+            // of item j-1 has long left the stage item j+1 goes into, so lane 0 does not wait for it to drain
+            bulk_wait_read<0>();
+            PANSIM_CM_LOAD(nprow, nreg, s ^ 1u);
+        }
+        // first recombination window of the next item, fetched into the registers just consumed: its donor
+        // loads are in flight while this item's SNP events are applied
+        if (hr_on && more) hw_cur = hr_window_fetch(a, hr_gen, m.hr_thr, hr_thr_s, nprow, blk_reg0 + nreg, lane, 0u, 0u);
 
         if (RNG && a.mut_nsub) {
             // ---- SNP mutation (population.rs:512-539) ----
@@ -504,13 +527,12 @@ __device__ __forceinline__ void mut_cta_items(const CoreMutArgs &a, const MutSme
             }
         }
         __syncwarp();
-        row += d_row; breg += d_reg;
-        if (breg >= blk_regs) { breg -= blk_regs; row++; }
-        prow = nprow;
+        row = nrow; breg = nreg; prow = nprow;
         if (++s == (uint32_t)CM_STAGES) { s = 0; par ^= 1u; }
     }
     if (lane == 0) bulk_wait<0>();
 #undef PANSIM_CM_ISSUE_LOAD
+#undef PANSIM_CM_LOAD
 #undef PANSIM_CM_PARENT
 }
 

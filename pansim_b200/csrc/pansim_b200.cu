@@ -1422,6 +1422,13 @@ int pansim_create(const pansim_config *cfg, pansim_ctx **out)
 
         // launch shape of the core kernel
         c->core_smem = core_mut_smem_bytes(c->tab_mut.size, c->tab_hr.nsub ? c->tab_hr.size : 0u);
+        {
+            // at most CM_RESIDENT_CTAS core CTAs per SM: the registers and shared memory they leave free hold
+            // the selection chain's CTAs while the core kernel runs (core_mut.cuh)
+            const size_t fit = prop.sharedMemPerMultiprocessor / (CM_RESIDENT_CTAS + 1) + 1;
+            if (fit > prop.reservedSharedMemPerBlock)
+                c->core_smem = std::max(c->core_smem, std::min(fit - prop.reservedSharedMemPerBlock, prop.sharedMemPerBlockOptin));
+        }
         if (const char *e = getenv("PANSIM_CORE_SMEM_PAD_KB")) c->core_smem += (size_t)std::max(0, atoi(e)) * 1024;   // experiment: cap the CTAs per SM
         if (const char *e = getenv("PANSIM_HR_DEFER")) c->hr_defer = atoi(e) != 0;
         CU(c, cudaFuncSetAttribute(core_mut_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->core_smem));
@@ -1441,13 +1448,11 @@ int pansim_create(const pansim_config *cfg, pansim_ctx **out)
             c->core_items_per_warp = (uint32_t)std::max<uint64_t>(1, (items + ctas * CM_WARPS - 1) / (ctas * CM_WARPS));
         }
         if (const char *e = getenv("PANSIM_CORE_ITEMS_PER_WARP")) c->core_items_per_warp = (uint32_t)std::max(1, atoi(e));
-        // Items per warp in the device-resident batch. A CTA of this kernel fills its SM slot completely
-        // (registers and shared memory), so a selection-chain kernel of the NEXT generation can only start
-        // where a core CTA has just retired: the shorter the CTAs live, the sooner the chain gets its slots,
-        // and the chain (select + accessory step, ~150 us serial under contention) is what the core step waits
-        // for once the kernel itself is fast enough. Measured at cfg2 (round 2, us per generation): 3 items 168.7,
-        // 4 items 164.2, 6 items 171.1, 8 items 179.7, 12 items 182.8.
-        c->core_items_batch = std::max(c->core_items_per_warp, 5u);     // cfg2 sweep with the tcgen05 selection chain: 4 -> 161, 5 -> 155, 6 -> 160 us per generation
+        // Items per warp in the device-resident batch. Short-lived CTAs turn SM slots over often, so the chain
+        // (select + accessory step) of the NEXT generation finds room sooner; longer ones pay the per-warp
+        // prologue less often. Measured at cfg2 with the two-stage kernel at 4 resident CTAs (us per
+        // generation): 4 items 146.9-147.4, 5 items 143.8-144.3, 6 items 152.6-153.0.
+        c->core_items_batch = std::max(c->core_items_per_warp, 5u);
         if (const char *e = getenv("PANSIM_CORE_ITEMS_BATCH")) c->core_items_batch = (uint32_t)std::max(0, atoi(e));
         const uint64_t per_cta = (uint64_t)CM_WARPS * c->core_items_per_warp;
         c->core_grid = (uint32_t)std::max<uint64_t>(1, (items + per_cta - 1) / per_cta);
