@@ -5,24 +5,15 @@
 // (population.rs:817) = number of differing sites. On 2-bit codes a site
 // differs iff either bit of the XOR is set:
 //   d = a ^ b;  m = (d | d >> 1) & 0x5555...;  differing sites = popc(m)
-// Two words share one POPC by parking the second mask in the odd bits.
-// Row padding is zero in every row, so it never contributes.
+// The pair kernels compare the bit-plane form of the rows (core_planes_kernel),
+// where the mask is one OR of two XORs. Row padding is zero in every row, so it
+// never contributes.
 #pragma once
 #include <cuda.h>          // CUtensorMap (the encoder is fetched through cudaGetDriverEntryPoint: no libcuda link)
 
 #include "common.cuh"
 
 namespace pansim {
-
-__device__ __forceinline__ uint32_t diff_sites4(const uint4 a, const uint4 b)
-{
-    const uint32_t d0 = a.x ^ b.x, d1 = a.y ^ b.y, d2 = a.z ^ b.z, d3 = a.w ^ b.w;
-    const uint32_t m0 = (d0 | (d0 >> 1)) & 0x55555555u;
-    const uint32_t m1 = (d1 | (d1 << 1)) & 0xAAAAAAAAu;
-    const uint32_t m2 = (d2 | (d2 >> 1)) & 0x55555555u;
-    const uint32_t m3 = (d3 | (d3 << 1)) & 0xAAAAAAAAu;
-    return __popc(m0 | m1) + __popc(m2 | m3);
-}
 
 __device__ __forceinline__ uint4 ld_stream(const uint4 *p)
 {
@@ -33,52 +24,13 @@ __device__ __forceinline__ uint4 ld_stream(const uint4 *p)
     return r;
 }
 
-// v1: one CTA per (pair, column chunk). Chunks are the slow grid dimension so
-// that concurrently running CTAs touch the same column slab of all rows
-// (N * chunk bytes is sized to stay L2-resident); partial counts are combined
-// with integer atomics (order-independent, exact).
 constexpr int PAIR_THREADS = 256;
 
-__global__ void __launch_bounds__(PAIR_THREADS) pair_core_kernel(const uint8_t *state, uint64_t row_stride,
-                                                                 uint32_t chunk_vec4, uint32_t row_vec4,
-                                                                 const uint32_t *range1, const uint32_t *range2,
-                                                                 uint32_t n_pairs, uint32_t *core_diff)
-{
-    __shared__ uint32_t wsum[PAIR_THREADS / 32];
-    const uint32_t chunk = blockIdx.y;
-    const uint32_t v_lo = chunk * chunk_vec4;
-    const uint32_t v_hi = min(row_vec4, v_lo + chunk_vec4);
-    for (uint32_t p = blockIdx.x; p < n_pairs; p += gridDim.x) {
-        const uint4 *ra = reinterpret_cast<const uint4 *>(state + (uint64_t)range1[p] * row_stride);
-        const uint4 *rb = reinterpret_cast<const uint4 *>(state + (uint64_t)range2[p] * row_stride);
-        uint32_t acc = 0;
-        uint32_t v = v_lo + threadIdx.x;
-        for (; v + 3 * PAIR_THREADS < v_hi; v += 4 * PAIR_THREADS) {
-            const uint4 a0 = ld_stream(ra + v), b0 = ld_stream(rb + v);
-            const uint4 a1 = ld_stream(ra + v + PAIR_THREADS), b1 = ld_stream(rb + v + PAIR_THREADS);
-            const uint4 a2 = ld_stream(ra + v + 2 * PAIR_THREADS), b2 = ld_stream(rb + v + 2 * PAIR_THREADS);
-            const uint4 a3 = ld_stream(ra + v + 3 * PAIR_THREADS), b3 = ld_stream(rb + v + 3 * PAIR_THREADS);
-            acc += diff_sites4(a0, b0) + diff_sites4(a1, b1) + diff_sites4(a2, b2) + diff_sites4(a3, b3);
-        }
-        for (; v < v_hi; v += PAIR_THREADS) acc += diff_sites4(ld_stream(ra + v), ld_stream(rb + v));
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-        if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = acc;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            uint32_t t = 0;
-            for (int q = 0; q < PAIR_THREADS / 32; q++) t += wsum[q];
-            if (gridDim.y == 1) core_diff[p] = t; else atomicAdd(&core_diff[p], t);
-        }
-        __syncthreads();
-    }
-}
-
-// v1.5: row-stationary groups. Pairs are sorted by their first row on the host (plan
+// Row-stationary groups. Pairs are sorted by their first row on the host (plan
 // cached while the pair list is unchanged, as in the reference where the pairs are
 // fixed for the whole run, main.rs:413-427). A CTA handles one group = one row i and up
 // to PAIR_GROUP partner rows j: row i's words are loaded once per thread and compared
-// against every partner, which almost halves the L2 traffic of the pair-per-CTA kernel.
+// against every partner, which almost halves the L2 traffic of one CTA per pair.
 constexpr int PAIR_GROUP = 8;
 
 struct PairGroup {
@@ -86,54 +38,6 @@ struct PairGroup {
     uint32_t first;      // index into the sorted partner / original-index arrays
     uint32_t count;      // 1..PAIR_GROUP
 };
-
-__global__ void __launch_bounds__(PAIR_THREADS) pair_core_grouped_kernel(
-    const uint8_t *state, uint64_t row_stride, uint32_t chunk_vec4, uint32_t row_vec4, const PairGroup *groups,
-    uint32_t n_groups, const uint32_t *partner, const uint32_t *orig_index, uint32_t *core_diff)
-{
-    __shared__ uint32_t wsum[PAIR_THREADS / 32][PAIR_GROUP];
-    const uint32_t chunk = blockIdx.y;
-    const uint32_t v_lo = chunk * chunk_vec4;
-    const uint32_t v_hi = min(row_vec4, v_lo + chunk_vec4);
-    for (uint32_t g = blockIdx.x; g < n_groups; g += gridDim.x) {
-        const PairGroup grp = groups[g];
-        const uint4 *ra = reinterpret_cast<const uint4 *>(state + (uint64_t)grp.row_i * row_stride);
-        const uint4 *rb[PAIR_GROUP];
-#pragma unroll
-        for (int q = 0; q < PAIR_GROUP; q++) {
-            const uint32_t j = partner[grp.first + (q < (int)grp.count ? q : 0)];
-            rb[q] = reinterpret_cast<const uint4 *>(state + (uint64_t)j * row_stride);
-        }
-        uint32_t acc[PAIR_GROUP];
-#pragma unroll
-        for (int q = 0; q < PAIR_GROUP; q++) acc[q] = 0;
-        for (uint32_t v = v_lo + threadIdx.x; v < v_hi; v += PAIR_THREADS) {
-            const uint4 a = ld_stream(ra + v);
-            uint4 b[PAIR_GROUP];
-#pragma unroll
-            for (int q = 0; q < PAIR_GROUP; q++) b[q] = ld_stream(rb[q] + v);
-#pragma unroll
-            for (int q = 0; q < PAIR_GROUP; q++) acc[q] += diff_sites4(a, b[q]);
-        }
-#pragma unroll
-        for (int q = 0; q < PAIR_GROUP; q++) {
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) acc[q] += __shfl_xor_sync(0xffffffffu, acc[q], o);
-        }
-        if ((threadIdx.x & 31) == 0) {
-#pragma unroll
-            for (int q = 0; q < PAIR_GROUP; q++) wsum[threadIdx.x >> 5][q] = acc[q];
-        }
-        __syncthreads();
-        if (threadIdx.x < grp.count) {
-            uint32_t t = 0;
-            for (int w = 0; w < PAIR_THREADS / 32; w++) t += wsum[w][threadIdx.x];
-            const uint32_t out = orig_index[grp.first + threadIdx.x];
-            atomicAdd(&core_diff[out], t);
-        }
-        __syncthreads();
-    }
-}
 
 // Exact all-pairs mode: the pair list of a row block [row_begin, row_end) -- every (i, j) with
 // i < j < N, ordered by i then j -- and its row-stationary groups are generated on the device, so
@@ -184,7 +88,7 @@ struct TileBatch {
 //
 // The XOR-popcount on 2-bit cells costs three logic operations per 32-bit word before the POPC
 // ((a ^ b), >> 1, (x | s) & 0x5555...), all on the ALU pipe the POPC shares (64 lanes/clk/SM, POPC a
-// quarter of that): 12 ALU slots per 32 sites, which is what bounded the row-stationary kernel at
+// quarter of that): 12 ALU slots per 32 sites, which is what bounded a row-stationary kernel on 2-bit cells at
 // 4.3e7 pairs/s. A site differs iff its low bits differ OR its high bits differ, so with the low bits
 // and the high bits of 32 sites in two separate words the mask is two operations:
 //     m = (aL ^ bL) | (aH ^ bH)            (LOP3, LOP3)           -> 7 slots per 32 sites with the POPC
@@ -217,7 +121,7 @@ __device__ __forceinline__ uint32_t diff_planes(const uint4 a, const uint4 b)
     return __popc(m0) + __popc(m1);
 }
 
-// row-stationary groups (see pair_core_grouped_kernel) on the plane form: the sparse remainder of a
+// row-stationary groups (PairGroup) on the plane form: the sparse remainder of a
 // sampled pair list and the exact all-pairs row blocks
 __global__ void __launch_bounds__(PAIR_THREADS, 4) pair_planes_grouped_kernel(
     const uint8_t *planes, uint64_t row_stride, uint32_t chunk_vec4, uint32_t row_vec4, const PairGroup *groups,

@@ -13,8 +13,8 @@
 //
 // Pair kernel: all tile pairs I <= J over tiles of 128 used genes, the tile pair of a CTA found by binary search
 // over the closed form of ld_pair_kernel's tile-pair offsets (tile I pairs with every J >= I). The operand pipeline
-// of ld_pair_kernel (ld_pipe_*: u8 expansion, tcgen05.mma.kind::i8, tcgen05.ld) puts c = the rows carrying both
-// genes in tensor memory. The epilogue forms D, r^2 and q per pair and keeps the class totals in registers while the
+// of bitmma.cuh (u8 expansion, tcgen05.mma.kind::i8, tcgen05.ld) puts c = the rows carrying both genes in tensor
+// memory. The epilogue forms D, r^2 and q per pair and keeps the class totals in registers while the
 // class does not change along a thread's columns (groups are one contiguous gene range, so at most twice), then in
 // shared memory; the r^2 histogram is counted in shared u32 counters. At CTA exit both go to global u64 counters
 // (r^2 as a 128-bit sum).
@@ -149,7 +149,7 @@ __global__ void __launch_bounds__(LD_THREADS, 3) gene_ld_pair_kernel(const GeneL
     __shared__ double s_inv[LD_TILE];
     __shared__ unsigned long long s_cls[3][GL_CLASS_WORDS - 1];      // pairs, four-gamete, sum of q, associated, dissociated
     __shared__ uint32_t s_ij[2];
-    const LdPipe m = ld_pipe(um_smem);
+    const BitMma m = bitmma_smem<LD_KB>(um_smem);
     uint32_t *s_hist = reinterpret_cast<uint32_t *>(um_smem + LD_OPERAND_SMEM);
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
@@ -163,12 +163,12 @@ __global__ void __launch_bounds__(LD_THREADS, 3) gene_ld_pair_kernel(const GeneL
         }
         s_ij[0] = lo;
         s_ij[1] = lo + (uint32_t)(blockIdx.x - gene_ld_tile_off(lo, p.n_tiles));
-        ld_pipe_init(m);
+        bitmma_init<LD_KB>(m);
     }
     for (uint32_t b = threadIdx.x; b < 3 * p.r2_bins; b += LD_THREADS) s_hist[b] = 0;
     if (threadIdx.x < 3 * (GL_CLASS_WORDS - 1)) (&s_cls[0][0])[threadIdx.x] = 0;
-    if (warp == UB_EXP_WARPS) ld_pipe_alloc(m);
-    const uint32_t tmem = ld_pipe_tmem(m);
+    if (warp == UB_EXP_WARPS) bitmma_alloc(m);
+    const uint32_t tmem = bitmma_tmem(m);
     const uint32_t bi = s_ij[0], bj = s_ij[1];
     if (threadIdx.x < LD_TILE) {
         const uint32_t j = bj * LD_TILE + threadIdx.x;
@@ -178,13 +178,13 @@ __global__ void __launch_bounds__(LD_THREADS, 3) gene_ld_pair_kernel(const GeneL
         s_inv[threadIdx.x] = ok ? p.inv[j] : 0.0;
     }
 
-    ld_pipe_mma(m, tmem, p.x, p.kw, p.k_iters, p.n_used, bi, bj, warp, lane);
+    bitmma_mainloop<LD_KB>(m, tmem, p.x, p.kw, p.n_used, p.k_iters, bi, bj, warp, lane);
     __syncthreads();                                   // s_a / s_grp / s_inv / s_cls / s_hist written
 
     // ---- epilogue: warps w and w + 4 share the accumulator lanes 32 * (w % 4) .. + 31 (genes i of the I tile)
     //      and split the 128 columns (genes j of the J tile) ----
     if (warp < UB_EXP_WARPS) {
-        ld_pipe_wait(m);
+        bitmma_wait(m);
         const uint32_t quad = warp & 3u;
         const uint32_t ci = bi * LD_TILE + quad * 32u + lane;
         const bool i_ok = ci < p.n_used;
@@ -206,7 +206,7 @@ __global__ void __launch_bounds__(LD_THREADS, 3) gene_ld_pair_kernel(const GeneL
 #pragma unroll 1
         for (uint32_t c0 = (warp >> 2) * 64u; c0 < (warp >> 2) * 64u + 64u; c0 += 16) {
             uint32_t v[16];
-            ld_pipe_load16(tmem, quad, c0, v);
+            bitmma_load16(tmem, quad, c0, v);
             if (!i_ok) continue;
 #pragma unroll
             for (uint32_t q = 0; q < 16; q++) {
@@ -230,7 +230,7 @@ __global__ void __launch_bounds__(LD_THREADS, 3) gene_ld_pair_kernel(const GeneL
         }
         flush();
     }
-    ld_pipe_free(tmem, warp);
+    bitmma_free(tmem, warp);
     if (threadIdx.x < 3 && s_cls[threadIdx.x][0]) {
         unsigned long long *g = p.out + GL_CLASS_WORDS * threadIdx.x;
         atomicAdd(g, s_cls[threadIdx.x][0]);

@@ -14,7 +14,7 @@
 // Tile list: used sites in tiles of 128. Tile I pairs with J = I .. the tile of the last used site within max_dist
 // of I's last site (ld_tiles_kernel: a binary search per I), scanned into tile-pair offsets.
 //
-// Pair kernel: one CTA per tile pair, the structure of acc_inter_umma_bits_kernel<64> (select.cuh): eight warps
+// Pair kernel: one CTA per tile pair on the operand pipeline of bitmma.cuh with 64-byte swizzled rows: eight warps
 // expand the bit rows of both tiles into the swizzled K-major u8 operand layout, one thread issues
 // tcgen05.mma.kind::i8 into a 128 x 128 s32 accumulator in tensor memory, which holds c = the rows derived at both
 // sites. The same eight warps then read it with tcgen05.ld and form D, r^2, q and the four-gamete test per pair,
@@ -22,8 +22,8 @@
 // memory, then global u64 adds (r^2 as a 128-bit sum: lo with carry into hi). About 50 KB of shared memory and
 // 128 tensor-memory columns per CTA, so several CTAs share an SM and one's epilogue overlaps another's MMAs.
 #pragma once
+#include "bitmma.cuh"
 #include "common.cuh"
-#include "select.cuh"
 #include "vcf.cuh"
 
 namespace pansim {
@@ -221,151 +221,13 @@ __device__ __forceinline__ void ld_add128(unsigned long long *hi, unsigned long 
     if (old + x < old) atomicAdd(hi, 1ull);
 }
 
-// operand stages and barriers (UbCfg<LD_KB>::smem_bytes()), then the per-CTA bins when they fit
-constexpr uint32_t LD_OPERAND_SMEM = 1024 + 2 * UbCfg<LD_KB>::STAGES * UbCfg<LD_KB>::TILE_BYTES + (2 * UbCfg<LD_KB>::STAGES + 1) * 8 + 16;
+// operand stages and barriers, then the per-CTA bins when they fit
+constexpr uint32_t LD_OPERAND_SMEM = (uint32_t)UbCfg<LD_KB>::smem_bytes();
 static_assert(LD_OPERAND_SMEM % 8 == 0, "per-CTA bins are 8-byte words");
 
 static inline size_t ld_pair_smem_bytes(uint32_t n_bins)
 {
     return LD_OPERAND_SMEM + (n_bins <= LD_SMEM_BINS ? 3 * (size_t)n_bins * sizeof(unsigned long long) : 0);
-}
-
-// ---- the operand pipeline of the pair kernels (ld_pair_kernel here, gene_ld_pair_kernel in gene_ld.cuh) ----
-// Shared-memory addresses of the operand stages, the barriers and the tensor-memory slot in the dynamic shared memory.
-struct LdPipe {
-    uint32_t a_s, b_s, full_s, empty_s, done_s, slot_s;
-};
-
-__device__ __forceinline__ LdPipe ld_pipe(const uint8_t *smem)
-{
-    using Cfg = UbCfg<LD_KB>;
-    constexpr uint32_t STAGES = Cfg::STAGES, TILE_BYTES = Cfg::TILE_BYTES;
-    LdPipe m;
-    const uint32_t base_s = (smem_u32(smem) + 1023u) & ~1023u;
-    m.a_s = base_s;
-    m.b_s = base_s + STAGES * TILE_BYTES;
-    m.full_s = m.b_s + STAGES * TILE_BYTES;
-    m.empty_s = m.full_s + STAGES * 8u;
-    m.done_s = m.empty_s + STAGES * 8u;
-    m.slot_s = m.done_s + 8u;
-    return m;
-}
-
-// one thread: the stage barriers and the accumulator's
-__device__ __forceinline__ void ld_pipe_init(const LdPipe &m)
-{
-    for (uint32_t s = 0; s < UbCfg<LD_KB>::STAGES; s++) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(m.full_s + s * 8u), "r"((uint32_t)UB_EXP_WARPS) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(m.empty_s + s * 8u), "r"(1u) : "memory");
-    }
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(m.done_s), "r"(1u) : "memory");
-    fence_mbar_init();
-}
-
-// the MMA warp: the accumulator's tensor-memory columns
-__device__ __forceinline__ void ld_pipe_alloc(const LdPipe &m)
-{
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(m.slot_s), "r"(UM_TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-
-// every thread, after ld_pipe_init and ld_pipe_alloc: a CTA barrier, then the accumulator's address
-__device__ __forceinline__ uint32_t ld_pipe_tmem(const LdPipe &m)
-{
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    uint32_t tmem;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem) : "r"(m.slot_s) : "memory");
-    return tmem;
-}
-
-// Main loop: threads 0..127 expand the bit rows of tile bi, 128..255 those of tile bj (rows at or past n_all are
-// zero) into the swizzled K-major u8 stages; lane 0 of the MMA warp issues tcgen05.mma.kind::i8 into the
-// 128 x 128 s32 accumulator, which then holds the rows set in both rows of x, and commits to done_s.
-__device__ __forceinline__ void ld_pipe_mma(const LdPipe &m, uint32_t tmem, const uint32_t *x, uint32_t kw, uint32_t k_iters,
-                                            uint32_t n_all, uint32_t bi, uint32_t bj, uint32_t warp, uint32_t lane)
-{
-    using Cfg = UbCfg<LD_KB>;
-    constexpr uint32_t STAGES = Cfg::STAGES, TILE_BYTES = Cfg::TILE_BYTES, WORDS = LD_KB / 32;
-    if (warp < UB_EXP_WARPS) {
-        // ---- expansion: threads 0..127 = rows of the I tile, 128..255 = rows of the J tile ----
-        const uint32_t tr = threadIdx.x & 127u;
-        const bool is_b = threadIdx.x >= 128u;
-        const uint32_t grow = (is_b ? bj : bi) * LD_TILE + tr;
-        const bool row_ok = grow < n_all;
-        const uint2 *src = reinterpret_cast<const uint2 *>(x + (uint64_t)(row_ok ? grow : 0u) * kw);
-        const uint32_t row_s = (is_b ? m.b_s : m.a_s) + tr * LD_KB;
-        const uint32_t sw = ((tr >> 1) & 3u) << 4;                          // SWIZZLE_64B
-        uint2 nxt = row_ok ? __ldg(src) : make_uint2(0, 0);
-        for (uint32_t it = 0; it < k_iters; it++) {
-            const uint32_t s = it % STAGES, n = it / STAGES;
-            const uint2 cur = nxt;
-            if (it + 1u < k_iters) nxt = row_ok ? __ldg(src + it + 1u) : make_uint2(0, 0);
-            if (n) mbar_wait_or_trap(m.empty_s + s * 8u, (n - 1u) & 1u);
-            const uint32_t dst = row_s + s * TILE_BYTES;
-#pragma unroll
-            for (uint32_t q = 0; q < WORDS; q++) {
-                const uint32_t v = q ? cur.y : cur.x;
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + (((2u * q) << 4) ^ sw)), "r"(v & 0x01010101u),
-                             "r"((v >> 1) & 0x01010101u), "r"((v >> 2) & 0x01010101u), "r"((v >> 3) & 0x01010101u) : "memory");
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + (((2u * q + 1u) << 4) ^ sw)), "r"((v >> 4) & 0x01010101u),
-                             "r"((v >> 5) & 0x01010101u), "r"((v >> 6) & 0x01010101u), "r"((v >> 7) & 0x01010101u) : "memory");
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(m.full_s + s * 8u) : "memory");
-        }
-    } else {
-        if (lane == 0) {
-            // ---- MMA issue ----
-            for (uint32_t it = 0; it < k_iters; it++) {
-                const uint32_t s = it % STAGES, n = it / STAGES;
-                mbar_wait_or_trap(m.full_s + s * 8u, n & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint32_t a_lo = (((m.a_s + s * TILE_BYTES) & 0x3FFFFu) >> 4) | (1u << 16);
-                const uint32_t b_lo = (((m.b_s + s * TILE_BYTES) & 0x3FFFFu) >> 4) | (1u << 16);
-#pragma unroll
-                for (uint32_t k = 0; k < LD_KB / 32; k++) {
-                    const uint64_t da = ((uint64_t)Cfg::DESC_HI << 32) | (a_lo + 2u * k);
-                    const uint64_t db = ((uint64_t)Cfg::DESC_HI << 32) | (b_lo + 2u * k);
-                    const uint32_t accumulate = (it | k) ? 1u : 0u;
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                 "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                                 ::"r"(tmem), "l"(da), "l"(db), "r"(UM_IDESC), "r"(accumulate) : "memory");
-                }
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(m.empty_s + s * 8u) : "memory");
-            }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(m.done_s) : "memory");
-        }
-        __syncwarp();
-    }
-}
-
-// an epilogue warp: wait until the accumulator is complete
-__device__ __forceinline__ void ld_pipe_wait(const LdPipe &m)
-{
-    mbar_wait_or_trap(m.done_s, 0u);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-}
-
-// columns c0 .. c0 + 15 of accumulator lanes 32 * quad .. + 31 (the warp's lane = its row)
-__device__ __forceinline__ void ld_pipe_load16(uint32_t tmem, uint32_t quad, uint32_t c0, uint32_t (&v)[16])
-{
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(tmem + ((quad * 32u) << 16) + c0) : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// every thread: a CTA barrier, then the MMA warp frees the accumulator
-__device__ __forceinline__ void ld_pipe_free(uint32_t tmem, uint32_t warp)
-{
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == UB_EXP_WARPS) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(UM_TMEM_COLS) : "memory");
 }
 
 __global__ void __launch_bounds__(LD_THREADS, 3) ld_pair_kernel(const LdPairArgs p)
@@ -374,7 +236,7 @@ __global__ void __launch_bounds__(LD_THREADS, 3) ld_pair_kernel(const LdPairArgs
     __shared__ uint32_t s_pos[LD_TILE], s_a[LD_TILE];
     __shared__ double s_inv[LD_TILE];
     __shared__ uint32_t s_ij[2];
-    const LdPipe m = ld_pipe(um_smem);
+    const BitMma m = bitmma_smem<LD_KB>(um_smem);
     // per-CTA bins after the operand stages and barriers: pairs, four-gamete, sum of q
     unsigned long long *s_bins = reinterpret_cast<unsigned long long *>(um_smem + LD_OPERAND_SMEM);
     const bool smem_bins = p.n_bins <= LD_SMEM_BINS;
@@ -390,12 +252,12 @@ __global__ void __launch_bounds__(LD_THREADS, 3) ld_pair_kernel(const LdPairArgs
         }
         s_ij[0] = lo;
         s_ij[1] = lo + (uint32_t)(blockIdx.x - p.tile_off[lo]);
-        ld_pipe_init(m);
+        bitmma_init<LD_KB>(m);
     }
     if (smem_bins)
         for (uint32_t b = threadIdx.x; b < 3 * p.n_bins; b += LD_THREADS) s_bins[b] = 0;
-    if (warp == UB_EXP_WARPS) ld_pipe_alloc(m);
-    const uint32_t tmem = ld_pipe_tmem(m);
+    if (warp == UB_EXP_WARPS) bitmma_alloc(m);
+    const uint32_t tmem = bitmma_tmem(m);
     const uint32_t bi = s_ij[0], bj = s_ij[1];
     if (threadIdx.x < LD_TILE) {
         const uint32_t j = bj * LD_TILE + threadIdx.x;
@@ -405,13 +267,13 @@ __global__ void __launch_bounds__(LD_THREADS, 3) ld_pair_kernel(const LdPairArgs
         s_inv[threadIdx.x] = ok ? p.inv[j] : 0.0;
     }
 
-    ld_pipe_mma(m, tmem, p.x, p.kw, p.k_iters, p.n_all, bi, bj, warp, lane);
+    bitmma_mainloop<LD_KB>(m, tmem, p.x, p.kw, p.n_all, p.k_iters, bi, bj, warp, lane);
     __syncthreads();                                   // s_pos / s_a / s_inv written
 
     // ---- epilogue: warps w and w + 4 share the accumulator lanes 32 * (w % 4) .. + 31 (sites i of the I tile)
     //      and split the 128 columns (sites j of the J tile) ----
     if (warp < UB_EXP_WARPS) {
-        ld_pipe_wait(m);
+        bitmma_wait(m);
         const uint32_t quad = warp & 3u;
         const uint32_t ci = bi * LD_TILE + quad * 32u + lane;
         const bool i_ok = ci < p.n_own;
@@ -438,7 +300,7 @@ __global__ void __launch_bounds__(LD_THREADS, 3) ld_pair_kernel(const LdPairArgs
 #pragma unroll 1
         for (uint32_t c0 = (warp >> 2) * 64u; c0 < (warp >> 2) * 64u + 64u; c0 += 16) {
             uint32_t v[16];
-            ld_pipe_load16(tmem, quad, c0, v);
+            bitmma_load16(tmem, quad, c0, v);
             if (!i_ok) continue;
 #pragma unroll
             for (uint32_t q = 0; q < 16; q++) {
@@ -458,7 +320,7 @@ __global__ void __launch_bounds__(LD_THREADS, 3) ld_pair_kernel(const LdPairArgs
         }
         flush();
     }
-    ld_pipe_free(tmem, warp);
+    bitmma_free(tmem, warp);
     if (smem_bins)
         for (uint32_t b = threadIdx.x; b < p.n_bins; b += LD_THREADS) {
             const unsigned long long np = s_bins[b];

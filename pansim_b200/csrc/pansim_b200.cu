@@ -185,22 +185,8 @@ struct pansim_ctx {
     bool avgdist_valid = false;
     bool fitness_valid = false;   // d_logfit / d_num_genes match the current accessory state
     bool neutral = true;          // every selection coefficient is 0 (ln(1 + s_j) = +0.0 for all genes)
-    bool inter_popc = false;      // competition term: AND/popcount tiles instead of the tensor-core kernel
-    // PANSIM_INTER_UMMA: 2 / 3 = tcgen05 intersection kernel that expands the bit rows to bytes inside the CTA (128- / 64-byte
-    // swizzled operand rows: 128 KiB / 48 KiB of shared memory), 1 = tcgen05 kernel fed by TMA from a byte-expanded copy of the
-    // presence matrix, 0 = warp-level mma.sync on the bit matrix. Generation step at cfg2: 155 (2), 165 (3), 164 (1), 161-165 (0) us.
-    int inter_umma = 2;
-    bool umma_bits_ready = false;
-    uint8_t *d_acc_bytes = nullptr;   // [N][acc_kpad] one byte per gene (operand of the tcgen05 kernel), made per call
-    uint32_t acc_kpad = 0;            // genes per row of d_acc_bytes (a multiple of UM_KBYTES)
-    CUtensorMap acc_bytes_tmap;
-    bool acc_bytes_tmap_ok = false;
-    // PANSIM_AVG_RCP: 0 = IEEE division in the mean-distance kernel; 1 = quotients from a reciprocal table (bit-identical,
-    // 12 % fewer instructions, but a second dependent load per round: 157.8 against 155.0 us per generation at cfg2);
-    // 2 = the table kernel software-pipelined over the rounds (avg_distance_pipe_kernel: 3.6 -> 2.2 M instructions per
-    // launch, 154.4 against 154.7 us per generation)
-    int avg_rcp = 2;
-    double *d_rcp = nullptr;          // RN(1 / b), b = 0 .. G + core_genes
+    bool umma_bits_ready = false;     // the intersection kernel's dynamic shared-memory limit is raised
+    double *d_rcp = nullptr;          // RN(1 / b), b = 0 .. G + core_genes; only when G + core_genes <= AVG_RCP_MAX
     bool fitness_blocked = false; // large shapes: blocked (fixed-association) fitness sum instead of the sequential chain
 
     HostPoissonTable tab_mut, tab_hr;    // per 256-site block (SNPs), per 8192-site region (HR)
@@ -598,42 +584,16 @@ int launch_fitness(pansim_ctx *c, cudaStream_t st = nullptr)
     return 0;
 }
 
-// operand of the tcgen05 intersection kernel: byte matrix + its 2-D tensor map (x = genes, y = individuals;
-// box = 128 genes x 128 individuals, 128-byte swizzle), and the reciprocal table of the lane distance kernel
+// the intersection matrix, the intersection kernel's shared-memory limit, and the reciprocal table of the mean-distance
+// kernel when the shape allows it
 int ensure_competition_buffers(pansim_ctx *c)
 {
     if (!c->d_inter) CU(c, cudaMalloc(&c->d_inter, (size_t)c->N * c->N * sizeof(uint32_t)));
-    if (c->inter_umma >= 2 && !c->inter_popc && !c->umma_bits_ready) {
-        CU(c, cudaFuncSetAttribute(acc_inter_umma_bits_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UbCfg<128>::smem_bytes()));
-        CU(c, cudaFuncSetAttribute(acc_inter_umma_bits_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UbCfg<64>::smem_bytes()));
+    if (!c->umma_bits_ready) {
+        CU(c, cudaFuncSetAttribute(acc_inter_umma_bits_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UbCfg<128>::smem_bytes()));
         c->umma_bits_ready = true;
     }
-    if (c->inter_umma == 1 && !c->inter_popc && !c->d_acc_bytes) {
-        c->acc_kpad = (uint32_t)div_up64(std::max<uint64_t>(c->G, 1), UM_KBYTES) * UM_KBYTES;
-        const size_t bytes = (size_t)c->N * c->acc_kpad;
-        if (cudaMalloc(&c->d_acc_bytes, bytes) != cudaSuccess) FAIL(c, PANSIM_ERR_NOMEM, "cudaMalloc of %zu bytes (byte-expanded accessory matrix) failed", bytes);
-        c->acc_bytes_tmap_ok = false;
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess && fn &&
-            qres == cudaDriverEntryPointSuccess) {
-            typedef CUresult (*encode_t)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                         const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                         CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-            const cuuint64_t gdim[2] = {c->acc_kpad, c->N};
-            const cuuint64_t gstride[1] = {c->acc_kpad};
-            const cuuint32_t box[2] = {UM_KBYTES, UM_TILE};
-            const cuuint32_t estr[2] = {1, 1};
-            const CUresult r = reinterpret_cast<encode_t>(fn)(&c->acc_bytes_tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, c->d_acc_bytes, gdim, gstride,
-                                                             box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            c->acc_bytes_tmap_ok = r == CUDA_SUCCESS;
-        }
-        cudaGetLastError();
-        if (!c->acc_bytes_tmap_ok) FAIL(c, PANSIM_ERR_CUDA, "no TMA descriptor for the byte-expanded accessory matrix (cuTensorMapEncodeTiled unavailable)");
-        CU(c, cudaFuncSetAttribute(acc_inter_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)inter_umma_smem_bytes()));
-    }
-    if (c->avg_rcp && !c->d_rcp && (uint64_t)c->G + c->cfg.core_genes <= AVG_RCP_MAX) {
+    if (!c->d_rcp && (uint64_t)c->G + c->cfg.core_genes <= AVG_RCP_MAX) {
         const size_t n = (size_t)c->G + c->cfg.core_genes + 1;
         std::vector<double> h(n);
         for (size_t b = 0; b < n; b++) h[b] = 1.0 / (double)b;            // IEEE division: correctly rounded; b = 0 -> inf
@@ -659,44 +619,18 @@ int launch_competition(pansim_ctx *c)
         CU(c, cudaEventRecord(c->ev_join, c->stream_aux));
         c->fitness_join_pending = true;
     }
-    if (c->inter_popc) {     // PANSIM_INTER_POPC=1: the AND/popcount tile kernel instead of the tensor-core one
-        const uint32_t nb = div_up64(c->N, 32);
-        acc_inter_kernel<<<dim3(nb, nb), 256, 0, c->stream>>>(c->acc[c->acc_cur], c->N, c->acc_stride_words,
-                                                              c->acc_words, c->d_inter, c->d_inter_diag);
-    } else if (c->inter_umma >= 2) {
-        const uint32_t nb = div_up64(c->N, UM_TILE);
-        const uint64_t genes = std::max<uint64_t>(c->G, 1);
-        if (c->inter_umma == 2)
-            acc_inter_umma_bits_kernel<128><<<nb * (nb + 1) / 2, UB_THREADS, UbCfg<128>::smem_bytes(), c->stream>>>(
-                c->acc[c->acc_cur], c->N, c->acc_stride_words, (uint32_t)div_up64(genes, 128), c->d_inter, c->d_inter_diag);
-        else
-            acc_inter_umma_bits_kernel<64><<<nb * (nb + 1) / 2, UB_THREADS, UbCfg<64>::smem_bytes(), c->stream>>>(
-                c->acc[c->acc_cur], c->N, c->acc_stride_words, (uint32_t)div_up64(genes, 64), c->d_inter, c->d_inter_diag);
-    } else if (c->inter_umma == 1) {
-        const uint32_t kw = c->acc_kpad / 32u;
-        acc_expand_bytes_kernel<<<div_up64((uint64_t)c->N * kw, 256), 256, 0, c->stream>>>(c->acc[c->acc_cur], c->N, c->acc_stride_words,
-                                                                                         kw, c->d_acc_bytes);
-        LAUNCH_CHECK(c);
-        const uint32_t nb = div_up64(c->N, UM_TILE);
-        acc_inter_umma_kernel<<<nb * (nb + 1) / 2, UM_THREADS, inter_umma_smem_bytes(), c->stream>>>(
-            c->acc_bytes_tmap, c->N, c->acc_kpad / UM_KBYTES, c->d_inter, c->d_inter_diag);
-    } else {
-        const uint32_t nb = div_up64(c->N, IM_TILE);
-        acc_inter_mma_kernel<<<nb * (nb + 1) / 2, 256, 0, c->stream>>>(c->acc[c->acc_cur], c->N, c->acc_stride_words,
-                                                                  c->acc_words, c->d_inter, c->d_inter_diag);
-    }
+    const uint32_t nb = div_up64(c->N, UM_TILE);
+    acc_inter_umma_bits_kernel<<<nb * (nb + 1) / 2, UB_THREADS, UbCfg<128>::smem_bytes(), c->stream>>>(
+        c->acc[c->acc_cur], c->N, c->acc_stride_words, (uint32_t)div_up64(std::max<uint64_t>(c->G, 1), 128), c->d_inter, c->d_inter_diag);
     LAUNCH_CHECK(c);
     fs.reset();
     FineSpan fs2(c, TG_D_AVG);
-    if (c->avg_rcp == 2 && c->d_rcp)
+    if (c->d_rcp)          // the reciprocal table exists iff G + core_genes <= AVG_RCP_MAX
         avg_distance_pipe_kernel<<<div_up64(c->N, AVG_WARPS), AVG_WARPS * 32, 0, c->stream>>>(c->d_inter, c->d_inter_diag, c->N,
                                                                              c->cfg.core_genes, c->d_rcp, c->d_avgdist);
-    else if (c->avg_rcp && c->d_rcp)
-        avg_distance_kernel<true><<<div_up64(c->N, AVG_WARPS), AVG_WARPS * 32, 0, c->stream>>>(c->d_inter, c->d_inter_diag, c->N,
-                                                                              c->cfg.core_genes, c->d_rcp, c->d_avgdist);
     else
-        avg_distance_kernel<false><<<div_up64(c->N, AVG_WARPS), AVG_WARPS * 32, 0, c->stream>>>(c->d_inter, c->d_inter_diag, c->N,
-                                                                               c->cfg.core_genes, nullptr, c->d_avgdist);
+        avg_distance_kernel<<<div_up64(c->N, AVG_WARPS), AVG_WARPS * 32, 0, c->stream>>>(c->d_inter, c->d_inter_diag, c->N,
+                                                                        c->cfg.core_genes, c->d_avgdist);
     LAUNCH_CHECK(c);
     c->avgdist_valid = true;
     return 0;
@@ -1160,7 +1094,7 @@ void pansim_destroy(pansim_ctx *c)
     if (c->stream_core) cudaStreamSynchronize(c->stream_core);
     if (c->stream_aux) cudaStreamSynchronize(c->stream_aux);
     void *ptrs[] = {c->core[0], c->core[1], c->d_hr_slots, c->d_hr_counts, c->d_hr_ovf, c->d_hr_ovf_count, c->d_core_img, c->acc[0], c->acc[1], c->d_parents_buf[0], c->d_parents_buf[1], c->d_parents_buf[2], c->d_lw, c->d_lethal, c->d_logfit, c->d_avgdist,
-                    c->d_num_genes, c->d_inter_diag, c->d_tmp_a, c->d_tmp_b, c->d_weights, c->d_cum, c->d_err, c->d_inter, c->d_acc_bytes, c->d_rcp, c->d_rowInvK, c->d_gain_planes,
+                    c->d_num_genes, c->d_inter_diag, c->d_tmp_a, c->d_tmp_b, c->d_weights, c->d_cum, c->d_err, c->d_inter, c->d_rcp, c->d_rowInvK, c->d_gain_planes,
                     c->d_gain_thr, c->tab_mut.d_thr, c->tab_hr.d_thr, c->d_r1, c->d_r2, c->d_cd, c->d_in, c->d_un,
                     c->d_planes, c->d_work_counter, c->d_replay, c->d_hkeys, c->d_hvals, c->d_stage, c->d_groups, c->d_partner, c->d_orig, c->d_batches, c->d_tile_slots, c->d_tile_orig, c->d_dump_counters, c->d_mut_row, c->d_mut_site,
                     c->d_mut_seq, c->d_mut_allele, c->d_hr_rec, c->d_hr_locus, c->d_hr_donor, c->d_hr_seq,
@@ -1359,9 +1293,6 @@ int pansim_create(const pansim_config *cfg, pansim_ctx **out)
         // the bit-exact sequential fitness chain is kept up to 2^25 accessory cells (cfg1-3: 4e6)
         c->fitness_blocked = (uint64_t)c->N * c->G > (1ull << 25);
         if (const char *e = getenv("PANSIM_FITNESS_BLOCKED")) c->fitness_blocked = atoi(e) != 0;
-        if (const char *e = getenv("PANSIM_INTER_POPC")) c->inter_popc = atoi(e) != 0;
-        if (const char *e = getenv("PANSIM_INTER_UMMA")) c->inter_umma = atoi(e);
-        if (const char *e = getenv("PANSIM_AVG_RCP")) c->avg_rcp = atoi(e);
         if (const char *e = getenv("PANSIM_TILES2")) c->use_tiles2 = atoi(e) != 0;
         if (const char *e = getenv("PANSIM_GRAPH")) c->use_graph = atoi(e) != 0;
         if (const char *e = getenv("PANSIM_GRAPH_SPANS")) c->graph_spans = atoi(e) != 0;

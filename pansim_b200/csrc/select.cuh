@@ -4,7 +4,7 @@
 //   K3 weights + draw    population.rs:325-447
 #pragma once
 #include <cfloat>
-#include <cuda.h>          // CUtensorMap (acc_inter_umma_kernel)
+#include "bitmma.cuh"
 #include "common.cuh"
 
 namespace pansim {
@@ -303,443 +303,41 @@ __global__ void __launch_bounds__(FIT_WARPS * 32) fitness_blocked_kernel(const u
 }
 
 // ---------------------------------------------------------------------------
-// K2a: all-vs-all intersection counts I[i][j] = popc(row_i & row_j), 32x32 tiles,
-// upper triangle computed, mirrored on store.
+// K2a: all-vs-all intersection counts I[i][j] = popc(row_i & row_j), the dense contraction X * X^T of the 0/1
+// presence matrix on the tensor cores (bitmma.cuh). One CTA per upper-triangle tile of 128 x 128 pairs, mirrored on
+// store. The diagonal I[i][i] = |row_i| is also written as a compact vector: the distance kernel takes its gene
+// counts from there, so it does not have to wait for the (much longer) fitness kernel.
+// Rows are zero-padded to stride_words = a multiple of 4 words (at least 4), so k_iters = ceil(max(G, 1) / 128)
+// stages of 4 words never read past a row (the pipeline's precondition).
 // ---------------------------------------------------------------------------
-constexpr int INTER_CHUNK = 32;   // words per shared-memory chunk
-
-__global__ void __launch_bounds__(256) acc_inter_kernel(const uint32_t *acc, uint32_t n_rows,
-                                                        uint32_t stride_words, uint32_t n_words,
-                                                        uint32_t *inter, int32_t *diag)
+__global__ void __launch_bounds__(UB_THREADS, 1) acc_inter_umma_bits_kernel(const uint32_t *__restrict__ acc, uint32_t n_rows,
+                                                                           uint32_t stride_words, uint32_t k_iters,
+                                                                           uint32_t *inter, int32_t *diag)
 {
-    const uint32_t bi = blockIdx.y, bj = blockIdx.x;
-    if (bj < bi) return;
-    __shared__ uint32_t Ri[32][INTER_CHUNK + 1];
-    __shared__ uint32_t Rj[32][INTER_CHUNK + 1];
-    const uint32_t tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    uint32_t acc4[4] = {0, 0, 0, 0};
-    for (uint32_t w0 = 0; w0 < n_words; w0 += INTER_CHUNK) {
-        for (uint32_t q = ty; q < 32; q += 8) {
-            const uint32_t w = w0 + tx;
-            const uint32_t ri = bi * 32 + q, rj = bj * 32 + q;
-            Ri[q][tx] = (w < n_words && ri < n_rows) ? acc[(uint64_t)ri * stride_words + w] : 0u;
-            Rj[q][tx] = (w < n_words && rj < n_rows) ? acc[(uint64_t)rj * stride_words + w] : 0u;
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (uint32_t w = 0; w < INTER_CHUNK; w++) {
-            const uint32_t vj = Rj[tx][w];
-#pragma unroll
-            for (uint32_t q = 0; q < 4; q++) acc4[q] += __popc(Ri[ty + 8 * q][w] & vj);
-        }
-        __syncthreads();
-    }
-    for (uint32_t q = 0; q < 4; q++) {
-        const uint32_t i = bi * 32 + ty + 8 * q, j = bj * 32 + tx;
-        if (i < n_rows && j < n_rows) {
-            inter[(uint64_t)i * n_rows + j] = acc4[q];
-            inter[(uint64_t)j * n_rows + i] = acc4[q];
-            if (i == j) diag[i] = (int32_t)acc4[q];           // |row_i|: the gene count the distances need
-        }
-    }
-}
-
-// K2a (tensor cores): the intersection counts are the dense contraction X * X^T of the 0/1
-// presence matrix, so they run on the tensor cores as an integer MMA with exact s32 accumulation:
-// warp-level mma.sync m16n8k32 u8 x u8 (IMMA.16832 in SASS), the bits of a 32-gene word expanded
-// to 0/1 bytes in registers. A dot product does not care in which k slot a gene sits as long as
-// both operands agree, so the expansion is the cheapest one: the thread with t = lane % 4 takes
-// bits {t, t+8, t+16, t+24} ((w >> t) & 0x01010101) for the low k half of the fragment and bits
-// {t+4, ...} for the high half -- over t = 0..3 every bit of the word exactly once.
-// CTA = 64 x 64 pairs, 8 warps of 16 x 32; upper-triangle tiles only, mirrored on store. The
-// diagonal I[i][i] = |row_i| is also written as a compact vector: the distance kernel takes its
-// gene counts from there, so it does not have to wait for the (much longer) fitness kernel.
-constexpr int IM_TILE = 64;
-constexpr int IM_CHUNK = 32;      // words per shared-memory chunk
-
-__device__ __forceinline__ void imma_16832_u8(int (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
-                                              uint32_t b0, uint32_t b1)
-{
-    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-
-__global__ void __launch_bounds__(256) acc_inter_mma_kernel(const uint32_t *acc, uint32_t n_rows,
-                                                            uint32_t stride_words, uint32_t n_words,
-                                                            uint32_t *inter, int32_t *diag)
-{
+    extern __shared__ uint8_t um_smem[];
+    const BitMma m = bitmma_smem<128>(um_smem);
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     // blockIdx.x enumerates the upper-triangle tiles row by row: (0,0..nb-1), (1,1..nb-1), ...
-    const uint32_t nb = (n_rows + IM_TILE - 1) / IM_TILE;
-    uint32_t t_lin = blockIdx.x, bi = 0;
-    while (t_lin >= nb - bi) { t_lin -= nb - bi; bi++; }
-    const uint32_t bj = bi + t_lin;
-    __shared__ uint32_t Ri[IM_TILE][IM_CHUNK + 1];
-    __shared__ uint32_t Rj[IM_TILE][IM_CHUNK + 1];
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t g = lane >> 2, t = lane & 3;
-    const uint32_t mrow = (warp & 3u) * 16u;          // this warp's 16 rows of the i tile
-    const uint32_t ncol = (warp >> 2) * 32u;          // and 32 columns (4 n-tiles of 8) of the j tile
-    int c[4][4];
-#pragma unroll
-    for (int n = 0; n < 4; n++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) c[n][q] = 0;
-    for (uint32_t w0 = 0; w0 < n_words; w0 += IM_CHUNK) {
-        __syncthreads();
-        const uint32_t w = w0 + lane;
-#pragma unroll
-        for (uint32_t q = 0; q < IM_TILE / 8; q++) {
-            const uint32_t rr = warp + 8u * q;
-            const uint32_t ri = bi * IM_TILE + rr, rj = bj * IM_TILE + rr;
-            Ri[rr][lane] = (w < n_words && ri < n_rows) ? acc[(uint64_t)ri * stride_words + w] : 0u;
-            Rj[rr][lane] = (w < n_words && rj < n_rows) ? acc[(uint64_t)rj * stride_words + w] : 0u;
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (uint32_t ks = 0; ks < IM_CHUNK; ks++) {
-            const uint32_t wa = Ri[mrow + g][ks] >> t, wb = Ri[mrow + g + 8][ks] >> t;
-            const uint32_t a0 = wa & 0x01010101u, a1 = wb & 0x01010101u;
-            const uint32_t a2 = (wa >> 4) & 0x01010101u, a3 = (wb >> 4) & 0x01010101u;
-#pragma unroll
-            for (int n = 0; n < 4; n++) {
-                const uint32_t wj = Rj[ncol + n * 8 + g][ks] >> t;
-                imma_16832_u8(c[n], a0, a1, a2, a3, wj & 0x01010101u, (wj >> 4) & 0x01010101u);
-            }
-        }
-    }
-    // accumulator layout: c[n][0..1] = (row g, cols 2t, 2t+1), c[n][2..3] = (row g + 8, same cols)
-#pragma unroll
-    for (int n = 0; n < 4; n++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-            const uint32_t i = bi * IM_TILE + mrow + g + ((q >> 1) ? 8u : 0u);
-            const uint32_t j = bj * IM_TILE + ncol + n * 8 + 2 * t + (q & 1);
-            if (i < n_rows && j < n_rows) {
-                inter[(uint64_t)i * n_rows + j] = (uint32_t)c[n][q];
-                inter[(uint64_t)j * n_rows + i] = (uint32_t)c[n][q];
-                if (i == j) diag[i] = c[n][q];                // |row_i|: the gene count the distances need
-            }
-        }
-}
-
-// K2a (tcgen05): the same contraction X * X^T on the 5th-generation tensor cores. The presence matrix
-// is first expanded to one byte per gene (acc_expand_bytes_kernel: 0/1 bytes, K-major rows padded to
-// whole 128-byte swizzle rows; the order of the 32 genes of a word inside their 32 bytes is a fixed
-// permutation, which a dot product does not see). One CTA per upper-triangle tile of 128 x 128
-// pairs: a producer thread streams [128 rows x 128 genes] operand tiles through a 4-stage
-// TMA/mbarrier ring (2-D tensor map, 128-byte swizzle, out-of-range rows are zero-filled by the
-// TMA unit), one thread issues tcgen05.mma.kind::i8 (u8 x u8 -> s32, M = N = 128, K = 32 per
-// instruction, four per stage) with the accumulator tile in tensor memory (128 lanes x 128
-// columns), tcgen05.commit releases the stages and finally signals the epilogue: every warp reads
-// its 32 accumulator lanes with tcgen05.ld (32x32b.x32) and stores the counts directly and
-// mirrored. Exact: the products are 0/1 and the s32 accumulation cannot overflow.
-constexpr int UM_TILE = 128;                 // rows per operand tile = UMMA M = UMMA N
-constexpr int UM_KBYTES = 128;               // genes per stage = one swizzle row
-constexpr int UM_STAGES = 4;
-constexpr int UM_THREADS = 128;
-constexpr uint32_t UM_TILE_BYTES = UM_TILE * UM_KBYTES;
-constexpr uint32_t UM_TMEM_COLS = 128;
-// instruction descriptor (kind::i8): D = s32 (bits 4-5 = 2), A = B = u8 (0), both K-major (0), N >> 3 at bit 17, M >> 4 at bit 24
-constexpr uint32_t UM_IDESC = (2u << 4) | ((uint32_t)(UM_TILE >> 3) << 17) | ((uint32_t)(UM_TILE >> 4) << 24);
-// shared-memory matrix descriptor, K-major, 128-byte swizzle: stride between 8-row groups 1024 B (bits 32-45, in 16 B),
-// leading byte offset 1 (unused with this swizzle), descriptor version 1 (bit 46), layout SWIZZLE_128B = 2 (bits 61-63)
-constexpr uint32_t UM_DESC_HI = (1024u >> 4) | (1u << 14) | (2u << 29);
-
-static inline size_t inter_umma_smem_bytes()
-{
-    return 1024 /* alignment slack */ + 2 * (size_t)UM_STAGES * UM_TILE_BYTES + (2 * UM_STAGES + 1) * sizeof(uint64_t) + 16;
-}
-
-// row r, 32-gene word w -> 32 bytes: byte 4t + q = bit t + 8q of the word
-__global__ void __launch_bounds__(256) acc_expand_bytes_kernel(const uint32_t *acc, uint32_t n_rows, uint32_t stride_words,
-                                                               uint32_t kpad_words, uint8_t *bytes)
-{
-    const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= (uint64_t)n_rows * kpad_words) return;
-    const uint32_t row = (uint32_t)(idx / kpad_words), w = (uint32_t)(idx % kpad_words);
-    const uint32_t v = w < stride_words ? acc[(uint64_t)row * stride_words + w] : 0u;
-    uint4 lo, hi;
-    lo.x = v & 0x01010101u; lo.y = (v >> 1) & 0x01010101u; lo.z = (v >> 2) & 0x01010101u; lo.w = (v >> 3) & 0x01010101u;
-    hi.x = (v >> 4) & 0x01010101u; hi.y = (v >> 5) & 0x01010101u; hi.z = (v >> 6) & 0x01010101u; hi.w = (v >> 7) & 0x01010101u;
-    uint4 *dst = reinterpret_cast<uint4 *>(bytes + idx * 32u);
-    dst[0] = lo;
-    dst[1] = hi;
-}
-
-// mbarrier wait that traps instead of spinning forever (a wrong tensor map or descriptor would otherwise hang the device)
-__device__ __forceinline__ void mbar_wait_or_trap(uint32_t bar_s, uint32_t parity)
-{
-    for (uint32_t spin = 0; spin < (1u << 24); spin++) {
-        uint32_t ok;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(bar_s), "r"(parity) : "memory");
-        if (ok) return;
-    }
-    __trap();
-}
-
-__device__ __forceinline__ void tma_load_2d_s(uint32_t smem_dst, const void *tmap, uint32_t x, uint32_t y, uint32_t bar_s)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"(smem_dst), "l"(tmap), "r"(x), "r"(y), "r"(bar_s) : "memory");
-}
-
-__global__ void __launch_bounds__(UM_THREADS, 1) acc_inter_umma_kernel(const __grid_constant__ CUtensorMap tmap, uint32_t n_rows,
-                                                                       uint32_t k_iters, uint32_t *inter, int32_t *diag)
-{
-    extern __shared__ uint8_t um_smem[];
-    const uint32_t base_s = (smem_u32(um_smem) + 1023u) & ~1023u;      // operand tiles on 1 KiB boundaries (swizzle atom)
-    const uint32_t a_s = base_s, b_s = base_s + UM_STAGES * UM_TILE_BYTES;
-    const uint32_t full_s = b_s + UM_STAGES * UM_TILE_BYTES, empty_s = full_s + UM_STAGES * 8u, done_s = empty_s + UM_STAGES * 8u;
-    const uint32_t slot_s = done_s + 8u;
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t nb = (n_rows + UM_TILE - 1) / UM_TILE;
     uint32_t t_lin = blockIdx.x, bi = 0;
     while (t_lin >= nb - bi) { t_lin -= nb - bi; bi++; }
     const uint32_t bj = bi + t_lin;
 
-    if (threadIdx.x == 0) {
-        for (uint32_t s = 0; s < 2 * UM_STAGES + 1; s++)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(full_s + s * 8u), "r"(1u) : "memory");
-        fence_mbar_init();
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot_s), "r"(UM_TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    uint32_t tmem;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem) : "r"(slot_s) : "memory");
-
-    if (warp == 0) {
-        if (lane == 0) {
-            // ---- TMA producer ----
-            for (uint32_t it = 0; it < k_iters; it++) {
-                const uint32_t s = it % UM_STAGES, n = it / UM_STAGES;
-                if (n) mbar_wait_or_trap(empty_s + s * 8u, (n - 1u) & 1u);       // the MMAs that read the stage's previous fill have completed
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full_s + s * 8u), "r"(2u * UM_TILE_BYTES) : "memory");
-                tma_load_2d_s(a_s + s * UM_TILE_BYTES, &tmap, it * UM_KBYTES, bi * UM_TILE, full_s + s * 8u);
-                tma_load_2d_s(b_s + s * UM_TILE_BYTES, &tmap, it * UM_KBYTES, bj * UM_TILE, full_s + s * 8u);
-            }
-        }
-        __syncwarp();
-    } else if (warp == 1) {
-        if (lane == 0) {
-            // ---- MMA issue ----
-            for (uint32_t it = 0; it < k_iters; it++) {
-                const uint32_t s = it % UM_STAGES, n = it / UM_STAGES;
-                mbar_wait_or_trap(full_s + s * 8u, n & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint32_t a_lo = (((a_s + s * UM_TILE_BYTES) & 0x3FFFFu) >> 4) | (1u << 16);
-                const uint32_t b_lo = (((b_s + s * UM_TILE_BYTES) & 0x3FFFFu) >> 4) | (1u << 16);
-#pragma unroll
-                for (uint32_t k = 0; k < UM_KBYTES / 32; k++) {           // K = 32 bytes per instruction: +32 B inside the swizzle row
-                    const uint64_t da = ((uint64_t)UM_DESC_HI << 32) | (a_lo + 2u * k);
-                    const uint64_t db = ((uint64_t)UM_DESC_HI << 32) | (b_lo + 2u * k);
-                    const uint32_t accumulate = (it | k) ? 1u : 0u;
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                 "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                                 ::"r"(tmem), "l"(da), "l"(db), "r"(UM_IDESC), "r"(accumulate) : "memory");
-                }
-                // arrives on the barrier once the MMAs issued so far have read their operands (implies fence::before_thread_sync)
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(empty_s + s * 8u) : "memory");
-            }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(done_s) : "memory");
-        }
-        __syncwarp();
-    }
-
-    // ---- epilogue: accumulator lane 32 * warp + lane = row of the i tile, columns = rows of the j tile ----
-    mbar_wait_or_trap(done_s, 0u);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t i = bi * UM_TILE + warp * 32u + lane;
-    const bool vec_ok = (n_rows & 3u) == 0u;
-#pragma unroll 1
-    for (uint32_t c0 = 0; c0 < (uint32_t)UM_TILE; c0 += 32) {
-        uint32_t v[32];
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-                     "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-                     "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-                     : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                       "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-                       "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-                       "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-                     : "r"(tmem + ((warp * 32u) << 16) + c0) : "memory");
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        const uint32_t j0 = bj * UM_TILE + c0;
-        if (i < n_rows) {
-            uint32_t *dst = inter + (uint64_t)i * n_rows + j0;
-            if (vec_ok && j0 + 32u <= n_rows) {
-#pragma unroll
-                for (int q = 0; q < 32; q += 4) *reinterpret_cast<uint4 *>(dst + q) = make_uint4(v[q], v[q + 1], v[q + 2], v[q + 3]);
-            } else {
-#pragma unroll
-                for (int q = 0; q < 32; q++)
-                    if (j0 + q < n_rows) dst[q] = v[q];
-            }
-#pragma unroll
-            for (int q = 0; q < 32; q++) {
-                const uint32_t j = j0 + q;
-                if (j < n_rows) {
-                    if (bi != bj) inter[(uint64_t)j * n_rows + i] = v[q];      // lanes = consecutive i: coalesced
-                    else if (i == j) diag[i] = (int32_t)v[q];                  // |row_i|: the gene count the distances need
-                }
-            }
-        }
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(UM_TMEM_COLS) : "memory");
-}
-
-// K2a (tcgen05, operands expanded inside the CTA): the kernel above is bound by the L2 -> SM traffic of the
-// byte matrix (1 MiB per 128 x 128 tile). Here the CTA reads the BIT rows (an eighth of that), eight warps
-// expand them to 0/1 bytes straight into the swizzled K-major operand layout the tensor core expects, make the
-// writes visible to the async proxy (fence.proxy.async) and hand the stage to the MMA thread through an
-// mbarrier; tcgen05.commit returns it. Thread = one row of the stage (128 rows of the i tile, 128 of the j
-// tile), KB / 8 bytes of bits per row per stage, fetched one stage ahead. The 32 genes of a word go to 32
-// consecutive bytes, byte 4t + q = bit t + 8q: a fixed permutation of the k index, which a dot product does not see.
-//   KB = 128: rows of 128 bytes, 16-byte chunk c of row r stored at chunk c ^ (r % 8) (SWIZZLE_128B, what a TMA load
-//             would have produced; 8-row groups 1024 bytes apart), four stages of 32 KiB.
-//   KB = 64:  rows of 64 bytes, chunk c of row r at c ^ ((r / 2) % 4) (SWIZZLE_64B; 8-row groups 512 bytes apart),
-//             three stages of 16 KiB: 48 KiB of shared memory and <= 56 registers x 288 threads, i.e. the CTA fits
-//             into the slot ONE retiring core_mut_kernel CTA leaves on an SM (the generation pipeline keeps every SM
-//             full of those), instead of waiting for three.
-constexpr int UB_EXP_WARPS = 8;
-constexpr int UB_THREADS = 32 * (UB_EXP_WARPS + 1);       // + the MMA warp
-
-template <int KB> struct UbCfg {
-    static constexpr uint32_t STAGES = KB == 128 ? 4u : 3u;
-    static constexpr uint32_t TILE_BYTES = UM_TILE * KB;
-    // matrix descriptor, high word: stride between 8-row groups (8 * KB bytes, in 16 B), version 1, layout 2 = SWIZZLE_128B / 4 = SWIZZLE_64B
-    static constexpr uint32_t DESC_HI = ((8u * KB) >> 4) | (1u << 14) | ((KB == 128 ? 2u : 4u) << 29);
-    static constexpr size_t smem_bytes() { return 1024 + 2 * (size_t)STAGES * TILE_BYTES + (2 * STAGES + 1) * sizeof(uint64_t) + 16; }
-};
-
-template <int KB>
-__global__ void __launch_bounds__(UB_THREADS, KB == 128 ? 1 : 4) acc_inter_umma_bits_kernel(const uint32_t *__restrict__ acc, uint32_t n_rows,
-                                                                                            uint32_t stride_words, uint32_t k_iters,
-                                                                                            uint32_t *inter, int32_t *diag)
-{
-    using Cfg = UbCfg<KB>;
-    constexpr uint32_t STAGES = Cfg::STAGES, TILE_BYTES = Cfg::TILE_BYTES, WORDS = KB / 32;      // bit words per row per stage
-    extern __shared__ uint8_t um_smem[];
-    const uint32_t base_s = (smem_u32(um_smem) + 1023u) & ~1023u;
-    const uint32_t a_s = base_s, b_s = base_s + STAGES * TILE_BYTES;
-    const uint32_t full_s = b_s + STAGES * TILE_BYTES, empty_s = full_s + STAGES * 8u, done_s = empty_s + STAGES * 8u;
-    const uint32_t slot_s = done_s + 8u;
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t nb = (n_rows + UM_TILE - 1) / UM_TILE;
-    uint32_t t_lin = blockIdx.x, bi = 0;
-    while (t_lin >= nb - bi) { t_lin -= nb - bi; bi++; }
-    const uint32_t bj = bi + t_lin;
-
-    if (threadIdx.x == 0) {
-        for (uint32_t s = 0; s < STAGES; s++) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(full_s + s * 8u), "r"((uint32_t)UB_EXP_WARPS) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(empty_s + s * 8u), "r"(1u) : "memory");
-        }
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(done_s), "r"(1u) : "memory");
-        fence_mbar_init();
-    }
-    if (warp == UB_EXP_WARPS) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot_s), "r"(UM_TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    uint32_t tmem;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem) : "r"(slot_s) : "memory");
-
-    if (warp < UB_EXP_WARPS) {
-        // ---- expansion: threads 0..127 = rows of the i tile, 128..255 = rows of the j tile ----
-        const uint32_t tr = threadIdx.x & 127u;                          // row inside the tile
-        const bool is_b = threadIdx.x >= 128u;
-        const uint32_t grow = (is_b ? bj : bi) * UM_TILE + tr;
-        const bool row_ok = grow < n_rows;
-        const uint32_t *src = acc + (uint64_t)(row_ok ? grow : 0u) * stride_words;      // rows: zero-padded to a multiple of 4 words
-        const uint32_t row_s = (is_b ? b_s : a_s) + tr * KB;
-        const uint32_t sw = (KB == 128 ? (tr & 7u) : ((tr >> 1) & 3u)) << 4;             // XOR term of the swizzle
-        auto fetch = [&](uint32_t it, uint32_t (&w)[WORDS]) {
-            const bool ok = row_ok && (it + 1u) * WORDS <= stride_words;
-            if (KB == 128) {
-                const uint4 v = ok ? __ldg(reinterpret_cast<const uint4 *>(src) + it) : make_uint4(0, 0, 0, 0);
-                w[0] = v.x; w[1] = v.y; w[WORDS - 2] = v.z; w[WORDS - 1] = v.w;
-            } else {
-                const uint2 v = ok ? __ldg(reinterpret_cast<const uint2 *>(src) + it) : make_uint2(0, 0);
-                w[0] = v.x; w[WORDS - 1] = v.y;
-            }
-        };
-        uint32_t nxt[WORDS];
-        fetch(0u, nxt);
-        for (uint32_t it = 0; it < k_iters; it++) {
-            const uint32_t s = it % STAGES, n = it / STAGES;
-            uint32_t cur[WORDS];
-#pragma unroll
-            for (uint32_t q = 0; q < WORDS; q++) cur[q] = nxt[q];
-            if (it + 1u < k_iters) fetch(it + 1u, nxt);
-            if (n) mbar_wait_or_trap(empty_s + s * 8u, (n - 1u) & 1u);      // the MMAs that read the stage's previous contents have completed
-            const uint32_t dst = row_s + s * TILE_BYTES;
-#pragma unroll
-            for (uint32_t q = 0; q < WORDS; q++) {
-                const uint32_t v = cur[q];
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + (((2u * q) << 4) ^ sw)), "r"(v & 0x01010101u),
-                             "r"((v >> 1) & 0x01010101u), "r"((v >> 2) & 0x01010101u), "r"((v >> 3) & 0x01010101u) : "memory");
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst + (((2u * q + 1u) << 4) ^ sw)), "r"((v >> 4) & 0x01010101u),
-                             "r"((v >> 5) & 0x01010101u), "r"((v >> 6) & 0x01010101u), "r"((v >> 7) & 0x01010101u) : "memory");
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy writes -> visible to the tensor core's reads
-            __syncwarp();
-            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(full_s + s * 8u) : "memory");
-        }
-    } else {
-        if (lane == 0) {
-            // ---- MMA issue ----
-            for (uint32_t it = 0; it < k_iters; it++) {
-                const uint32_t s = it % STAGES, n = it / STAGES;
-                mbar_wait_or_trap(full_s + s * 8u, n & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint32_t a_lo = (((a_s + s * TILE_BYTES) & 0x3FFFFu) >> 4) | (1u << 16);
-                const uint32_t b_lo = (((b_s + s * TILE_BYTES) & 0x3FFFFu) >> 4) | (1u << 16);
-#pragma unroll
-                for (uint32_t k = 0; k < KB / 32; k++) {                     // K = 32 bytes per instruction: +32 B inside the swizzled row
-                    const uint64_t da = ((uint64_t)Cfg::DESC_HI << 32) | (a_lo + 2u * k);
-                    const uint64_t db = ((uint64_t)Cfg::DESC_HI << 32) | (b_lo + 2u * k);
-                    const uint32_t accumulate = (it | k) ? 1u : 0u;
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                 "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                                 ::"r"(tmem), "l"(da), "l"(db), "r"(UM_IDESC), "r"(accumulate) : "memory");
-                }
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(empty_s + s * 8u) : "memory");
-            }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(done_s) : "memory");
-        }
-        __syncwarp();
-    }
+    if (threadIdx.x == 0) bitmma_init<128>(m);
+    if (warp == UB_EXP_WARPS) bitmma_alloc(m);
+    const uint32_t tmem = bitmma_tmem(m);
+    bitmma_mainloop<128>(m, tmem, acc, stride_words, n_rows, k_iters, bi, bj, warp, lane);
 
     // ---- epilogue: warps w and w + 4 share the accumulator lanes 32 * (w % 4) .. + 31 and split the columns ----
     if (warp < UB_EXP_WARPS) {
-        mbar_wait_or_trap(done_s, 0u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        bitmma_wait(m);
         const uint32_t quad = warp & 3u;
         const uint32_t i = bi * UM_TILE + quad * 32u + lane;
         const bool vec_ok = (n_rows & 3u) == 0u;
 #pragma unroll 1
         for (uint32_t c0 = (warp >> 2) * 64u; c0 < (warp >> 2) * 64u + 64u; c0 += 16) {
             uint32_t v[16];
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                         "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                         : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                           "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                         : "r"(tmem + ((quad * 32u) << 16) + c0) : "memory");
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            bitmma_load16(tmem, quad, c0, v);
             const uint32_t j0 = bj * UM_TILE + c0;
             if (i < n_rows) {
                 uint32_t *dst = inter + (uint64_t)i * n_rows + j0;
@@ -762,9 +360,7 @@ __global__ void __launch_bounds__(UB_THREADS, KB == 128 ? 1 : 4) acc_inter_umma_
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == UB_EXP_WARPS) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(UM_TMEM_COLS) : "memory");
+    bitmma_free(tmem, warp);
 }
 
 // K2b: mean Jaccard distance of individual i to all j != i, summed in j order
@@ -773,20 +369,9 @@ constexpr int AVG_WARPS = 8;
 constexpr int AVG_RING = 256;       // distances evaluated per round (8 per lane)
 constexpr int AVG_BATCH = 8;
 
-// RCP = true: the quotient a / b of the two small integers a = |i & j| + core_genes <= b = |i | j| + core_genes is
-// formed from the correctly rounded reciprocal r = RN(1 / b) (host table indexed by b) instead of the ~100-instruction
-// IEEE division sequence:
-//     q0 = RN(a * r);  e = a - q0 * b (exact, one FMA);  q = RN(q0 + e * r)
-// which is the correctly rounded quotient RN(a / b) (Markstein's division step; checked exhaustively for every
-// 0 <= a <= b <= 131072 by tools/check_recip_division.c), i.e. bit for bit what the division of population.rs:144-145
-// returns; b = 0 (two empty genomes, no core genes) gives r = inf and a NaN, as 0.0 / 0.0 does.
-constexpr uint32_t AVG_RCP_MAX = 131072;        // largest denominator the table may serve (range of the exhaustive check)
-
-template <bool RCP>
 __global__ void __launch_bounds__(AVG_WARPS * 32) avg_distance_kernel(const uint32_t *inter,
                                                                       const int32_t *num_genes, uint32_t n_rows,
-                                                                      uint32_t core_genes, const double *__restrict__ rcp,
-                                                                      double *avgdist)
+                                                                      uint32_t core_genes, double *avgdist)
 {
     // One warp per individual. Per round the 32 lanes evaluate 256 distances in parallel (the
     // f64 divisions are independent) into shared memory, then the values are added one by one in
@@ -813,23 +398,11 @@ __global__ void __launch_bounds__(AVG_WARPS * 32) avg_distance_kernel(const uint
             in[q] = irow[j];
             kj[q] = (uint32_t)num_genes[j];
         }
-        double rr[AVG_RING / 32];
-        if (RCP) {
-#pragma unroll
-            for (int q = 0; q < AVG_RING / 32; q++) rr[q] = __ldg(rcp + (ki + kj[q] - in[q] + core_genes));
-        }
 #pragma unroll
         for (int q = 0; q < AVG_RING / 32; q++) {
             const uint32_t j = j0 + q * 32 + lane;
             const uint32_t un = ki + kj[q] - in[q];
-            double d;
-            if (RCP) {
-                const double da = (double)(in[q] + core_genes), db = (double)(un + core_genes);
-                const double r = rr[q], q0 = da * r;
-                d = 1.0 - fma(fma(-q0, db, da), r, q0);
-            } else {
-                d = 1.0 - (((double)in[q] + 0.0 + cg) / ((double)un + 0.0 + cg));   // :144-145
-            }
+            const double d = 1.0 - (((double)in[q] + 0.0 + cg) / ((double)un + 0.0 + cg));   // :144-145
             mine[q * 32 + lane] = (j < n_rows && j != i) ? d : 0.0;
         }
         __syncwarp();
@@ -855,14 +428,23 @@ __global__ void __launch_bounds__(AVG_WARPS * 32) avg_distance_kernel(const uint
     }
 }
 
-// The same kernel (warp per individual, reciprocal-table quotients) software-pipelined over the rounds, for the
-// generation pipeline where the warp shares its scheduler with eight core-kernel warps and every exposed global-load
-// latency is paid in full: while the chain of round r runs over one half of a double-buffered ring,
+// The same mean distance for shapes with G + core_genes <= AVG_RCP_MAX. The quotient a / b of the two small integers
+// a = |i & j| + core_genes <= b = |i | j| + core_genes is formed from the correctly rounded reciprocal r = RN(1 / b)
+// (host table indexed by b) instead of the ~100-instruction IEEE division sequence:
+//     q0 = RN(a * r);  e = a - q0 * b (exact, one FMA);  q = RN(q0 + e * r)
+// which is the correctly rounded quotient RN(a / b) (Markstein's division step; checked exhaustively for every
+// 0 <= a <= b <= 131072 by tools/check_recip_division.c), i.e. bit for bit what the division of population.rs:144-145
+// returns; b = 0 (two empty genomes, no core genes) gives r = inf and a NaN, as 0.0 / 0.0 does.
+// The kernel is software-pipelined over the rounds, for the generation pipeline where the warp shares its scheduler
+// with eight core-kernel warps and every exposed global-load latency is paid in full: while the chain of round r runs
+// over one half of a double-buffered ring,
 //   * the reciprocals of round r + 1 are fetched (their addresses come from intersection counts loaded a round earlier),
 //   * its quotients are evaluated into the other half of the ring between the two halves of the chain,
 //   * the intersection counts and gene counts of round r + 2 are requested.
 // The loads are volatile asm so that they are issued where they are written; two values per shared-memory load in the
 // chain. Same additions in the same order: same bits.
+constexpr uint32_t AVG_RCP_MAX = 131072;        // largest denominator the table may serve (range of the exhaustive check)
+
 __device__ __forceinline__ uint32_t ldg_u32_v(const void *p)
 {
     uint32_t v;

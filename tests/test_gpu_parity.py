@@ -203,26 +203,26 @@ def test_competition_and_fitness_kernels_over_shapes(N, G, dens):
     np.testing.assert_allclose(w / w.sum(), ow / ow.sum(), rtol=1e-11)
 
 
-@pytest.mark.parametrize("umma", ["0", "1", "2", "3"])
-@pytest.mark.parametrize("rcp", ["0", "1", "2"])
-def test_competition_kernel_variants_are_bit_exact(monkeypatch, umma, rcp):
-    """Every implementation of the competition term behind PANSIM_INTER_UMMA / PANSIM_AVG_RCP gives the oracle's
-    bits: tcgen05.mma with operands expanded in the CTA (2: 128-byte, 3: 64-byte swizzled rows) or fed by TMA from a
-    byte-expanded matrix (1), warp-level mma.sync (0); IEEE division (0) or the reciprocal-table quotient
-    (tools/check_recip_division.c; 1, and 2 = software-pipelined over the rounds). Shapes: several 128-row tiles with a ragged last one, gene counts off the
-    64 / 128-gene stage size, fewer rows than a tile, no core genes (denominator 0 is not reachable here)."""
-    monkeypatch.setenv("PANSIM_INTER_UMMA", umma)
-    monkeypatch.setenv("PANSIM_AVG_RCP", rcp)
-    for N, pan, cg, dens in [(300, 900, 200, 0.5), (130, 37, 0, 0.9), (1025, 4229, 100, 0.02), (257, 300, 0, 1.0), (5, 40, 37, 0.3)]:
-        rng = np.random.default_rng(N + pan)
-        G = pan - cg
-        core, acc = random_state(rng, N, 20, G, dens)
-        p = pb.Params(pop_size=N, core_size=20, pan_genes=pan, core_genes=cg, competition_strength=0.5)
-        oavg = ob.Population(acc, False, cg).average_distance()
-        with make(p) as sim:
-            sim.upload(core, acc)
-            avg = sim.average_distance()
-        assert np.array_equal(avg, oavg), (N, pan, cg, dens, int((avg != oavg).sum()))
+@pytest.mark.parametrize("N,pan,cg,dens", [
+    (300, 900, 200, 0.5), (130, 37, 0, 0.9), (1025, 4229, 100, 0.02), (257, 300, 0, 1.0), (5, 40, 37, 0.3),
+    (1000, 6000, 2000, 0.25), (640, 12800, 0, 0.4),
+    (2, 1, 0, 1.0), (128, 128, 0, 0.5), (129, 129, 0, 0.5), (384, 641, 1, 0.5),
+    (200, 131072, 131000, 0.5), (300, 131100, 131000, 0.5)])
+def test_competition_kernel_variants_are_bit_exact(N, pan, cg, dens):
+    """The competition term gives the oracle's bits: intersection counts on tcgen05.mma with the operands expanded in
+    the CTA, mean distances from the reciprocal-table quotient (tools/check_recip_division.c) while G + core_genes <=
+    131072 and from the IEEE division above. Shapes: several 128-row tiles with a ragged last one, gene counts off the
+    128-gene stage size, exactly one tile and one stage and one past each, more stages than the ring holds, fewer rows
+    than a tile, no core genes (denominator 0 is not reachable here), the last shape of the table and the first past it."""
+    rng = np.random.default_rng(N + pan)
+    G = pan - cg
+    core, acc = random_state(rng, N, 20, G, dens)
+    p = pb.Params(pop_size=N, core_size=20, pan_genes=pan, core_genes=cg, competition_strength=0.5)
+    oavg = ob.Population(acc, False, cg).average_distance()
+    with make(p) as sim:
+        sim.upload(core, acc)
+        avg = sim.average_distance()
+    assert np.array_equal(avg, oavg), (N, pan, cg, dens, int((avg != oavg).sum()))
 
 
 def test_average_distance_identical_population_is_min_positive():

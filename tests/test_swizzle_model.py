@@ -1,4 +1,4 @@
-"""Byte placement of acc_inter_umma_bits_kernel<KB> (select.cuh) against the canonical shared-memory swizzles of the
+"""Byte placement of bitmma_mainloop<KB> (bitmma.cuh) against the canonical shared-memory swizzles of the
 tensor-core operand layouts (CuTe Swizzle<B, M, S>: the B address bits from bit M + S up are XOR-ed into the B bits
 from bit M up; K-major SWIZZLE_128B = Swizzle<3,4,3>, SWIZZLE_64B = Swizzle<2,4,3>; tile base aligned to 1 KiB). CPU only."""
 import pytest
