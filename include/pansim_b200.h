@@ -518,6 +518,57 @@ int pansim_parsimony_kernel_ms(pansim_ctx *ctx, const uint32_t *parent, uint32_t
 /* CI and RI of a summary (either may be NULL); needs no device */
 void pansim_parsimony_indices(const pansim_parsimony *p, double *ci, double *ri);
 
+/* ---- neighbour-joining trees from the all-pairs distances (extension) -----
+ * The tree PopPUNK or snp-dists -> RapidNJ would infer from the present rows, on the device (DESIGN.md section 18),
+ * and an exact split comparison with any other tree over the same leaves (the true genealogy, for instance).
+ * DISTANCES. metric 0 (core): d_ij = pansim_core_distance(core_diff, core_size). metric 1 (acc): d_ij =
+ * pansim_acc_distance(inter, uni, core_genes), except d = 0 where uni + core_genes = 0. These are the values of
+ * <outpref>.tsv over every pair i < j, whatever max_distances is. pansim_nj_tree_matrix takes a caller's matrix as its
+ * upper triangle, row-major (d(0,1), d(0,2), .. d(0,n-1), d(1,2), ..); a non-finite or negative entry ->
+ * PANSIM_ERR_INVALID. Core on a context with core_size = 0 -> PANSIM_ERR_INVALID; core on a column shard without a
+ * communicator -> PANSIM_ERR_STATE (its counts are partial). Under a communicator the counts are summed first
+ * (comm_allreduce_counts), so every rank computes the same tree.
+ * ALGORITHM (Saitou & Nei 1987, with Studier & Keppler's 1988 Q). IEEE binary64, round-to-nearest, nothing contracted,
+ * every operation in the order written here, so a float64 numpy transcription reproduces every bit.
+ *  - Active nodes sit in an ordered list of slots, initially leaves 0 .. N-1 in order.
+ *  - R_a = sum_b d_ab, summed left to right over ascending b (d_aa = 0), once.
+ *  - While k = active > 3: the slots a < b minimising Q_ab = ((k - 2) * d_ab - R_a) - R_b, compared as doubles, ties to
+ *    the smaller a, then the smaller b (no grid, tile or reduction order enters).
+ *  - delta_a = (d_ab + (R_a - R_b) / (k - 2)) * 0.5, delta_b = d_ab - delta_a (negative lengths are kept, as ape::nj
+ *    keeps them).
+ *  - Join t (from 0) makes node N + t; it takes slot a, slot b leaves the list, the other slots keep their order.
+ *  - Every other active c: d_uc = ((d_ac + d_bc) - d_ab) * 0.5; R_c = ((R_c - d_ac) - d_bc) + d_uc;
+ *    R_u = (((R_a - d_ab) + (R_b - d_ab)) - (k - 2) * d_ab) * 0.5.
+ *  - The last slots x < y < z become the root 2N - 3, children in that order, delta_x = ((d_xy + d_xz) - d_yz) * 0.5,
+ *    delta_y = ((d_xy + d_yz) - d_xz) * 0.5, delta_z = ((d_xz + d_yz) - d_xy) * 0.5.
+ *  - N = 2: root 2, both branches d_01 * 0.5. N = 1: the single leaf.
+ * OUTPUT. parent[n_nodes] (root 0xFFFFFFFF) and length[n_nodes] (branch above each node, root 0), n_nodes = 2N - 2
+ * for N >= 3, 3 for N = 2, 1 for N = 1: a node table in the sense of pansim_core_parsimony (parents above children,
+ * root last, every internal node with >= 2 children), so the parsimony calls take it unchanged.
+ * The matrix (N x N doubles, padded rows; plus a second buffer for the first compaction) is allocated for the call and
+ * freed before it returns: PANSIM_ERR_NOMEM if it cannot be, and the context keeps working. No state
+ * (pansim_set_initial or pansim_upload_*) -> PANSIM_ERR_STATE. */
+int pansim_nj_tree(pansim_ctx *ctx, int metric /* 0 core, 1 acc */, uint32_t *parent, double *length);
+int pansim_nj_tree_matrix(pansim_ctx *ctx, const double *upper /* n (n - 1) / 2 */, uint32_t n, uint32_t *parent,
+                          double *length);
+/* measurement: one warm-up call, then `repeats` calls; mean device ms of the matrix build (pair counts, scatter, R)
+ * and of the join loop (scans, joins, compactions, the last three) by CUDA events; bytes_scanned = sum over the
+ * iterations of the stored upper triangle the scan reads x 8 bytes; compactions of one call. Any output may be NULL. */
+int pansim_nj_kernel_ms(pansim_ctx *ctx, int metric, uint32_t repeats, float *build_ms, float *join_ms,
+                        uint64_t *bytes_scanned, uint32_t *compactions);
+/* Newick of a node table with branch lengths (no device): leaves ind_<i>, children ordered by their smallest leaf,
+ * lengths "%.17g" (they round-trip), the same writer as pansim_genealogy_newick; out / cap / len as there. A table
+ * that breaks the node-table rules -> PANSIM_ERR_INVALID. */
+int pansim_tree_newick(const uint32_t *parent, const double *length, uint32_t n_nodes, uint32_t n_leaves, char *out,
+                       size_t cap, size_t *len);
+/* SPLITS (no device). Every non-root edge of a node table over n_leaves leaves cuts the leaves in two; splits(T) is
+ * the set of distinct bipartitions with both sides of >= 2 leaves (trivial splits excluded; the two edges of a binary
+ * root give one split). out = {|splits(A)|, |splits(B)|, |shared|}; Robinson-Foulds = out[0] + out[1] - 2 out[2].
+ * Exact (leaf sets, not hashes), for polytomies and a virtual root alike. A table that breaks the rules ->
+ * PANSIM_ERR_INVALID. */
+int pansim_tree_compare_splits(const uint32_t *parent_a, uint32_t n_a, const uint32_t *parent_b, uint32_t n_b,
+                               uint32_t n_leaves, uint64_t out[3]);
+
 /* ---- multi-GPU: column shards of one alignment --------------------------
  * (SURVEY.md 8e; the reference is one shared-memory process, population.rs has no analogue.)
  * Every shard context holds all individuals for [site_begin, site_end) and a replica of the
@@ -606,6 +657,10 @@ int pansim_group_core_parsimony(pansim_group *g, const uint32_t *parent, uint32_
                                 uint32_t *site_changes, uint64_t *branch_changes);
 int pansim_group_gene_parsimony(pansim_group *g, const uint32_t *parent, uint32_t n_nodes, pansim_parsimony *out,
                                 uint32_t *gene_changes, uint64_t *gains, uint64_t *losses);
+/* neighbour-joining tree of the group (pansim_nj_tree). Core: every shard counts its columns per row block, the counts
+ * are summed over the shards (ncclAllReduce) and shard 0 builds the matrix and joins. Acc: the accessory matrix is
+ * replicated, so shard 0 answers. Bit-identical to one context. */
+int pansim_group_nj_tree(pansim_group *g, int metric, uint32_t *parent, double *length);
 
 /* ---- introspection / instrumentation ----------------------------------- */
 typedef struct {

@@ -4,8 +4,9 @@ Wright-Fisher step and pairwise distance pass, behind a C ABI
 reference's `Population` API. No CPU fallback."""
 from .params import Derived, Params, derive, fmt_f64, validate  # noqa: F401
 from .population import (CoreFasta, CoreLD, CoreParsimony, Diversity, GeneAccumulation, GeneLD, GeneParsimony,  # noqa: F401
-                         Genealogy, Pansim, PansimError, diversity_stats, genealogy_newick, make_config, pangenome_classes,
-                         parsimony_indices, standard_deviation)
+                         Genealogy, NJTree, Pansim, PansimError, SplitComparison, compare_splits, diversity_stats,
+                         genealogy_newick, make_config, pangenome_classes, parsimony_indices, standard_deviation,
+                         tree_newick)
 from .group import PansimGroup  # noqa: F401
 
 __version__ = "0.1.0"

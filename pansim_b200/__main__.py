@@ -7,7 +7,7 @@ threads and seed are parsed as integers (main.rs:169, 177, 180). --threads is
 accepted and ignored (the work runs on the GPU). Extra flags: --device, --all_pairs, --print_diversity, --print_vcf,
 --print_ld, --ld_max_dist, --ld_bin_width, --ld_min_minor, --print_genealogy, --print_fasta, --print_snp_alignment,
 --print_gene_ld, --gene_ld_bins, --gene_ld_min_minor, --print_gene_accumulation, --gene_accumulation_perms,
---print_parsimony.
+--print_parsimony, --print_nj.
 """
 from __future__ import annotations
 
@@ -101,6 +101,10 @@ def build_parser() -> argparse.ArgumentParser:
                     help="(extension) parsimony changes on the true genealogy of the last generation: <outpref>_parsimony.tsv "
                          "(core and gene summaries with CI and RI), <outpref>_core_site_changes.txt, <outpref>_gene_changes.txt, "
                          "<outpref>_branch_changes.tsv")
+    ap.add_argument("--print_nj", action="store_true",
+                    help="(extension) neighbour-joining trees of the last generation on the core and accessory distances: "
+                         "<outpref>_core_nj.nwk, <outpref>_acc_nj.nwk, and their splits against the true genealogy in "
+                         "<outpref>_nj_rf.tsv")
     return ap
 
 
@@ -115,7 +119,7 @@ def main(argv=None) -> int:
     print_snp_alignment = ns.pop("print_snp_alignment")
     ld = {k: ns.pop(k) for k in ("print_ld", "ld_max_dist", "ld_bin_width", "ld_min_minor")}
     ld.update({k: ns.pop(k) for k in ("print_gene_ld", "gene_ld_bins", "gene_ld_min_minor", "print_gene_accumulation",
-                                      "gene_accumulation_perms", "print_parsimony")})
+                                      "gene_accumulation_perms", "print_parsimony", "print_nj")})
     p = Params(**ns)
     run(p, outpref=p.outpref, device=device, all_pairs=all_pairs, print_diversity=print_diversity, print_vcf=print_vcf,
         print_genealogy=print_genealogy, print_fasta=print_fasta, print_snp_alignment=print_snp_alignment, **ld)

@@ -40,6 +40,8 @@ EXPORTED = [
     "pansim_gene_spectrum", "pansim_group_gene_spectrum", "pansim_pangenome_classes",
     "pansim_core_parsimony", "pansim_gene_parsimony", "pansim_parsimony_kernel_ms", "pansim_parsimony_indices",
     "pansim_group_core_parsimony", "pansim_group_gene_parsimony",
+    "pansim_nj_tree", "pansim_nj_tree_matrix", "pansim_nj_kernel_ms", "pansim_tree_newick", "pansim_tree_compare_splits",
+    "pansim_group_nj_tree",
     "pansim_enable_genealogy", "pansim_genealogy", "pansim_genealogy_history", "pansim_genealogy_tmrca",
     "pansim_genealogy_newick", "pansim_group_enable_genealogy", "pansim_group_genealogy", "pansim_group_genealogy_tmrca",
 ]
@@ -271,6 +273,13 @@ def lib():
     sig("pansim_parsimony_kernel_ms", cint, vp, vp, u32, cint, u32, C.POINTER(C.c_float), C.POINTER(C.c_uint64),
         C.POINTER(C.c_uint32))
     sig("pansim_parsimony_indices", None, C.POINTER(Parsimony), C.POINTER(C.c_double), C.POINTER(C.c_double))
+    sig("pansim_nj_tree", cint, vp, cint, vp, vp)
+    sig("pansim_group_nj_tree", cint, vp, cint, vp, vp)
+    sig("pansim_nj_tree_matrix", cint, vp, vp, u32, vp, vp)
+    sig("pansim_nj_kernel_ms", cint, vp, cint, u32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint64),
+        C.POINTER(C.c_uint32))
+    sig("pansim_tree_newick", cint, vp, vp, u32, u32, vp, sz, C.POINTER(sz))
+    sig("pansim_tree_compare_splits", cint, vp, u32, vp, u32, u32, vp)
     sig("pansim_enable_genealogy", cint, vp, u32)
     sig("pansim_genealogy", cint, vp, vp, C.POINTER(GenealogyInfo))
     sig("pansim_genealogy_history", cint, vp, vp)

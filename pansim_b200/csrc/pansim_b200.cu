@@ -24,6 +24,7 @@
 #include "gene_ld.cuh"
 #include "genealogy.cuh"
 #include "ld.cuh"
+#include "nj.cuh"
 #include "pack.cuh"
 #include "pangenome.cuh"
 #include "parsimony.cuh"
@@ -3987,29 +3988,50 @@ void pansim_pangenome_classes(const uint64_t *spectrum, uint32_t pop_size, uint6
 // PANSIM_PARSIMONY_SCRATCH_MB=<n> replaces it (a small value forces many slabs; the results are the same).
 constexpr uint64_t PS_BUDGET_CAP_MB = 16384;
 
-// The rules of the node table (include/pansim_b200.h), checked on the host. On success csr = child_off[n_internal + 1]
-// followed by child[n_nodes - 1]: the children of each internal node in ascending id.
-static int parsimony_tree(pansim_ctx *c, const uint32_t *parent, uint32_t n_nodes, std::vector<uint32_t> &csr)
+// The rules of the node table (include/pansim_b200.h), checked on the host: an empty string, or what is wrong. With
+// csr, on success csr = child_off[n_internal + 1] followed by child[n_nodes - 1]: the children of each internal node
+// in ascending id.
+static std::string node_table_error(const uint32_t *parent, uint32_t n_nodes, uint32_t N, std::vector<uint32_t> *csr)
 {
-    const uint32_t N = c->N;
-    if (!parent) FAIL(c, PANSIM_ERR_INVALID, "parsimony: null node table");
-    if (n_nodes < N || (uint64_t)n_nodes > 2ull * N - 1)
-        FAIL(c, PANSIM_ERR_INVALID, "parsimony: %u nodes for %u leaves (a tree has N .. 2N - 1)", n_nodes, N);
+    char b[160];
+    if (!parent) return "null node table";
+    if (n_nodes < N || (uint64_t)n_nodes > 2ull * N - 1) {
+        snprintf(b, sizeof b, "%u nodes for %u leaves (a tree has N .. 2N - 1)", n_nodes, N);
+        return b;
+    }
     const uint32_t root = n_nodes - 1, n_int = n_nodes - N;
-    if (parent[root] != GEN_NONE) FAIL(c, PANSIM_ERR_INVALID, "parsimony: the last node (%u) must be the root, parent 0xFFFFFFFF", root);
-    csr.assign((size_t)n_int + 1 + root, 0);
+    if (parent[root] != GEN_NONE) {
+        snprintf(b, sizeof b, "the last node (%u) must be the root, parent 0xFFFFFFFF", root);
+        return b;
+    }
+    std::vector<uint32_t> local;
+    std::vector<uint32_t> &off = csr ? *csr : local;
+    off.assign((size_t)n_int + 1 + (csr ? root : 0), 0);
     for (uint32_t k = 0; k < root; k++) {
         const uint32_t p = parent[k];
-        if (p <= k || p < N || p >= n_nodes)
-            FAIL(c, PANSIM_ERR_INVALID, "parsimony: node %u has parent %u (an internal node with a larger id)", k, p);
-        csr[p - N + 1]++;
+        if (p <= k || p < N || p >= n_nodes) {
+            snprintf(b, sizeof b, "node %u has parent %u (an internal node with a larger id)", k, p);
+            return b;
+        }
+        off[p - N + 1]++;
     }
     for (uint32_t v = 0; v < n_int; v++)
-        if (csr[v + 1] < 2) FAIL(c, PANSIM_ERR_INVALID, "parsimony: internal node %u has %u children (at least 2)", N + v, csr[v + 1]);
-    for (uint32_t v = 0; v < n_int; v++) csr[v + 1] += csr[v];
-    std::vector<uint32_t> fill(csr.begin(), csr.begin() + n_int);
-    uint32_t *child = csr.data() + n_int + 1;
+        if (off[v + 1] < 2) {
+            snprintf(b, sizeof b, "internal node %u has %u children (at least 2)", N + v, off[v + 1]);
+            return b;
+        }
+    if (!csr) return "";
+    for (uint32_t v = 0; v < n_int; v++) off[v + 1] += off[v];
+    std::vector<uint32_t> fill(off.begin(), off.begin() + n_int);
+    uint32_t *child = off.data() + n_int + 1;
     for (uint32_t k = 0; k < root; k++) child[fill[parent[k] - N]++] = k;
+    return "";
+}
+
+static int parsimony_tree(pansim_ctx *c, const uint32_t *parent, uint32_t n_nodes, std::vector<uint32_t> &csr)
+{
+    const std::string e = node_table_error(parent, n_nodes, c->N, &csr);
+    if (!e.empty()) FAIL(c, PANSIM_ERR_INVALID, "parsimony: %s", e.c_str());
     return 0;
 }
 
@@ -4204,6 +4226,266 @@ void pansim_parsimony_indices(const pansim_parsimony *p, double *ci, double *ri)
     if (ri) *ri = p->max_changes != p->min_changes ? (G - S) / (G - M) : nan;
 }
 
+// ---- neighbour-joining (nj.cuh, DESIGN.md section 18) ------------------------------------------
+// Pairs per row block of the matrix build (the context's pair buffers hold one block).
+constexpr uint64_t NJ_BLOCK_PAIRS = 1ull << 26;
+// A compaction repacks the active rows when k <= NJ_COMPACT_FRACTION x the stored dimension, and only while that
+// dimension is above NJ_COMPACT_MIN (below it the scan is bound by latency, not bytes). PANSIM_NJ_COMPACT=<f> (0 < f
+// < 1) replaces the fraction for measurements; the tree is the same for every schedule.
+constexpr double NJ_COMPACT_FRACTION = 0.9;
+constexpr uint32_t NJ_COMPACT_MIN = 512;
+
+static uint32_t nj_nodes(uint32_t n) { return n >= 3 ? 2 * n - 2 : n == 2 ? 3 : 1; }
+static uint64_t nj_pitch(uint64_t m) { return (m + 31) / 32 * 32; }
+
+// the k at which the loop compacts, largest first
+static std::vector<uint32_t> nj_schedule(uint32_t n)
+{
+    double f = NJ_COMPACT_FRACTION;
+    if (const char *e = std::getenv("PANSIM_NJ_COMPACT")) {
+        const double v = std::strtod(e, nullptr);
+        if (v > 0.0 && v < 1.0) f = v;
+    }
+    std::vector<uint32_t> ks;
+    uint32_t M = n;
+    for (uint32_t k = n; k > 3; k--)
+        if (M > NJ_COMPACT_MIN && (double)k <= f * (double)M) { ks.push_back(k); M = k; }
+    return ks;
+}
+
+// the device buffers of one call, freed when it returns
+struct NjCall {
+    uint32_t n = 0;
+    double *D[2] = {nullptr, nullptr};
+    void *scratch = nullptr;
+    double *R[2] = {nullptr, nullptr}, *length = nullptr;
+    uint32_t *node[2] = {nullptr, nullptr}, *old_of = nullptr, *parent = nullptr, *done = nullptr;
+    NjBest *part = nullptr, *best = nullptr;
+    uint32_t max_grid = 0;
+    std::vector<uint32_t> compact_at;
+    ~NjCall()
+    {
+        for (void *p : {(void *)D[0], (void *)D[1], scratch})
+            if (p) cudaFree(p);
+    }
+};
+
+static int nj_alloc(pansim_ctx *c, uint32_t n, NjCall &w)
+{
+    CU(c, cudaSetDevice(c->cfg.device));
+    w.n = n;
+    w.compact_at = nj_schedule(n);
+    w.max_grid = (uint32_t)c->sm_count * 8;
+    const uint64_t k1 = w.compact_at.empty() ? 0 : w.compact_at[0];
+    const size_t bytes[2] = {(size_t)n * nj_pitch(n) * 8, (size_t)k1 * nj_pitch(k1) * 8};
+    const size_t scratch = (size_t)n * (2 * 8 + 2 * 4 + 4) + (size_t)nj_nodes(n) * 12 + ((size_t)w.max_grid + 1) * sizeof(NjBest) + 10 * 16;   // + the rounding of ten pieces
+    for (int i = 0; i < 2; i++)
+        if (bytes[i] && cudaMalloc(&w.D[i], bytes[i]) != cudaSuccess) {
+            cudaGetLastError();
+            w.D[i] = nullptr;
+            FAIL(c, PANSIM_ERR_NOMEM, "neighbour-joining: cudaMalloc of the %u x %u distance matrix (%zu bytes) failed", n, n, bytes[i]);
+        }
+    if (cudaMalloc(&w.scratch, scratch) != cudaSuccess) {
+        cudaGetLastError();
+        w.scratch = nullptr;
+        FAIL(c, PANSIM_ERR_NOMEM, "neighbour-joining: cudaMalloc of %zu bytes of scratch failed", scratch);
+    }
+    char *p = (char *)w.scratch;
+    auto take = [&](size_t b) { char *q = p; p += (b + 15) / 16 * 16; return q; };
+    w.best = (NjBest *)take(sizeof(NjBest));
+    w.part = (NjBest *)take((size_t)w.max_grid * sizeof(NjBest));
+    w.R[0] = (double *)take((size_t)n * 8);
+    w.R[1] = (double *)take((size_t)n * 8);
+    w.length = (double *)take((size_t)nj_nodes(n) * 8);
+    w.node[0] = (uint32_t *)take((size_t)n * 4);
+    w.node[1] = (uint32_t *)take((size_t)n * 4);
+    w.old_of = (uint32_t *)take((size_t)n * 4);
+    w.parent = (uint32_t *)take((size_t)nj_nodes(n) * 4);
+    w.done = (uint32_t *)take(4);
+    CU(c, cudaMemsetAsync(w.done, 0, 4, c->stream));
+    CU(c, cudaMemsetAsync(w.D[0], 0, bytes[0], c->stream));
+    return 0;
+}
+
+// D[0] is filled: R, the joins, the last two or three, and the table back to the host. Times the join loop between
+// ev[0] and ev[1] when ev is given; *scanned / *compactions as pansim_nj_kernel_ms reports them.
+static int nj_join_loop(pansim_ctx *c, NjCall &w, uint32_t *parent, double *length, cudaEvent_t *ev, uint64_t *scanned,
+                        uint32_t *compactions)
+{
+    const uint32_t n = w.n;
+    int cur = 0;
+    uint32_t M = n;
+    uint64_t pitch = nj_pitch(n);
+    nj_rowsum_kernel<<<div_up64(n, 256), 256, 0, c->stream>>>(w.D[0], pitch, n, w.R[0], w.node[0]);
+    LAUNCH_CHECK(c);
+    if (ev) CU(c, cudaEventRecord(ev[0], c->stream));
+    uint64_t bytes = 0;
+    size_t next = 0;
+    for (uint32_t k = n; k > 3; k--) {
+        if (next < w.compact_at.size() && w.compact_at[next] == k) {
+            const uint64_t np = nj_pitch(k);
+            nj_compact_index_kernel<<<1, 1024, 0, c->stream>>>(w.R[cur], w.node[cur], M, w.old_of, w.R[cur ^ 1], w.node[cur ^ 1]);
+            LAUNCH_CHECK(c);
+            nj_compact_copy_kernel<<<std::min<uint32_t>(k, w.max_grid), 256, 0, c->stream>>>(w.D[cur], pitch, w.D[cur ^ 1], np, w.old_of, k);
+            LAUNCH_CHECK(c);
+            cur ^= 1;
+            M = k;
+            pitch = np;
+            next++;
+        }
+        const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(div_up64(M - 1, NJ_THREADS / 32), w.max_grid));
+        nj_scan_kernel<<<grid, NJ_THREADS, 0, c->stream>>>(w.D[cur], pitch, M, (double)(k - 2), w.R[cur], w.part, w.done, w.best);
+        LAUNCH_CHECK(c);
+        nj_join_kernel<<<div_up64(M, NJ_THREADS), NJ_THREADS, 0, c->stream>>>(w.D[cur], pitch, M, w.R[cur], w.node[cur], w.best, k, n,
+                                                                              w.parent, w.length);
+        LAUNCH_CHECK(c);
+        bytes += (uint64_t)M * (M - 1) / 2 * 8;
+    }
+    if (n >= 2) {
+        nj_finish_kernel<<<1, 1, 0, c->stream>>>(w.D[cur], pitch, M, w.R[cur], w.node[cur], n, w.parent, w.length);
+        LAUNCH_CHECK(c);
+    }
+    if (ev) CU(c, cudaEventRecord(ev[1], c->stream));
+    const size_t nn = nj_nodes(n);
+    CU(c, cudaMemcpyAsync(parent, w.parent, nn * 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(length, w.length, nn * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (scanned) *scanned = bytes;
+    if (compactions) *compactions = (uint32_t)w.compact_at.size();
+    return 0;
+}
+
+// the distances of the pairs of the current block (c->d_r1 / d_r2 and the counts) into D[0]
+static int nj_scatter(pansim_ctx *c, NjCall &w, int metric, size_t P)
+{
+    if (!P) return 0;
+    const uint32_t grid = (uint32_t)std::min<uint64_t>(div_up64(P, 256), (uint64_t)c->sm_count * 16);
+    nj_scatter_pairs_kernel<<<grid, 256, 0, c->stream>>>(c->d_r1, c->d_r2, c->d_cd, c->d_in, c->d_un, (uint32_t)P, metric,
+                                                        (double)c->L, (double)c->cfg.core_genes, w.D[0], nj_pitch(w.n));
+    LAUNCH_CHECK(c);
+    return 0;
+}
+
+// row blocks [i0, i1) of at most NJ_BLOCK_PAIRS pairs over rows 0 .. n-2
+static std::vector<std::pair<uint32_t, uint32_t>> nj_blocks(uint32_t n, uint64_t *max_pairs)
+{
+    std::vector<std::pair<uint32_t, uint32_t>> out;
+    *max_pairs = 0;
+    uint32_t i0 = 0;
+    while (i0 + 1 < n) {
+        uint64_t P = 0;
+        uint32_t i1 = i0;
+        while (i1 + 1 < n && (i1 == i0 || P + (n - 1 - i1) <= NJ_BLOCK_PAIRS)) P += n - 1 - i1++;
+        out.push_back({i0, i1});
+        *max_pairs = std::max(*max_pairs, P);
+        i0 = i1;
+    }
+    return out;
+}
+
+// The refusals of pansim_nj_tree; shard = false skips the column-shard check (a group sums its shards itself).
+static int nj_check(pansim_ctx *c, int metric, bool shard)
+{
+    if (metric != 0 && metric != 1) FAIL(c, PANSIM_ERR_INVALID, "neighbour-joining: metric %d (0 core, 1 acc)", metric);
+    if (int rc = require_state(c)) return rc;
+    if (metric == 0 && c->L == 0) FAIL(c, PANSIM_ERR_INVALID, "neighbour-joining: core distances need core_size > 0");
+    if (metric == 0 && shard)
+        if (int rc = require_whole_alignment(c, "neighbour-joining on core distances")) return rc;
+    return 0;
+}
+
+// One context's matrix: per row block, the pair counts (summed over the communicator for core) and the scatter.
+static int nj_build_ctx(pansim_ctx *c, int metric, NjCall &w)
+{
+    uint64_t maxP = 0;
+    const auto blocks = nj_blocks(w.n, &maxP);
+    if (maxP)
+        if (int rc = ensure_pairs(c, (size_t)maxP)) return rc;
+    for (const auto &b : blocks) {
+        size_t P = 0;
+        if (int rc = pair_counts_rows_impl(c, b.first, b.second, metric == 0 ? c->d_cd : nullptr, metric ? c->d_in : nullptr,
+                                           metric ? c->d_un : nullptr, &P)) return rc;
+        if (metric == 0)
+            if (int rc = comm_allreduce_counts(c, c->d_cd, P)) return rc;
+        if (int rc = nj_scatter(c, w, metric, P)) return rc;
+    }
+    return 0;
+}
+
+static void nj_single_leaf(uint32_t *parent, double *length)
+{
+    parent[0] = NJ_NONE;
+    length[0] = 0.0;
+}
+
+int pansim_nj_tree(pansim_ctx *c, int metric, uint32_t *parent, double *length)
+{
+    if (!c || !parent || !length) return PANSIM_ERR_INVALID;
+    if (int rc = nj_check(c, metric, true)) return rc;
+    if (c->N == 1) { nj_single_leaf(parent, length); return 0; }
+    NjCall w;
+    if (int rc = nj_alloc(c, c->N, w)) return rc;
+    if (int rc = nj_build_ctx(c, metric, w)) return rc;
+    if (int rc = nj_join_loop(c, w, parent, length, nullptr, nullptr, nullptr)) return rc;
+    return check_device_flag(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG);
+}
+
+int pansim_nj_tree_matrix(pansim_ctx *c, const double *upper, uint32_t n, uint32_t *parent, double *length)
+{
+    if (!c || !parent || !length || n == 0 || (n > 1 && !upper)) return PANSIM_ERR_INVALID;
+    const uint64_t m = (uint64_t)n * (n - 1) / 2;
+    for (uint64_t e = 0; e < m; e++)
+        if (!std::isfinite(upper[e]) || upper[e] < 0.0)
+            FAIL(c, PANSIM_ERR_INVALID, "neighbour-joining: matrix entry %llu is %g (finite and >= 0 required)", (unsigned long long)e, upper[e]);
+    if (n == 1) { nj_single_leaf(parent, length); return 0; }
+    NjCall w;
+    if (int rc = nj_alloc(c, n, w)) return rc;
+    double *d_upper = nullptr;
+    if (cudaMalloc(&d_upper, m * 8) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL(c, PANSIM_ERR_NOMEM, "neighbour-joining: cudaMalloc of the %llu matrix entries failed", (unsigned long long)m);
+    }
+    cudaError_t e = cudaMemcpyAsync(d_upper, upper, m * 8, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) {
+        nj_scatter_upper_kernel<<<std::min<uint32_t>(n, w.max_grid), 256, 0, c->stream>>>(d_upper, n, w.D[0], nj_pitch(n));
+        e = cudaGetLastError();
+    }
+    cudaStreamSynchronize(c->stream);
+    cudaFree(d_upper);
+    CU(c, e);
+    return nj_join_loop(c, w, parent, length, nullptr, nullptr, nullptr);
+}
+
+int pansim_nj_kernel_ms(pansim_ctx *c, int metric, uint32_t repeats, float *build_ms, float *join_ms, uint64_t *bytes_scanned,
+                        uint32_t *compactions)
+{
+    if (!c || !repeats) return PANSIM_ERR_INVALID;
+    if (int rc = nj_check(c, metric, true)) return rc;
+    if (c->N < 2) FAIL(c, PANSIM_ERR_INVALID, "neighbour-joining measurement needs pop_size >= 2");
+    std::vector<uint32_t> parent(nj_nodes(c->N));
+    std::vector<double> length(parent.size());
+    cudaEvent_t ev[3];
+    for (auto &x : ev) CU(c, cudaEventCreate(&x));
+    double tb = 0.0, tj = 0.0;
+    int rc = 0;
+    for (uint32_t r = 0; r <= repeats && !rc; r++) {             // r = 0 warms up
+        NjCall w;
+        if ((rc = nj_alloc(c, c->N, w))) break;
+        cudaEventRecord(ev[0], c->stream);
+        if ((rc = nj_build_ctx(c, metric, w))) break;
+        if ((rc = nj_join_loop(c, w, parent.data(), length.data(), ev + 1, bytes_scanned, compactions))) break;
+        float b = 0.f, j = 0.f;
+        cudaEventElapsedTime(&b, ev[0], ev[1]);
+        cudaEventElapsedTime(&j, ev[1], ev[2]);
+        if (r) { tb += b; tj += j; }
+    }
+    for (auto &x : ev) cudaEventDestroy(x);
+    if (rc) return rc;
+    if (build_ms) *build_ms = (float)(tb / repeats);
+    if (join_ms) *join_ms = (float)(tj / repeats);
+    return check_device_flag(c, PANSIM_ERR_WEIGHTS, PANSIM_WEIGHTS_MSG);
+}
+
 // ---- clonal genealogy (genealogy.cuh, DESIGN.md section 13) ------------------
 // trace scratch and node table: owner, cnt, newid [N]; lineage nodes and ancestors [2][N] each; parent, individual,
 // time [2N] each; n_nodes and lineages_at_start
@@ -4340,44 +4622,39 @@ int pansim_genealogy_tmrca(pansim_ctx *c, const uint32_t *r1, const uint32_t *r2
     return 0;
 }
 
-// Newick of a node table, no device. A checked table has its root last and every other node's parent above it, so
-// the tree is walked with an explicit stack (no recursion: a caterpillar of any size is fine).
-int pansim_genealogy_newick(const pansim_genealogy_node *nodes, uint32_t n_nodes, uint32_t n_leaves, char *out,
-                            size_t cap, size_t *len)
+// Newick of a checked node table, no device: root last, every other node's parent above it, so the tree is walked with
+// an explicit stack (no recursion: a caterpillar of any size is fine). Leaves are ind_<i>, children go in the order of
+// their smallest leaf; put_length(v, put) writes the ":<length>" of non-root node v. Returns the text's length.
+extern "C++" {
+template <class Parent, class PutLength>
+static size_t newick_write(uint32_t n_nodes, uint32_t n_leaves, Parent parent_of, PutLength put_length, char *out, size_t cap)
 {
-    if (!nodes || !len || n_leaves == 0 || n_nodes < n_leaves || (uint64_t)n_nodes > 2ull * n_leaves) return PANSIM_ERR_INVALID;
     const uint32_t root = n_nodes - 1;
-    if (nodes[root].parent != GEN_NONE) return PANSIM_ERR_INVALID;
-    for (uint32_t k = 0; k < root; k++) {
-        const uint32_t p = nodes[k].parent;
-        if (p <= k || p < n_leaves || p >= n_nodes || nodes[p].time < nodes[k].time) return PANSIM_ERR_INVALID;
-    }
     // smallest leaf below every node; the children of every node in that order (CSR)
     std::vector<uint32_t> minleaf(n_nodes, GEN_NONE), first(n_nodes + 1, 0), child(root);
     for (uint32_t k = 0; k < n_leaves; k++) minleaf[k] = k;
     for (uint32_t k = 0; k < root; k++) {
-        minleaf[nodes[k].parent] = std::min(minleaf[nodes[k].parent], minleaf[k]);
-        first[nodes[k].parent + 1]++;
+        minleaf[parent_of(k)] = std::min(minleaf[parent_of(k)], minleaf[k]);
+        first[parent_of(k) + 1]++;
     }
     for (uint32_t k = 0; k < n_nodes; k++) first[k + 1] += first[k];
     std::vector<uint32_t> order(root), fill(first.begin(), first.end() - 1);
     for (uint32_t k = 0; k < root; k++) order[k] = k;
     std::sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return minleaf[x] != minleaf[y] ? minleaf[x] < minleaf[y] : x < y; });
-    for (uint32_t k : order) child[fill[nodes[k].parent]++] = k;
+    for (uint32_t k : order) child[fill[parent_of(k)]++] = k;
     size_t pos = 0;
     auto put = [&](const char *s, size_t n) {
         if (out && pos + n <= cap) memcpy(out + pos, s, n);
         pos += n;
     };
-    auto put_u = [&](const char *prefix, size_t np, uint32_t v) {
-        char b[24];
-        const int n = snprintf(b, sizeof b, "%u", v);
-        put(prefix, np);
-        put(b, (size_t)n);
-    };
     auto enter = [&](uint32_t v) {
-        if (v < n_leaves) put_u("ind_", 4, v);
-        else put("(", 1);
+        if (v < n_leaves) {
+            char b[24];
+            const int n = snprintf(b, sizeof b, "ind_%u", v);
+            put(b, (size_t)n);
+        } else {
+            put("(", 1);
+        }
     };
     struct Frame { uint32_t node, next; };
     std::vector<Frame> stack{{root, 0}};
@@ -4393,14 +4670,139 @@ int pansim_genealogy_newick(const pansim_genealogy_node *nodes, uint32_t n_nodes
             continue;
         }
         if (v >= n_leaves) put(")", 1);
-        if (v != root) put_u(":", 1, nodes[nodes[v].parent].time - nodes[v].time);
+        if (v != root) put_length(v, put);
         stack.pop_back();
     }
     put(";\n", 2);
+    return pos;
+}
+}  // extern "C++"
+
+// the text into out when it fits with its terminating NUL (out = NULL: only the length)
+static int newick_finish(char *out, size_t cap, size_t pos, size_t *len)
+{
     *len = pos;
     if (!out) return 0;
     if (cap < pos + 1) return PANSIM_ERR_INVALID;
     out[pos] = '\0';
+    return 0;
+}
+
+int pansim_genealogy_newick(const pansim_genealogy_node *nodes, uint32_t n_nodes, uint32_t n_leaves, char *out,
+                            size_t cap, size_t *len)
+{
+    if (!nodes || !len || n_leaves == 0 || n_nodes < n_leaves || (uint64_t)n_nodes > 2ull * n_leaves) return PANSIM_ERR_INVALID;
+    const uint32_t root = n_nodes - 1;
+    if (nodes[root].parent != GEN_NONE) return PANSIM_ERR_INVALID;
+    for (uint32_t k = 0; k < root; k++) {
+        const uint32_t p = nodes[k].parent;
+        if (p <= k || p < n_leaves || p >= n_nodes || nodes[p].time < nodes[k].time) return PANSIM_ERR_INVALID;
+    }
+    const size_t pos = newick_write(
+        n_nodes, n_leaves, [&](uint32_t k) { return nodes[k].parent; },
+        [&](uint32_t v, auto &put) {
+            char b[24];
+            const int n = snprintf(b, sizeof b, ":%u", nodes[nodes[v].parent].time - nodes[v].time);
+            put(b, (size_t)n);
+        },
+        out, cap);
+    return newick_finish(out, cap, pos, len);
+}
+
+int pansim_tree_newick(const uint32_t *parent, const double *length, uint32_t n_nodes, uint32_t n_leaves, char *out,
+                       size_t cap, size_t *len)
+{
+    if (!parent || !length || !len || n_leaves == 0 || !node_table_error(parent, n_nodes, n_leaves, nullptr).empty())
+        return PANSIM_ERR_INVALID;
+    const size_t pos = newick_write(
+        n_nodes, n_leaves, [&](uint32_t k) { return parent[k]; },
+        [&](uint32_t v, auto &put) {
+            char b[40];
+            const int n = snprintf(b, sizeof b, ":%.17g", length[v]);
+            put(b, (size_t)n);
+        },
+        out, cap);
+    return newick_finish(out, cap, pos, len);
+}
+
+// ---- split comparison (no device) -------------------------------------------------------------
+// The leaves of a checked table in an order where every subtree is a contiguous run and leaf 0 comes first (at every
+// node the child holding leaf 0 is laid out first). Then the side of a split without leaf 0 is a run too: the subtree
+// [lo, hi] itself, or [hi + 1, N - 1] when the subtree holds leaf 0. sides = those runs with 2 .. N - 2 leaves, as
+// lo << 32 | hi, sorted, distinct. pos[leaf] = its place in the order, order[place] = the leaf.
+static void tree_sides(const uint32_t *parent, uint32_t n_nodes, uint32_t N, std::vector<uint32_t> &pos,
+                       std::vector<uint32_t> &order, std::vector<uint64_t> &sides)
+{
+    const uint32_t root = n_nodes - 1;
+    std::vector<uint32_t> cnt(n_nodes, 0), start(n_nodes, 0), off(n_nodes + 1, 0), child(root);
+    std::vector<uint8_t> has0(n_nodes, 0);
+    for (uint32_t k = 0; k < N; k++) cnt[k] = 1;
+    has0[0] = 1;
+    for (uint32_t k = 0; k < root; k++) {
+        cnt[parent[k]] += cnt[k];
+        has0[parent[k]] |= has0[k];
+        off[parent[k] + 1]++;
+    }
+    for (uint32_t k = 0; k < n_nodes; k++) off[k + 1] += off[k];
+    std::vector<uint32_t> fill(off.begin(), off.end() - 1);
+    for (uint32_t k = 0; k < root; k++) child[fill[parent[k]]++] = k;
+    for (uint32_t v = root + 1; v-- > N;) {                  // parents before children
+        uint32_t run = start[v];
+        for (int pass = 0; pass < 2; pass++)                 // the child holding leaf 0 first
+            for (uint32_t e = off[v]; e < off[v + 1]; e++)
+                if (has0[child[e]] == (pass == 0)) { start[child[e]] = run; run += cnt[child[e]]; }
+    }
+    pos.assign(N, 0);
+    order.assign(N, 0);
+    for (uint32_t k = 0; k < N; k++) { pos[k] = start[k]; order[start[k]] = k; }
+    sides.clear();
+    for (uint32_t v = 0; v < root; v++) {
+        uint64_t lo = start[v], hi = (uint64_t)start[v] + cnt[v] - 1;
+        if (lo == 0) { lo = hi + 1; hi = N - 1; }
+        const uint64_t size = hi + 1 - lo;
+        if (size >= 2 && size + 2 <= N) sides.push_back(lo << 32 | hi);
+    }
+    std::sort(sides.begin(), sides.end());
+    sides.erase(std::unique(sides.begin(), sides.end()), sides.end());
+}
+
+// A side of B (a run of B's order) is a split of A iff its leaves occupy a run [m, M] of A's order (M - m + 1 = its
+// size; min and max by a sparse table over A's places in B's order) and [m, M] is one of A's sides.
+int pansim_tree_compare_splits(const uint32_t *parent_a, uint32_t n_a, const uint32_t *parent_b, uint32_t n_b,
+                               uint32_t n_leaves, uint64_t out[3])
+{
+    if (!out || n_leaves == 0 || !node_table_error(parent_a, n_a, n_leaves, nullptr).empty() ||
+        !node_table_error(parent_b, n_b, n_leaves, nullptr).empty())
+        return PANSIM_ERR_INVALID;
+    const uint32_t N = n_leaves;
+    std::vector<uint32_t> pos_a, order_a, pos_b, order_b;
+    std::vector<uint64_t> sides_a, sides_b;
+    tree_sides(parent_a, n_a, N, pos_a, order_a, sides_a);
+    tree_sides(parent_b, n_b, N, pos_b, order_b, sides_b);
+    uint32_t levels = 1;
+    while ((1ull << levels) <= N) levels++;
+    std::vector<std::vector<uint32_t>> mn(levels), mx(levels);
+    mn[0].resize(N);
+    for (uint32_t i = 0; i < N; i++) mn[0][i] = pos_a[order_b[i]];
+    mx[0] = mn[0];
+    for (uint32_t l = 1; l < levels; l++) {
+        const uint32_t w = 1u << (l - 1), n = N - (1u << l) + 1;
+        mn[l].resize(n);
+        mx[l].resize(n);
+        for (uint32_t i = 0; i < n; i++) {
+            mn[l][i] = std::min(mn[l - 1][i], mn[l - 1][i + w]);
+            mx[l][i] = std::max(mx[l - 1][i], mx[l - 1][i + w]);
+        }
+    }
+    uint64_t shared = 0;
+    for (uint64_t s : sides_b) {
+        const uint32_t lo = (uint32_t)(s >> 32), hi = (uint32_t)s, l = 31 - __builtin_clz(hi - lo + 1);
+        const uint32_t m = std::min(mn[l][lo], mn[l][hi + 1 - (1u << l)]), M = std::max(mx[l][lo], mx[l][hi + 1 - (1u << l)]);
+        if (M - m == hi - lo && std::binary_search(sides_a.begin(), sides_a.end(), (uint64_t)m << 32 | M)) shared++;
+    }
+    out[0] = sides_a.size();
+    out[1] = sides_b.size();
+    out[2] = shared;
     return 0;
 }
 

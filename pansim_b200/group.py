@@ -13,9 +13,9 @@ import numpy as np
 
 from . import _ffi
 from .params import Params
-from .population import (OK, CoreFasta, CoreLD, CoreParsimony, GeneAccumulation, GeneLD, GeneParsimony, Genealogy, PansimError,
-                         _core_ld, _diversity, _gene_accumulation, _gene_ld, _gene_spectrum, _genealogy, _genealogy_history,
-                         _ld_bins, _ld_params, _pairs_or_none, _parent_table, _parsimony, _ptr, _tmrca, _write_fasta,
+from .population import (NJ_METRICS, OK, CoreFasta, CoreLD, CoreParsimony, GeneAccumulation, GeneLD, GeneParsimony, Genealogy,
+                         NJTree, PansimError, _core_ld, _diversity, _gene_accumulation, _gene_ld, _gene_spectrum, _genealogy, _genealogy_history,
+                         _ld_bins, _ld_params, _nj_tree, _pairs_or_none, _parent_table, _parsimony, _ptr, _tmrca, _write_fasta,
                          make_config)
 
 
@@ -175,6 +175,12 @@ class PansimGroup:
         """Pansim.gene_parsimony: the accessory matrix is replicated, so shard 0 answers."""
         parent = _parent_table(self.genealogy() if genealogy is None else genealogy)
         return _parsimony(lambda *a: self._lib.pansim_group_gene_parsimony(self._h, *a), self._check, parent, self.G, True)
+
+    def nj_tree(self, metric: str = "core") -> NJTree:
+        """Pansim.nj_tree of the group: core counts summed over the shards, shard 0 joins; the same tree as one
+        context."""
+        m = NJ_METRICS[metric]
+        return _nj_tree(lambda *a: self._lib.pansim_group_nj_tree(self._h, m, *a), self._check, self.N)
 
     def enable_genealogy(self, capacity: int):
         """Pansim.enable_genealogy for the group: shard 0 records (every shard draws the same parents)."""

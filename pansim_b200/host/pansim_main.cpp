@@ -48,7 +48,8 @@ const char *VALUE_FLAGS[] = {"pop_size", "core_size", "pan_genes", "core_genes",
 const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection", "verbose", "no_control_genome_size",
                               "all_pairs", "print_diversity", "print_vcf", "print_ld", "print_genealogy",
                               "print_fasta", "print_snp_alignment", "print_gene_ld",
-                              "print_gene_accumulation", "print_parsimony"};  // extensions: all_pairs (every pair i < j in <outpref>.tsv),
+                              "print_gene_accumulation", "print_parsimony",
+                              "print_nj"};                                    // extensions: all_pairs (every pair i < j in <outpref>.tsv),
                                                                               // print_diversity (<outpref>_diversity.tsv, <outpref>_core_sfs.txt),
                                                                               // print_vcf (<outpref>_core_genome.vcf),
                                                                               // print_ld (<outpref>_core_ld.tsv),
@@ -59,7 +60,8 @@ const char *SWITCH_FLAGS[] = {"print_dist", "print_matrices", "print_selection",
                                                                               // print_gene_accumulation (<outpref>_number_of_*.Rtab,
                                                                               //   <outpref>_gene_spectrum.txt, <outpref>_summary_statistics.txt),
                                                                               // print_parsimony (<outpref>_parsimony.tsv, <outpref>_core_site_changes.txt,
-                                                                              //   <outpref>_gene_changes.txt, <outpref>_branch_changes.tsv)
+                                                                              //   <outpref>_gene_changes.txt, <outpref>_branch_changes.tsv),
+                                                                              // print_nj (<outpref>_core_nj.nwk, <outpref>_acc_nj.nwk, <outpref>_nj_rf.tsv)
 
 bool parse(int argc, char **argv, Flags &f)
 {
@@ -152,6 +154,7 @@ int main(int argc, char **argv)
     const bool print_gene_ld = fl.sw["print_gene_ld"];
     const bool print_gene_accumulation = fl.sw["print_gene_accumulation"];
     const bool print_parsimony = fl.sw["print_parsimony"];
+    const bool print_nj = fl.sw["print_nj"];
     const uint32_t gene_accumulation_perms = (uint32_t)std::strtoul(fl.val["gene_accumulation_perms"].c_str(), nullptr, 10);
     const pansim_gene_ld_params gene_ld_params = {(uint32_t)std::strtoul(fl.val["gene_ld_bins"].c_str(), nullptr, 10),
                                                   (uint32_t)std::strtoul(fl.val["gene_ld_min_minor"].c_str(), nullptr, 10)};
@@ -242,7 +245,7 @@ int main(int argc, char **argv)
         pansim::Populations pops(cfg, n_gpus);
         pops.set_initial(core_row, acc_row);
         pops.set_selection(selection);
-        if (print_genealogy || print_parsimony) pops.enable_genealogy((uint32_t)n_gen);   // extension: after set_initial, which clears the record
+        if (print_genealogy || print_parsimony || print_nj) pops.enable_genealogy((uint32_t)n_gen);   // extension: after set_initial, which clears the record
         std::vector<double> avg_core(n_gen, 0.0), avg_acc(n_gen, 0.0), std_core(n_gen, 0.0), std_acc(n_gen, 0.0);
         std::vector<double> core_d, acc_d;
         std::vector<pansim_diversity> diversity;
@@ -414,6 +417,20 @@ int main(int argc, char **argv)
             for (size_t k = 0; k + 1 < n; k++)
                 f << k << "\t" << parent[k] << "\t" << first[k] << "\t" << below[k] << "\t" << nodes[parent[k]].time - nodes[k].time
                   << "\t" << core.branch_changes[k] << "\t" << genes.gains[k] << "\t" << genes.losses[k] << "\n";
+        }
+        if (print_nj) {                                                     // extension: NJ trees against the true genealogy
+            const std::vector<pansim_genealogy_node> nodes = pops.genealogy();
+            std::vector<uint32_t> gparent(nodes.size());
+            for (size_t k = 0; k < nodes.size(); k++) gparent[k] = nodes[k].parent;
+            std::ofstream rf(outpref + "_nj_rf.tsv");
+            for (const char *metric : {"core", "acc"}) {
+                const auto t = pops.nj_tree(metric[0] == 'c' ? 0 : 1);
+                std::ofstream(outpref + "_" + metric + "_nj.nwk") << pops.tree_newick(t.parent, t.length);
+                const auto s = pops.compare_splits(t.parent, gparent);
+                const uint64_t total = s[0] + s[1], d = total - 2 * s[2];
+                rf << metric << "\t" << s[0] << "\t" << s[1] << "\t" << s[2] << "\t" << d << "\t"
+                   << fmt(total ? (double)d / (double)total : std::nan("")) << "\n";
+            }
         }
     } catch (const pansim::Error &e) {
         // the reference aborts with a panic message (exit status 101)

@@ -275,6 +275,32 @@ public:
                                            r.gains.data(), r.losses.data()));
         return r;
     }
+    // (extension) the neighbour-joining tree of the present rows, metric 0 core / 1 acc (pansim_group_nj_tree)
+    struct NJTree { std::vector<uint32_t> parent; std::vector<double> length; };
+    NJTree nj_tree(int metric)
+    {
+        const uint32_t n = cfg_.pop_size, nodes = n >= 3 ? 2 * n - 2 : n == 2 ? 3 : 1;
+        NJTree t{std::vector<uint32_t>(nodes), std::vector<double>(nodes)};
+        gcheck(pansim_group_nj_tree(grp_, metric, t.parent.data(), t.length.data()));
+        return t;
+    }
+    // (extension) the Newick text of a node table with branch lengths (pansim_tree_newick)
+    std::string tree_newick(const std::vector<uint32_t> &parent, const std::vector<double> &length)
+    {
+        size_t len = 0;
+        check_table(pansim_tree_newick(parent.data(), length.data(), (uint32_t)parent.size(), cfg_.pop_size, nullptr, 0, &len));
+        std::string s(len + 1, '\0');
+        check_table(pansim_tree_newick(parent.data(), length.data(), (uint32_t)parent.size(), cfg_.pop_size, &s[0], s.size(), &len));
+        s.resize(len);
+        return s;
+    }
+    // (extension) {splits of a, splits of b, shared} of two node tables over the rows (pansim_tree_compare_splits)
+    std::array<uint64_t, 3> compare_splits(const std::vector<uint32_t> &a, const std::vector<uint32_t> &b)
+    {
+        std::array<uint64_t, 3> out{};
+        check_table(pansim_tree_compare_splits(a.data(), (uint32_t)a.size(), b.data(), (uint32_t)b.size(), cfg_.pop_size, out.data()));
+        return out;
+    }
     // (extension) the canonical Newick text of a node table (pansim_genealogy_newick)
     std::string newick(const std::vector<pansim_genealogy_node> &nodes)
     {
@@ -298,6 +324,10 @@ private:
     void gcheck(int rc)
     {
         if (rc != PANSIM_OK) throw Error(rc, pansim_group_last_error(grp_));
+    }
+    void check_table(int rc)
+    {
+        if (rc != PANSIM_OK) throw Error(rc, "the node table breaks the rules of include/pansim_b200.h (section 17 tables)");
     }
     void check_newick(int rc)
     {

@@ -315,6 +315,72 @@ def genealogy_newick(parent, individual, time, n_leaves: int) -> str:
     return buf.raw[:n.value].decode()
 
 
+NJ_METRICS = {"core": 0, "acc": 1}
+
+
+def nj_nodes(n_leaves: int) -> int:
+    """Nodes of a neighbour-joining table over n_leaves leaves: 2N - 2 for N >= 3, 3 for N = 2, 1 for N = 1."""
+    return 2 * n_leaves - 2 if n_leaves >= 3 else 3 if n_leaves == 2 else 1
+
+
+def tree_newick(parent, length, n_leaves: int) -> str:
+    """pansim_tree_newick of a node table with branch lengths (no device): leaves ind_<i>, children ordered by their
+    smallest leaf, lengths %.17g."""
+    lib = _ffi.lib()
+    parent = np.ascontiguousarray(parent, np.uint32)
+    length = np.ascontiguousarray(length, np.float64)
+    if len(length) != len(parent):
+        raise ValueError("parent and length differ in length")
+    n = C.c_size_t(0)
+    rc = lib.pansim_tree_newick(_ptr(parent), _ptr(length), len(parent), n_leaves, None, 0, C.byref(n))
+    if rc != OK:
+        raise PansimError(rc, "pansim_tree_newick: not a node table over that many leaves")
+    buf = C.create_string_buffer(n.value + 1)
+    rc = lib.pansim_tree_newick(_ptr(parent), _ptr(length), len(parent), n_leaves, buf, n.value + 1, C.byref(n))
+    if rc != OK:
+        raise PansimError(rc, "pansim_tree_newick failed")
+    return buf.raw[:n.value].decode()
+
+
+class NJTree(NamedTuple):
+    """A neighbour-joining tree (pansim_nj_tree, include/pansim_b200.h): parent (uint32, root 0xFFFFFFFF) and the
+    branch length above each node (float64, root 0) over n_leaves leaves, a node table the parsimony calls accept."""
+    parent: np.ndarray
+    length: np.ndarray
+    n_leaves: int
+
+    def newick(self) -> str:
+        return tree_newick(self.parent, self.length, self.n_leaves)
+
+
+class SplitComparison(NamedTuple):
+    """pansim_tree_compare_splits: the non-trivial splits of each tree, those they share, and Robinson-Foulds
+    rf = splits_a + splits_b - 2 shared."""
+    splits_a: int
+    splits_b: int
+    shared: int
+    rf: int
+
+
+def compare_splits(a, b, n_leaves: int) -> SplitComparison:
+    """The split comparison of two node tables over the same leaves (NJTree, Genealogy or parent arrays; no device)."""
+    pa, pb = _parent_table(a), _parent_table(b)
+    out = np.zeros(3, np.uint64)
+    rc = _ffi.lib().pansim_tree_compare_splits(_ptr(pa), len(pa), _ptr(pb), len(pb), n_leaves, _ptr(out))
+    if rc != OK:
+        raise PansimError(rc, "pansim_tree_compare_splits: not node tables over that many leaves")
+    sa, sb, sh = (int(x) for x in out)
+    return SplitComparison(sa, sb, sh, sa + sb - 2 * sh)
+
+
+def _nj_tree(call, check, n_leaves: int) -> NJTree:
+    """call(parent, length) -> status."""
+    parent = np.zeros(nj_nodes(n_leaves), np.uint32)
+    length = np.zeros(len(parent), np.float64)
+    check(call(_ptr(parent), _ptr(length)))
+    return NJTree(parent, length, n_leaves)
+
+
 def _genealogy(call, check, N: int) -> Genealogy:
     nodes = np.empty((2 * N, 3), np.uint32)
     info = _ffi.GenealogyInfo()
@@ -708,6 +774,28 @@ class Pansim:
                                                          C.byref(ms), C.byref(nb), C.byref(sl)))
         return ms.value, nb.value, sl.value
 
+    # -- neighbour-joining (extension) -----------------------------------------
+    def nj_tree(self, metric: str = "core") -> NJTree:
+        """The neighbour-joining tree of the present rows on the core or accessory distances of <outpref>.tsv over
+        every pair (pansim_nj_tree)."""
+        m = NJ_METRICS[metric]
+        return _nj_tree(lambda *a: self._lib.pansim_nj_tree(self._h, m, *a), self._check, self.N)
+
+    def nj_tree_matrix(self, upper, n: int) -> NJTree:
+        """The neighbour-joining tree of a caller's distances given as the upper triangle, row-major (n (n - 1) / 2
+        values), on this context's device (pansim_nj_tree_matrix)."""
+        upper = np.ascontiguousarray(upper, np.float64)
+        if len(upper) != n * (n - 1) // 2:
+            raise ValueError(f"{len(upper)} values for the upper triangle of {n} leaves")
+        return _nj_tree(lambda *a: self._lib.pansim_nj_tree_matrix(self._h, _ptr(upper), n, *a), self._check, n)
+
+    def nj_kernel_ms(self, metric: str = "core", repeats: int = 3):
+        """Measurement: device ms of the matrix build and of the join loop, bytes the scans read, compactions."""
+        b, j, nb, nc = C.c_float(), C.c_float(), C.c_uint64(), C.c_uint32()
+        self._check(self._lib.pansim_nj_kernel_ms(self._h, NJ_METRICS[metric], repeats, C.byref(b), C.byref(j), C.byref(nb),
+                                                  C.byref(nc)))
+        return b.value, j.value, nb.value, nc.value
+
     # -- multi-GPU: communicator over column shards (one process per GPU) --
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -878,5 +966,6 @@ class Pansim:
 
 
 __all__ = ["Pansim", "PansimError", "Diversity", "diversity_stats", "CoreLD", "ld_mean_r2", "GeneLD", "GeneAccumulation",
-           "pangenome_classes", "CoreParsimony", "GeneParsimony", "parsimony_indices", "Genealogy", "genealogy_newick",
+           "pangenome_classes", "CoreParsimony", "GeneParsimony", "parsimony_indices", "NJTree", "SplitComparison",
+           "compare_splits", "tree_newick", "Genealogy", "genealogy_newick",
            "make_config", "standard_deviation", "fmt_f64"]

@@ -11,13 +11,14 @@ stream cannot be reproduced without the crate, so only the distributions match.
 """
 from __future__ import annotations
 
+import math
 import sys
 from dataclasses import dataclass, field
 
 import numpy as np
 
 from .params import Derived, Params, derive, fmt_f64, validate
-from .population import Pansim, diversity_stats, pangenome_classes, standard_deviation
+from .population import Pansim, compare_splits, diversity_stats, pangenome_classes, standard_deviation
 
 
 def selection_coefficients(p: Params, pan_size: int, rng: np.random.Generator) -> np.ndarray:
@@ -68,6 +69,8 @@ class RunResult:
     genealogy: object = None                      # Genealogy of the last generation (--print_genealogy)
     core_parsimony: object = None                 # CoreParsimony on the genealogy (--print_parsimony)
     gene_parsimony: object = None                 # GeneParsimony on the genealogy (--print_parsimony)
+    nj: dict = None                               # {"core", "acc"}: NJTree of the last generation (--print_nj)
+    nj_splits: dict = None                        # {"core", "acc"}: SplitComparison with the genealogy (--print_nj)
     tmrca: np.ndarray = None                      # TMRCA of the sampled pairs (--print_genealogy without --all_pairs)
     selection: np.ndarray = None
     stdout: list = field(default_factory=list)
@@ -78,7 +81,7 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
         ld_bin_width: int = 100, ld_min_minor: int = 1, print_genealogy: bool = False, print_fasta: bool = False,
         print_snp_alignment: bool = False, print_gene_ld: bool = False, gene_ld_bins: int = 20,
         gene_ld_min_minor: int = 1, print_gene_accumulation: bool = False,
-        gene_accumulation_perms: int = 100, print_parsimony: bool = False) -> RunResult | None:
+        gene_accumulation_perms: int = 100, print_parsimony: bool = False, print_nj: bool = False) -> RunResult | None:
     """main.rs:15-564. Returns None where the reference prints a validation message and exits 0.
     all_pairs (extension, BASELINE config 5): `<outpref>.tsv` holds the distances of every pair i < j
     in (i, j) order instead of the max_distances sampled pairs; res.core/acc_distances stay None.
@@ -105,7 +108,10 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     write_gene_accumulation).
     print_parsimony (extension): the parents are recorded from generation 0 as for print_genealogy (without its files
     unless that is also given); after every other output, the parsimony changes of the core sites and the accessory
-    genes on the genealogy of the last generation (Pansim.core_parsimony, Pansim.gene_parsimony; write_parsimony)."""
+    genes on the genealogy of the last generation (Pansim.core_parsimony, Pansim.gene_parsimony; write_parsimony).
+    print_nj (extension): the parents are recorded as for print_parsimony; after every other output, the
+    neighbour-joining trees of the last generation on the core and the accessory distances, and their splits against
+    the genealogy (Pansim.nj_tree, compare_splits; write_nj)."""
     out = out or sys.stdout
     msgs = validate(p)
     if msgs:
@@ -130,7 +136,7 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
     with Pansim.from_params(p, device=device) as sim:
         sim.set_initial(core_row, acc_row)
         sim.set_selection(sel)
-        if print_genealogy or print_parsimony:
+        if print_genealogy or print_parsimony or print_nj:
             sim.enable_genealogy(p.n_gen)                                        # after set_initial, which clears the record
         def last_generation_outputs():                                           # main.rs:467-499
             if not all_pairs:
@@ -230,7 +236,27 @@ def run(p: Params, outpref: str | None = None, device: int = 0, out=None, all_pa
             res.gene_parsimony = sim.gene_parsimony(g)
             if outpref:
                 write_parsimony(outpref, g, res.core_parsimony, res.gene_parsimony)
+        if print_nj:
+            g = res.genealogy if res.genealogy is not None else sim.genealogy()
+            res.nj = {m: sim.nj_tree(m) for m in ("core", "acc")}
+            res.nj_splits = {m: compare_splits(t, g, p.pop_size) for m, t in res.nj.items()}
+            if outpref:
+                write_nj(outpref, res.nj, res.nj_splits)
     return res
+
+
+def write_nj(outpref: str, trees, splits):
+    """`<outpref>_core_nj.nwk` and `<outpref>_acc_nj.nwk`: the neighbour-joining trees (pansim_tree_newick);
+    `<outpref>_nj_rf.tsv`: two lines, `core` then `acc`, each NJ splits, genealogy splits, shared, Robinson-Foulds and
+    RF / (NJ splits + genealogy splits) (NaN if both are 0), no header."""
+    for m in ("core", "acc"):
+        with open(f"{outpref}_{m}_nj.nwk", "w") as f:
+            f.write(trees[m].newick())
+    with open(outpref + "_nj_rf.tsv", "w") as f:
+        for m in ("core", "acc"):
+            s = splits[m]
+            total = s.splits_a + s.splits_b
+            f.write(f"{m}\t{s.splits_a}\t{s.splits_b}\t{s.shared}\t{s.rf}\t{fmt_f64(s.rf / total if total else math.nan)}\n")
 
 
 def clades(parent, n_leaves: int) -> tuple[np.ndarray, np.ndarray]:
